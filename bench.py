@@ -7,7 +7,7 @@ A "step" is one pass of the hot path over one frame: BASELINE.json configs[1], t
 samples [k*spp/N, (k+1)*spp/N) of every pixel and the fp32 sum buffers are combined with one NCCL
 reduce to rank 0 (strong scaling: the frame is fixed).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scene NAME ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  `value` = whole-job Mpaths/s with the scene resident in HBM,
 timed with CUDA events on the stream every kernel and the reduce run on, max over ranks.
@@ -19,6 +19,8 @@ the scene's working set lives in), the bound named by whichever is larger.  `oth
 are short runs of BASELINE.json's other four configurations so that they appear in the driver's record too.
 `--impl reference` times the CPU restatement of the reference (oracle/, the Rust itself cannot be
 built here) on the host cores with the same config, on a bounded sample of the frame's spp.
+`--dump-outputs DIR` writes the frame the last timed step finished (see dump_frame) so that two builds can be
+compared output for output: the seeds of the timed steps are fixed, so the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -48,6 +50,24 @@ def load_json(path, default=None):
         return json.load(open(path))
     except Exception:
         return default
+
+
+DUMP_LIMIT = 64 * 10**6  # bytes of --dump-outputs, all files together
+
+
+def dump_frame(out_dir, frame):
+    """The finished (H, W, 3) float32 frame as out_dir/frame.npy.  A frame over DUMP_LIMIT (stress_1m at 4K) is
+    replaced by a fixed sample of 2^20 pixels drawn with seed 0: out_dir/frame_sample.npy (N, 3) and the row-major
+    pixel indices of that sample as out_dir/frame_sample_pixels.npy (float64, exact below 2^53)."""
+    os.makedirs(out_dir, exist_ok=True)
+    frame = np.ascontiguousarray(frame, dtype=np.float32)
+    if frame.nbytes <= DUMP_LIMIT:
+        np.save(os.path.join(out_dir, "frame.npy"), frame)
+        return
+    px = frame.reshape(-1, 3)
+    idx = np.sort(np.random.default_rng(0).choice(len(px), size=1 << 20, replace=False))
+    np.save(os.path.join(out_dir, "frame_sample.npy"), px[idx])
+    np.save(os.path.join(out_dir, "frame_sample_pixels.npy"), idx.astype(np.float64))
 
 
 def alg_work(scene_name):
@@ -204,10 +224,12 @@ def run_reference(args, cfg):
     paths = rays = 0
     t0 = time.perf_counter()
     for i in range(args.steps):
-        _, _, st = o.render(cam, vb.render_params(W, H, cpu_spp, depth, seed=200 + i), threads=cores)
+        frame, _, st = o.render(cam, vb.render_params(W, H, cpu_spp, depth, seed=200 + i), threads=cores)
         paths += st.paths
         rays += st.rays
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_frame(args.dump_outputs, frame)
     v = paths / dt / 1e6
     line = {"impl": "reference", "metric": "Mpaths/s", "value": v, "unit": "Mpaths/s", "mrays_per_s": rays / dt / 1e6,
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt / args.steps * 1e3,
@@ -318,6 +340,8 @@ def run_ours(args, cfg):
     paths, rays, dropped, launches = [float(x) for x in counts.tolist()]
     value = paths / (ms * 1e-3) / 1e6
     mrays = rays / (ms * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:  # before the kernel-only and e2e runs below reuse the device buffers
+        dump_frame(args.dump_outputs, d_rgb.cpu().numpy().reshape(H, W, 3))
 
     # ---- kernel-only time of the dominant kernel (CUDA events inside the library) ---------------
     kst = ctx.render_device(cam, params(77), d_sum.data_ptr(), want_stats=True)
@@ -386,7 +410,10 @@ def main():
     ap.add_argument("--variant", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-other-configs", action="store_true", help="skip the short runs of the other four BASELINE.json configurations")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the frame of the last timed step to DIR as .npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = list(CONFIGS[args.config])
     if args.spp:
         cfg[4] = args.spp

@@ -1,3 +1,4 @@
+import ctypes
 import os
 import subprocess
 import sys
@@ -6,6 +7,22 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+
+
+def cuda_device_count():
+    """CUDA devices the driver reports, 0 without a driver or a device.  Asked of the driver rather than read off
+    /dev/nvidia0: a container may expose its only GPU under another index, and CUDA_VISIBLE_DEVICES may hide all."""
+    try:
+        cuda = ctypes.CDLL("libcuda.so.1")
+    except OSError:
+        return 0
+    n = ctypes.c_int(0)
+    if cuda.cuInit(0) != 0 or cuda.cuDeviceGetCount(ctypes.byref(n)) != 0:
+        return 0
+    return n.value
+
+
+HAS_GPU = cuda_device_count() > 0
 
 
 def pytest_configure(config):

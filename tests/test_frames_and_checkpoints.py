@@ -9,7 +9,7 @@ import subprocess
 import numpy as np
 import pytest
 
-from conftest import ROOT, get_scene
+from conftest import HAS_GPU, ROOT, get_scene
 
 RENDER_BIN = os.path.join(ROOT, "vecchio_b200", "lib", "vecchio_gpu_render")
 
@@ -92,7 +92,7 @@ def test_render_program_usage_and_scene_numbers():
         assert subprocess.run([RENDER_BIN] + bad, capture_output=True).returncode == 2
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="a GPU is present")
+@pytest.mark.skipif(HAS_GPU, reason="a GPU is present")
 def test_render_program_has_no_cpu_path(tmp_path):
     r = subprocess.run([RENDER_BIN, "--width", "32", "--spp", "2", "--out-dir", str(tmp_path)], capture_output=True,
                        text=True, cwd=ROOT)
