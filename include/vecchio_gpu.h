@@ -318,6 +318,26 @@ int vk_render(vk_ctx* ctx, const vk_camera* cam, const vk_render_params* params,
 int vk_render_rgb8(vk_ctx* ctx, const vk_camera* cam, const vk_render_params* params,
                    uint8_t* out_rgb8, vk_stats* stats);
 
+/* K cameras of one scene in one launch.  Frame f uses cams[f] and Philox key params->seed + f (the rule of
+ * vecchio_gpu_render --seed); every other field of params applies to every frame.  Frame f of the output, at offset
+ * f * W*H*3, is what vk_render / vk_render_rgb8 return for (cams[f], seed + f) ON THE SAME KERNEL, bit for bit.
+ * The frames' units share the warps (frame-major: the batch drains once), and VK_VARIANT_AUTO decides on the batch's
+ * path count n_frames * W * H * spp_count, so a batch may run another kernel than its frames would one by one (config 1's
+ * turntable, 400x225x16: the step queues from 3 frames on, the lane megakernel for one).  With VK_FLAG_STRICT_MATH every
+ * kernel computes the reference's operation sequence and the batch equals the single-frame calls bit for bit whatever
+ * ran; in the render build each kernel contracts FMAs its own way, so there the guarantee needs an explicit variant:
+ * with AUTO a batch that changes kernel renders the same estimate with other rounding (individual samples can differ).
+ * stats: totals of the batch (paths, rays, dropped samples, kernel time) and
+ * the variant that ran.  No sums of squares (vk_render keeps them).  n_frames == 1 is vk_render / vk_render_rgb8.
+ * Errors, before anything is launched: VK_ERR_INVALID for n_frames == 0, a null pointer, a camera with
+ * time0 >= time1 (the message names the frame) or n_frames * W*H*3 >= 2^31; VK_ERR_OOM when the batch's accumulators
+ * cannot be allocated; VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED / VK_VARIANT_WAVEFRONT with n_frames > 1;
+ * VK_ERR_NO_SCENE without a scene. */
+int vk_render_frames(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                     float* out_rgb, vk_stats* stats);
+int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                          uint8_t* out_rgb8, vk_stats* stats);
+
 /* Same loop, device-resident result: writes per-pixel SUMS (not means) of samples
  * [spp_begin, spp_begin+spp_count) to d_sum (and d_sumsq, nullable), both device
  * pointers of W*H*3 floats, enqueued on the context stream; synchronised before return
@@ -357,6 +377,8 @@ int vk_multi_render(vk_multi* m, const vk_camera* cam, const vk_render_params* p
                     vk_stats* stats);                                           /* vk_render over all devices              */
 int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* params, uint8_t* out_rgb8,
                          vk_stats* stats);                                      /* vk_render_rgb8 over all devices         */
+int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                                uint8_t* out_rgb8, vk_stats* stats);            /* vk_render_frames_rgb8 over all devices  */
 
 /* Parity hook: closest hit of `world.hit(&r, tmin, tmax)` (src/accel.rs:58-83) for
  * a batch of rays.  medium_xi (nullable): n * VK_MEDIUM_XI_SLOTS uniform variates

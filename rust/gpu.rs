@@ -102,6 +102,12 @@ extern "C" {
     pub fn vk_finalize_device(ctx: *mut vk_ctx, d_sum: *const f32, d_rgb: *mut f32, n_floats: usize, spp: u32) -> c_int;
     pub fn vk_set_stream(ctx: *mut vk_ctx, stream: *mut c_void) -> c_int;
     pub fn vk_flush_stats(ctx: *mut vk_ctx, stats: *mut vk_stats) -> c_int;
+    // K cameras in one launch: frame f uses cams[f] and seed + f, and equals vk_render / vk_render_rgb8 of that camera bit for bit
+    // on the same kernel (AUTO decides on the batch's path count; the render build's kernels round differently)
+    pub fn vk_render_frames(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                            out_rgb: *mut f32, stats: *mut vk_stats) -> c_int;
+    pub fn vk_render_frames_rgb8(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                                 out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
     // one context over several GPUs of the node (samples split by global index, peer-memory reduce on devices[0])
     pub fn vk_multi_create(devices: *const c_int, n_devices: c_int, out: *mut *mut vk_multi) -> c_int;
     pub fn vk_multi_destroy(m: *mut vk_multi);
@@ -111,6 +117,8 @@ extern "C" {
                            out_rgb: *mut f32, out_sumsq: *mut f32, stats: *mut vk_stats) -> c_int;
     pub fn vk_multi_render_rgb8(m: *mut vk_multi, cam: *const vk_camera, params: *const vk_render_params,
                                 out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
+    pub fn vk_multi_render_frames_rgb8(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                                       out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
 }
 #[repr(C)] pub struct vk_multi { _private: [u8; 0] }
 
@@ -267,6 +275,21 @@ impl Gpu {
         self.check(unsafe { vk_render_rgb8(self.ctx, cam, &p, out.as_mut_ptr(), &mut st) })?;
         Ok((out, st))
     }
+    /// Several cameras of the turntable (`config.cam_iter`, src/main.rs:176) in one launch: frame f is
+    /// `render_rgb8(&cams[f], .., seed + f)`, at offset f * W*H*3 of the result -- byte for byte when both run the same
+    /// kernel; AUTO decides on the batch's path count, so a large batch may run a faster kernel, whose rounding differs
+    /// in this (render) build.  The frames share the
+    /// GPU's warps, so small frames fill it and the batch drains once.
+    pub fn render_frames_rgb8(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64)
+                              -> Result<(Vec<u8>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_frames_rgb8: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; cams.len() * width * height * 3];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_frames_rgb8(self.ctx, cams.as_ptr(), cams.len() as u32, &p, out.as_mut_ptr(), &mut st) })?;
+        Ok((out, st))
+    }
     /// One spp slice [begin, begin+count) of the frame, already divided by the full `spp`: slices of disjoint
     /// sample ranges ADD to the frame (the Philox counter holds the global sample index).
     pub fn render_slice(&mut self, cam: &vk_camera, width: usize, height: usize, spp: u32, begin: u32, count: u32,
@@ -309,6 +332,17 @@ impl MultiGpu {
         let mut out = vec![0f32; width * height * 3];
         let mut st = vk_stats::default();
         self.check(unsafe { vk_multi_render(self.m, cam, &p, out.as_mut_ptr(), std::ptr::null_mut(), &mut st) })?;
+        Ok((out, st))
+    }
+    /// `Gpu::render_frames_rgb8` over all devices (every device renders its sample slice of every frame): the same bytes as one GPU's batch.
+    pub fn render_frames_rgb8(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64)
+                              -> Result<(Vec<u8>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_frames_rgb8: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; cams.len() * width * height * 3];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_multi_render_frames_rgb8(self.m, cams.as_ptr(), cams.len() as u32, &p, out.as_mut_ptr(), &mut st) })?;
         Ok((out, st))
     }
 }

@@ -103,10 +103,17 @@ def gpu_lib():
         L.vk_multi_scene_upload.argtypes = [vp, C.POINTER(_abi.vk_scene_desc)]
         L.vk_multi_render.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), vp, vp, C.POINTER(_abi.vk_stats)]
         L.vk_multi_render_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), vp, C.POINTER(_abi.vk_stats)]
-        for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8"):
+        L.vk_render_frames.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), vp, C.POINTER(_abi.vk_stats)]
+        L.vk_render_frames_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), vp,
+                                            C.POINTER(_abi.vk_stats)]
+        L.vk_multi_render_frames_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), vp,
+                                                  C.POINTER(_abi.vk_stats)]
+        for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
+                  "vk_multi_render_frames_rgb8"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
-                  "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info"):
+                  "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
+                  "vk_render_frames", "vk_render_frames_rgb8"):
             getattr(L, f).restype = C.c_int
         _gpu = L
     return _gpu
@@ -115,7 +122,8 @@ def gpu_lib():
 GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device",
                "vk_finalize_device", "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks",
                "vk_device_info", "vk_multi_create", "vk_multi_destroy", "vk_multi_last_error", "vk_multi_device_count",
-               "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8"]
+               "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8", "vk_render_frames", "vk_render_frames_rgb8",
+               "vk_multi_render_frames_rgb8"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
                 "vkh_frame_filename", "vkh_last_error"]
@@ -243,6 +251,15 @@ def render_params(width, height, spp, max_depth=100, seed=1, spp_begin=0, spp_co
     return p
 
 
+def _camera_array(cams):
+    """A list of vk_camera as one contiguous C array (what vk_render_frames* take).  An empty list is rejected here,
+    before the library is called."""
+    cams = list(cams)
+    if not cams:
+        raise ValueError("render_frames: at least one camera")
+    return (_abi.vk_camera * len(cams))(*cams), len(cams)
+
+
 class Context:
     """One GPU context (``vk_create``).  Fails loudly without the CUDA library or a device."""
 
@@ -281,6 +298,25 @@ class Context:
         st = _abi.vk_stats()
         self._check(self._L.vk_render_rgb8(self._h, C.byref(cam), C.byref(params), out.ctypes.data, C.byref(st)))
         return out.reshape(params.height, params.width, 3), st
+
+    def render_frames(self, cams, params):
+        """``vk_render_frames``: K cameras in one launch, frame f with seed ``params.seed + f``; frame f equals
+        ``render(cams[f], params with seed + f)`` bit for bit on the same kernel: always with VK_FLAG_STRICT_MATH or an
+        explicit variant; with AUTO in the render build a batch large enough to change kernel rounds differently.  Returns ((K, H, W, 3) float32, stats of the batch)."""
+        arr, k = _camera_array(cams)
+        out = np.empty(k * params.width * params.height * 3, dtype=np.float32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_frames(self._h, arr, k, C.byref(params), out.ctypes.data, C.byref(st)))
+        return out.reshape(k, params.height, params.width, 3), st
+
+    def render_frames_rgb8(self, cams, params):
+        """``vk_render_frames_rgb8``: as render_frames, every frame as render_rgb8 returns it (rows top-down).
+        Returns ((K, H, W, 3) uint8, stats of the batch)."""
+        arr, k = _camera_array(cams)
+        out = np.empty(k * params.width * params.height * 3, dtype=np.uint8)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_frames_rgb8(self._h, arr, k, C.byref(params), out.ctypes.data, C.byref(st)))
+        return out.reshape(k, params.height, params.width, 3), st
 
     def render_device(self, cam, params, d_sum_ptr, d_sumsq_ptr=None, want_stats=True):
         """``vk_render_device``: per-pixel SUMS of an spp slice into device memory.  With
@@ -377,6 +413,14 @@ class MultiContext:
         st = _abi.vk_stats()
         self._check(self._L.vk_multi_render_rgb8(self._h, C.byref(cam), C.byref(params), out.ctypes.data, C.byref(st)))
         return out.reshape(params.height, params.width, 3), st
+
+    def render_frames_rgb8(self, cams, params):
+        """``vk_multi_render_frames_rgb8``: Context.render_frames_rgb8 over all devices, the same frames bit for bit as one GPU's batch."""
+        arr, k = _camera_array(cams)
+        out = np.empty(k * params.width * params.height * 3, dtype=np.uint8)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_multi_render_frames_rgb8(self._h, arr, k, C.byref(params), out.ctypes.data, C.byref(st)))
+        return out.reshape(k, params.height, params.width, 3), st
 
     def close(self):
         if getattr(self, "_h", None):

@@ -52,6 +52,9 @@ struct vk_ctx {
     size_t frame_floats = 0;
     float* pinned = nullptr; // pinned host staging for the D2H of vk_render
     size_t pinned_floats = 0;
+    DCamera* cams = nullptr; // vk_render_frames: the batch's cameras on the device (FrameArgs::cams)
+    size_t cams_cap = 0;
+    std::vector<DCamera> cams_host;
     // wavefront variant: the slot pool (allocated on first use) and a pinned word block for the
     // host's termination checks
     WfState wf{};
@@ -98,6 +101,18 @@ __global__ void k_to_color(const float* __restrict__ sum, uint8_t* __restrict__ 
     float v = sqrtf(c);
     v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v); // Vec3::clamp keeps NaN
     out[i] = (uint8_t)__float2uint_rz(256.0f * v);   // `as u32`: NaN -> 0
+}
+// k_to_color over n_frames frames of a batch (contiguous planes), each frame top-down on its own
+__global__ void k_to_color_frames(const float* __restrict__ sum, uint8_t* __restrict__ out, uint32_t width, uint32_t height, uint32_t n_frames,
+                                  float spp) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, plane = (size_t)width * height * 3;
+    if (i >= plane * n_frames) return;
+    const size_t f = i / plane, j = i - f * plane;
+    const size_t row = j / ((size_t)width * 3), col = j - row * (size_t)width * 3;
+    const float c = sum[f * plane + (size_t)(height - 1 - row) * width * 3 + col] / spp;
+    float v = sqrtf(c);
+    v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v);
+    out[i] = (uint8_t)__float2uint_rz(256.0f * v);
 }
 // FP32 peak: 8 independent FFMA chains per thread, no memory traffic
 __global__ void k_ffma_peak(float* out, int iters) {
@@ -244,6 +259,7 @@ void vk_destroy(vk_ctx* c) {
     if (c->wf_host_counts) cudaFreeHost(c->wf_host_counts);
     if (c->frame) cudaFree(c->frame);
     if (c->pinned) cudaFreeHost(c->pinned);
+    if (c->cams) cudaFree(c->cams);
     if (c->counters) cudaFree(c->counters);
     if (c->debug) cudaFree(c->debug);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -462,7 +478,8 @@ static int wf_render(vk_ctx* c, bool strict, const FlatProgram* flat, const DCam
 //   BVH scenes                               -> MEGAKERNEL (final scene: 49 ms against 78 ms staged and
 //       98 ms wavefront: while-while traversal diverges whatever the staging, and the lane
 //       megakernel keeps 32 warps per SM against 24)
-static uint32_t choose_variant(const vk_ctx* c, const vk_render_params* P) {
+// (n_frames: a batch of frames is decided on its path count, all frames together)
+static uint32_t choose_variant(const vk_ctx* c, const vk_render_params* P, uint32_t n_frames = 1) {
     if (P->variant != VK_VARIANT_AUTO) return P->variant;
     const bool flat = c->flat.n && !(P->flags & VK_FLAG_FORCE_BVH);
     // (a hybrid program holds subtrees whose traversal lengths vary: the lane megakernel, not the
@@ -478,7 +495,7 @@ static uint32_t choose_variant(const vk_ctx* c, const vk_render_params* P) {
     // -- and only for frames that fill the pools a few dozen times over: 227 000 slots are resident, and below ~3 M paths
     // their start-up and drain cost more than the fuller warps gain (random spheres 400x225: 16 spp 1.32 against 1.21 ms,
     // 32 spp 1.85 against 1.83, 64 spp 2.78 against 3.30; profiles/r2_sweep_9.log)
-    const uint64_t paths = (uint64_t)P->width * P->height * (P->spp_count ? P->spp_count : P->spp - P->spp_begin);
+    const uint64_t paths = (uint64_t)P->width * P->height * (P->spp_count ? P->spp_count : P->spp - P->spp_begin) * n_frames;
     return c->levels_sub == 0u && paths >= (4ull << 20) ? (uint32_t)VK_VARIANT_STEPQ : (uint32_t)VK_VARIANT_MEGAKERNEL;
 }
 
@@ -516,11 +533,28 @@ static void apply_l2_window(vk_ctx* c) {
     cudaGetLastError();
 }
 
-// shared body of vk_render / vk_render_device
+// What vk_render_frames* reject before anything is allocated or launched (`who` names the call in the message).
+static int check_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P) {
+    if (!cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, std::string(who) + ": null argument or no frames");
+    if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, std::string(who) + ": no scene uploaded");
+    for (uint32_t f = 0; f < n_frames; ++f)
+        if (!(cams[f].time0 < cams[f].time1))
+            return fail(c, VK_ERR_INVALID, std::string(who) + ": frame " + std::to_string(f) + ": camera time0 >= time1 (gen_range panics, src/main.rs:118)");
+    // the kernels index the accumulators of the whole batch with 32-bit pixels: render_into's bound for one frame, on the batch
+    if ((uint64_t)P->width * P->height * n_frames > 0x7FFFFFFFull / 3)
+        return fail(c, VK_ERR_INVALID, std::string(who) + ": batch too large (n_frames * width * height * 3 exceeds 2^31 - 1)");
+    if (n_frames > 1 && (P->variant == VK_VARIANT_STAGED || P->variant == VK_VARIANT_WAVEFRONT))
+        return fail(c, VK_ERR_UNSUPPORTED, std::string(who) + ": the staged and wavefront kernels render one frame per call");
+    return VK_OK;
+}
+
+// shared body of vk_render / vk_render_device / vk_render_frames*
 // acc_only: leave the result in the context's integer accumulators (c->partial) and skip the conversion to fp32 sums
 // (the multi-GPU context reduces the accumulators of all its devices itself); want_sq then says whether squares are kept
+// n_frames > 1: cam points to n_frames cameras and the result is n_frames contiguous planes (check_frames has passed; the
+// batch kernels take FrameArgs, everything else is the single-frame path)
 static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* d_sum, float* d_sumsq, vk_stats* stats,
-                       bool acc_only = false, bool want_sq = false) {
+                       bool acc_only = false, bool want_sq = false, uint32_t n_frames = 1) {
     if (!c) return VK_ERR_INVALID;
     if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, "render: no scene uploaded");
     if (!cam || !P || (!d_sum && !acc_only)) return fail(c, VK_ERR_INVALID, "render: null argument");
@@ -538,7 +572,7 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     const FlatProgram* flat = (c->flat.n && !(P->flags & VK_FLAG_FORCE_BVH)) ? &c->flat : nullptr;
     int bps = 0, bt = 0;
     const bool legacy = (P->flags & VK_FLAG_LEGACY_SCATTER) != 0;
-    uint32_t variant = choose_variant(c, P);
+    uint32_t variant = choose_variant(c, P, n_frames);
     if (legacy && variant != VK_VARIANT_WARPQ && variant != VK_VARIANT_STEPQ) variant = VK_VARIANT_MEGAKERNEL; // legacy integrator: lane megakernel and warp queues
     // a hybrid program (flat top + homogeneous subtrees) is the warp-queue kernel's: every other variant walks the BVH
     // (lane megakernel on it: 51.5 against 46.1 ms on the final scene, profiles/r2_sweep_12.log)
@@ -547,6 +581,8 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         return fail(c, VK_ERR_UNSUPPORTED, "render: SpecDiffuse has no legacy scatter (the reference's default unwraps a missing specular ray and panics, src/material.rs:21-28)");
     if (!legacy && c->scene.n_lights == 0)
         return fail(c, VK_ERR_INVALID, "render: empty light list (the reference panics: choose().unwrap(), src/hittable.rs:431); only VK_FLAG_LEGACY_SCATTER renders without lights");
+    if (n_frames > 1 && (variant == VK_VARIANT_STAGED || variant == VK_VARIANT_WAVEFRONT))
+        return fail(c, VK_ERR_UNSUPPORTED, "render: the staged and wavefront kernels render one frame per call");
     // the render build compiled for a light list of one unflipped Rect (VK_LIGHT0, see vk_device.cuh)
     const bool l0 = !strict && !legacy && c->one_rect_light && !c->has_specdiffuse && !std::getenv("VECCHIO_NO_LIGHT0");
     CU(c, strict ? vkstrict::megakernel_occupancy(flat != nullptr, c->scene.has_media, legacy, &bps, &bt)
@@ -569,7 +605,7 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     a.tiles_x = (P->width + 7) / 8;
     a.tiles_y = (P->height + 3) / 4;
     // Accumulators (see RenderBuffers): u64 fixed-point sums, plus double sums of squares when asked for.
-    const size_t plane = (size_t)P->width * P->height * 3;
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
     RenderBuffers b{};
     b.counters = c->counters;
     b.debug = c->debug;
@@ -582,7 +618,7 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     }
     // Lane megakernel: chunks of samples, sized for ~48 work items per resident warp (small items keep
     // the end-of-kernel tail short; an item costs one atomic).
-    const uint32_t n_tiles = a.tiles_x * a.tiles_y;
+    const uint32_t n_tiles = a.tiles_x * a.tiles_y * n_frames; // (a batch: the items of all its frames share the warps)
     uint32_t n_chunks = (48u * resident_warps + n_tiles - 1) / n_tiles;
     if (n_chunks > count) n_chunks = count;
     if (n_chunks < 1) n_chunks = 1;
@@ -593,6 +629,25 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     apply_l2_window(c);
     CU(c, cudaEventRecord(c->ev0, c->stream));
     const DCamera dc = to_dcam(cam);
+    // a batch: its cameras go to the device with the call (read at regeneration only), FrameArgs selects the batch kernels
+    FrameArgs fa{};
+    const FrameArgs* fr = nullptr;
+    if (n_frames > 1) {
+        if (c->cams_cap < n_frames) {
+            if (c->cams) cudaFree(c->cams);
+            c->cams = nullptr;
+            c->cams_cap = 0;
+            CU(c, cudaMalloc((void**)&c->cams, n_frames * sizeof(DCamera)));
+            c->cams_cap = n_frames;
+        }
+        c->cams_host.resize(n_frames);
+        for (uint32_t f = 0; f < n_frames; ++f) c->cams_host[f] = to_dcam(cam + f);
+        CU(c, cudaMemcpyAsync(c->cams, c->cams_host.data(), n_frames * sizeof(DCamera), cudaMemcpyHostToDevice, c->stream));
+        fa.cams = c->cams;
+        fa.n_frames = n_frames;
+        fa.n_pix = P->width * P->height;
+        fr = &fa;
+    }
     uint32_t launches = 0;
     if (variant == VK_VARIANT_STEPQ && flat && flat->n_bvh == 0) variant = VK_VARIANT_WARPQ; // step queues are the BVH traversal; a flat program has none
     if (variant == VK_VARIANT_STEPQ) {
@@ -606,9 +661,9 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         }
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
         CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
-        CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream)
-              : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream)
-                     : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream));
+        CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr)
+              : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr)
+                     : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr));
         launches = 1;
     } else if (variant == VK_VARIANT_WARPQ) {
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
@@ -616,10 +671,10 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         // (a hybrid program -- flat top, homogeneous subtrees walked inside extend -- runs k_warpq_hybrid)
         const FlatProgram* sflat = flat;
         const bool simple = !strict && !legacy && sflat && sflat->n_bvh == 0 && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
-        CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream)
-              : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream)
-              : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream)
-                       : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream));
+        CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
+              : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
+              : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
+                       : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr));
         launches = 1;
     } else if (variant == VK_VARIANT_WAVEFRONT) {
         int rc = wf_render(c, strict, flat, dc, a, b, &launches);
@@ -638,14 +693,14 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         launches = 1;
     } else if (!flat && !legacy && use_dynamic_megakernel(c)) {
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream)
-              : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream)
-                     : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream));
+        CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr)
+              : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr)
+                     : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr));
         launches = 1;
     } else {
-        CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream)
-              : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream)
-                     : vkfast::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream));
+        CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr)
+              : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr)
+                     : vkfast::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr));
         launches = 1;
     }
     if (!acc_only) {
@@ -655,7 +710,7 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     CU(c, cudaGetLastError());
     CU(c, cudaEventRecord(c->ev1, c->stream));
     c->launches += launches;
-    c->paths += (uint64_t)P->width * P->height * count;
+    c->paths += (uint64_t)P->width * P->height * count * n_frames;
     if (stats) { // reading the counters synchronises; with stats == NULL the call is fully asynchronous
         int rc = vk_flush_stats(c, stats);
         if (rc != VK_OK) return rc;
@@ -785,6 +840,62 @@ int vk_render_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, u
     CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
     if (stats) *stats = st;
     return VK_OK;
+}
+
+// shared body of vk_render_frames / vk_render_frames_rgb8 (n_frames > 1; one frame is vk_render / vk_render_rgb8): one
+// launch over every frame's units, then the conversion of all planes and one copy back through the pinned staging
+static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb,
+                         uint8_t* out_rgb8, vk_stats* stats) {
+    int rc = check_frames(c, who, cams, n_frames, P);
+    if (rc != VK_OK) return rc;
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames; // all frames
+    CU(c, cudaSetDevice(c->device));
+    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane * 2)) != VK_OK) return rc; // sums | rgb
+    const size_t out_floats = out_rgb ? plane : (plane + 3) / 4;
+    if (c->pinned_floats < out_floats) {
+        if (c->pinned) cudaFreeHost(c->pinned);
+        c->pinned = nullptr;
+        c->pinned_floats = 0;
+        CU(c, cudaMallocHost((void**)&c->pinned, out_floats * sizeof(float)));
+        c->pinned_floats = out_floats;
+    }
+    float *d_sum = c->frame, *d_rgb = c->frame + plane;
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    vk_stats st{};
+    rc = render_into(c, cams, P, d_sum, nullptr, &st, false, false, n_frames);
+    if (rc != VK_OK) return rc;
+    if (out_rgb) {
+        k_finalize<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, d_rgb, plane, (float)P->spp);
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned, d_rgb, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    } else {
+        k_to_color_frames<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, (uint8_t*)d_rgb, P->width, P->height, n_frames, (float)P->spp);
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned, d_rgb, plane, cudaMemcpyDeviceToHost, c->stream));
+    }
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (out_rgb) std::memcpy(out_rgb, c->pinned, plane * sizeof(float));
+    else std::memcpy(out_rgb8, c->pinned, plane);
+    st.launches += 1;
+    c->launches = 0;
+    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!cams || !P || !out_rgb || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames: null argument or no frames");
+    if (n_frames == 1) return vk_render(c, cams, P, out_rgb, nullptr, stats);
+    return render_frames(c, "vk_render_frames", cams, n_frames, P, out_rgb, nullptr, stats);
+}
+
+int vk_render_frames_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!cams || !P || !out_rgb8 || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_rgb8: null argument or no frames");
+    if (n_frames == 1) return vk_render_rgb8(c, cams, P, out_rgb8, stats);
+    return render_frames(c, "vk_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, stats);
 }
 
 int vk_intersect(vk_ctx* c, const vk_ray* rays, size_t n, const float* medium_xi, uint32_t flags, vk_hit* out) {
@@ -926,13 +1037,15 @@ int vk_multi_scene_upload(vk_multi* m, const vk_scene_desc* scene) {
 }
 
 // shared body of vk_multi_render / vk_multi_render_rgb8: every device accumulates its slice, device 0 reduces
-static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_params* P, bool want_sq, float** d_sum, float** d_sq, vk_stats* st) {
+// (n_frames > 1: a batch, every device renders its sample slice of every frame; check_frames has passed on every device)
+static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_params* P, bool want_sq, float** d_sum, float** d_sq, vk_stats* st,
+                             uint32_t n_frames = 1) {
     if (!m || !cam || !P) return mfail(m, VK_ERR_INVALID, "vk_multi_render: null argument");
     const int n = (int)m->ctx.size();
     const uint32_t begin = P->spp_begin, count = P->spp_count ? P->spp_count : (P->spp > P->spp_begin ? P->spp - P->spp_begin : 0u);
     if (P->spp == 0 || count == 0 || (uint64_t)begin + count > P->spp) return mfail(m, VK_ERR_INVALID, "vk_multi_render: bad spp range");
     vk_ctx* c0 = m->ctx[0];
-    const size_t plane = (size_t)P->width * P->height * 3;
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
     cudaSetDevice(c0->device);
     cudaEventRecord(c0->ev2, c0->stream);
     int active = 0;
@@ -944,7 +1057,7 @@ static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_
         q.spp_begin = s0;
         q.spp_count = s1 - s0;
         vk_ctx* c = m->ctx[k];
-        const int rc = render_into(c, cam, &q, nullptr, nullptr, nullptr, true, want_sq);
+        const int rc = render_into(c, cam, &q, nullptr, nullptr, nullptr, true, want_sq, n_frames);
         if (rc != VK_OK) return mfail(m, rc, c->err);
         cudaSetDevice(c->device);
         cudaEventRecord(m->done[k], c->stream);
@@ -1031,6 +1144,35 @@ int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_para
     cudaEventRecord(c0->ev1, c0->stream);
     cudaError_t e = cudaStreamSynchronize(c0->stream);
     if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("vk_multi_render_rgb8: ") + cudaGetErrorString(e));
+    std::memcpy(out_rgb8, c0->pinned, plane);
+    cudaEventElapsedTime(&st.ms_total, c0->ev2, c0->ev1);
+    st.launches += 1;
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8,
+                                vk_stats* stats) {
+    if (!m || !cams || !P || !out_rgb8 || n_frames == 0) return mfail(m, VK_ERR_INVALID, "vk_multi_render_frames_rgb8: null argument or no frames");
+    if (n_frames == 1) return vk_multi_render_rgb8(m, cams, P, out_rgb8, stats);
+    for (vk_ctx* c : m->ctx) { // every device, before any of them launches
+        const int rc = check_frames(c, "vk_multi_render_frames_rgb8", cams, n_frames, P);
+        if (rc != VK_OK) return mfail(m, rc, c->err);
+    }
+    float *d_sum = nullptr, *d_sq = nullptr;
+    vk_stats st{};
+    int rc = multi_render_sums(m, cams, P, false, &d_sum, &d_sq, &st, n_frames);
+    if (rc != VK_OK) return rc;
+    vk_ctx* c0 = m->ctx[0];
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
+    if ((rc = multi_pinned(m, c0, (plane + 3) / 4)) != VK_OK) return rc;
+    cudaSetDevice(c0->device);
+    uint8_t* d_rgb8 = (uint8_t*)(c0->frame + 2 * plane);
+    k_to_color_frames<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(d_sum, d_rgb8, P->width, P->height, n_frames, (float)P->spp);
+    cudaMemcpyAsync(c0->pinned, d_rgb8, plane, cudaMemcpyDeviceToHost, c0->stream);
+    cudaEventRecord(c0->ev1, c0->stream);
+    cudaError_t e = cudaStreamSynchronize(c0->stream);
+    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("vk_multi_render_frames_rgb8: ") + cudaGetErrorString(e));
     std::memcpy(out_rgb8, c0->pinned, plane);
     cudaEventElapsedTime(&st.ms_total, c0->ev2, c0->ev1);
     st.launches += 1;

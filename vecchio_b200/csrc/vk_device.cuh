@@ -120,6 +120,17 @@ struct PathRng {
         return philox4x32_10(make_uint4(pixel, sample, (depth << 8) | blk, w), key);
     }
 };
+// Philox key of frame f of a batch (FrameArgs): seed + f, the key vecchio_gpu_render --seed gives frame f of a frame loop
+VKD uint2 frame_key(const RenderArgs& a, uint32_t f) {
+    const unsigned long long k = (((unsigned long long)a.seed_hi << 32) | a.seed_lo) + f;
+    return make_uint2((uint32_t)k, (uint32_t)(k >> 32));
+}
+// A batch-wide pixel index (f * n_pix + the pixel within frame f, see FrameArgs) -> the frame's own counter pixel and key
+VKD void frame_rng(PathRng& rng, const RenderArgs& a, uint32_t n_pix, uint32_t gpix) {
+    const uint32_t f = gpix / n_pix;
+    rng.pixel = gpix - f * n_pix;
+    rng.key = frame_key(a, f);
+}
 // Source of the ConstantMedium free-flight variate (src/hittable.rs:473): an injected table for
 // vk_intersect (VK_MEDIUM_XI_SLOTS entries per ray: scenes of up to four media), and for the render
 // Philox block 1 of the current segment with the counter's fourth word counting groups of four

@@ -189,6 +189,19 @@ struct RenderArgs {
     uint32_t tiles_x, tiles_y, n_chunks, chunk_spp;
 };
 
+// A batch of frames (vk_render_frames): frame f renders with cams[f] and Philox key seed + f (64-bit add) into the
+// accumulator plane that starts at f * n_pix * 3; pixel and sample of the Philox counter are the frame's own, so every frame
+// equals its single-frame render.  Only the batch instantiations of the kernels take it, as a kernel parameter behind all
+// the others: RenderArgs and everything in front of it keep the single-frame kernels' layout.  Their work units are
+// frame-major (the frame is the outermost dimension): a warp whose frame has run dry takes the next frame's units, and the
+// batch drains once.  Inside the warp-queue slots a pixel is the batch-wide index f * n_pix + y * width + x (the slot does
+// not grow); the frame is recovered from it where a PathRng is rebuilt.
+struct FrameArgs {
+    const DCamera* cams; // device array, n_frames entries
+    uint32_t n_frames;
+    uint32_t n_pix;      // width * height
+};
+
 // Accumulation.  Every finished sample is added to its pixel with three 64-bit integer atomics
 // (fixed point, VK_ACC_SCALE = 2^30 units per 1.0): integer addition is associative, so the frame is
 // bit-identical for a (seed, sample range, image size) whatever the kernel variant, the scheduling of
@@ -239,9 +252,11 @@ struct WfState {
 #define VK_DECLARE_LAUNCHERS(NS)                                                                                       \
     namespace NS {                                                                                                     \
     cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,  \
-                                  const RenderBuffers& b, int grid, bool legacy, cudaStream_t st);                     \
+                                  const RenderBuffers& b, int grid, bool legacy, cudaStream_t st,                      \
+                                  const FrameArgs* fr = nullptr);                                                      \
     cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, \
-                                      unsigned long long* unit_head, int sm_count, cudaStream_t st);                   \
+                                      unsigned long long* unit_head, int sm_count, cudaStream_t st,                     \
+                                      const FrameArgs* fr = nullptr);                                                  \
     cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk_ray* rays, size_t n,              \
                                  const float* medium_xi, vk_hit* out, cudaStream_t st);                                \
     cudaError_t megakernel_occupancy(bool flat, bool media, bool legacy, int* blocks_per_sm, int* block_threads);      \
@@ -252,11 +267,11 @@ struct WfState {
                               const RenderBuffers& b, unsigned long long* unit_head, int sm_count, cudaStream_t st);   \
     cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,       \
                              const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy,         \
-                             cudaStream_t st);                                                                         \
+                             cudaStream_t st, const FrameArgs* fr = nullptr);                                          \
     size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t* levels);                          \
     cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,        \
                              unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, \
-                             bool legacy, cudaStream_t st);                                                            \
+                             bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr);                             \
     cudaError_t launch_wf_generate(const DCamera& cam, const RenderArgs& a, const WfState& w, cudaStream_t st);        \
     cudaError_t launch_wf_extend(const DScene& sc, const FlatProgram* flat, const RenderArgs& a, const WfState& w,     \
                                  const RenderBuffers& b, uint32_t set, cudaStream_t st);                               \
@@ -270,5 +285,5 @@ namespace vkfast_simple { // vk_staged.cu / vk_warpq.cu compiled with VK_SIMPLE=
 cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
                           unsigned long long* unit_head, int sm_count, cudaStream_t st);
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st);
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr);
 }

@@ -25,19 +25,27 @@ namespace VK_NS {
 #define VK_MINB_BVH 5
 #endif
 
+// accumulator pixel of a lane's sample: in a batch (FR) the frame's plane starts at pixel pbase
+template <bool FR> VKD uint32_t frame_pixel(uint32_t pbase, uint32_t pixel) {
+    if constexpr (FR) return pbase + pixel;
+    else return pixel;
+}
+
 // Work decomposition (deterministic for a seed whatever the grid):
 //   item  = one 8x4 pixel tile x one chunk of samples, fetched by a whole warp from a global queue;
 //   unit  = one pixel of the tile x one sample.  The 32 lanes of the warp draw units from a
 //           warp-local counter (ballot + popc, no memory traffic): a lane whose path has ended takes
 //           the next one, so lanes only idle for the last unit of an item.
 // A finished sample goes straight into its pixel's integer accumulators (accumulate_sample).
-template <bool FLAT, bool MEDIA, bool LEGACY>
+// FR: a batch of frames (FrameArgs, k_megakernel*_frames): item = frame x chunk x tile, frame outermost.
+template <bool FLAT, bool MEDIA, bool LEGACY, bool FR = false>
 VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,
-                         const RenderBuffers& buf) {
+                         const RenderBuffers& buf, const FrameArgs* fr = nullptr) {
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t lanes_below = (1u << lane) - 1u;
     const uint32_t n_tiles = a.tiles_x * a.tiles_y;
-    const uint32_t total = n_tiles * a.n_chunks;
+    uint32_t total = n_tiles * a.n_chunks;
+    if constexpr (FR) total *= fr->n_frames;
     const uint32_t spp_end = a.spp_begin + a.spp_count;
     uint32_t n_rays = 0, n_drop = 0, n_nodes = 0, n_prims = 0; // per lane: far below 2^32 for any frame
 
@@ -47,6 +55,12 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
         if (lane == 0) item = (uint32_t)atomicAdd(&buf.counters[2], 1ull);
         item = __shfl_sync(0xFFFFFFFFu, item, 0);
         if (item >= total) break;
+        uint32_t f = 0, pbase = 0; // (FR) frame of the item, its first pixel in the accumulators
+        if constexpr (FR) {
+            f = item / (n_tiles * a.n_chunks);
+            item -= f * (n_tiles * a.n_chunks);
+            pbase = f * fr->n_pix;
+        }
         const uint32_t chunk = item / n_tiles, tile = item - chunk * n_tiles;
         const uint32_t px0 = (tile % a.tiles_x) * 8u, py0 = (tile / a.tiles_x) * 4u;
         const uint32_t c0 = a.spp_begin + chunk * a.chunk_spp;
@@ -58,6 +72,7 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
         rng.pixel = 0;
         rng.sample = 0;
         rng.key = make_uint2(a.seed_lo, a.seed_hi);
+        if constexpr (FR) rng.key = frame_key(a, f);
         float3 o = f3(0.0f, 0.0f, 0.0f), d = o, beta = o, L = o;
         float time = 0.0f;
         uint32_t depth = 0, s = 0, s_end = 0, px = 0, py = 0;
@@ -89,7 +104,8 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
             // ---- one path segment ---------------------------------------------------------------
             if (!alive) { // regenerate: this lane starts its next sample while others keep bouncing
                 rng.sample = s++;
-                camera_get_ray(cam, rng, px, py, a.width, a.height, o, d, time);
+                if constexpr (FR) camera_get_ray(fr->cams[f], rng, px, py, a.width, a.height, o, d, time);
+                else camera_get_ray(cam, rng, px, py, a.width, a.height, o, d, time);
                 beta = f3(1.0f, 1.0f, 1.0f);
                 L = f3(0.0f, 0.0f, 0.0f);
                 depth = 1; // ray_color(ray, .., 1) src/main.rs:190
@@ -125,7 +141,7 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
                 }
             }
             if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                if (valid && finite3(L)) accumulate_sample(buf, rng.pixel, L);
+                if (valid && finite3(L)) accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
                 else ++n_drop;
             }
         }
@@ -169,12 +185,15 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VK_DYN_NODE_STEPS
 #define VK_DYN_NODE_STEPS 4
 #endif
-template <bool MEDIA>
+// FR: a batch of frames (FrameArgs, k_megakernel_dyn_frames): unit = frame x sample x pixel, frame outermost.
+template <bool MEDIA, bool FR = false>
 VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                             unsigned long long* unit_head) {
+                             unsigned long long* unit_head, const FrameArgs* fr = nullptr) {
     const uint32_t lane = threadIdx.x & 31u, lanes_below = (1u << lane) - 1u;
     const uint32_t n_pixels = a.width * a.height;
-    const unsigned long long n_units = (unsigned long long)n_pixels * a.spp_count;
+    unsigned long long n_units = (unsigned long long)n_pixels * a.spp_count;
+    if constexpr (FR) n_units *= fr->n_frames;
+    uint32_t pbase = 0; // (FR) first accumulator pixel of this lane's frame
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
 
@@ -218,7 +237,7 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
                     }
                 }
                 if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                    if (valid && finite3(L)) accumulate_sample(buf, rng.pixel, L);
+                    if (valid && finite3(L)) accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
                     else ++n_drop;
                 }
             }
@@ -231,12 +250,21 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
             if (lane == 0) base = atomicAdd(unit_head, (unsigned long long)__popc(mu));
             base = __shfl_sync(0xFFFFFFFFu, base, 0);
             if (need_unit) {
-                const unsigned long long u = base + __popc(mu & lanes_below);
+                unsigned long long u = base + __popc(mu & lanes_below);
                 if (u < n_units) {
+                    uint32_t f = 0;
+                    if constexpr (FR) {
+                        const unsigned long long per_frame = (unsigned long long)n_pixels * a.spp_count;
+                        f = (uint32_t)(u / per_frame);
+                        u -= (unsigned long long)f * per_frame;
+                        pbase = f * n_pixels;
+                        rng.key = frame_key(a, f);
+                    }
                     const uint32_t sb = (uint32_t)(u / n_pixels);
                     rng.pixel = (uint32_t)(u - (unsigned long long)sb * n_pixels); // i = y*width + x (src/main.rs:182-183)
                     rng.sample = a.spp_begin + sb;
-                    camera_get_ray(cam, rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
+                    if constexpr (FR) camera_get_ray(fr->cams[f], rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
+                    else camera_get_ray(cam, rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
                     beta = f3(1.0f, 1.0f, 1.0f);
                     depth = 1;
                     new_ray = true;
@@ -292,6 +320,12 @@ __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn(const 
                                                                       const RenderBuffers buf, unsigned long long* unit_head) {
     megakernel_dyn_body<MEDIA>(sc, cam, a, buf, unit_head);
 }
+template <bool MEDIA>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn_frames(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                             const RenderBuffers buf, unsigned long long* unit_head,
+                                                                             const __grid_constant__ FrameArgs fr) {
+    megakernel_dyn_body<MEDIA, true>(sc, cam, a, buf, unit_head, &fr);
+}
 
 // instantiations: {BVH, flat program} x {scene without / with ConstantMedium} x {HEAD integrator, legacy scatter}
 template <bool MEDIA, bool LEGACY>
@@ -303,6 +337,18 @@ template <bool MEDIA, bool LEGACY>
 __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat(const DScene sc, const __grid_constant__ FlatProgram flat,
                                                                        const DCamera cam, const RenderArgs a, const RenderBuffers buf) {
     megakernel_body<true, MEDIA, LEGACY>(sc, &flat, cam, a, buf);
+}
+// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_frames(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                         const RenderBuffers buf, const __grid_constant__ FrameArgs fr) {
+    megakernel_body<false, MEDIA, LEGACY, true>(sc, nullptr, cam, a, buf, &fr);
+}
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat_frames(const DScene sc, const __grid_constant__ FlatProgram flat,
+                                                                              const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                              const __grid_constant__ FrameArgs fr) {
+    megakernel_body<true, MEDIA, LEGACY, true>(sc, &flat, cam, a, buf, &fr);
 }
 
 template <bool FLAT>
@@ -416,14 +462,20 @@ __global__ void k_philox_kat(const uint32_t* in6, uint32_t* out4) {
 }
 
 // *unit_head must be zero on the stream before the launch
+// fr != nullptr: a batch of frames (k_megakernel_dyn_frames)
 cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                                  unsigned long long* unit_head, int sm_count, cudaStream_t st) {
+                                  unsigned long long* unit_head, int sm_count, cudaStream_t st, const FrameArgs* fr) {
     int bps = 0;
-    cudaError_t e = sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<true>, VK_BLOCK, 0)
-                                 : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<false>, VK_BLOCK, 0);
+    cudaError_t e = fr ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<true>, VK_BLOCK, 0)
+                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<false>, VK_BLOCK, 0))
+                       : (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<true>, VK_BLOCK, 0)
+                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<false>, VK_BLOCK, 0));
     if (e != cudaSuccess) return e;
     const int grid = sm_count * (bps < 1 ? 1 : bps);
-    if (sc.has_media) k_megakernel_dyn<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
+    if (fr) {
+        if (sc.has_media) k_megakernel_dyn_frames<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
+        else k_megakernel_dyn_frames<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
+    } else if (sc.has_media) k_megakernel_dyn<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
     else k_megakernel_dyn<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
     return cudaGetLastError();
 }
@@ -435,9 +487,18 @@ cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const Re
         if (media) { if (legacy) { CALL_BVH(true, true); } else { CALL_BVH(true, false); } }                           \
         else { if (legacy) { CALL_BVH(false, true); } else { CALL_BVH(false, false); } }                               \
     }
+// fr != nullptr: a batch of frames (k_megakernel*_frames; the grid is the single-frame kernels', same registers)
 cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flatp, const DCamera& cam, const RenderArgs& a,
-                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st) {
+                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const FrameArgs* fr) {
     const bool flat = flatp && flatp->n, media = sc.has_media;
+    if (fr) {
+#define VK_LB(M, G) k_megakernel_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, *fr)
+#define VK_LF(M, G) k_megakernel_flat_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, *fr)
+        VK_MEGA_DISPATCH(VK_LB, VK_LF)
+#undef VK_LB
+#undef VK_LF
+        return cudaGetLastError();
+    }
 #define VK_LB(M, G) k_megakernel<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b)
 #define VK_LF(M, G) k_megakernel_flat<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b)
     VK_MEGA_DISPATCH(VK_LB, VK_LF)

@@ -139,13 +139,14 @@ VKD bool sq_pick(const W& S, uint32_t last_q, uint32_t& q, uint32_t& n_q, uint32
     return (key >> 4) != 0u;
 }
 
-template <bool MEDIA, bool LEGACY, class W>
+// FR: a batch of frames (FrameArgs, the *_frames kernels)
+template <bool MEDIA, bool LEGACY, class W, bool FR = false>
 VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
-                    uint32_t* gstack, uint32_t glevels) {
+                    uint32_t* gstack, uint32_t glevels, const FrameArgs* fr = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W> C = wq_ctx(cam, a, S, unit_head, lane);
+    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -322,6 +323,7 @@ VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, c
                                 xi.rng.key = make_uint2(a.seed_lo, a.seed_hi);
                                 xi.rng.pixel = S.px[slot];
                                 xi.rng.sample = __float_as_uint(S.bt[slot].w);
+                                if constexpr (FR) frame_rng(xi.rng, a, fr->n_pix, xi.rng.pixel);
                                 hit = medium_t(sc, leaf, to, td, time, tmin, best_t, xi, t);
                             } else {
                                 hit = leaf_t(sc, leaf, to, td, rcp3(td), time, tmin, best_t, t, face);
@@ -380,6 +382,19 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst(co
                                                                           unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels) {
     stepq_body<MEDIA, LEGACY, WqStepInst>(sc, cam, a, buf, unit_head, gstack, glevels);
 }
+// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB) k_stepq_frames(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                       unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
+                                                                       const __grid_constant__ FrameArgs fr) {
+    stepq_body<MEDIA, LEGACY, WqStepWorld, true>(sc, cam, a, buf, unit_head, gstack, glevels, &fr);
+}
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst_frames(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                                 const RenderBuffers buf, unsigned long long* unit_head, uint32_t* gstack,
+                                                                                 uint32_t glevels, const __grid_constant__ FrameArgs fr) {
+    stepq_body<MEDIA, LEGACY, WqStepInst, true>(sc, cam, a, buf, unit_head, gstack, glevels, &fr);
+}
 
 // What the launch needs of the overflow stack: `words` 32-bit words for a scene whose traversal may hold `stack_need`
 // entries (vk_scene_info); 0 when the shared-memory part is enough.
@@ -389,25 +404,30 @@ size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t*
     return warps * *levels * (inst ? VKS_N_INST : VKS_N);
 }
 
+// fr != nullptr: a batch of frames, the *_frames kernels
 cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, unsigned long long* unit_head,
-                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st) {
+                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
-#define VKS_LAUNCH(KERNEL, WARP)                                                                                       \
+#define VKS_LAUNCH(KERNEL, WARP, ...)                                                                                  \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WARP);                                                                  \
         if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
         if (bps > 8) bps = 8;                                                                                          \
-        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head, gstack, glevels); \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head, gstack, glevels __VA_ARGS__); \
     }
-    if (inst) {
-        if (media) { if (legacy) VKS_LAUNCH((k_stepq_inst<true, true>), WqStepInst) else VKS_LAUNCH((k_stepq_inst<true, false>), WqStepInst) }
-        else { if (legacy) VKS_LAUNCH((k_stepq_inst<false, true>), WqStepInst) else VKS_LAUNCH((k_stepq_inst<false, false>), WqStepInst) }
-    } else {
-        if (media) { if (legacy) VKS_LAUNCH((k_stepq<true, true>), WqStepWorld) else VKS_LAUNCH((k_stepq<true, false>), WqStepWorld) }
-        else { if (legacy) VKS_LAUNCH((k_stepq<false, true>), WqStepWorld) else VKS_LAUNCH((k_stepq<false, false>), WqStepWorld) }
+#define VKS_DISPATCH(FRAMES, ...)                                                                                      \
+    if (inst) {                                                                                                        \
+        if (media) { if (legacy) VKS_LAUNCH((k_stepq_inst##FRAMES<true, true>), WqStepInst, __VA_ARGS__) else VKS_LAUNCH((k_stepq_inst##FRAMES<true, false>), WqStepInst, __VA_ARGS__) } \
+        else { if (legacy) VKS_LAUNCH((k_stepq_inst##FRAMES<false, true>), WqStepInst, __VA_ARGS__) else VKS_LAUNCH((k_stepq_inst##FRAMES<false, false>), WqStepInst, __VA_ARGS__) } \
+    } else {                                                                                                           \
+        if (media) { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<true, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<true, false>), WqStepWorld, __VA_ARGS__) } \
+        else { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<false, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<false, false>), WqStepWorld, __VA_ARGS__) } \
     }
+    if (fr) { VKS_DISPATCH(_frames, , *fr) }
+    else { VKS_DISPATCH(, ) }
+#undef VKS_DISPATCH
 #undef VKS_LAUNCH
     return cudaGetLastError();
 }

@@ -34,13 +34,14 @@ namespace VK_NS {
 // cluster) are traversed inside the extend stage, every lane for its own ray; what differs between the lanes of a batch is
 // then only how long a walk through ONE kind of tree takes -- the heterogeneous top of the scene (loose spheres, media,
 // rects) is typed batches, and the shading runs on whole batches of a class.
-template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID = false>
+// FR: a batch of frames (FrameArgs, the *_frames kernels)
+template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID = false, bool FR = false>
 VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                         unsigned long long* unit_head) {
+                         unsigned long long* unit_head, const FrameArgs* fr = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W> C = wq_ctx(cam, a, S, unit_head, lane);
+    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0, n_prims = 0;
     TraceCounters tc = {0u, 0u};
     constexpr uint32_t EXT_CAP = 32u * K;
@@ -78,6 +79,7 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
             xi[k].rng.key = make_uint2(a.seed_lo, a.seed_hi);
             xi[k].rng.pixel = MEDIA ? S.px[slot[k]] : 0u;
             xi[k].rng.sample = MEDIA ? __float_as_uint(S.bt[slot[k]].w) : 0u;
+            if constexpr (FR && MEDIA) frame_rng(xi[k].rng, a, fr->n_pix, xi[k].rng.pixel);
         }
         TraceHit sub[K];
         trace_flat_k<K, MEDIA, HYBRID>(sc, *flat, o, d, tm, live, 0.001f, xi, best_t, best_hit, sub, &tc);
@@ -129,12 +131,13 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VKQ_NODE_STEPS
 #define VKQ_NODE_STEPS 4
 #endif
-template <bool MEDIA, bool LEGACY, class W>
-VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head) {
+template <bool MEDIA, bool LEGACY, class W, bool FR = false>
+VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
+                        const FrameArgs* fr = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W> C = wq_ctx(cam, a, S, unit_head, lane);
+    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -195,6 +198,7 @@ VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& 
                     if (MEDIA) {
                         xi.rng.pixel = S.px[cur];
                         xi.rng.sample = __float_as_uint(S.bt[cur].w);
+                        if constexpr (FR) frame_rng(xi.rng, a, fr->n_pix, xi.rng.pixel);
                     }
                     trav_init(T, sc, o, d, CUDART_INF_F); // world.hit(&r, 0.001, inf) src/main.rs:130
                     ++n_rays;
@@ -249,42 +253,74 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid(c
     warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true>(sc, &flat, cam, a, buf, unit_head);
 }
 #endif
+// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_BVH) k_warpq_frames(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                           unsigned long long* unit_head, const __grid_constant__ FrameArgs fr) {
+    warpq_bvh_body<MEDIA, LEGACY, WqBvh, true>(sc, cam, a, buf, unit_head, &fr);
+}
+template <bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat_frames(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
+                                                                                 const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                                 const __grid_constant__ FrameArgs fr) {
+    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false, true>(sc, &flat, cam, a, buf, unit_head, &fr);
+}
+template <bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media_frames(const DScene sc, const __grid_constant__ FlatProgram flat,
+                                                                                        const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                                        unsigned long long* unit_head, const __grid_constant__ FrameArgs fr) {
+    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA, false, true>(sc, &flat, cam, a, buf, unit_head, &fr);
+}
+#if !VK_SIMPLE
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid_frames(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
+                                                                                   const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                                   const __grid_constant__ FrameArgs fr) {
+    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true, true>(sc, &flat, cam, a, buf, unit_head, &fr);
+}
+#endif
 
 // grid = sm_count * resident CTAs (persistent); *unit_head must be zero on the stream before the launch
+// fr != nullptr: a batch of frames, the *_frames kernels (the same choice of kernel, FrameArgs as one more argument)
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st) {
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
-#define VKQ_LAUNCH_FLAT(KERNEL, WARP)                                                                                  \
+#define VKQ_LAUNCH_FLAT(KERNEL, WARP, ...)                                                                             \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WARP);                                                                  \
         if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
-        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, *flat, cam, a, b, unit_head);          \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, *flat, cam, a, b, unit_head __VA_ARGS__); \
     }
-#define VKQ_LAUNCH_BVH(M, G)                                                                                           \
+#define VKQ_LAUNCH_BVH(KERNEL, ...)                                                                                    \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WqBvh);                                                                 \
-        if ((e = warpq_prepare(k_warpq<M, G>, smem, &bps)) != cudaSuccess) return e;                                   \
-        k_warpq<M, G><<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head);          \
+        if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head __VA_ARGS__);   \
     }
 #if VK_SIMPLE
     (void)legacy; // the trimmed build exists for the HEAD integrator on flat scenes only
-    if (media) VKQ_LAUNCH_FLAT(k_warpq_flat_media<false>, WqMedia) else VKQ_LAUNCH_FLAT(k_warpq_flat<false>, WqFlat)
+#define VKQ_DISPATCH(FRAMES, ...)                                                                                      \
+    if (media) VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<false>, WqMedia, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<false>, WqFlat, __VA_ARGS__)
 #else
-    if (flat && flat->n && flat->n_bvh) {
-#define VKQ_LAUNCH_HYB(M, G) VKQ_LAUNCH_FLAT((k_warpq_hybrid<M, G>), WqHyb)
-        if (media) { if (legacy) VKQ_LAUNCH_HYB(true, true) else VKQ_LAUNCH_HYB(true, false) }
-        else { if (legacy) VKQ_LAUNCH_HYB(false, true) else VKQ_LAUNCH_HYB(false, false) }
-#undef VKQ_LAUNCH_HYB
-    } else if (flat && flat->n) {
-        if (media) { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat_media<true>, WqMedia) else VKQ_LAUNCH_FLAT(k_warpq_flat_media<false>, WqMedia) }
-        else { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat<true>, WqFlat) else VKQ_LAUNCH_FLAT(k_warpq_flat<false>, WqFlat) }
-    } else {
-        if (media) { if (legacy) VKQ_LAUNCH_BVH(true, true) else VKQ_LAUNCH_BVH(true, false) }
-        else { if (legacy) VKQ_LAUNCH_BVH(false, true) else VKQ_LAUNCH_BVH(false, false) }
+#define VKQ_LAUNCH_HYB(M, G, FRAMES, ...) VKQ_LAUNCH_FLAT((k_warpq_hybrid##FRAMES<M, G>), WqHyb, __VA_ARGS__)
+#define VKQ_DISPATCH(FRAMES, ...)                                                                                      \
+    if (flat && flat->n && flat->n_bvh) {                                                                              \
+        if (media) { if (legacy) VKQ_LAUNCH_HYB(true, true, FRAMES, __VA_ARGS__) else VKQ_LAUNCH_HYB(true, false, FRAMES, __VA_ARGS__) } \
+        else { if (legacy) VKQ_LAUNCH_HYB(false, true, FRAMES, __VA_ARGS__) else VKQ_LAUNCH_HYB(false, false, FRAMES, __VA_ARGS__) } \
+    } else if (flat && flat->n) {                                                                                      \
+        if (media) { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<true>, WqMedia, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<false>, WqMedia, __VA_ARGS__) } \
+        else { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<true>, WqFlat, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<false>, WqFlat, __VA_ARGS__) } \
+    } else {                                                                                                           \
+        if (media) { if (legacy) VKQ_LAUNCH_BVH((k_warpq##FRAMES<true, true>), __VA_ARGS__) else VKQ_LAUNCH_BVH((k_warpq##FRAMES<true, false>), __VA_ARGS__) } \
+        else { if (legacy) VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, true>), __VA_ARGS__) else VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, false>), __VA_ARGS__) } \
     }
 #endif
+    if (fr) { VKQ_DISPATCH(_frames, , *fr) }
+    else { VKQ_DISPATCH(, ) }
+#undef VKQ_DISPATCH
+#undef VKQ_LAUNCH_HYB
 #undef VKQ_LAUNCH_FLAT
 #undef VKQ_LAUNCH_BVH
     return cudaGetLastError();

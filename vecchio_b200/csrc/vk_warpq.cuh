@@ -103,8 +103,16 @@ VKD void wq_converge() {
     asm volatile("barrier.sync.aligned %0, 32;" ::"r"((threadIdx.x >> 5) + 1u) : "memory");
 #endif
 }
-template <class W>
-struct WqCtx {
+// FR: a batch of frames (FrameArgs; separate instantiations, the single-frame code is untouched).  Its chunks are frame-major,
+// and the unit cursor's row is then the batch-wide row f * height + y.
+template <bool FR>
+struct WqFrameRef {}; // (one frame: nothing, not even a null pointer -- the single-frame kernels stay as they were)
+template <>
+struct WqFrameRef<true> {
+    const FrameArgs* fr;
+};
+template <class W, bool FR = false>
+struct WqCtx : WqFrameRef<FR> {
     const DCamera& cam;
     const RenderArgs& a;
     W& S;
@@ -137,8 +145,8 @@ VKD void wq_push(W& S, uint32_t cls, uint32_t slot, uint32_t lane, uint32_t belo
 // sample, so the lanes' units are (s, y, x0 + i) with nothing to wrap and nothing to divide; lane 0 splits the chunk
 // number into (sample, row, row segment) once per chunk.  Which warp renders which unit does not show in the image
 // (Philox is keyed by pixel and sample, the accumulators are integers).
-template <class W>
-VKD bool wq_regen(const WqCtx<W>& C, bool want, uint32_t slot) {
+template <class W, bool FR>
+VKD bool wq_regen(const WqCtx<W, FR>& C, bool want, uint32_t slot) {
     W& S = C.S;
     const uint32_t m = __ballot_sync(0xFFFFFFFFu, want);
     if (m == 0u) return false;
@@ -156,7 +164,18 @@ VKD bool wq_regen(const WqCtx<W>& C, bool want, uint32_t slot) {
             if (C.lane == 0) {
                 const unsigned long long c = atomicAdd(C.unit_head, 1ull);
                 if (c >= C.n_chunks) S.exhausted = 1u;
-                else {
+                else if constexpr (FR) {
+                    // c = ((f * spp_count + sample) * height + row) * chunks_per_row + segment; f * spp_count + sample stays
+                    // 64-bit until the frame is split off (it passes 2^32 long before the batch's pixel index does)
+                    const unsigned long long fs = c / C.chunks_per_sample;
+                    const uint32_t f = (uint32_t)(fs / C.a.spp_count);
+                    const uint32_t r = (uint32_t)(c - fs * C.chunks_per_sample);
+                    const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
+                    S.left = min(VKQ_CHUNK, C.a.width - x0);
+                    S.cur_s = (uint32_t)(fs - (unsigned long long)f * C.a.spp_count);
+                    S.cur_y = f * C.a.height + row;
+                    S.cur_x = x0;
+                } else {
                     const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
                     const uint32_t r = (uint32_t)(c - (unsigned long long)sb * C.chunks_per_sample);
                     const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
@@ -187,14 +206,22 @@ VKD bool wq_regen(const WqCtx<W>& C, bool want, uint32_t slot) {
         served += take;
     }
     if (got) {
-        const uint32_t p = y * C.a.width + x; // i = y*width + x, row 0 = bottom (src/main.rs:182-183)
+        const uint32_t p = y * C.a.width + x; // i = y*width + x, row 0 = bottom (src/main.rs:182-183); FR: + f * n_pix
         PathRng rng;
         rng.pixel = p;
         rng.sample = C.a.spp_begin + s;
         rng.key = make_uint2(C.a.seed_lo, C.a.seed_hi);
         float3 o, d;
         float time;
-        camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
+        if constexpr (FR) {
+            const uint32_t f = y / C.a.height;
+            y -= f * C.a.height;
+            rng.pixel = y * C.a.width + x;
+            rng.key = frame_key(C.a, f);
+            camera_get_ray(C.fr->cams[f], rng, x, y, C.a.width, C.a.height, o, d, time);
+        } else {
+            camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
+        }
         S.ro[slot] = make_float4(o.x, o.y, o.z, time);
         S.rd[slot] = make_float4(d.x, d.y, d.z, __uint_as_float(1u)); // ray_color(ray, .., 1)
         S.bt[slot] = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(rng.sample));
@@ -207,7 +234,18 @@ VKD bool wq_regen(const WqCtx<W>& C, bool want, uint32_t slot) {
 template <class W>
 VKD WqCtx<W> wq_ctx(const DCamera& cam, const RenderArgs& a, W& S, unsigned long long* unit_head, uint32_t lane) {
     const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
-    return WqCtx<W>{cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count, unit_head, lane, (1u << lane) - 1u};
+    return WqCtx<W>{{}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count, unit_head, lane, (1u << lane) - 1u};
+}
+// the context of a body instantiated for one frame (FR false: wq_ctx, `fr` unused) or for a batch
+template <bool FR, class W>
+VKD WqCtx<W, FR> wq_ctx_fr(const DCamera& cam, const RenderArgs& a, const FrameArgs* fr, W& S, unsigned long long* unit_head, uint32_t lane) {
+    if constexpr (FR) {
+        const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
+        return WqCtx<W, true>{{fr}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count * fr->n_frames,
+                              unit_head, lane, (1u << lane) - 1u};
+    } else {
+        return wq_ctx(cam, a, S, unit_head, lane);
+    }
 }
 VKD bool wq_black_miss(const RenderArgs& a) {
     return !(a.flags & VK_FLAG_SKY_BACKGROUND) && a.background.x == 0.0f && a.background.y == 0.0f && a.background.z == 0.0f;
@@ -281,8 +319,8 @@ VKD uint32_t wq_pop(W& S, uint32_t q, uint32_t n_q, uint32_t tail_q, uint32_t ca
 #ifndef VKQ_FAST_RESOLVE
 #define VKQ_FAST_RESOLVE 1 // (Cornell, 1000 spp: 37.9 against 40.0 ms per frame)
 #endif
-template <bool LEGACY, bool FLAT, class W>
-VKD void wq_shade_batch(const DScene& sc, const WqCtx<W>& C, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
+template <bool LEGACY, bool FLAT, class W, bool FR>
+VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR>& C, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
     W& S = C.S;
     const RenderArgs& a = C.a;
     const uint32_t lane = C.lane;
@@ -305,6 +343,7 @@ VKD void wq_shade_batch(const DScene& sc, const WqCtx<W>& C, const RenderBuffers
                 rng.pixel = pixel;
                 rng.sample = __float_as_uint(bt.w);
                 rng.key = make_uint2(a.seed_lo, a.seed_hi);
+                if constexpr (FR) frame_rng(rng, a, C.fr->n_pix, pixel); // (the slot's pixel is batch-wide, the accumulator index too)
                 HitRecD rec;
                 bool direct = false;
                 uint32_t leaf = prim, hi = hp.z;

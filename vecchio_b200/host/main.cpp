@@ -39,6 +39,7 @@ struct Options {
     std::vector<int> devices{0};
     std::string out_dir, assets_dir = "assets";
     uint32_t variant = VK_VARIANT_AUTO, flags = 0;
+    uint32_t batch = 1; // cameras per launch (vk_render_frames_rgb8); 1 = one vk_render_rgb8 per camera
     bool quiet = false;
 };
 
@@ -56,6 +57,9 @@ void usage(FILE* f) {
         "  --frames K         stop after K frames (default: the whole camera iterator)\n"
         "  --first-frame F    skip the first F cameras (file numbering is kept)\n"
         "  --seed S           Philox key of the render (default 1); frame f uses S + f\n"
+        "  --batch K          render up to K cameras per launch (default 1).  Same files, byte for byte, with\n"
+        "                     --strict or an explicit --variant; with auto in the render build a batch may run a\n"
+        "                     faster kernel than one frame does, whose rounding differs (DESIGN.md section 7)\n"
         "  --scene-seed S     host RNG seed for scene generation and BVH axis choices (default 1)\n"
         "  --gpus N           render each frame on devices 0..N-1 (spp split N ways)\n"
         "  --devices a,b,..   explicit device list\n"
@@ -114,6 +118,8 @@ int parse(int argc, char** argv, Options& o) {
             if (!need(v) || !parse_u32(v, o.max_depth)) return 2;
         } else if (a == "--frames") {
             if (!need(v) || !parse_u32(v, o.frames)) return 2;
+        } else if (a == "--batch") {
+            if (!need(v) || !parse_u32(v, o.batch) || o.batch == 0) return 2;
         } else if (a == "--first-frame") {
             if (!need(v) || !parse_u32(v, o.first_frame)) return 2;
         } else if (a == "--seed") {
@@ -190,6 +196,106 @@ void destroy_all(Gpus& g, vkh_scene* scene) {
     if (scene) vkh_scene_free(scene);
 }
 
+// --batch K > 1: the frame loop with up to K cameras of cam_iter per vk_render_frames_rgb8 (or
+// vk_multi_render_frames_rgb8) call.  Frame f of a batch is file number n0 + f with seed + n0 + f -- the numbers and seeds
+// of the one-camera loop, so the files are the same byte for byte whenever the batch runs the kernel a single frame runs:
+// always with --strict (every kernel computes the reference's operation sequence) or an explicit --variant; with AUTO in
+// the render build a batch that crosses AUTO's path-count rule runs another kernel, which rounds differently.  The P3 files of a batch are written by a helper
+// thread while the next batch renders; one "Wrote frame" line per file.  Returns the exit code.
+int render_batched(const Options& opt, Gpus& gpus, vkh_scene* scene, uint32_t width, uint32_t height) {
+    const uint32_t world = (uint32_t)opt.devices.size();
+    const size_t n_bytes = (size_t)width * height * 3;
+    std::vector<uint8_t> rgb8_buf[2] = {std::vector<uint8_t>(n_bytes * opt.batch), std::vector<uint8_t>(n_bytes * opt.batch)};
+    std::vector<vk_camera> cams;
+    cams.reserve(opt.batch);
+    struct Pending {
+        std::future<std::string> done; // "" = written, else the writer's error message
+        std::vector<std::string> filenames;
+        std::chrono::steady_clock::time_point start;
+        uint64_t rays = 0;
+    } pending;
+    auto finish_pending = [&]() -> bool {
+        if (!pending.done.valid()) return true;
+        std::string err = pending.done.get();
+        if (!err.empty()) {
+            std::fprintf(stderr, "vecchio_gpu_render: %s\n", err.c_str());
+            return false;
+        }
+        if (!opt.quiet) { // the batch's time, shared evenly by its frames
+            const double k = (double)pending.filenames.size();
+            const double s = std::chrono::duration<double>(std::chrono::steady_clock::now() - pending.start).count() / k;
+            for (const std::string& name : pending.filenames)
+                std::fprintf(stderr, "Wrote frame %s in %.3fs (%.1f Mpaths/s, %.1f Mrays/s)\n", name.c_str(), s,
+                             (double)width * height * opt.spp / s * 1e-6, (double)pending.rays / k / s * 1e-6);
+        }
+        return true;
+    };
+    uint32_t file_idx = 0, written = 0, n_batches = 0;
+    bool cameras_left = true;
+    while (cameras_left && !(opt.frames && written >= opt.frames)) {
+        // the next up to K cameras of cam_iter (main.rs:176), after --first-frame, within --frames
+        cams.clear();
+        uint32_t first_idx = 0;
+        while (cams.size() < opt.batch && !(opt.frames && written + cams.size() >= opt.frames)) {
+            vk_camera cam;
+            if (!vkh_scene_next_camera(scene, &cam)) {
+                cameras_left = false;
+                break;
+            }
+            if (file_idx < opt.first_frame) {
+                file_idx++;
+                continue;
+            }
+            if (cams.empty()) first_idx = file_idx;
+            cams.push_back(cam);
+            file_idx++;
+        }
+        if (cams.empty()) break;
+        const uint32_t n = (uint32_t)cams.size();
+        auto start = std::chrono::steady_clock::now();
+        std::vector<uint8_t>& rgb8 = rgb8_buf[n_batches & 1];
+
+        vk_render_params P{};
+        P.width = width;
+        P.height = height;
+        P.spp = opt.spp;
+        P.max_depth = opt.max_depth;
+        P.seed = opt.seed + first_idx; // frame f of the batch: seed + first_idx + f
+        P.variant = opt.variant;
+        P.flags = opt.flags;
+        vk_stats stats{};
+        if ((world == 1 ? vk_render_frames_rgb8(gpus.one, cams.data(), n, &P, rgb8.data(), &stats)
+                        : vk_multi_render_frames_rgb8(gpus.many, cams.data(), n, &P, rgb8.data(), &stats)) != VK_OK) {
+            std::fprintf(stderr, "vecchio_gpu_render: %s\n", gpus.error());
+            finish_pending();
+            return 1;
+        }
+        // the previous batch's files are done before its buffer is reused by the batch after this one
+        if (!finish_pending()) return 1;
+        std::vector<std::string> names;
+        for (uint32_t f = 0; f < n; f++) {
+            char filename[4096];
+            if (vkh_frame_filename(opt.out_dir.c_str(), first_idx + f, filename, sizeof filename) < 0) {
+                std::fprintf(stderr, "vecchio_gpu_render: output path too long\n");
+                return 1;
+            }
+            names.push_back(filename);
+        }
+        pending.filenames = names;
+        pending.start = start;
+        pending.rays = stats.rays;
+        const uint8_t* data = rgb8.data();
+        pending.done = std::async(std::launch::async, [data, width, height, n_bytes, names = std::move(names)]() -> std::string {
+            for (size_t f = 0; f < names.size(); f++) // vkh_last_error is per thread: read it on the thread that failed
+                if (vkh_write_ppm(names[f].c_str(), data + f * n_bytes, width, height) != VK_OK) return std::string(vkh_last_error());
+            return std::string();
+        });
+        written += n;
+        n_batches++;
+    }
+    return finish_pending() ? 0 : 1;
+}
+
 } // namespace
 
 int main(int argc, char** argv) {
@@ -234,6 +340,11 @@ int main(int argc, char** argv) {
         std::fprintf(stderr, "vecchio_gpu_render: %s\n", gpus.error());
         destroy_all(gpus, scene);
         return 1;
+    }
+    if (opt.batch > 1) {
+        const int rc = render_batched(opt, gpus, scene, width, height);
+        destroy_all(gpus, scene);
+        return rc;
     }
     const size_t n_floats = (size_t)width * height * 3;
     // two output buffers: the P3 text of frame f is written by a helper thread while frame f+1 renders
