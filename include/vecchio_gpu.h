@@ -338,6 +338,36 @@ int vk_render_frames(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, cons
 int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
                           uint8_t* out_rgb8, vk_stats* stats);
 
+/* Adaptive sampling: every pixel renders until its displayed noise is below max_error, or until params->spp samples.
+ * Passes: pass 0 renders global samples [0, pass_spp) of every pixel; pass k renders [k*pass_spp, min((k+1)*pass_spp, spp))
+ * of every pixel still active.  A pixel therefore ends with n_p in {pass_spp, 2*pass_spp, ..} or n_p = spp samples, and
+ * they are exactly its samples [0, n_p): its mean is, bit for bit, what vk_render returns for that pixel with spp = n_p on
+ * the same kernel (Philox is keyed by pixel and global sample, the accumulators are integers).
+ * Stopping rule, after each pass, per channel of the pixel (in the reference's output units, Vec3::to_color's sqrt x 256):
+ *     m = sum / n,  se = sqrt(max(Q / n - m^2, 0) / (n - 1))   (Q: sum of squares),
+ *     e = 128 * (sqrt(max(m + se, 0)) - sqrt(max(m - se, 0))),  half the width of sqrt(m +- se) in 8-bit steps;
+ * the pixel stops when the largest e of its three channels is <= max_error, or when n == spp.  max_error == 0 never stops
+ * early; a pixel with one sample (pass_spp == 1, pass 0) has no standard error and renders on.
+ * The squares behind the rule are 64-bit fixed-point sums (2^32 units per 1.0, the sample's channel clamped to 255 first:
+ * the clamp touches the statistic only, never the image), exact and order independent, and the decision is deterministic;
+ * this bounds spp to 65536.
+ * The rule looks at the samples, so the estimate is slightly BIASED: pixels that happen to look smooth stop early.
+ * Kernel: VK_VARIANT_AUTO decides once, by vk_render's rule on pass 0's path count W*H*pass_spp, and every pass runs that
+ * kernel, so a pass boundary never changes rounding (render build included).
+ * out_rgb: the means sum / n_p in vk_render's layout; out_rgb8: to_color of the same means, top-down like vk_render_rgb8;
+ * out_spp (nullable): n_p, W*H in the order of the image it accompanies.  stats: paths = sum of n_p; rays, dropped
+ * samples, ms_kernels and launches are totals over all passes; variant is the kernel that ran.  Each pass costs one 4-byte
+ * D2H of the active count and a stream synchronisation.  One frame on one device: no batches, no multi-GPU context.
+ * Errors, before anything is launched: VK_ERR_INVALID for pass_spp == 0, max_error negative or NaN, spp_begin != 0,
+ * spp_count not 0 or spp, spp > 65536, and every check of vk_render; VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED /
+ * VK_VARIANT_WAVEFRONT; VK_ERR_NO_SCENE without a scene. */
+int vk_render_adaptive(vk_ctx* ctx, const vk_camera* cam, const vk_render_params* params,
+                       uint32_t pass_spp, float max_error,
+                       float* out_rgb, uint32_t* out_spp, vk_stats* stats);
+int vk_render_adaptive_rgb8(vk_ctx* ctx, const vk_camera* cam, const vk_render_params* params,
+                            uint32_t pass_spp, float max_error,
+                            uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats);
+
 /* Same loop, device-resident result: writes per-pixel SUMS (not means) of samples
  * [spp_begin, spp_begin+spp_count) to d_sum (and d_sumsq, nullable), both device
  * pointers of W*H*3 floats, enqueued on the context stream; synchronised before return

@@ -108,6 +108,12 @@ extern "C" {
                             out_rgb: *mut f32, stats: *mut vk_stats) -> c_int;
     pub fn vk_render_frames_rgb8(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
                                  out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
+    // adaptive sampling: passes of pass_spp samples until a pixel's displayed noise is <= max_error (8-bit steps) or spp;
+    // a pixel that stopped at n samples equals vk_render with spp = n on the same kernel (the header states the rule)
+    pub fn vk_render_adaptive(ctx: *mut vk_ctx, cam: *const vk_camera, params: *const vk_render_params, pass_spp: u32, max_error: f32,
+                              out_rgb: *mut f32, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
+    pub fn vk_render_adaptive_rgb8(ctx: *mut vk_ctx, cam: *const vk_camera, params: *const vk_render_params, pass_spp: u32,
+                                   max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
     // one context over several GPUs of the node (samples split by global index, peer-memory reduce on devices[0])
     pub fn vk_multi_create(devices: *const c_int, n_devices: c_int, out: *mut *mut vk_multi) -> c_int;
     pub fn vk_multi_destroy(m: *mut vk_multi);
@@ -289,6 +295,31 @@ impl Gpu {
         let mut st = vk_stats::default();
         self.check(unsafe { vk_render_frames_rgb8(self.ctx, cams.as_ptr(), cams.len() as u32, &p, out.as_mut_ptr(), &mut st) })?;
         Ok((out, st))
+    }
+    /// Adaptive sampling with `spp` as the cap: every pixel renders passes of `pass_spp` samples until half the width of
+    /// sqrt(mean +- standard error) is <= `max_error` 8-bit steps in every channel (vk_render_adaptive in vecchio_gpu.h).
+    /// Returns the linear means in `render`'s layout and each pixel's sample count in the same order.  A pixel that
+    /// stopped at n samples is `render(.., spp = n, ..)`'s pixel; the stopping rule makes the frame slightly biased.
+    pub fn render_adaptive(&mut self, cam: &vk_camera, width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                           pass_spp: u32, max_error: f32) -> Result<(Vec<f32>, Vec<u32>, vk_stats), GpuError> {
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0f32; width * height * 3];
+        let mut n = vec![0u32; width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_adaptive(self.ctx, cam, &p, pass_spp, max_error, out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
+    }
+    /// `render_adaptive` as `render_rgb8` returns a frame: the P3 file's numbers, the counts top-down as well.
+    pub fn render_adaptive_rgb8(&mut self, cam: &vk_camera, width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                                pass_spp: u32, max_error: f32) -> Result<(Vec<u8>, Vec<u32>, vk_stats), GpuError> {
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; width * height * 3];
+        let mut n = vec![0u32; width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_adaptive_rgb8(self.ctx, cam, &p, pass_spp, max_error, out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
     }
     /// One spp slice [begin, begin+count) of the frame, already divided by the full `spp`: slices of disjoint
     /// sample ranges ADD to the frame (the Philox counter holds the global sample index).

@@ -108,12 +108,16 @@ def gpu_lib():
                                             C.POINTER(_abi.vk_stats)]
         L.vk_multi_render_frames_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), vp,
                                                   C.POINTER(_abi.vk_stats)]
+        L.vk_render_adaptive.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), C.c_uint32, C.c_float, vp, vp,
+                                         C.POINTER(_abi.vk_stats)]
+        L.vk_render_adaptive_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), C.c_uint32, C.c_float, vp,
+                                              vp, C.POINTER(_abi.vk_stats)]
         for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
                   "vk_multi_render_frames_rgb8"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
                   "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
-                  "vk_render_frames", "vk_render_frames_rgb8"):
+                  "vk_render_frames", "vk_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8"):
             getattr(L, f).restype = C.c_int
         _gpu = L
     return _gpu
@@ -123,7 +127,7 @@ GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk
                "vk_finalize_device", "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks",
                "vk_device_info", "vk_multi_create", "vk_multi_destroy", "vk_multi_last_error", "vk_multi_device_count",
                "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8", "vk_render_frames", "vk_render_frames_rgb8",
-               "vk_multi_render_frames_rgb8"]
+               "vk_multi_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
                 "vkh_frame_filename", "vkh_last_error"]
@@ -260,6 +264,14 @@ def _camera_array(cams):
     return (_abi.vk_camera * len(cams))(*cams), len(cams)
 
 
+def _check_adaptive(pass_spp, max_error):
+    """What vk_render_adaptive* refuse of their two own arguments, refused here before the library is called."""
+    if int(pass_spp) < 1:
+        raise ValueError("render_adaptive: pass_spp must be >= 1")
+    if not float(max_error) >= 0.0:  # (NaN fails the comparison)
+        raise ValueError("render_adaptive: max_error must be >= 0 (and not NaN)")
+
+
 class Context:
     """One GPU context (``vk_create``).  Fails loudly without the CUDA library or a device."""
 
@@ -317,6 +329,33 @@ class Context:
         st = _abi.vk_stats()
         self._check(self._L.vk_render_frames_rgb8(self._h, arr, k, C.byref(params), out.ctypes.data, C.byref(st)))
         return out.reshape(k, params.height, params.width, 3), st
+
+    def render_adaptive(self, cam, params, pass_spp, max_error):
+        """``vk_render_adaptive``: each pixel renders passes of ``pass_spp`` samples until its displayed noise (half the
+        width of sqrt(mean +- standard error) in 8-bit steps) is <= ``max_error``, or until ``params.spp`` samples
+        (the header states the rule).  A pixel that stopped at n samples equals ``render`` with spp = n on the same kernel,
+        bit for bit; the stopping rule makes the frame slightly biased.  ``max_error = 0`` renders ``params.spp`` everywhere.
+        Returns (rgb (H, W, 3) float32 with row 0 = bottom like ``render``, spp (H, W) uint32 in the same order, stats)."""
+        _check_adaptive(pass_spp, max_error)
+        n = params.width * params.height
+        rgb = np.empty(n * 3, dtype=np.float32)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_adaptive(self._h, C.byref(cam), C.byref(params), int(pass_spp), float(max_error),
+                                               rgb.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return rgb.reshape(params.height, params.width, 3), spp.reshape(params.height, params.width), st
+
+    def render_adaptive_rgb8(self, cam, params, pass_spp, max_error):
+        """``vk_render_adaptive_rgb8``: render_adaptive's frame as ``render_rgb8`` returns one (row 0 = top).
+        Returns (rgb8 (H, W, 3) uint8, spp (H, W) uint32 with row 0 = top, stats)."""
+        _check_adaptive(pass_spp, max_error)
+        n = params.width * params.height
+        out = np.empty(n * 3, dtype=np.uint8)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_adaptive_rgb8(self._h, C.byref(cam), C.byref(params), int(pass_spp), float(max_error),
+                                                    out.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return out.reshape(params.height, params.width, 3), spp.reshape(params.height, params.width), st
 
     def render_device(self, cam, params, d_sum_ptr, d_sumsq_ptr=None, want_stats=True):
         """``vk_render_device``: per-pixel SUMS of an spp slice into device memory.  With

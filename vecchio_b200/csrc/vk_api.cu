@@ -8,6 +8,8 @@
 #include <string>
 #include <vector>
 
+#include <cub/device/device_select.cuh>
+
 #include "vk_internal.h"
 #include "vk_relayout.h"
 
@@ -55,6 +57,8 @@ struct vk_ctx {
     DCamera* cams = nullptr; // vk_render_frames: the batch's cameras on the device (FrameArgs::cams)
     size_t cams_cap = 0;
     std::vector<DCamera> cams_host;
+    void* adapt = nullptr; // vk_render_adaptive: squares | per-pixel counts | two pixel lists | flags | count | compaction scratch
+    size_t adapt_bytes = 0;
     // wavefront variant: the slot pool (allocated on first use) and a pinned word block for the
     // host's termination checks
     WfState wf{};
@@ -113,6 +117,56 @@ __global__ void k_to_color_frames(const float* __restrict__ sum, uint8_t* __rest
     float v = sqrtf(c);
     v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v);
     out[i] = (uint8_t)__float2uint_rz(256.0f * v);
+}
+// ---- adaptive sampling (vk_render_adaptive) ----
+__global__ void k_iota(uint32_t* list, uint32_t n) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) list[i] = i;
+}
+// The stopping rule of vk_render_adaptive (include/vecchio_gpu.h) for every listed pixel after a pass that brought it to
+// n_done samples: records n_done as its count, keep[i] = 1 when it renders on.  Computed from the integer sums alone, so
+// the decision does not depend on the order the samples arrived in.
+__global__ void k_adaptive_select(const uint32_t* __restrict__ list, uint32_t n, const unsigned long long* __restrict__ acc,
+                                  const unsigned long long* __restrict__ sq, uint32_t n_done, uint32_t spp, float max_error,
+                                  uint32_t* __restrict__ nspp, uint8_t* __restrict__ keep) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t p = list[i];
+    nspp[p] = n_done;
+    bool stop = n_done >= spp;
+    if (!stop && max_error > 0.0f && n_done > 1u) { // (one sample has no standard error)
+        double e = 0.0;
+        for (uint32_t ch = 0; ch < 3u; ++ch) {
+            const double m = (double)(long long)acc[3u * p + ch] * VK_ACC_INV_SCALE / n_done;
+            const double q = (double)sq[3u * p + ch] * VK_SQ_INV_SCALE / n_done;
+            const double se = sqrt(fmax(q - m * m, 0.0) / (double)(n_done - 1u));
+            e = fmax(e, 128.0 * (sqrt(fmax(m + se, 0.0)) - sqrt(fmax(m - se, 0.0))));
+        }
+        stop = e <= (double)max_error;
+    }
+    keep[i] = stop ? 0u : 1u;
+}
+// mean = sum / n_p with k_acc_to_sum's and k_finalize's operations, so a pixel that stopped at n equals vk_render(spp = n)
+__global__ void k_finalize_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, float* __restrict__ rgb,
+                                    size_t n) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float sum = (float)((double)(long long)acc[i] * VK_ACC_INV_SCALE);
+    rgb[i] = sum / (float)nspp[i / 3];
+}
+// k_to_color of the same means, rows top-down; the counts follow the image's order
+__global__ void k_to_color_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, uint8_t* __restrict__ out,
+                                    uint32_t* __restrict__ spp_out, uint32_t width, uint32_t height) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, n = (size_t)width * height * 3;
+    if (i >= n) return;
+    const size_t row = i / ((size_t)width * 3), col = i - row * (size_t)width * 3;
+    const size_t j = (size_t)(height - 1 - row) * width * 3 + col;
+    const uint32_t np = nspp[j / 3];
+    const float c = (float)((double)(long long)acc[j] * VK_ACC_INV_SCALE) / (float)np;
+    float v = sqrtf(c);
+    v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v);
+    out[i] = (uint8_t)__float2uint_rz(256.0f * v);
+    if (col % 3 == 0) spp_out[i / 3] = np;
 }
 // FP32 peak: 8 independent FFMA chains per thread, no memory traffic
 __global__ void k_ffma_peak(float* out, int iters) {
@@ -260,6 +314,7 @@ void vk_destroy(vk_ctx* c) {
     if (c->frame) cudaFree(c->frame);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->cams) cudaFree(c->cams);
+    if (c->adapt) cudaFree(c->adapt);
     if (c->counters) cudaFree(c->counters);
     if (c->debug) cudaFree(c->debug);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -548,17 +603,10 @@ static int check_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint3
     return VK_OK;
 }
 
-// shared body of vk_render / vk_render_device / vk_render_frames*
-// acc_only: leave the result in the context's integer accumulators (c->partial) and skip the conversion to fp32 sums
-// (the multi-GPU context reduces the accumulators of all its devices itself); want_sq then says whether squares are kept
-// n_frames > 1: cam points to n_frames cameras and the result is n_frames contiguous planes (check_frames has passed; the
-// batch kernels take FrameArgs, everything else is the single-frame path)
-static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* d_sum, float* d_sumsq, vk_stats* stats,
-                       bool acc_only = false, bool want_sq = false, uint32_t n_frames = 1) {
-    if (!c) return VK_ERR_INVALID;
+// What every render call checks of its camera and parameters before anything is launched.
+static int check_render(vk_ctx* c, const vk_camera* cam, const vk_render_params* P) {
     if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, "render: no scene uploaded");
-    if (!cam || !P || (!d_sum && !acc_only)) return fail(c, VK_ERR_INVALID, "render: null argument");
-    if (!acc_only) want_sq = d_sumsq != nullptr;
+    if (!cam || !P) return fail(c, VK_ERR_INVALID, "render: null argument");
     if (P->width < 2 || P->height < 2) return fail(c, VK_ERR_INVALID, "render: width/height must be >= 2 ((width-1) divides, src/main.rs:187)");
     if (P->spp == 0 || P->spp_begin >= P->spp) return fail(c, VK_ERR_INVALID, "render: bad spp / spp_begin");
     const uint32_t count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
@@ -566,9 +614,20 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     if ((uint64_t)P->width * P->height > 0x7FFFFFFFull / 3) return fail(c, VK_ERR_INVALID, "render: image too large");
     if (P->variant > VK_VARIANT_STEPQ) return fail(c, VK_ERR_INVALID, "render: unknown variant");
     if (!(cam->time0 < cam->time1)) return fail(c, VK_ERR_INVALID, "render: camera time0 >= time1 (gen_range panics, src/main.rs:118)");
-    CU(c, cudaSetDevice(c->device));
-    const bool strict = (P->flags & VK_FLAG_STRICT_MATH) != 0;
+    return VK_OK;
+}
 
+// The kernel a call runs and how it is launched, decided once per call (an adaptive render runs every pass on it).
+struct RenderPlan {
+    bool strict, legacy, l0;
+    const FlatProgram* flat;
+    uint32_t variant;
+    int grid;
+    uint32_t resident_warps;
+};
+static int plan_render(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, RenderPlan* R) {
+    R->strict = (P->flags & VK_FLAG_STRICT_MATH) != 0;
+    const bool strict = R->strict;
     const FlatProgram* flat = (c->flat.n && !(P->flags & VK_FLAG_FORCE_BVH)) ? &c->flat : nullptr;
     int bps = 0, bt = 0;
     const bool legacy = (P->flags & VK_FLAG_LEGACY_SCATTER) != 0;
@@ -589,13 +648,28 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
           : l0   ? vkfast_l0::megakernel_occupancy(flat != nullptr, c->scene.has_media, legacy, &bps, &bt)
                  : vkfast::megakernel_occupancy(flat != nullptr, c->scene.has_media, legacy, &bps, &bt));
     if (bps < 1) bps = 1;
-    const int grid = c->sm_count * bps;
-    const uint32_t resident_warps = (uint32_t)grid * (uint32_t)bt / 32u;
+    R->legacy = legacy;
+    R->l0 = l0;
+    R->flat = flat;
+    R->grid = c->sm_count * bps;
+    R->resident_warps = (uint32_t)R->grid * (uint32_t)bt / 32u;
+    if (variant == VK_VARIANT_STEPQ && flat && flat->n_bvh == 0) variant = VK_VARIANT_WARPQ; // step queues are the BVH traversal; a flat program has none
+    R->variant = variant;
+    return VK_OK;
+}
 
+// One launch of the sample loop over global samples [spp_begin, spp_begin + count) into the accumulators of b (which the
+// caller has zeroed), on the kernel R names.  n_frames > 1: cam points to n_frames cameras (the batch kernels take
+// FrameArgs); ls != nullptr: only the listed pixels (the list kernels, one frame).  Adds the kernels it launched to *launches.
+static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, const vk_render_params* P, uint32_t spp_begin, uint32_t count,
+                       const RenderBuffers& b, uint32_t n_frames, const ListArgs* ls, uint32_t* launches) {
+    const bool strict = R.strict, legacy = R.legacy, l0 = R.l0;
+    const FlatProgram* flat = R.flat;
+    const uint32_t variant = R.variant;
     RenderArgs a{};
     a.width = P->width;
     a.height = P->height;
-    a.spp_begin = P->spp_begin;
+    a.spp_begin = spp_begin;
     a.spp_count = count;
     a.max_depth = P->max_depth;
     a.seed_lo = (uint32_t)P->seed;
@@ -604,30 +678,20 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     a.flags = P->flags;
     a.tiles_x = (P->width + 7) / 8;
     a.tiles_y = (P->height + 3) / 4;
-    // Accumulators (see RenderBuffers): u64 fixed-point sums, plus double sums of squares when asked for.
-    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
-    RenderBuffers b{};
-    b.counters = c->counters;
-    b.debug = c->debug;
-    {
-        const int rc = ensure(c, &c->partial, &c->partial_floats, plane * (want_sq ? 4 : 2));
-        if (rc != VK_OK) return rc;
-        b.acc = (unsigned long long*)c->partial;
-        b.accsq = want_sq ? (double*)(c->partial + plane * 2) : nullptr;
-        CU(c, cudaMemsetAsync(c->partial, 0, plane * (want_sq ? 4 : 2) * sizeof(float), c->stream));
+    if (ls) { // the lane megakernel's items over a list: groups of 32 consecutive entries
+        a.tiles_x = (ls->n + 31) / 32;
+        a.tiles_y = 1;
     }
     // Lane megakernel: chunks of samples, sized for ~48 work items per resident warp (small items keep
     // the end-of-kernel tail short; an item costs one atomic).
     const uint32_t n_tiles = a.tiles_x * a.tiles_y * n_frames; // (a batch: the items of all its frames share the warps)
-    uint32_t n_chunks = (48u * resident_warps + n_tiles - 1) / n_tiles;
+    uint32_t n_chunks = (48u * R.resident_warps + n_tiles - 1) / n_tiles;
     if (n_chunks > count) n_chunks = count;
     if (n_chunks < 1) n_chunks = 1;
     a.chunk_spp = (count + n_chunks - 1) / n_chunks;
     a.n_chunks = (count + a.chunk_spp - 1) / a.chunk_spp;
 
     CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // work-queue head only
-    apply_l2_window(c);
-    CU(c, cudaEventRecord(c->ev0, c->stream));
     const DCamera dc = to_dcam(cam);
     // a batch: its cameras go to the device with the call (read at regeneration only), FrameArgs selects the batch kernels
     FrameArgs fa{};
@@ -648,8 +712,6 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         fa.n_pix = P->width * P->height;
         fr = &fa;
     }
-    uint32_t launches = 0;
-    if (variant == VK_VARIANT_STEPQ && flat && flat->n_bvh == 0) variant = VK_VARIANT_WARPQ; // step queues are the BVH traversal; a flat program has none
     if (variant == VK_VARIANT_STEPQ) {
         const bool inst = c->levels_sub != 0u;
         uint32_t glevels = 0;
@@ -661,24 +723,26 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         }
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
         CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
-        CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr)
-              : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr)
-                     : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr));
-        launches = 1;
+        CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls)
+              : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls)
+                     : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls));
+        *launches += 1;
     } else if (variant == VK_VARIANT_WARPQ) {
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
         CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
         // (a hybrid program -- flat top, homogeneous subtrees walked inside extend -- runs k_warpq_hybrid)
         const FlatProgram* sflat = flat;
         const bool simple = !strict && !legacy && sflat && sflat->n_bvh == 0 && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
-        CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
-              : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
-              : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr)
-                       : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr));
-        launches = 1;
+        CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
+              : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
+              : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
+                       : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls));
+        *launches += 1;
     } else if (variant == VK_VARIANT_WAVEFRONT) {
-        int rc = wf_render(c, strict, flat, dc, a, b, &launches);
+        uint32_t n = 0;
+        int rc = wf_render(c, strict, flat, dc, a, b, &n);
         if (rc != VK_OK) return rc;
+        *launches += n;
     } else if (variant == VK_VARIANT_STAGED) {
         CU(c, cudaMemsetAsync(c->counters + 5, 0xFF, 2 * sizeof(unsigned long long), c->stream)); // CTA start / first end: minima
         CU(c, cudaMemsetAsync(c->counters + 7, 0, sizeof(unsigned long long), c->stream));        // last end: maximum
@@ -690,19 +754,55 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
         CU(c, strict   ? vkstrict::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
               : simple ? vkfast_simple::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
                        : vkfast::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream));
-        launches = 1;
+        *launches += 1;
     } else if (!flat && !legacy && use_dynamic_megakernel(c)) {
         CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr)
-              : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr)
-                     : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr));
-        launches = 1;
+        CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls)
+              : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls)
+                     : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls));
+        *launches += 1;
     } else {
-        CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr)
-              : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr)
-                     : vkfast::launch_megakernel(c->scene, flat, dc, a, b, grid, legacy, c->stream, fr));
-        launches = 1;
+        CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls)
+              : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls)
+                     : vkfast::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls));
+        *launches += 1;
     }
+    return VK_OK;
+}
+
+// shared body of vk_render / vk_render_device / vk_render_frames*
+// acc_only: leave the result in the context's integer accumulators (c->partial) and skip the conversion to fp32 sums
+// (the multi-GPU context reduces the accumulators of all its devices itself); want_sq then says whether squares are kept
+// n_frames > 1: cam points to n_frames cameras and the result is n_frames contiguous planes (check_frames has passed; the
+// batch kernels take FrameArgs, everything else is the single-frame path)
+static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* d_sum, float* d_sumsq, vk_stats* stats,
+                       bool acc_only = false, bool want_sq = false, uint32_t n_frames = 1) {
+    if (!c) return VK_ERR_INVALID;
+    int rc = check_render(c, cam, P);
+    if (rc != VK_OK) return rc;
+    if (!d_sum && !acc_only) return fail(c, VK_ERR_INVALID, "render: null argument");
+    if (!acc_only) want_sq = d_sumsq != nullptr;
+    const uint32_t count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
+    CU(c, cudaSetDevice(c->device));
+    RenderPlan R;
+    if ((rc = plan_render(c, P, n_frames, &R)) != VK_OK) return rc;
+
+    // Accumulators (see RenderBuffers): u64 fixed-point sums, plus double sums of squares when asked for.
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
+    RenderBuffers b{};
+    b.counters = c->counters;
+    b.debug = c->debug;
+    {
+        rc = ensure(c, &c->partial, &c->partial_floats, plane * (want_sq ? 4 : 2));
+        if (rc != VK_OK) return rc;
+        b.acc = (unsigned long long*)c->partial;
+        b.accsq = want_sq ? (double*)(c->partial + plane * 2) : nullptr;
+        CU(c, cudaMemsetAsync(c->partial, 0, plane * (want_sq ? 4 : 2) * sizeof(float), c->stream));
+    }
+    apply_l2_window(c);
+    CU(c, cudaEventRecord(c->ev0, c->stream));
+    uint32_t launches = 0;
+    if ((rc = launch_pass(c, R, cam, P, P->spp_begin, count, b, n_frames, nullptr, &launches)) != VK_OK) return rc;
     if (!acc_only) {
         k_acc_to_sum<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, b.accsq, plane, d_sum, d_sumsq);
         ++launches;
@@ -712,11 +812,11 @@ static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* 
     c->launches += launches;
     c->paths += (uint64_t)P->width * P->height * count * n_frames;
     if (stats) { // reading the counters synchronises; with stats == NULL the call is fully asynchronous
-        int rc = vk_flush_stats(c, stats);
+        rc = vk_flush_stats(c, stats);
         if (rc != VK_OK) return rc;
         CU(c, cudaEventElapsedTime(&stats->ms_kernels, c->ev0, c->ev1));
         stats->ms_total = stats->ms_kernels;
-        stats->variant = variant;
+        stats->variant = R.variant;
     }
     return VK_OK;
 }
@@ -882,6 +982,151 @@ static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint
     CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
     if (stats) *stats = st;
     return VK_OK;
+}
+
+// shared body of vk_render_adaptive / vk_render_adaptive_rgb8 (include/vecchio_gpu.h states the passes and the rule)
+static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
+                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    const std::string w(who);
+    if (!cam || !P || (!out_rgb && !out_rgb8)) return fail(c, VK_ERR_INVALID, w + ": null argument");
+    int rc = check_render(c, cam, P);
+    if (rc != VK_OK) return rc;
+    if (pass_spp == 0) return fail(c, VK_ERR_INVALID, w + ": pass_spp must be >= 1");
+    if (!(max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, w + ": max_error must be >= 0 (and not NaN)");
+    if (P->spp_begin != 0 || (P->spp_count != 0 && P->spp_count != P->spp))
+        return fail(c, VK_ERR_INVALID, w + ": an adaptive render draws samples [0, n_p) of every pixel: spp_begin must be 0, spp_count 0 or spp");
+    if (P->spp > VK_ADAPTIVE_MAX_SPP)
+        return fail(c, VK_ERR_INVALID, w + ": spp above " + std::to_string(VK_ADAPTIVE_MAX_SPP) +
+                                           ", the limit of the fixed-point sums of squares (2^16 samples of at most 255^2 * 2^32 units)");
+    if (P->variant == VK_VARIANT_STAGED || P->variant == VK_VARIANT_WAVEFRONT)
+        return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
+    CU(c, cudaSetDevice(c->device));
+    // AUTO decides once, on pass 0's path count; every pass runs that kernel
+    vk_render_params Q = *P;
+    Q.spp_count = pass_spp < P->spp ? pass_spp : P->spp;
+    RenderPlan R;
+    if ((rc = plan_render(c, &Q, 1, &R)) != VK_OK) return rc;
+    if (R.variant == VK_VARIANT_STAGED || R.variant == VK_VARIANT_WAVEFRONT)
+        return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
+
+    const uint32_t n_pix = P->width * P->height;
+    const size_t plane = (size_t)n_pix * 3;
+    // buffers: fixed-point sums (c->partial) | the adaptive block | the output staging (c->frame, pinned)
+    if ((rc = ensure(c, &c->partial, &c->partial_floats, plane * 2)) != VK_OK) return rc;
+    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane + n_pix)) != VK_OK) return rc; // rgb or rgb8 | counts in output order
+    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    size_t cub_bytes = 0;
+    CU(c, cub::DeviceSelect::Flagged(nullptr, cub_bytes, (const uint32_t*)nullptr, (const uint8_t*)nullptr, (uint32_t*)nullptr, (int*)nullptr,
+                                     (int)n_pix, c->stream));
+    const size_t o_sq = 0, o_n = o_sq + al(plane * 8), o_l0 = o_n + al(n_pix * 4ull), o_l1 = o_l0 + al(n_pix * 4ull),
+                 o_keep = o_l1 + al(n_pix * 4ull), o_cnt = o_keep + al(n_pix), o_cub = o_cnt + 256, need = o_cub + al(cub_bytes);
+    if (c->adapt_bytes < need) {
+        if (c->adapt) cudaFree(c->adapt);
+        c->adapt = nullptr;
+        c->adapt_bytes = 0;
+        CU(c, cudaMalloc(&c->adapt, need));
+        c->adapt_bytes = need;
+    }
+    const size_t pinned_need = plane + n_pix + 1; // floats: rgb | counts | the active count
+    if (c->pinned_floats < pinned_need) {
+        if (c->pinned) cudaFreeHost(c->pinned);
+        c->pinned = nullptr;
+        c->pinned_floats = 0;
+        CU(c, cudaMallocHost((void**)&c->pinned, pinned_need * sizeof(float)));
+        c->pinned_floats = pinned_need;
+    }
+    char* base = (char*)c->adapt;
+    unsigned long long* sq = (unsigned long long*)(base + o_sq);
+    uint32_t* nspp = (uint32_t*)(base + o_n);
+    uint32_t* cur = (uint32_t*)(base + o_l0);
+    uint32_t* nxt = (uint32_t*)(base + o_l1);
+    uint8_t* keep = (uint8_t*)(base + o_keep);
+    int* d_count = (int*)(base + o_cnt);
+    void* cub_tmp = base + o_cub;
+    uint32_t* h_count = (uint32_t*)(c->pinned + plane + n_pix);
+
+    RenderBuffers b{};
+    b.counters = c->counters;
+    b.debug = c->debug;
+    b.acc = (unsigned long long*)c->partial;
+    b.accsq = nullptr;
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    // the accumulators are zeroed once per call: pass k adds samples [k * pass_spp, ..) to what passes 0 .. k-1 left
+    CU(c, cudaMemsetAsync(c->partial, 0, plane * 2 * sizeof(float), c->stream));
+    CU(c, cudaMemsetAsync(sq, 0, plane * sizeof(unsigned long long), c->stream));
+    uint32_t launches = 1;
+    k_iota<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(cur, n_pix); // pass 0: every pixel, ascending
+    apply_l2_window(c);
+    uint32_t n_active = n_pix, done = 0;
+    uint64_t paths = 0;
+    float ms_kernels = 0.0f;
+    for (;;) {
+        const uint32_t cnt = P->spp - done < pass_spp ? P->spp - done : pass_spp;
+        const ListArgs la{cur, n_active, sq};
+        CU(c, cudaEventRecord(c->ev0, c->stream));
+        if ((rc = launch_pass(c, R, cam, P, done, cnt, b, 1, &la, &launches)) != VK_OK) return rc;
+        paths += (uint64_t)n_active * cnt;
+        done += cnt;
+        k_adaptive_select<<<(n_active + 255) / 256, 256, 0, c->stream>>>(cur, n_active, b.acc, sq, done, P->spp, max_error, nspp, keep);
+        ++launches;
+        const bool last = done == P->spp;
+        if (!last) { // the next list: the kept entries, compacted in their (ascending) order
+            CU(c, cub::DeviceSelect::Flagged(cub_tmp, cub_bytes, cur, keep, nxt, d_count, (int)n_active, c->stream));
+            launches += 2; // (its init and select kernels)
+        }
+        CU(c, cudaGetLastError());
+        CU(c, cudaEventRecord(c->ev1, c->stream));
+        // one 4-byte D2H and a stream synchronisation per pass: the host sizes the next pass's work from the count
+        if (!last) CU(c, cudaMemcpyAsync(h_count, d_count, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream));
+        float ms = 0.0f;
+        CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+        ms_kernels += ms;
+        if (last || *h_count == 0u) break;
+        n_active = *h_count;
+        std::swap(cur, nxt);
+    }
+    uint32_t* d_spp = (uint32_t*)(c->frame + plane);
+    if (out_rgb) {
+        k_finalize_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, c->frame, plane);
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        d_spp = nspp; // (vk_render's layout: the counts are already in pixel order)
+    } else {
+        k_to_color_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, (uint8_t*)c->frame, d_spp, P->width, P->height);
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane, cudaMemcpyDeviceToHost, c->stream));
+    }
+    ++launches;
+    if (out_spp) CU(c, cudaMemcpyAsync(c->pinned + plane, d_spp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (out_rgb) std::memcpy(out_rgb, c->pinned, plane * sizeof(float));
+    else std::memcpy(out_rgb8, c->pinned, plane);
+    if (out_spp) std::memcpy(out_spp, c->pinned + plane, n_pix * sizeof(uint32_t));
+    c->launches += launches;
+    c->paths += paths;
+    vk_stats st{};
+    if ((rc = vk_flush_stats(c, &st)) != VK_OK) return rc;
+    st.ms_kernels = ms_kernels;
+    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
+    st.variant = R.variant;
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+int vk_render_adaptive(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error, float* out_rgb,
+                       uint32_t* out_spp, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!out_rgb) return fail(c, VK_ERR_INVALID, "vk_render_adaptive: null argument");
+    return render_adaptive(c, "vk_render_adaptive", cam, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats);
+}
+
+int vk_render_adaptive_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
+                            uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!out_rgb8) return fail(c, VK_ERR_INVALID, "vk_render_adaptive_rgb8: null argument");
+    return render_adaptive(c, "vk_render_adaptive_rgb8", cam, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats);
 }
 
 int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {

@@ -1732,6 +1732,16 @@ VKD void accumulate_sample(const RenderBuffers& buf, uint32_t pixel, float3 L) {
         if (L.z != 0.0f) atomicAdd(q + 2, (double)L.z * (double)L.z);
     }
 }
+// The list kernels of an adaptive pass (ListArgs) add, next to accumulate_sample, each channel's square to the pixel's
+// fixed-point sums of squares: |L| clamped to VK_SQ_CLAMP, squared exactly in double (a float product fits its mantissa),
+// rounded to VK_SQ_SCALE units.  Integer sums again, so the stopping statistic does not depend on arrival order.
+VKD void accumulate_square(unsigned long long* sq, uint32_t pixel, float3 L) {
+    unsigned long long* q = sq + (size_t)pixel * 3u;
+    const double cx = fminf(fabsf(L.x), VK_SQ_CLAMP), cy = fminf(fabsf(L.y), VK_SQ_CLAMP), cz = fminf(fabsf(L.z), VK_SQ_CLAMP);
+    if (L.x != 0.0f) atomicAdd(q + 0, __double2ull_rn(cx * cx * (double)VK_SQ_SCALE));
+    if (L.y != 0.0f) atomicAdd(q + 1, __double2ull_rn(cy * cy * (double)VK_SQ_SCALE));
+    if (L.z != 0.0f) atomicAdd(q + 2, __double2ull_rn(cz * cz * (double)VK_SQ_SCALE));
+}
 
 // A ray that leaves the scene: the constant background of src/main.rs:124,151, or with
 // VK_FLAG_SKY_BACKGROUND the book-1 sky (1-t)*white + t*(0.5,0.7,1.0), t = 0.5*(unit(d).y + 1).

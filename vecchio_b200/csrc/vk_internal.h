@@ -202,6 +202,24 @@ struct FrameArgs {
     uint32_t n_pix;      // width * height
 };
 
+// A pass of an adaptive render (vk_render_adaptive): the work units run over a list of active pixels instead of the dense
+// frame.  An entry is a frame pixel index y * width + x, so the accumulators keep their dense W*H*3 layout and a slot keeps
+// the frame pixel.  Only the list instantiations of the kernels take it, as their last kernel parameter (like FrameArgs;
+// frame x list is not instantiated).  Every kept sample also adds its per-channel square to `sq` (accumulate_square): 64-bit
+// fixed point, so the sums, and the stopping decision made from them, do not depend on the order samples arrive in.
+struct ListArgs {
+    const uint32_t* list;   // active pixels, ascending
+    uint32_t n;             // list length
+    unsigned long long* sq; // W*H*3 fixed-point sums of squares (VK_SQ_SCALE)
+};
+// Squares: VK_SQ_SCALE = 2^32 units per 1.0, each channel of a sample clamped to VK_SQ_CLAMP before it is squared (the clamp
+// touches the statistic only, never the image).  One sample adds at most 255^2 * 2^32 < 2^48 units, so VK_ADAPTIVE_MAX_SPP =
+// 2^16 samples stay below 2^64.
+#define VK_SQ_SCALE 4294967296.0f
+#define VK_SQ_INV_SCALE (1.0 / 4294967296.0)
+#define VK_SQ_CLAMP 255.0f
+#define VK_ADAPTIVE_MAX_SPP 65536u
+
 // Accumulation.  Every finished sample is added to its pixel with three 64-bit integer atomics
 // (fixed point, VK_ACC_SCALE = 2^30 units per 1.0): integer addition is associative, so the frame is
 // bit-identical for a (seed, sample range, image size) whatever the kernel variant, the scheduling of
@@ -253,10 +271,10 @@ struct WfState {
     namespace NS {                                                                                                     \
     cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,  \
                                   const RenderBuffers& b, int grid, bool legacy, cudaStream_t st,                      \
-                                  const FrameArgs* fr = nullptr);                                                      \
+                                  const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);                        \
     cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, \
                                       unsigned long long* unit_head, int sm_count, cudaStream_t st,                     \
-                                      const FrameArgs* fr = nullptr);                                                  \
+                                      const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);                    \
     cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk_ray* rays, size_t n,              \
                                  const float* medium_xi, vk_hit* out, cudaStream_t st);                                \
     cudaError_t megakernel_occupancy(bool flat, bool media, bool legacy, int* blocks_per_sm, int* block_threads);      \
@@ -267,11 +285,11 @@ struct WfState {
                               const RenderBuffers& b, unsigned long long* unit_head, int sm_count, cudaStream_t st);   \
     cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,       \
                              const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy,         \
-                             cudaStream_t st, const FrameArgs* fr = nullptr);                                          \
+                             cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);            \
     size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t* levels);                          \
     cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,        \
                              unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, \
-                             bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr);                             \
+                             bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr); \
     cudaError_t launch_wf_generate(const DCamera& cam, const RenderArgs& a, const WfState& w, cudaStream_t st);        \
     cudaError_t launch_wf_extend(const DScene& sc, const FlatProgram* flat, const RenderArgs& a, const WfState& w,     \
                                  const RenderBuffers& b, uint32_t set, cudaStream_t st);                               \
@@ -285,5 +303,5 @@ namespace vkfast_simple { // vk_staged.cu / vk_warpq.cu compiled with VK_SIMPLE=
 cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
                           unsigned long long* unit_head, int sm_count, cudaStream_t st);
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr);
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);
 }

@@ -38,9 +38,11 @@ template <bool FR> VKD uint32_t frame_pixel(uint32_t pbase, uint32_t pixel) {
 //           the next one, so lanes only idle for the last unit of an item.
 // A finished sample goes straight into its pixel's integer accumulators (accumulate_sample).
 // FR: a batch of frames (FrameArgs, k_megakernel*_frames): item = frame x chunk x tile, frame outermost.
-template <bool FLAT, bool MEDIA, bool LEGACY, bool FR = false>
+// LS: a pass over a list of active pixels (ListArgs, k_megakernel*_list): a "tile" is 32 consecutive list entries (the host
+// sets tiles_x to their number, tiles_y to 1), unit u of an item is list entry tile * 32 + (u & 31) x sample c0 + (u >> 5).
+template <bool FLAT, bool MEDIA, bool LEGACY, bool FR = false, bool LS = false>
 VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,
-                         const RenderBuffers& buf, const FrameArgs* fr = nullptr) {
+                         const RenderBuffers& buf, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t lanes_below = (1u << lane) - 1u;
     const uint32_t n_tiles = a.tiles_x * a.tiles_y;
@@ -85,7 +87,17 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
             const uint32_t want = __ballot_sync(0xFFFFFFFFu, need);
             if (need) {
                 const uint32_t u = next_unit + __popc(want & lanes_below);
-                if (u < n_units) {
+                if constexpr (LS) {
+                    const uint32_t li = tile * 32u + (u & 31u);
+                    if (u < n_units && li < ls->n) { // the last group of the list is ragged
+                        rng.pixel = ls->list[li];
+                        py = rng.pixel / a.width;
+                        px = rng.pixel - py * a.width;
+                        s = c0 + (u >> 5);
+                        s_end = s + 1u;
+                        has_unit = true;
+                    }
+                } else if (u < n_units) {
                     px = px0 + (u & 7u);
                     py = py0 + ((u >> 3) & 3u);
                     if (px < a.width && py < a.height) { // ragged tiles: a unit outside the image is void
@@ -141,8 +153,12 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
                 }
             }
             if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                if (valid && finite3(L)) accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
-                else ++n_drop;
+                if (valid && finite3(L)) {
+                    accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
+                    if constexpr (LS) accumulate_square(ls->sq, rng.pixel, L);
+                } else {
+                    ++n_drop;
+                }
             }
         }
     }
@@ -186,11 +202,13 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #define VK_DYN_NODE_STEPS 4
 #endif
 // FR: a batch of frames (FrameArgs, k_megakernel_dyn_frames): unit = frame x sample x pixel, frame outermost.
-template <bool MEDIA, bool FR = false>
+// LS: a pass over a list of active pixels (ListArgs, k_megakernel_dyn_list): unit = sample x list entry.
+template <bool MEDIA, bool FR = false, bool LS = false>
 VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                             unsigned long long* unit_head, const FrameArgs* fr = nullptr) {
+                             unsigned long long* unit_head, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
     const uint32_t lane = threadIdx.x & 31u, lanes_below = (1u << lane) - 1u;
-    const uint32_t n_pixels = a.width * a.height;
+    uint32_t n_pixels = a.width * a.height;
+    if constexpr (LS) n_pixels = ls->n; // (the units' "pixels" are list entries)
     unsigned long long n_units = (unsigned long long)n_pixels * a.spp_count;
     if constexpr (FR) n_units *= fr->n_frames;
     uint32_t pbase = 0; // (FR) first accumulator pixel of this lane's frame
@@ -237,8 +255,12 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
                     }
                 }
                 if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                    if (valid && finite3(L)) accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
-                    else ++n_drop;
+                    if (valid && finite3(L)) {
+                        accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
+                        if constexpr (LS) accumulate_square(ls->sq, rng.pixel, L);
+                    } else {
+                        ++n_drop;
+                    }
                 }
             }
             if (alive) new_ray = true;
@@ -262,6 +284,7 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
                     }
                     const uint32_t sb = (uint32_t)(u / n_pixels);
                     rng.pixel = (uint32_t)(u - (unsigned long long)sb * n_pixels); // i = y*width + x (src/main.rs:182-183)
+                    if constexpr (LS) rng.pixel = ls->list[rng.pixel];
                     rng.sample = a.spp_begin + sb;
                     if constexpr (FR) camera_get_ray(fr->cams[f], rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
                     else camera_get_ray(cam, rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
@@ -326,6 +349,12 @@ __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn_frames
                                                                              const __grid_constant__ FrameArgs fr) {
     megakernel_dyn_body<MEDIA, true>(sc, cam, a, buf, unit_head, &fr);
 }
+template <bool MEDIA>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn_list(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                           const RenderBuffers buf, unsigned long long* unit_head,
+                                                                           const __grid_constant__ ListArgs ls) {
+    megakernel_dyn_body<MEDIA, false, true>(sc, cam, a, buf, unit_head, nullptr, &ls);
+}
 
 // instantiations: {BVH, flat program} x {scene without / with ConstantMedium} x {HEAD integrator, legacy scatter}
 template <bool MEDIA, bool LEGACY>
@@ -349,6 +378,18 @@ __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat_fram
                                                                               const DCamera cam, const RenderArgs a, const RenderBuffers buf,
                                                                               const __grid_constant__ FrameArgs fr) {
     megakernel_body<true, MEDIA, LEGACY, true>(sc, &flat, cam, a, buf, &fr);
+}
+// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_list(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                       const RenderBuffers buf, const __grid_constant__ ListArgs ls) {
+    megakernel_body<false, MEDIA, LEGACY, false, true>(sc, nullptr, cam, a, buf, nullptr, &ls);
+}
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat_list(const DScene sc, const __grid_constant__ FlatProgram flat,
+                                                                            const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                            const __grid_constant__ ListArgs ls) {
+    megakernel_body<true, MEDIA, LEGACY, false, true>(sc, &flat, cam, a, buf, nullptr, &ls);
 }
 
 template <bool FLAT>
@@ -462,17 +503,22 @@ __global__ void k_philox_kat(const uint32_t* in6, uint32_t* out4) {
 }
 
 // *unit_head must be zero on the stream before the launch
-// fr != nullptr: a batch of frames (k_megakernel_dyn_frames)
+// fr != nullptr: a batch of frames (k_megakernel_dyn_frames); ls != nullptr: a pass over a pixel list (k_megakernel_dyn_list)
 cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                                  unsigned long long* unit_head, int sm_count, cudaStream_t st, const FrameArgs* fr) {
+                                  unsigned long long* unit_head, int sm_count, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
     int bps = 0;
-    cudaError_t e = fr ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<true>, VK_BLOCK, 0)
+    cudaError_t e = ls ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_list<true>, VK_BLOCK, 0)
+                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_list<false>, VK_BLOCK, 0))
+                  : fr ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<true>, VK_BLOCK, 0)
                                        : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<false>, VK_BLOCK, 0))
                        : (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<true>, VK_BLOCK, 0)
                                        : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<false>, VK_BLOCK, 0));
     if (e != cudaSuccess) return e;
     const int grid = sm_count * (bps < 1 ? 1 : bps);
-    if (fr) {
+    if (ls) {
+        if (sc.has_media) k_megakernel_dyn_list<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *ls);
+        else k_megakernel_dyn_list<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *ls);
+    } else if (fr) {
         if (sc.has_media) k_megakernel_dyn_frames<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
         else k_megakernel_dyn_frames<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
     } else if (sc.has_media) k_megakernel_dyn<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
@@ -488,9 +534,18 @@ cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const Re
         else { if (legacy) { CALL_BVH(false, true); } else { CALL_BVH(false, false); } }                               \
     }
 // fr != nullptr: a batch of frames (k_megakernel*_frames; the grid is the single-frame kernels', same registers)
+// ls != nullptr: a pass over a pixel list (k_megakernel*_list; a.tiles_x * a.tiles_y = groups of 32 list entries)
 cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flatp, const DCamera& cam, const RenderArgs& a,
-                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const FrameArgs* fr) {
+                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
     const bool flat = flatp && flatp->n, media = sc.has_media;
+    if (ls) {
+#define VK_LB(M, G) k_megakernel_list<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, *ls)
+#define VK_LF(M, G) k_megakernel_flat_list<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, *ls)
+        VK_MEGA_DISPATCH(VK_LB, VK_LF)
+#undef VK_LB
+#undef VK_LF
+        return cudaGetLastError();
+    }
     if (fr) {
 #define VK_LB(M, G) k_megakernel_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, *fr)
 #define VK_LF(M, G) k_megakernel_flat_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, *fr)

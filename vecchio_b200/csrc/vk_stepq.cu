@@ -140,13 +140,14 @@ VKD bool sq_pick(const W& S, uint32_t last_q, uint32_t& q, uint32_t& n_q, uint32
 }
 
 // FR: a batch of frames (FrameArgs, the *_frames kernels)
-template <bool MEDIA, bool LEGACY, class W, bool FR = false>
+// LS: a pass over a list of active pixels (ListArgs, the *_list kernels)
+template <bool MEDIA, bool LEGACY, class W, bool FR = false, bool LS = false>
 VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
-                    uint32_t* gstack, uint32_t glevels, const FrameArgs* fr = nullptr) {
+                    uint32_t* gstack, uint32_t glevels, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
+    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -395,6 +396,19 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst_fr
                                                                                  uint32_t glevels, const __grid_constant__ FrameArgs fr) {
     stepq_body<MEDIA, LEGACY, WqStepInst, true>(sc, cam, a, buf, unit_head, gstack, glevels, &fr);
 }
+// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB) k_stepq_list(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                     unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
+                                                                     const __grid_constant__ ListArgs ls) {
+    stepq_body<MEDIA, LEGACY, WqStepWorld, false, true>(sc, cam, a, buf, unit_head, gstack, glevels, nullptr, &ls);
+}
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst_list(const DScene sc, const DCamera cam, const RenderArgs a,
+                                                                               const RenderBuffers buf, unsigned long long* unit_head, uint32_t* gstack,
+                                                                               uint32_t glevels, const __grid_constant__ ListArgs ls) {
+    stepq_body<MEDIA, LEGACY, WqStepInst, false, true>(sc, cam, a, buf, unit_head, gstack, glevels, nullptr, &ls);
+}
 
 // What the launch needs of the overflow stack: `words` 32-bit words for a scene whose traversal may hold `stack_need`
 // entries (vk_scene_info); 0 when the shared-memory part is enough.
@@ -404,9 +418,10 @@ size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t*
     return warps * *levels * (inst ? VKS_N_INST : VKS_N);
 }
 
-// fr != nullptr: a batch of frames, the *_frames kernels
+// fr != nullptr: a batch of frames, the *_frames kernels; ls != nullptr: a pass over a pixel list, the *_list kernels
 cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, unsigned long long* unit_head,
-                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr) {
+                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr,
+                         const ListArgs* ls) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
@@ -425,7 +440,8 @@ cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs&
         if (media) { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<true, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<true, false>), WqStepWorld, __VA_ARGS__) } \
         else { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<false, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<false, false>), WqStepWorld, __VA_ARGS__) } \
     }
-    if (fr) { VKS_DISPATCH(_frames, , *fr) }
+    if (ls) { VKS_DISPATCH(_list, , *ls) }
+    else if (fr) { VKS_DISPATCH(_frames, , *fr) }
     else { VKS_DISPATCH(, ) }
 #undef VKS_DISPATCH
 #undef VKS_LAUNCH

@@ -35,13 +35,14 @@ namespace VK_NS {
 // then only how long a walk through ONE kind of tree takes -- the heterogeneous top of the scene (loose spheres, media,
 // rects) is typed batches, and the shading runs on whole batches of a class.
 // FR: a batch of frames (FrameArgs, the *_frames kernels)
-template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID = false, bool FR = false>
+// LS: a pass over a list of active pixels (ListArgs, the *_list kernels)
+template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID = false, bool FR = false, bool LS = false>
 VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                         unsigned long long* unit_head, const FrameArgs* fr = nullptr) {
+                         unsigned long long* unit_head, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
+    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
     uint32_t n_rays = 0, n_drop = 0, n_prims = 0;
     TraceCounters tc = {0u, 0u};
     constexpr uint32_t EXT_CAP = 32u * K;
@@ -131,13 +132,13 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VKQ_NODE_STEPS
 #define VKQ_NODE_STEPS 4
 #endif
-template <bool MEDIA, bool LEGACY, class W, bool FR = false>
+template <bool MEDIA, bool LEGACY, class W, bool FR = false, bool LS = false>
 VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
-                        const FrameArgs* fr = nullptr) {
+                        const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR> C = wq_ctx_fr<FR>(cam, a, fr, S, unit_head, lane);
+    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -279,11 +280,38 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid_f
     warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true, true>(sc, &flat, cam, a, buf, unit_head, &fr);
 }
 #endif
+// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_BVH) k_warpq_list(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                         unsigned long long* unit_head, const __grid_constant__ ListArgs ls) {
+    warpq_bvh_body<MEDIA, LEGACY, WqBvh, false, true>(sc, cam, a, buf, unit_head, nullptr, &ls);
+}
+template <bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat_list(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
+                                                                               const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                               const __grid_constant__ ListArgs ls) {
+    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
+}
+template <bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media_list(const DScene sc, const __grid_constant__ FlatProgram flat,
+                                                                                      const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                                      unsigned long long* unit_head, const __grid_constant__ ListArgs ls) {
+    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA, false, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
+}
+#if !VK_SIMPLE
+template <bool MEDIA, bool LEGACY>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid_list(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
+                                                                                 const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                                 const __grid_constant__ ListArgs ls) {
+    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
+}
+#endif
 
 // grid = sm_count * resident CTAs (persistent); *unit_head must be zero on the stream before the launch
 // fr != nullptr: a batch of frames, the *_frames kernels (the same choice of kernel, FrameArgs as one more argument)
+// ls != nullptr: a pass over a pixel list, the *_list kernels (likewise, ListArgs)
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr) {
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
@@ -317,7 +345,8 @@ cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamer
         else { if (legacy) VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, true>), __VA_ARGS__) else VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, false>), __VA_ARGS__) } \
     }
 #endif
-    if (fr) { VKQ_DISPATCH(_frames, , *fr) }
+    if (ls) { VKQ_DISPATCH(_list, , *ls) }
+    else if (fr) { VKQ_DISPATCH(_frames, , *fr) }
     else { VKQ_DISPATCH(, ) }
 #undef VKQ_DISPATCH
 #undef VKQ_LAUNCH_HYB

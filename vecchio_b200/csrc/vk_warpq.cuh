@@ -105,14 +105,20 @@ VKD void wq_converge() {
 }
 // FR: a batch of frames (FrameArgs; separate instantiations, the single-frame code is untouched).  Its chunks are frame-major,
 // and the unit cursor's row is then the batch-wide row f * height + y.
-template <bool FR>
+// LS: a pass over a list of active pixels (ListArgs); its chunks are VKQ_CHUNK consecutive list entries of one sample, and the
+// unit cursor's column is then a list index.  (Frame x list is not instantiated.)
+template <bool FR, bool LS = false>
 struct WqFrameRef {}; // (one frame: nothing, not even a null pointer -- the single-frame kernels stay as they were)
 template <>
-struct WqFrameRef<true> {
+struct WqFrameRef<true, false> {
     const FrameArgs* fr;
 };
-template <class W, bool FR = false>
-struct WqCtx : WqFrameRef<FR> {
+template <>
+struct WqFrameRef<false, true> {
+    const ListArgs* ls;
+};
+template <class W, bool FR = false, bool LS = false>
+struct WqCtx : WqFrameRef<FR, LS> {
     const DCamera& cam;
     const RenderArgs& a;
     W& S;
@@ -145,8 +151,8 @@ VKD void wq_push(W& S, uint32_t cls, uint32_t slot, uint32_t lane, uint32_t belo
 // sample, so the lanes' units are (s, y, x0 + i) with nothing to wrap and nothing to divide; lane 0 splits the chunk
 // number into (sample, row, row segment) once per chunk.  Which warp renders which unit does not show in the image
 // (Philox is keyed by pixel and sample, the accumulators are integers).
-template <class W, bool FR>
-VKD bool wq_regen(const WqCtx<W, FR>& C, bool want, uint32_t slot) {
+template <class W, bool FR, bool LS>
+VKD bool wq_regen(const WqCtx<W, FR, LS>& C, bool want, uint32_t slot) {
     W& S = C.S;
     const uint32_t m = __ballot_sync(0xFFFFFFFFu, want);
     if (m == 0u) return false;
@@ -174,6 +180,13 @@ VKD bool wq_regen(const WqCtx<W, FR>& C, bool want, uint32_t slot) {
                     S.left = min(VKQ_CHUNK, C.a.width - x0);
                     S.cur_s = (uint32_t)(fs - (unsigned long long)f * C.a.spp_count);
                     S.cur_y = f * C.a.height + row;
+                    S.cur_x = x0;
+                } else if constexpr (LS) { // c = sample * chunks_per_sample + chunk of the list
+                    const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
+                    const uint32_t x0 = ((uint32_t)c - sb * C.chunks_per_sample) * VKQ_CHUNK;
+                    S.left = min(VKQ_CHUNK, C.ls->n - x0);
+                    S.cur_s = sb;
+                    S.cur_y = 0u;
                     S.cur_x = x0;
                 } else {
                     const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
@@ -219,13 +232,18 @@ VKD bool wq_regen(const WqCtx<W, FR>& C, bool want, uint32_t slot) {
             rng.pixel = y * C.a.width + x;
             rng.key = frame_key(C.a, f);
             camera_get_ray(C.fr->cams[f], rng, x, y, C.a.width, C.a.height, o, d, time);
+        } else if constexpr (LS) { // x is a list index
+            rng.pixel = C.ls->list[x];
+            y = rng.pixel / C.a.width;
+            x = rng.pixel - y * C.a.width;
+            camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
         } else {
             camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
         }
         S.ro[slot] = make_float4(o.x, o.y, o.z, time);
         S.rd[slot] = make_float4(d.x, d.y, d.z, __uint_as_float(1u)); // ray_color(ray, .., 1)
         S.bt[slot] = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(rng.sample));
-        S.px[slot] = p;
+        S.px[slot] = LS ? rng.pixel : p;
         S.mark_new(slot);
     }
     return got;
@@ -236,10 +254,14 @@ VKD WqCtx<W> wq_ctx(const DCamera& cam, const RenderArgs& a, W& S, unsigned long
     const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
     return WqCtx<W>{{}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count, unit_head, lane, (1u << lane) - 1u};
 }
-// the context of a body instantiated for one frame (FR false: wq_ctx, `fr` unused) or for a batch
-template <bool FR, class W>
-VKD WqCtx<W, FR> wq_ctx_fr(const DCamera& cam, const RenderArgs& a, const FrameArgs* fr, W& S, unsigned long long* unit_head, uint32_t lane) {
-    if constexpr (FR) {
+// the context of a body instantiated for one frame (FR, LS false: wq_ctx, `fr` and `ls` unused), for a batch or for a list
+template <bool FR, bool LS = false, class W>
+VKD WqCtx<W, FR, LS> wq_ctx_fr(const DCamera& cam, const RenderArgs& a, const FrameArgs* fr, W& S, unsigned long long* unit_head, uint32_t lane,
+                               const ListArgs* ls = nullptr) {
+    if constexpr (LS) {
+        const uint32_t cps = (ls->n + VKQ_CHUNK - 1u) / VKQ_CHUNK;
+        return WqCtx<W, false, true>{{ls}, cam, a, S, cps, cps, (unsigned long long)cps * a.spp_count, unit_head, lane, (1u << lane) - 1u};
+    } else if constexpr (FR) {
         const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
         return WqCtx<W, true>{{fr}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count * fr->n_frames,
                               unit_head, lane, (1u << lane) - 1u};
@@ -319,8 +341,8 @@ VKD uint32_t wq_pop(W& S, uint32_t q, uint32_t n_q, uint32_t tail_q, uint32_t ca
 #ifndef VKQ_FAST_RESOLVE
 #define VKQ_FAST_RESOLVE 1 // (Cornell, 1000 spp: 37.9 against 40.0 ms per frame)
 #endif
-template <bool LEGACY, bool FLAT, class W, bool FR>
-VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR>& C, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
+template <bool LEGACY, bool FLAT, class W, bool FR, bool LS>
+VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR, LS>& C, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
     W& S = C.S;
     const RenderArgs& a = C.a;
     const uint32_t lane = C.lane;
@@ -391,8 +413,12 @@ VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR>& C, const RenderBuf
                 S.bt[slot] = make_float4(beta.x, beta.y, beta.z, bt.w);
                 S.mark_new(slot);
             } else {
-                if (valid && finite3(L)) accumulate_sample(buf, pixel, L);
-                else ++n_drop;
+                if (valid && finite3(L)) {
+                    accumulate_sample(buf, pixel, L);
+                    if constexpr (LS) accumulate_square(C.ls->sq, pixel, L);
+                } else {
+                    ++n_drop;
+                }
                 ended = true;
             }
         }

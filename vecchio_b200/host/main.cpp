@@ -14,6 +14,7 @@
 #include "../../include/vecchio_host.h"
 
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -40,6 +41,8 @@ struct Options {
     std::string out_dir, assets_dir = "assets";
     uint32_t variant = VK_VARIANT_AUTO, flags = 0;
     uint32_t batch = 1; // cameras per launch (vk_render_frames_rgb8); 1 = one vk_render_rgb8 per camera
+    float adaptive = -1.0f; // >= 0: vk_render_adaptive_rgb8 with this max_error, --spp the cap
+    uint32_t pass_spp = 0;  // its samples per pass (0 = not given: 64)
     bool quiet = false;
 };
 
@@ -60,6 +63,11 @@ void usage(FILE* f) {
         "  --batch K          render up to K cameras per launch (default 1).  Same files, byte for byte, with\n"
         "                     --strict or an explicit --variant; with auto in the render build a batch may run a\n"
         "                     faster kernel than one frame does, whose rounding differs (DESIGN.md section 7)\n"
+        "  --adaptive E       adaptive sampling (vk_render_adaptive_rgb8): a pixel stops when half the width of\n"
+        "                     sqrt(mean +- standard error) is <= E 8-bit steps in every channel, or at --spp samples\n"
+        "                     (the cap).  E = 0 writes the same files as without --adaptive.  The stopping rule\n"
+        "                     makes the estimate slightly biased.  One device, --batch 1 (DESIGN.md section 7)\n"
+        "  --pass-spp M       samples per adaptive pass (default 64)\n"
         "  --scene-seed S     host RNG seed for scene generation and BVH axis choices (default 1)\n"
         "  --gpus N           render each frame on devices 0..N-1 (spp split N ways)\n"
         "  --devices a,b,..   explicit device list\n"
@@ -120,6 +128,20 @@ int parse(int argc, char** argv, Options& o) {
             if (!need(v) || !parse_u32(v, o.frames)) return 2;
         } else if (a == "--batch") {
             if (!need(v) || !parse_u32(v, o.batch) || o.batch == 0) return 2;
+        } else if (a == "--adaptive") {
+            if (!need(v)) return 2;
+            char* end = nullptr;
+            const float e = std::strtof(v, &end);
+            if (!v[0] || *end || !std::isfinite(e) || e < 0.0f) {
+                std::fprintf(stderr, "vecchio_gpu_render: --adaptive needs a finite value >= 0\n");
+                return 2;
+            }
+            o.adaptive = e;
+        } else if (a == "--pass-spp") {
+            if (!need(v) || !parse_u32(v, o.pass_spp) || o.pass_spp == 0) {
+                std::fprintf(stderr, "vecchio_gpu_render: --pass-spp needs an integer >= 1\n");
+                return 2;
+            }
         } else if (a == "--first-frame") {
             if (!need(v) || !parse_u32(v, o.first_frame)) return 2;
         } else if (a == "--seed") {
@@ -178,6 +200,15 @@ int parse(int argc, char** argv, Options& o) {
         std::fprintf(stderr, "vecchio_gpu_render: need width >= 2 and spp >= number of devices\n");
         return 2;
     }
+    if (o.pass_spp && o.adaptive < 0.0f) {
+        std::fprintf(stderr, "vecchio_gpu_render: --pass-spp needs --adaptive\n");
+        return 2;
+    }
+    if (o.adaptive >= 0.0f && (o.batch > 1 || o.devices.size() > 1)) {
+        std::fprintf(stderr, "vecchio_gpu_render: --adaptive renders one frame per call on one device (no --batch > 1, no --gpus > 1)\n");
+        return 2;
+    }
+    if (!o.pass_spp) o.pass_spp = 64;
     return 0;
 }
 
@@ -353,7 +384,7 @@ int main(int argc, char** argv) {
         std::future<std::string> done; // "" = written, else the writer's error message
         std::string filename;
         std::chrono::steady_clock::time_point start;
-        uint64_t rays = 0;
+        uint64_t rays = 0, paths = 0;
     } pending;
     auto finish_pending = [&]() -> bool {
         if (!pending.done.valid()) return true;
@@ -365,7 +396,7 @@ int main(int argc, char** argv) {
         if (!opt.quiet) {
             double s = std::chrono::duration<double>(std::chrono::steady_clock::now() - pending.start).count();
             std::fprintf(stderr, "Wrote frame %s in %.3fs (%.1f Mpaths/s, %.1f Mrays/s)\n", pending.filename.c_str(), s,
-                         (double)width * height * opt.spp / s * 1e-6, (double)pending.rays / s * 1e-6);
+                         (double)pending.paths / s * 1e-6, (double)pending.rays / s * 1e-6);
         }
         return true;
     };
@@ -391,7 +422,10 @@ int main(int argc, char** argv) {
 
         // sample loop + Vec3::to_color on the device(s); a quarter of the bytes come back
         vk_stats stats{};
-        if ((world == 1 ? vk_render_rgb8(gpus.one, &cam, &P, rgb8.data(), &stats) : vk_multi_render_rgb8(gpus.many, &cam, &P, rgb8.data(), &stats)) != VK_OK) {
+        const int rc = opt.adaptive >= 0.0f ? vk_render_adaptive_rgb8(gpus.one, &cam, &P, opt.pass_spp, opt.adaptive, rgb8.data(), nullptr, &stats)
+                       : world == 1        ? vk_render_rgb8(gpus.one, &cam, &P, rgb8.data(), &stats)
+                                           : vk_multi_render_rgb8(gpus.many, &cam, &P, rgb8.data(), &stats);
+        if (rc != VK_OK) {
             std::fprintf(stderr, "vecchio_gpu_render: %s\n", gpus.error());
             destroy_all(gpus, scene);
             return 1;
@@ -413,6 +447,7 @@ int main(int argc, char** argv) {
         pending.filename = filename;
         pending.start = start;
         pending.rays = rays;
+        pending.paths = opt.adaptive >= 0.0f ? stats.paths : (uint64_t)width * height * opt.spp;
         const uint8_t* data = rgb8.data();
         pending.done = std::async(std::launch::async, [data, width, height, name = pending.filename]() -> std::string {
             // vkh_last_error is per thread: read it on the thread that failed
