@@ -229,6 +229,16 @@ int ensure(vk_ctx* c, float** buf, size_t* have, size_t want) {
     *have = want;
     return VK_OK;
 }
+// the pinned counterpart: c->pinned, the host staging of the results, holds at least `floats` floats
+static int ensure_pinned(vk_ctx* c, size_t floats) {
+    if (c->pinned_floats >= floats) return VK_OK;
+    if (c->pinned) cudaFreeHost(c->pinned);
+    c->pinned = nullptr;
+    c->pinned_floats = 0;
+    CU(c, cudaMallocHost((void**)&c->pinned, floats * sizeof(float)));
+    c->pinned_floats = floats;
+    return VK_OK;
+}
 DCamera to_dcam(const vk_camera* k) {
     DCamera c;
     auto v3 = [](const float* p) { return make_float3(p[0], p[1], p[2]); };
@@ -659,8 +669,9 @@ static int plan_render(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, 
 }
 
 // One launch of the sample loop over global samples [spp_begin, spp_begin + count) into the accumulators of b (which the
-// caller has zeroed), on the kernel R names.  n_frames > 1: cam points to n_frames cameras (the batch kernels take
-// FrameArgs); ls != nullptr: only the listed pixels (the list kernels, one frame).  Adds the kernels it launched to *launches.
+// caller has zeroed), on the kernel R names.  The work domain: n_frames > 1, cam points to n_frames cameras (FrameArgs);
+// ls != nullptr, only the listed pixels of one frame (ListArgs); otherwise one frame (OneFrame).  Adds the kernels it
+// launched to *launches.
 static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, const vk_render_params* P, uint32_t spp_begin, uint32_t count,
                        const RenderBuffers& b, uint32_t n_frames, const ListArgs* ls, uint32_t* launches) {
     const bool strict = R.strict, legacy = R.legacy, l0 = R.l0;
@@ -693,81 +704,80 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
 
     CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // work-queue head only
     const DCamera dc = to_dcam(cam);
-    // a batch: its cameras go to the device with the call (read at regeneration only), FrameArgs selects the batch kernels
-    FrameArgs fa{};
-    const FrameArgs* fr = nullptr;
-    if (n_frames > 1) {
-        if (c->cams_cap < n_frames) {
-            if (c->cams) cudaFree(c->cams);
-            c->cams = nullptr;
-            c->cams_cap = 0;
-            CU(c, cudaMalloc((void**)&c->cams, n_frames * sizeof(DCamera)));
-            c->cams_cap = n_frames;
-        }
-        c->cams_host.resize(n_frames);
-        for (uint32_t f = 0; f < n_frames; ++f) c->cams_host[f] = to_dcam(cam + f);
-        CU(c, cudaMemcpyAsync(c->cams, c->cams_host.data(), n_frames * sizeof(DCamera), cudaMemcpyHostToDevice, c->stream));
-        fa.cams = c->cams;
-        fa.n_frames = n_frames;
-        fa.n_pix = P->width * P->height;
-        fr = &fa;
-    }
-    if (variant == VK_VARIANT_STEPQ) {
-        const bool inst = c->levels_sub != 0u;
-        uint32_t glevels = 0;
-        const size_t words = strict ? vkstrict::stepq_stack_words(c->stack_need, inst, c->sm_count, &glevels)
-                                    : vkfast::stepq_stack_words(c->stack_need, inst, c->sm_count, &glevels);
-        if (words) {
-            const int rc = ensure(c, &c->sq_stack, &c->sq_stack_floats, words);
+    // the variant switch, for the work domain `dom` (staged and wavefront have none: plan_render and render_adaptive keep
+    // batches and pixel lists away from them)
+    auto run = [&](const auto& dom) -> int {
+        if (variant == VK_VARIANT_STEPQ) {
+            const bool inst = c->levels_sub != 0u;
+            uint32_t glevels = 0;
+            const size_t words = strict ? vkstrict::stepq_stack_words(c->stack_need, inst, c->sm_count, &glevels)
+                                        : vkfast::stepq_stack_words(c->stack_need, inst, c->sm_count, &glevels);
+            if (words) {
+                const int rc = ensure(c, &c->sq_stack, &c->sq_stack_floats, words);
+                if (rc != VK_OK) return rc;
+            }
+            CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
+            CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
+            CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, dom)
+                  : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, dom)
+                         : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, dom));
+            *launches += 1;
+        } else if (variant == VK_VARIANT_WARPQ) {
+            CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
+            CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
+            // (a hybrid program -- flat top, homogeneous subtrees walked inside extend -- runs k_warpq_hybrid)
+            const FlatProgram* sflat = flat;
+            const bool simple = !strict && !legacy && sflat && sflat->n_bvh == 0 && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
+            CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                  : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                  : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                           : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom));
+            *launches += 1;
+        } else if (variant == VK_VARIANT_WAVEFRONT) {
+            uint32_t n = 0;
+            int rc = wf_render(c, strict, flat, dc, a, b, &n);
             if (rc != VK_OK) return rc;
+            *launches += n;
+        } else if (variant == VK_VARIANT_STAGED) {
+            CU(c, cudaMemsetAsync(c->counters + 5, 0xFF, 2 * sizeof(unsigned long long), c->stream)); // CTA start / first end: minima
+            CU(c, cudaMemsetAsync(c->counters + 7, 0, sizeof(unsigned long long), c->stream));        // last end: maximum
+            CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
+            // a "simple" scene runs the build of the same kernel with the unreachable code compiled out
+            // (the staged kernel's K-ray flat trace has no subtree entries: a hybrid program means its BVH path)
+            const FlatProgram* sflat = flat && flat->n_bvh == 0 ? flat : nullptr;
+            const bool simple = !strict && sflat && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
+            CU(c, strict   ? vkstrict::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
+                  : simple ? vkfast_simple::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
+                           : vkfast::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream));
+            *launches += 1;
+        } else if (!flat && !legacy && use_dynamic_megakernel(c)) {
+            CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
+            CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, dom)
+                  : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, dom)
+                         : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, dom));
+            *launches += 1;
+        } else {
+            CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, dom)
+                  : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, dom)
+                         : vkfast::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, dom));
+            *launches += 1;
         }
-        CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
-        CU(c, strict ? vkstrict::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls)
-              : l0   ? vkfast_l0::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls)
-                     : vkfast::launch_stepq(c->scene, dc, a, b, c->counters + 2, (uint32_t*)c->sq_stack, glevels, inst, c->sm_count, legacy, c->stream, fr, ls));
-        *launches += 1;
-    } else if (variant == VK_VARIANT_WARPQ) {
-        CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        CU(c, cudaMemsetAsync(c->counters + 5, 0, sizeof(unsigned long long), c->stream)); // self-check violations (debug builds)
-        // (a hybrid program -- flat top, homogeneous subtrees walked inside extend -- runs k_warpq_hybrid)
-        const FlatProgram* sflat = flat;
-        const bool simple = !strict && !legacy && sflat && sflat->n_bvh == 0 && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
-        CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
-              : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
-              : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls)
-                       : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, fr, ls));
-        *launches += 1;
-    } else if (variant == VK_VARIANT_WAVEFRONT) {
-        uint32_t n = 0;
-        int rc = wf_render(c, strict, flat, dc, a, b, &n);
-        if (rc != VK_OK) return rc;
-        *launches += n;
-    } else if (variant == VK_VARIANT_STAGED) {
-        CU(c, cudaMemsetAsync(c->counters + 5, 0xFF, 2 * sizeof(unsigned long long), c->stream)); // CTA start / first end: minima
-        CU(c, cudaMemsetAsync(c->counters + 7, 0, sizeof(unsigned long long), c->stream));        // last end: maximum
-        CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        // a "simple" scene runs the build of the same kernel with the unreachable code compiled out
-        // (the staged kernel's K-ray flat trace has no subtree entries: a hybrid program means its BVH path)
-        const FlatProgram* sflat = flat && flat->n_bvh == 0 ? flat : nullptr;
-        const bool simple = !strict && sflat && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
-        CU(c, strict   ? vkstrict::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
-              : simple ? vkfast_simple::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream)
-                       : vkfast::launch_staged(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, c->stream));
-        *launches += 1;
-    } else if (!flat && !legacy && use_dynamic_megakernel(c)) {
-        CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // unit queue head
-        CU(c, strict ? vkstrict::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls)
-              : l0   ? vkfast_l0::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls)
-                     : vkfast::launch_megakernel_dyn(c->scene, dc, a, b, c->counters + 2, c->sm_count, c->stream, fr, ls));
-        *launches += 1;
-    } else {
-        CU(c, strict ? vkstrict::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls)
-              : l0   ? vkfast_l0::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls)
-                     : vkfast::launch_megakernel(c->scene, flat, dc, a, b, R.grid, legacy, c->stream, fr, ls));
-        *launches += 1;
+        return VK_OK;
+    };
+    if (ls) return run(*ls);
+    if (n_frames == 1) return run(OneFrame{});
+    // a batch: its cameras go to the device with the call (read at regeneration only)
+    if (c->cams_cap < n_frames) {
+        if (c->cams) cudaFree(c->cams);
+        c->cams = nullptr;
+        c->cams_cap = 0;
+        CU(c, cudaMalloc((void**)&c->cams, n_frames * sizeof(DCamera)));
+        c->cams_cap = n_frames;
     }
-    return VK_OK;
+    c->cams_host.resize(n_frames);
+    for (uint32_t f = 0; f < n_frames; ++f) c->cams_host[f] = to_dcam(cam + f);
+    CU(c, cudaMemcpyAsync(c->cams, c->cams_host.data(), n_frames * sizeof(DCamera), cudaMemcpyHostToDevice, c->stream));
+    return run(FrameArgs{c->cams, n_frames, P->width * P->height});
 }
 
 // shared body of vk_render / vk_render_device / vk_render_frames*
@@ -870,13 +880,7 @@ int vk_render(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float*
     CU(c, cudaSetDevice(c->device));
     int rc = ensure(c, &c->frame, &c->frame_floats, plane * 3);
     if (rc != VK_OK) return rc;
-    if (c->pinned_floats < plane * 2) {
-        if (c->pinned) cudaFreeHost(c->pinned);
-        c->pinned = nullptr;
-        c->pinned_floats = 0;
-        CU(c, cudaMallocHost((void**)&c->pinned, plane * 2 * sizeof(float)));
-        c->pinned_floats = plane * 2;
-    }
+    if ((rc = ensure_pinned(c, plane * 2)) != VK_OK) return rc;
     float *d_sum = c->frame, *d_sq = out_sumsq ? c->frame + plane : nullptr, *d_rgb = c->frame + 2 * plane;
     CU(c, cudaEventRecord(c->ev2, c->stream));
     vk_stats st{};
@@ -916,13 +920,7 @@ int vk_render_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, u
     CU(c, cudaSetDevice(c->device));
     int rc = ensure(c, &c->frame, &c->frame_floats, plane * 3);
     if (rc != VK_OK) return rc;
-    if (c->pinned_floats < plane * 2) {
-        if (c->pinned) cudaFreeHost(c->pinned);
-        c->pinned = nullptr;
-        c->pinned_floats = 0;
-        CU(c, cudaMallocHost((void**)&c->pinned, plane * 2 * sizeof(float)));
-        c->pinned_floats = plane * 2;
-    }
+    if ((rc = ensure_pinned(c, plane * 2)) != VK_OK) return rc;
     float* d_sum = c->frame;
     uint8_t* d_rgb8 = (uint8_t*)(c->frame + 2 * plane);
     CU(c, cudaEventRecord(c->ev2, c->stream));
@@ -951,14 +949,7 @@ static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint
     const size_t plane = (size_t)P->width * P->height * 3 * n_frames; // all frames
     CU(c, cudaSetDevice(c->device));
     if ((rc = ensure(c, &c->frame, &c->frame_floats, plane * 2)) != VK_OK) return rc; // sums | rgb
-    const size_t out_floats = out_rgb ? plane : (plane + 3) / 4;
-    if (c->pinned_floats < out_floats) {
-        if (c->pinned) cudaFreeHost(c->pinned);
-        c->pinned = nullptr;
-        c->pinned_floats = 0;
-        CU(c, cudaMallocHost((void**)&c->pinned, out_floats * sizeof(float)));
-        c->pinned_floats = out_floats;
-    }
+    if ((rc = ensure_pinned(c, out_rgb ? plane : (plane + 3) / 4)) != VK_OK) return rc;
     float *d_sum = c->frame, *d_rgb = c->frame + plane;
     CU(c, cudaEventRecord(c->ev2, c->stream));
     vk_stats st{};
@@ -1027,14 +1018,7 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
         CU(c, cudaMalloc(&c->adapt, need));
         c->adapt_bytes = need;
     }
-    const size_t pinned_need = plane + n_pix + 1; // floats: rgb | counts | the active count
-    if (c->pinned_floats < pinned_need) {
-        if (c->pinned) cudaFreeHost(c->pinned);
-        c->pinned = nullptr;
-        c->pinned_floats = 0;
-        CU(c, cudaMallocHost((void**)&c->pinned, pinned_need * sizeof(float)));
-        c->pinned_floats = pinned_need;
-    }
+    if ((rc = ensure_pinned(c, plane + n_pix + 1)) != VK_OK) return rc; // floats: rgb | counts | the active count
     char* base = (char*)c->adapt;
     unsigned long long* sq = (unsigned long long*)(base + o_sq);
     uint32_t* nspp = (uint32_t*)(base + o_n);
@@ -1341,12 +1325,7 @@ static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_
     return VK_OK;
 }
 static int multi_pinned(vk_multi* m, vk_ctx* c0, size_t floats) {
-    if (c0->pinned_floats >= floats) return VK_OK;
-    if (c0->pinned) cudaFreeHost(c0->pinned);
-    c0->pinned = nullptr;
-    c0->pinned_floats = 0;
-    if (cudaMallocHost((void**)&c0->pinned, floats * sizeof(float)) != cudaSuccess) return mfail(m, VK_ERR_OOM, "vk_multi_render: pinned staging");
-    c0->pinned_floats = floats;
+    if (ensure_pinned(c0, floats) != VK_OK) return mfail(m, VK_ERR_OOM, "vk_multi_render: pinned staging");
     return VK_OK;
 }
 int vk_multi_render(vk_multi* m, const vk_camera* cam, const vk_render_params* P, float* out_rgb, float* out_sumsq, vk_stats* stats) {

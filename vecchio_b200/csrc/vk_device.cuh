@@ -120,17 +120,6 @@ struct PathRng {
         return philox4x32_10(make_uint4(pixel, sample, (depth << 8) | blk, w), key);
     }
 };
-// Philox key of frame f of a batch (FrameArgs): seed + f, the key vecchio_gpu_render --seed gives frame f of a frame loop
-VKD uint2 frame_key(const RenderArgs& a, uint32_t f) {
-    const unsigned long long k = (((unsigned long long)a.seed_hi << 32) | a.seed_lo) + f;
-    return make_uint2((uint32_t)k, (uint32_t)(k >> 32));
-}
-// A batch-wide pixel index (f * n_pix + the pixel within frame f, see FrameArgs) -> the frame's own counter pixel and key
-VKD void frame_rng(PathRng& rng, const RenderArgs& a, uint32_t n_pix, uint32_t gpix) {
-    const uint32_t f = gpix / n_pix;
-    rng.pixel = gpix - f * n_pix;
-    rng.key = frame_key(a, f);
-}
 // Source of the ConstantMedium free-flight variate (src/hittable.rs:473): an injected table for
 // vk_intersect (VK_MEDIUM_XI_SLOTS entries per ray: scenes of up to four media), and for the render
 // Philox block 1 of the current segment with the counter's fourth word counting groups of four
@@ -1741,6 +1730,73 @@ VKD void accumulate_square(unsigned long long* sq, uint32_t pixel, float3 L) {
     if (L.x != 0.0f) atomicAdd(q + 0, __double2ull_rn(cx * cx * (double)VK_SQ_SCALE));
     if (L.y != 0.0f) atomicAdd(q + 1, __double2ull_rn(cy * cy * (double)VK_SQ_SCALE));
     if (L.z != 0.0f) atomicAdd(q + 2, __double2ull_rn(cz * cz * (double)VK_SQ_SCALE));
+}
+
+// ---------------------------------------------------------------------------------------------
+// Work domains (OneFrame, FrameArgs, ListArgs: vk_internal.h): what a render kernel's body asks its domain (the warp
+// queues' chunk dealing is next to WqCtx, vk_warpq.cuh).  Each question has a one-frame answer as its template and
+// an overload for each domain that answers differently; for OneFrame every answer is the single-frame code itself or
+// a constant that folds away.
+// ---------------------------------------------------------------------------------------------
+// Philox key of frame f of a batch: seed + f, the key vecchio_gpu_render --seed gives frame f of a frame loop
+VKD uint2 frame_key(const RenderArgs& a, uint32_t f) {
+    const unsigned long long k = (((unsigned long long)a.seed_hi << 32) | a.seed_lo) + f;
+    return make_uint2((uint32_t)k, (uint32_t)(k >> 32));
+}
+// the domain's unit count as a multiple of one frame's
+template <class D> VKD uint32_t dom_frames(const D&) { return 1u; }
+VKD uint32_t dom_frames(const FrameArgs& fr) { return fr.n_frames; }
+// the pixels a frame's units run over: W*H, or the list (a unit's "pixel" is then a list index, see dom_list_pixel)
+template <class D> VKD uint32_t dom_pixels(const D&, const RenderArgs& a) { return a.width * a.height; }
+VKD uint32_t dom_pixels(const ListArgs& ls, const RenderArgs&) { return ls.n; }
+template <class D> VKD uint32_t dom_list_pixel(const D&, uint32_t i) { return i; }
+VKD uint32_t dom_list_pixel(const ListArgs& ls, uint32_t i) { return ls.list[i]; }
+// Frame-major units: u of `per` units per frame -> its frame, and u within that frame (one frame: 0, u unchanged)
+template <class D, class T> VKD uint32_t dom_split_frame(const D&, T&, T) { return 0u; }
+template <class T> VKD uint32_t dom_split_frame(const FrameArgs&, T& u, T per) {
+    const uint32_t f = (uint32_t)(u / per);
+    u -= (T)f * per;
+    return f;
+}
+// frame f's first accumulator pixel, camera and Philox key (rng.key arrives as the seed's)
+template <class D> VKD uint32_t dom_plane(const D&, uint32_t) { return 0u; }
+VKD uint32_t dom_plane(const FrameArgs& fr, uint32_t f) { return f * fr.n_pix; }
+template <class D> VKD const DCamera& dom_camera(const D&, const DCamera& cam, uint32_t) { return cam; }
+VKD const DCamera& dom_camera(const FrameArgs& fr, const DCamera&, uint32_t f) { return fr.cams[f]; }
+template <class D> VKD void dom_frame_key(const D&, const RenderArgs&, uint32_t, PathRng&) {}
+VKD void dom_frame_key(const FrameArgs&, const RenderArgs& a, uint32_t f, PathRng& rng) { rng.key = frame_key(a, f); }
+// The pixel a warp-queue slot keeps (rng.pixel, the accumulator index: batch-wide in a batch) -> the Philox counter's
+// pixel and key of its frame
+template <class D> VKD void dom_slot_rng(const D&, const RenderArgs&, PathRng&) {}
+VKD void dom_slot_rng(const FrameArgs& fr, const RenderArgs& a, PathRng& rng) {
+    const uint32_t f = rng.pixel / fr.n_pix;
+    rng.pixel = rng.pixel - f * fr.n_pix;
+    rng.key = frame_key(a, f);
+}
+// a finished, finite sample into accumulator pixel `pixel`; an adaptive pass also keeps its squares
+template <class D> VKD void dom_accumulate(const D&, const RenderBuffers& buf, uint32_t pixel, float3 L) { accumulate_sample(buf, pixel, L); }
+VKD void dom_accumulate(const ListArgs& ls, const RenderBuffers& buf, uint32_t pixel, float3 L) {
+    accumulate_sample(buf, pixel, L);
+    accumulate_square(ls.sq, pixel, L);
+}
+// Unit u of a lane-megakernel item: pixel (px0, py0) + (u & 7, u >> 3 & 3) of an 8x4 tile -> (px, py) and the frame pixel
+// index; false for a unit outside the image.  A list's "tile" is 32 consecutive entries, unit u takes entry u & 31.
+template <class D>
+VKD bool mk_unit(const D&, const RenderArgs& a, uint32_t, uint32_t px0, uint32_t py0, uint32_t u, uint32_t& px, uint32_t& py, uint32_t& pixel) {
+    px = px0 + (u & 7u);
+    py = py0 + ((u >> 3) & 3u);
+    if (!(px < a.width && py < a.height)) return false; // ragged tiles: a unit outside the image is void
+    pixel = py * a.width + px;                          // i = y*width + x, row 0 = bottom (src/main.rs:182-183)
+    return true;
+}
+VKD bool mk_unit(const ListArgs& ls, const RenderArgs& a, uint32_t tile, uint32_t, uint32_t, uint32_t u, uint32_t& px, uint32_t& py,
+                 uint32_t& pixel) {
+    const uint32_t li = tile * 32u + (u & 31u);
+    if (!(li < ls.n)) return false; // the last group of the list is ragged
+    pixel = ls.list[li];
+    py = pixel / a.width;
+    px = pixel - py * a.width;
+    return true;
 }
 
 // A ray that leaves the scene: the constant background of src/main.rs:124,151, or with

@@ -189,13 +189,20 @@ struct RenderArgs {
     uint32_t tiles_x, tiles_y, n_chunks, chunk_spp;
 };
 
+// Work domains: what the units of a render kernel run over.  Every kernel AUTO can pick takes its domain as its last
+// template argument and as its last kernel parameter, behind all the others, so RenderArgs and everything in front of it
+// keep one layout.  The bodies ask the domain the few questions of the "work domains" section of vk_device.cuh.
+//   OneFrame   the W*H pixels of one frame (the single-frame kernels: the empty parameter adds nothing to their code)
+//   FrameArgs  a batch of frames
+//   ListArgs   a list of active pixels of one frame
+struct OneFrame {};
+
 // A batch of frames (vk_render_frames): frame f renders with cams[f] and Philox key seed + f (64-bit add) into the
 // accumulator plane that starts at f * n_pix * 3; pixel and sample of the Philox counter are the frame's own, so every frame
-// equals its single-frame render.  Only the batch instantiations of the kernels take it, as a kernel parameter behind all
-// the others: RenderArgs and everything in front of it keep the single-frame kernels' layout.  Their work units are
-// frame-major (the frame is the outermost dimension): a warp whose frame has run dry takes the next frame's units, and the
-// batch drains once.  Inside the warp-queue slots a pixel is the batch-wide index f * n_pix + y * width + x (the slot does
-// not grow); the frame is recovered from it where a PathRng is rebuilt.
+// equals its single-frame render.  The work units are frame-major (the frame is the outermost dimension): a warp whose
+// frame has run dry takes the next frame's units, and the batch drains once.  Inside the warp-queue slots a pixel is the
+// batch-wide index f * n_pix + y * width + x (the slot does not grow); the frame is recovered from it where a PathRng is
+// rebuilt.
 struct FrameArgs {
     const DCamera* cams; // device array, n_frames entries
     uint32_t n_frames;
@@ -204,9 +211,8 @@ struct FrameArgs {
 
 // A pass of an adaptive render (vk_render_adaptive): the work units run over a list of active pixels instead of the dense
 // frame.  An entry is a frame pixel index y * width + x, so the accumulators keep their dense W*H*3 layout and a slot keeps
-// the frame pixel.  Only the list instantiations of the kernels take it, as their last kernel parameter (like FrameArgs;
-// frame x list is not instantiated).  Every kept sample also adds its per-channel square to `sq` (accumulate_square): 64-bit
-// fixed point, so the sums, and the stopping decision made from them, do not depend on the order samples arrive in.
+// the frame pixel.  Every kept sample also adds its per-channel square to `sq` (accumulate_square): 64-bit fixed point, so
+// the sums, and the stopping decision made from them, do not depend on the order samples arrive in.
 struct ListArgs {
     const uint32_t* list;   // active pixels, ascending
     uint32_t n;             // list length
@@ -267,14 +273,15 @@ struct WfState {
     unsigned long long n_units;
 };
 
+// (the launchers that take a work domain D are instantiated for OneFrame, FrameArgs and ListArgs)
 #define VK_DECLARE_LAUNCHERS(NS)                                                                                       \
     namespace NS {                                                                                                     \
+    template <class D>                                                                                                 \
     cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,  \
-                                  const RenderBuffers& b, int grid, bool legacy, cudaStream_t st,                      \
-                                  const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);                        \
+                                  const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const D& dom);       \
+    template <class D>                                                                                                 \
     cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, \
-                                      unsigned long long* unit_head, int sm_count, cudaStream_t st,                     \
-                                      const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);                    \
+                                      unsigned long long* unit_head, int sm_count, cudaStream_t st, const D& dom);     \
     cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk_ray* rays, size_t n,              \
                                  const float* medium_xi, vk_hit* out, cudaStream_t st);                                \
     cudaError_t megakernel_occupancy(bool flat, bool media, bool legacy, int* blocks_per_sm, int* block_threads);      \
@@ -283,13 +290,15 @@ struct WfState {
                             cudaStream_t st);                                                                          \
     cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,      \
                               const RenderBuffers& b, unsigned long long* unit_head, int sm_count, cudaStream_t st);   \
+    template <class D>                                                                                                 \
     cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,       \
                              const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy,         \
-                             cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);            \
+                             cudaStream_t st, const D& dom);                                                           \
     size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t* levels);                          \
+    template <class D>                                                                                                 \
     cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,        \
                              unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, \
-                             bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr); \
+                             bool legacy, cudaStream_t st, const D& dom);                                              \
     cudaError_t launch_wf_generate(const DCamera& cam, const RenderArgs& a, const WfState& w, cudaStream_t st);        \
     cudaError_t launch_wf_extend(const DScene& sc, const FlatProgram* flat, const RenderArgs& a, const WfState& w,     \
                                  const RenderBuffers& b, uint32_t set, cudaStream_t st);                               \
@@ -302,6 +311,7 @@ VK_DECLARE_LAUNCHERS(vkfast_l0) // (vk_kernels.cu, vk_warpq.cu, vk_stepq.cu with
 namespace vkfast_simple { // vk_staged.cu / vk_warpq.cu compiled with VK_SIMPLE=1: kernels for "simple" flat scenes (see vk_device.cuh)
 cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
                           unsigned long long* unit_head, int sm_count, cudaStream_t st);
+template <class D>
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr);
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom);
 }

@@ -25,29 +25,22 @@ namespace VK_NS {
 #define VK_MINB_BVH 5
 #endif
 
-// accumulator pixel of a lane's sample: in a batch (FR) the frame's plane starts at pixel pbase
-template <bool FR> VKD uint32_t frame_pixel(uint32_t pbase, uint32_t pixel) {
-    if constexpr (FR) return pbase + pixel;
-    else return pixel;
-}
-
 // Work decomposition (deterministic for a seed whatever the grid):
 //   item  = one 8x4 pixel tile x one chunk of samples, fetched by a whole warp from a global queue;
 //   unit  = one pixel of the tile x one sample.  The 32 lanes of the warp draw units from a
 //           warp-local counter (ballot + popc, no memory traffic): a lane whose path has ended takes
 //           the next one, so lanes only idle for the last unit of an item.
 // A finished sample goes straight into its pixel's integer accumulators (accumulate_sample).
-// FR: a batch of frames (FrameArgs, k_megakernel*_frames): item = frame x chunk x tile, frame outermost.
-// LS: a pass over a list of active pixels (ListArgs, k_megakernel*_list): a "tile" is 32 consecutive list entries (the host
-// sets tiles_x to their number, tiles_y to 1), unit u of an item is list entry tile * 32 + (u & 31) x sample c0 + (u >> 5).
-template <bool FLAT, bool MEDIA, bool LEGACY, bool FR = false, bool LS = false>
+// A batch of frames: item = frame x chunk x tile, frame outermost.  A list of pixels: a "tile" is 32 consecutive list
+// entries (the host sets tiles_x to their number, tiles_y to 1), unit u of an item is entry tile * 32 + (u & 31) x sample
+// c0 + (u >> 5).
+template <bool FLAT, bool MEDIA, bool LEGACY, class D>
 VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,
-                         const RenderBuffers& buf, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
+                         const RenderBuffers& buf, const D& dom) {
     const uint32_t lane = threadIdx.x & 31u;
     const uint32_t lanes_below = (1u << lane) - 1u;
     const uint32_t n_tiles = a.tiles_x * a.tiles_y;
-    uint32_t total = n_tiles * a.n_chunks;
-    if constexpr (FR) total *= fr->n_frames;
+    const uint32_t total = n_tiles * a.n_chunks * dom_frames(dom);
     const uint32_t spp_end = a.spp_begin + a.spp_count;
     uint32_t n_rays = 0, n_drop = 0, n_nodes = 0, n_prims = 0; // per lane: far below 2^32 for any frame
 
@@ -57,12 +50,8 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
         if (lane == 0) item = (uint32_t)atomicAdd(&buf.counters[2], 1ull);
         item = __shfl_sync(0xFFFFFFFFu, item, 0);
         if (item >= total) break;
-        uint32_t f = 0, pbase = 0; // (FR) frame of the item, its first pixel in the accumulators
-        if constexpr (FR) {
-            f = item / (n_tiles * a.n_chunks);
-            item -= f * (n_tiles * a.n_chunks);
-            pbase = f * fr->n_pix;
-        }
+        const uint32_t f = dom_split_frame(dom, item, n_tiles * a.n_chunks); // frame of the item
+        const uint32_t pbase = dom_plane(dom, f);                            // its first pixel in the accumulators
         const uint32_t chunk = item / n_tiles, tile = item - chunk * n_tiles;
         const uint32_t px0 = (tile % a.tiles_x) * 8u, py0 = (tile / a.tiles_x) * 4u;
         const uint32_t c0 = a.spp_begin + chunk * a.chunk_spp;
@@ -74,7 +63,7 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
         rng.pixel = 0;
         rng.sample = 0;
         rng.key = make_uint2(a.seed_lo, a.seed_hi);
-        if constexpr (FR) rng.key = frame_key(a, f);
+        dom_frame_key(dom, a, f, rng);
         float3 o = f3(0.0f, 0.0f, 0.0f), d = o, beta = o, L = o;
         float time = 0.0f;
         uint32_t depth = 0, s = 0, s_end = 0, px = 0, py = 0;
@@ -87,26 +76,16 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
             const uint32_t want = __ballot_sync(0xFFFFFFFFu, need);
             if (need) {
                 const uint32_t u = next_unit + __popc(want & lanes_below);
-                if constexpr (LS) {
-                    const uint32_t li = tile * 32u + (u & 31u);
-                    if (u < n_units && li < ls->n) { // the last group of the list is ragged
-                        rng.pixel = ls->list[li];
-                        py = rng.pixel / a.width;
-                        px = rng.pixel - py * a.width;
-                        s = c0 + (u >> 5);
-                        s_end = s + 1u;
-                        has_unit = true;
-                    }
-                } else if (u < n_units) {
-                    px = px0 + (u & 7u);
-                    py = py0 + ((u >> 3) & 3u);
-                    if (px < a.width && py < a.height) { // ragged tiles: a unit outside the image is void
-                        s = c0 + (u >> 5);
-                        s_end = s + 1u;
-                        rng.pixel = py * a.width + px; // i = y*width + x, row 0 = bottom (src/main.rs:182-183)
-                        has_unit = true;
-                    }
+                // (through copies: px, py and rng.pixel passed by reference would change the single-frame kernels' code)
+                uint32_t x = px, y = py, pixel;
+                if (u < n_units && mk_unit(dom, a, tile, px0, py0, u, x, y, pixel)) {
+                    s = c0 + (u >> 5);
+                    s_end = s + 1u;
+                    rng.pixel = pixel;
+                    has_unit = true;
                 }
+                px = x;
+                py = y;
             }
             next_unit += __popc(want);
             const bool work = alive || (has_unit && s < s_end);
@@ -116,8 +95,7 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
             // ---- one path segment ---------------------------------------------------------------
             if (!alive) { // regenerate: this lane starts its next sample while others keep bouncing
                 rng.sample = s++;
-                if constexpr (FR) camera_get_ray(fr->cams[f], rng, px, py, a.width, a.height, o, d, time);
-                else camera_get_ray(cam, rng, px, py, a.width, a.height, o, d, time);
+                camera_get_ray(dom_camera(dom, cam, f), rng, px, py, a.width, a.height, o, d, time);
                 beta = f3(1.0f, 1.0f, 1.0f);
                 L = f3(0.0f, 0.0f, 0.0f);
                 depth = 1; // ray_color(ray, .., 1) src/main.rs:190
@@ -153,12 +131,8 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
                 }
             }
             if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                if (valid && finite3(L)) {
-                    accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
-                    if constexpr (LS) accumulate_square(ls->sq, rng.pixel, L);
-                } else {
-                    ++n_drop;
-                }
+                if (valid && finite3(L)) dom_accumulate(dom, buf, pbase + rng.pixel, L);
+                else ++n_drop;
             }
         }
     }
@@ -201,17 +175,14 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VK_DYN_NODE_STEPS
 #define VK_DYN_NODE_STEPS 4
 #endif
-// FR: a batch of frames (FrameArgs, k_megakernel_dyn_frames): unit = frame x sample x pixel, frame outermost.
-// LS: a pass over a list of active pixels (ListArgs, k_megakernel_dyn_list): unit = sample x list entry.
-template <bool MEDIA, bool FR = false, bool LS = false>
+// unit = frame x sample x pixel, frame outermost (a list of pixels: sample x list entry)
+template <bool MEDIA, class D>
 VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                             unsigned long long* unit_head, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
+                             unsigned long long* unit_head, const D& dom) {
     const uint32_t lane = threadIdx.x & 31u, lanes_below = (1u << lane) - 1u;
-    uint32_t n_pixels = a.width * a.height;
-    if constexpr (LS) n_pixels = ls->n; // (the units' "pixels" are list entries)
-    unsigned long long n_units = (unsigned long long)n_pixels * a.spp_count;
-    if constexpr (FR) n_units *= fr->n_frames;
-    uint32_t pbase = 0; // (FR) first accumulator pixel of this lane's frame
+    const uint32_t n_pixels = dom_pixels(dom, a);
+    const unsigned long long n_units = (unsigned long long)n_pixels * a.spp_count * dom_frames(dom);
+    uint32_t pbase = 0; // first accumulator pixel of this lane's frame
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
 
@@ -255,12 +226,8 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
                     }
                 }
                 if (!alive) { // sample finished: NaN/Inf filter of src/main.rs:191-194
-                    if (valid && finite3(L)) {
-                        accumulate_sample(buf, frame_pixel<FR>(pbase, rng.pixel), L);
-                        if constexpr (LS) accumulate_square(ls->sq, rng.pixel, L);
-                    } else {
-                        ++n_drop;
-                    }
+                    if (valid && finite3(L)) dom_accumulate(dom, buf, pbase + rng.pixel, L);
+                    else ++n_drop;
                 }
             }
             if (alive) new_ray = true;
@@ -274,20 +241,13 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
             if (need_unit) {
                 unsigned long long u = base + __popc(mu & lanes_below);
                 if (u < n_units) {
-                    uint32_t f = 0;
-                    if constexpr (FR) {
-                        const unsigned long long per_frame = (unsigned long long)n_pixels * a.spp_count;
-                        f = (uint32_t)(u / per_frame);
-                        u -= (unsigned long long)f * per_frame;
-                        pbase = f * n_pixels;
-                        rng.key = frame_key(a, f);
-                    }
+                    const uint32_t f = dom_split_frame(dom, u, (unsigned long long)n_pixels * a.spp_count);
+                    pbase = f * n_pixels;
+                    dom_frame_key(dom, a, f, rng);
                     const uint32_t sb = (uint32_t)(u / n_pixels);
-                    rng.pixel = (uint32_t)(u - (unsigned long long)sb * n_pixels); // i = y*width + x (src/main.rs:182-183)
-                    if constexpr (LS) rng.pixel = ls->list[rng.pixel];
+                    rng.pixel = dom_list_pixel(dom, (uint32_t)(u - (unsigned long long)sb * n_pixels)); // i = y*width + x (src/main.rs:182-183)
                     rng.sample = a.spp_begin + sb;
-                    if constexpr (FR) camera_get_ray(fr->cams[f], rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
-                    else camera_get_ray(cam, rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
+                    camera_get_ray(dom_camera(dom, cam, f), rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
                     beta = f3(1.0f, 1.0f, 1.0f);
                     depth = 1;
                     new_ray = true;
@@ -338,58 +298,23 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
         if (w_drop) atomicAdd(&buf.counters[1], w_drop);
     }
 }
-template <bool MEDIA>
+// instantiations: {BVH, flat program} x {scene without / with ConstantMedium} x {HEAD integrator, legacy scatter} x work domain
+template <bool MEDIA, class D>
 __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                      const RenderBuffers buf, unsigned long long* unit_head) {
-    megakernel_dyn_body<MEDIA>(sc, cam, a, buf, unit_head);
+                                                                      const RenderBuffers buf, unsigned long long* unit_head,
+                                                                      const __grid_constant__ D dom) {
+    megakernel_dyn_body<MEDIA>(sc, cam, a, buf, unit_head, dom);
 }
-template <bool MEDIA>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn_frames(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                             const RenderBuffers buf, unsigned long long* unit_head,
-                                                                             const __grid_constant__ FrameArgs fr) {
-    megakernel_dyn_body<MEDIA, true>(sc, cam, a, buf, unit_head, &fr);
-}
-template <bool MEDIA>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_dyn_list(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                           const RenderBuffers buf, unsigned long long* unit_head,
-                                                                           const __grid_constant__ ListArgs ls) {
-    megakernel_dyn_body<MEDIA, false, true>(sc, cam, a, buf, unit_head, nullptr, &ls);
-}
-
-// instantiations: {BVH, flat program} x {scene without / with ConstantMedium} x {HEAD integrator, legacy scatter}
-template <bool MEDIA, bool LEGACY>
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                  const RenderBuffers buf) {
-    megakernel_body<false, MEDIA, LEGACY>(sc, nullptr, cam, a, buf);
+                                                                  const RenderBuffers buf, const __grid_constant__ D dom) {
+    megakernel_body<false, MEDIA, LEGACY>(sc, nullptr, cam, a, buf, dom);
 }
-template <bool MEDIA, bool LEGACY>
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat(const DScene sc, const __grid_constant__ FlatProgram flat,
-                                                                       const DCamera cam, const RenderArgs a, const RenderBuffers buf) {
-    megakernel_body<true, MEDIA, LEGACY>(sc, &flat, cam, a, buf);
-}
-// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_frames(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                         const RenderBuffers buf, const __grid_constant__ FrameArgs fr) {
-    megakernel_body<false, MEDIA, LEGACY, true>(sc, nullptr, cam, a, buf, &fr);
-}
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat_frames(const DScene sc, const __grid_constant__ FlatProgram flat,
-                                                                              const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                              const __grid_constant__ FrameArgs fr) {
-    megakernel_body<true, MEDIA, LEGACY, true>(sc, &flat, cam, a, buf, &fr);
-}
-// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_BVH) k_megakernel_list(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                       const RenderBuffers buf, const __grid_constant__ ListArgs ls) {
-    megakernel_body<false, MEDIA, LEGACY, false, true>(sc, nullptr, cam, a, buf, nullptr, &ls);
-}
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(VK_BLOCK, VK_MINB_FLAT) k_megakernel_flat_list(const DScene sc, const __grid_constant__ FlatProgram flat,
-                                                                            const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                            const __grid_constant__ ListArgs ls) {
-    megakernel_body<true, MEDIA, LEGACY, false, true>(sc, &flat, cam, a, buf, nullptr, &ls);
+                                                                       const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                       const __grid_constant__ D dom) {
+    megakernel_body<true, MEDIA, LEGACY>(sc, &flat, cam, a, buf, dom);
 }
 
 template <bool FLAT>
@@ -503,26 +428,16 @@ __global__ void k_philox_kat(const uint32_t* in6, uint32_t* out4) {
 }
 
 // *unit_head must be zero on the stream before the launch
-// fr != nullptr: a batch of frames (k_megakernel_dyn_frames); ls != nullptr: a pass over a pixel list (k_megakernel_dyn_list)
+template <class D>
 cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                                  unsigned long long* unit_head, int sm_count, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
+                                  unsigned long long* unit_head, int sm_count, cudaStream_t st, const D& dom) {
     int bps = 0;
-    cudaError_t e = ls ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_list<true>, VK_BLOCK, 0)
-                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_list<false>, VK_BLOCK, 0))
-                  : fr ? (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<true>, VK_BLOCK, 0)
-                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn_frames<false>, VK_BLOCK, 0))
-                       : (sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<true>, VK_BLOCK, 0)
-                                       : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<false>, VK_BLOCK, 0));
+    cudaError_t e = sc.has_media ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<true, D>, VK_BLOCK, 0)
+                                 : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_megakernel_dyn<false, D>, VK_BLOCK, 0);
     if (e != cudaSuccess) return e;
     const int grid = sm_count * (bps < 1 ? 1 : bps);
-    if (ls) {
-        if (sc.has_media) k_megakernel_dyn_list<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *ls);
-        else k_megakernel_dyn_list<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *ls);
-    } else if (fr) {
-        if (sc.has_media) k_megakernel_dyn_frames<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
-        else k_megakernel_dyn_frames<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, *fr);
-    } else if (sc.has_media) k_megakernel_dyn<true><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
-    else k_megakernel_dyn<false><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head);
+    if (sc.has_media) k_megakernel_dyn<true, D><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, dom);
+    else k_megakernel_dyn<false, D><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, unit_head, dom);
     return cudaGetLastError();
 }
 #define VK_MEGA_DISPATCH(CALL_BVH, CALL_FLAT)                                                                         \
@@ -533,34 +448,28 @@ cudaError_t launch_megakernel_dyn(const DScene& sc, const DCamera& cam, const Re
         if (media) { if (legacy) { CALL_BVH(true, true); } else { CALL_BVH(true, false); } }                           \
         else { if (legacy) { CALL_BVH(false, true); } else { CALL_BVH(false, false); } }                               \
     }
-// fr != nullptr: a batch of frames (k_megakernel*_frames; the grid is the single-frame kernels', same registers)
-// ls != nullptr: a pass over a pixel list (k_megakernel*_list; a.tiles_x * a.tiles_y = groups of 32 list entries)
+// the grid is the single-frame kernels' whatever the domain (megakernel_occupancy: same registers); over a pixel list,
+// a.tiles_x * a.tiles_y = groups of 32 list entries
+template <class D>
 cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flatp, const DCamera& cam, const RenderArgs& a,
-                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
+                              const RenderBuffers& b, int grid, bool legacy, cudaStream_t st, const D& dom) {
     const bool flat = flatp && flatp->n, media = sc.has_media;
-    if (ls) {
-#define VK_LB(M, G) k_megakernel_list<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, *ls)
-#define VK_LF(M, G) k_megakernel_flat_list<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, *ls)
-        VK_MEGA_DISPATCH(VK_LB, VK_LF)
-#undef VK_LB
-#undef VK_LF
-        return cudaGetLastError();
-    }
-    if (fr) {
-#define VK_LB(M, G) k_megakernel_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, *fr)
-#define VK_LF(M, G) k_megakernel_flat_frames<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, *fr)
-        VK_MEGA_DISPATCH(VK_LB, VK_LF)
-#undef VK_LB
-#undef VK_LF
-        return cudaGetLastError();
-    }
-#define VK_LB(M, G) k_megakernel<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b)
-#define VK_LF(M, G) k_megakernel_flat<M, G><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b)
+#define VK_LB(M, G) k_megakernel<M, G, D><<<grid, VK_BLOCK, 0, st>>>(sc, cam, a, b, dom)
+#define VK_LF(M, G) k_megakernel_flat<M, G, D><<<grid, VK_BLOCK, 0, st>>>(sc, *flatp, cam, a, b, dom)
     VK_MEGA_DISPATCH(VK_LB, VK_LF)
 #undef VK_LB
 #undef VK_LF
     return cudaGetLastError();
 }
+#define VK_INSTANTIATE(D)                                                                                              \
+    template cudaError_t launch_megakernel_dyn(const DScene&, const DCamera&, const RenderArgs&, const RenderBuffers&, \
+                                               unsigned long long*, int, cudaStream_t, const D&);                      \
+    template cudaError_t launch_megakernel(const DScene&, const FlatProgram*, const DCamera&, const RenderArgs&,       \
+                                           const RenderBuffers&, int, bool, cudaStream_t, const D&);
+VK_INSTANTIATE(OneFrame)
+VK_INSTANTIATE(FrameArgs)
+VK_INSTANTIATE(ListArgs)
+#undef VK_INSTANTIATE
 cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk_ray* rays, size_t n, const float* medium_xi,
                              vk_hit* out, cudaStream_t st) {
     if (n == 0) return cudaSuccess;
@@ -572,8 +481,8 @@ cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk
 cudaError_t megakernel_occupancy(bool flat, bool media, bool legacy, int* blocks_per_sm, int* block_threads) {
     *block_threads = VK_BLOCK;
     cudaError_t e = cudaSuccess;
-#define VK_OB(M, G) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k_megakernel<M, G>, VK_BLOCK, 0)
-#define VK_OF(M, G) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k_megakernel_flat<M, G>, VK_BLOCK, 0)
+#define VK_OB(M, G) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k_megakernel<M, G, OneFrame>, VK_BLOCK, 0)
+#define VK_OF(M, G) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, k_megakernel_flat<M, G, OneFrame>, VK_BLOCK, 0)
     VK_MEGA_DISPATCH(VK_OB, VK_OF)
 #undef VK_OB
 #undef VK_OF

@@ -139,15 +139,13 @@ VKD bool sq_pick(const W& S, uint32_t last_q, uint32_t& q, uint32_t& n_q, uint32
     return (key >> 4) != 0u;
 }
 
-// FR: a batch of frames (FrameArgs, the *_frames kernels)
-// LS: a pass over a list of active pixels (ListArgs, the *_list kernels)
-template <bool MEDIA, bool LEGACY, class W, bool FR = false, bool LS = false>
+template <bool MEDIA, bool LEGACY, class W, class D>
 VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
-                    uint32_t* gstack, uint32_t glevels, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
+                    uint32_t* gstack, uint32_t glevels, const D& dom) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
+    const WqCtx<W> C = wq_ctx(dom, cam, a, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -163,7 +161,7 @@ VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, c
         if (!sq_pick(S, q, q, n_q, tail_q)) break; // every queue empty: all slots have retired
         const uint32_t n = wq_pop(S, q, n_q, tail_q, 32u, lane, head);
         if (q >= VKQ_END && q <= VKQ_DIFFI) {
-            wq_shade_batch<LEGACY, false>(sc, C, buf, q, n, head, n_drop);
+            wq_shade_batch<LEGACY, false>(sc, C, dom, buf, q, n, head, n_drop);
             continue;
         }
         wq_converge();
@@ -324,7 +322,7 @@ VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, c
                                 xi.rng.key = make_uint2(a.seed_lo, a.seed_hi);
                                 xi.rng.pixel = S.px[slot];
                                 xi.rng.sample = __float_as_uint(S.bt[slot].w);
-                                if constexpr (FR) frame_rng(xi.rng, a, fr->n_pix, xi.rng.pixel);
+                                dom_slot_rng(dom, a, xi.rng);
                                 hit = medium_t(sc, leaf, to, td, time, tmin, best_t, xi, t);
                             } else {
                                 hit = leaf_t(sc, leaf, to, td, rcp3(td), time, tmin, best_t, t, face);
@@ -373,41 +371,18 @@ VKD void stepq_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, c
 using WqStepWorld = WqStepWarp<VKS_N, VKS_RN, VKS_SD, false, VKS_MERGE != 0>;
 using WqStepInst = WqStepWarp<VKS_N_INST, VKS_RN, VKS_SD, true, VKS_MERGE_INST != 0>;
 
-template <bool MEDIA, bool LEGACY>
+// instantiations: {no medium, medium} x {HEAD integrator, legacy scatter} x work domain
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB) k_stepq(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels) {
-    stepq_body<MEDIA, LEGACY, WqStepWorld>(sc, cam, a, buf, unit_head, gstack, glevels);
+                                                                unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
+                                                                const __grid_constant__ D dom) {
+    stepq_body<MEDIA, LEGACY, WqStepWorld>(sc, cam, a, buf, unit_head, gstack, glevels, dom);
 }
-template <bool MEDIA, bool LEGACY>
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                          unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels) {
-    stepq_body<MEDIA, LEGACY, WqStepInst>(sc, cam, a, buf, unit_head, gstack, glevels);
-}
-// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB) k_stepq_frames(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                       unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
-                                                                       const __grid_constant__ FrameArgs fr) {
-    stepq_body<MEDIA, LEGACY, WqStepWorld, true>(sc, cam, a, buf, unit_head, gstack, glevels, &fr);
-}
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst_frames(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                                 const RenderBuffers buf, unsigned long long* unit_head, uint32_t* gstack,
-                                                                                 uint32_t glevels, const __grid_constant__ FrameArgs fr) {
-    stepq_body<MEDIA, LEGACY, WqStepInst, true>(sc, cam, a, buf, unit_head, gstack, glevels, &fr);
-}
-// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB) k_stepq_list(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                     unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
-                                                                     const __grid_constant__ ListArgs ls) {
-    stepq_body<MEDIA, LEGACY, WqStepWorld, false, true>(sc, cam, a, buf, unit_head, gstack, glevels, nullptr, &ls);
-}
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKS_MINB_INST) k_stepq_inst_list(const DScene sc, const DCamera cam, const RenderArgs a,
-                                                                               const RenderBuffers buf, unsigned long long* unit_head, uint32_t* gstack,
-                                                                               uint32_t glevels, const __grid_constant__ ListArgs ls) {
-    stepq_body<MEDIA, LEGACY, WqStepInst, false, true>(sc, cam, a, buf, unit_head, gstack, glevels, nullptr, &ls);
+                                                                          unsigned long long* unit_head, uint32_t* gstack, uint32_t glevels,
+                                                                          const __grid_constant__ D dom) {
+    stepq_body<MEDIA, LEGACY, WqStepInst>(sc, cam, a, buf, unit_head, gstack, glevels, dom);
 }
 
 // What the launch needs of the overflow stack: `words` 32-bit words for a scene whose traversal may hold `stack_need`
@@ -418,34 +393,35 @@ size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t*
     return warps * *levels * (inst ? VKS_N_INST : VKS_N);
 }
 
-// fr != nullptr: a batch of frames, the *_frames kernels; ls != nullptr: a pass over a pixel list, the *_list kernels
+template <class D>
 cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b, unsigned long long* unit_head,
-                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr,
-                         const ListArgs* ls) {
+                         uint32_t* gstack, uint32_t glevels, bool inst, int sm_count, bool legacy, cudaStream_t st, const D& dom) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
-#define VKS_LAUNCH(KERNEL, WARP, ...)                                                                                  \
+#define VKS_LAUNCH(KERNEL, WARP)                                                                                       \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WARP);                                                                  \
         if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
         if (bps > 8) bps = 8;                                                                                          \
-        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head, gstack, glevels __VA_ARGS__); \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head, gstack, glevels, dom); \
     }
-#define VKS_DISPATCH(FRAMES, ...)                                                                                      \
-    if (inst) {                                                                                                        \
-        if (media) { if (legacy) VKS_LAUNCH((k_stepq_inst##FRAMES<true, true>), WqStepInst, __VA_ARGS__) else VKS_LAUNCH((k_stepq_inst##FRAMES<true, false>), WqStepInst, __VA_ARGS__) } \
-        else { if (legacy) VKS_LAUNCH((k_stepq_inst##FRAMES<false, true>), WqStepInst, __VA_ARGS__) else VKS_LAUNCH((k_stepq_inst##FRAMES<false, false>), WqStepInst, __VA_ARGS__) } \
-    } else {                                                                                                           \
-        if (media) { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<true, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<true, false>), WqStepWorld, __VA_ARGS__) } \
-        else { if (legacy) VKS_LAUNCH((k_stepq##FRAMES<false, true>), WqStepWorld, __VA_ARGS__) else VKS_LAUNCH((k_stepq##FRAMES<false, false>), WqStepWorld, __VA_ARGS__) } \
+    if (inst) {
+        if (media) { if (legacy) VKS_LAUNCH((k_stepq_inst<true, true, D>), WqStepInst) else VKS_LAUNCH((k_stepq_inst<true, false, D>), WqStepInst) }
+        else { if (legacy) VKS_LAUNCH((k_stepq_inst<false, true, D>), WqStepInst) else VKS_LAUNCH((k_stepq_inst<false, false, D>), WqStepInst) }
+    } else {
+        if (media) { if (legacy) VKS_LAUNCH((k_stepq<true, true, D>), WqStepWorld) else VKS_LAUNCH((k_stepq<true, false, D>), WqStepWorld) }
+        else { if (legacy) VKS_LAUNCH((k_stepq<false, true, D>), WqStepWorld) else VKS_LAUNCH((k_stepq<false, false, D>), WqStepWorld) }
     }
-    if (ls) { VKS_DISPATCH(_list, , *ls) }
-    else if (fr) { VKS_DISPATCH(_frames, , *fr) }
-    else { VKS_DISPATCH(, ) }
-#undef VKS_DISPATCH
 #undef VKS_LAUNCH
     return cudaGetLastError();
 }
+#define VKS_INSTANTIATE(D)                                                                                             \
+    template cudaError_t launch_stepq(const DScene&, const DCamera&, const RenderArgs&, const RenderBuffers&, unsigned long long*, \
+                                      uint32_t*, uint32_t, bool, int, bool, cudaStream_t, const D&);
+VKS_INSTANTIATE(OneFrame)
+VKS_INSTANTIATE(FrameArgs)
+VKS_INSTANTIATE(ListArgs)
+#undef VKS_INSTANTIATE
 
 } // namespace VK_NS

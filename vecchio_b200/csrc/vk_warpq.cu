@@ -34,15 +34,13 @@ namespace VK_NS {
 // cluster) are traversed inside the extend stage, every lane for its own ray; what differs between the lanes of a batch is
 // then only how long a walk through ONE kind of tree takes -- the heterogeneous top of the scene (loose spheres, media,
 // rects) is typed batches, and the shading runs on whole batches of a class.
-// FR: a batch of frames (FrameArgs, the *_frames kernels)
-// LS: a pass over a list of active pixels (ListArgs, the *_list kernels)
-template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID = false, bool FR = false, bool LS = false>
+template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID, class D>
 VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
-                         unsigned long long* unit_head, const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
+                         unsigned long long* unit_head, const D& dom) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
+    const WqCtx<W> C = wq_ctx(dom, cam, a, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0, n_prims = 0;
     TraceCounters tc = {0u, 0u};
     constexpr uint32_t EXT_CAP = 32u * K;
@@ -56,7 +54,7 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
         if (!wq_pick(S, wq_counts(S), EXT_CAP, q, n_q, tail_q)) break; // every queue is empty: all slots have retired
         const uint32_t n = wq_pop(S, q, n_q, tail_q, q == VKQ_EXT ? EXT_CAP : 32u, lane, head);
         if (q != VKQ_EXT) {
-            wq_shade_batch<LEGACY, !HYBRID>(sc, C, buf, q, n, head, n_drop); // (no shading records for subtree hits)
+            wq_shade_batch<LEGACY, !HYBRID>(sc, C, dom, buf, q, n, head, n_drop); // (no shading records for subtree hits)
             continue;
         }
         // ---- extend: world.hit() (src/main.rs:130) for up to EXT_CAP rays, K per lane --------------------------------
@@ -80,7 +78,7 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
             xi[k].rng.key = make_uint2(a.seed_lo, a.seed_hi);
             xi[k].rng.pixel = MEDIA ? S.px[slot[k]] : 0u;
             xi[k].rng.sample = MEDIA ? __float_as_uint(S.bt[slot[k]].w) : 0u;
-            if constexpr (FR && MEDIA) frame_rng(xi[k].rng, a, fr->n_pix, xi[k].rng.pixel);
+            if (MEDIA) dom_slot_rng(dom, a, xi[k].rng);
         }
         TraceHit sub[K];
         trace_flat_k<K, MEDIA, HYBRID>(sc, *flat, o, d, tm, live, 0.001f, xi, best_t, best_hit, sub, &tc);
@@ -132,13 +130,13 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VKQ_NODE_STEPS
 #define VKQ_NODE_STEPS 4
 #endif
-template <bool MEDIA, bool LEGACY, class W, bool FR = false, bool LS = false>
+template <bool MEDIA, bool LEGACY, class W, class D>
 VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf, unsigned long long* unit_head,
-                        const FrameArgs* fr = nullptr, const ListArgs* ls = nullptr) {
+                        const D& dom) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
     const uint32_t lane = threadIdx.x & 31u, below = (1u << lane) - 1u;
     W& S = reinterpret_cast<W*>(vkq_raw)[threadIdx.x >> 5];
-    const WqCtx<W, FR, LS> C = wq_ctx_fr<FR, LS>(cam, a, fr, S, unit_head, lane, ls);
+    const WqCtx<W> C = wq_ctx(dom, cam, a, S, unit_head, lane);
     uint32_t n_rays = 0, n_drop = 0;
     TraceCounters tc = {0u, 0u};
     const uint32_t miss_cls = wq_black_miss(a) ? (uint32_t)VKQ_END : (uint32_t)VKQ_EMIT;
@@ -199,7 +197,7 @@ VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& 
                     if (MEDIA) {
                         xi.rng.pixel = S.px[cur];
                         xi.rng.sample = __float_as_uint(S.bt[cur].w);
-                        if constexpr (FR) frame_rng(xi.rng, a, fr->n_pix, xi.rng.pixel);
+                        dom_slot_rng(dom, a, xi.rng);
                     }
                     trav_init(T, sc, o, d, CUDART_INF_F); // world.hit(&r, 0.001, inf) src/main.rs:130
                     ++n_rays;
@@ -210,7 +208,7 @@ VKD void warpq_bvh_body(const DScene& sc, const DCamera& cam, const RenderArgs& 
                 uint32_t q, n_q, tail_q, head;
                 if (wq_pick(S, wq_counts(S), 0u, q, n_q, tail_q)) {
                     const uint32_t n = wq_pop(S, q, n_q, tail_q, 32u, lane, head);
-                    wq_shade_batch<LEGACY, false>(sc, C, buf, q, n, head, n_drop);
+                    wq_shade_batch<LEGACY, false>(sc, C, dom, buf, q, n, head, n_drop);
                     continue;
                 }
                 if (m_act == 0u) break; // nothing in flight, nothing queued: all slots have retired
@@ -231,128 +229,79 @@ using WqBvh = WqWarp<VKQ_N_BVH, VKQ_RN_BVH>;
 using WqHyb = WqWarp<VKQ_N_HYB, VKQ_RN_HYB>;
 static_assert(VKQ_WARPS <= 15, "one named barrier per warp of the CTA");
 
-template <bool MEDIA, bool LEGACY>
+// instantiations: {no medium, medium} x {HEAD integrator, legacy scatter} x work domain
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_BVH) k_warpq(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                    unsigned long long* unit_head) {
-    warpq_bvh_body<MEDIA, LEGACY, WqBvh>(sc, cam, a, buf, unit_head);
+                                                                    unsigned long long* unit_head, const __grid_constant__ D dom) {
+    warpq_bvh_body<MEDIA, LEGACY, WqBvh>(sc, cam, a, buf, unit_head, dom);
 }
-template <bool LEGACY>
+template <bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                          const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head) {
-    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT>(sc, &flat, cam, a, buf, unit_head);
+                                                                          const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                          const __grid_constant__ D dom) {
+    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false>(sc, &flat, cam, a, buf, unit_head, dom);
 }
-template <bool LEGACY>
+template <bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media(const DScene sc, const __grid_constant__ FlatProgram flat,
                                                                                  const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                                 unsigned long long* unit_head) {
-    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA>(sc, &flat, cam, a, buf, unit_head);
+                                                                                 unsigned long long* unit_head, const __grid_constant__ D dom) {
+    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA, false>(sc, &flat, cam, a, buf, unit_head, dom);
 }
 #if !VK_SIMPLE
-template <bool MEDIA, bool LEGACY>
+template <bool MEDIA, bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                            const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head) {
-    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true>(sc, &flat, cam, a, buf, unit_head);
-}
-#endif
-// the same kernels for a batch of frames (FrameArgs: the last parameter, so that everything in front keeps its place)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_BVH) k_warpq_frames(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                           unsigned long long* unit_head, const __grid_constant__ FrameArgs fr) {
-    warpq_bvh_body<MEDIA, LEGACY, WqBvh, true>(sc, cam, a, buf, unit_head, &fr);
-}
-template <bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat_frames(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                                 const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
-                                                                                 const __grid_constant__ FrameArgs fr) {
-    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false, true>(sc, &flat, cam, a, buf, unit_head, &fr);
-}
-template <bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media_frames(const DScene sc, const __grid_constant__ FlatProgram flat,
-                                                                                        const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                                        unsigned long long* unit_head, const __grid_constant__ FrameArgs fr) {
-    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA, false, true>(sc, &flat, cam, a, buf, unit_head, &fr);
-}
-#if !VK_SIMPLE
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid_frames(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                                   const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
-                                                                                   const __grid_constant__ FrameArgs fr) {
-    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true, true>(sc, &flat, cam, a, buf, unit_head, &fr);
-}
-#endif
-// ... and for a pass over a list of active pixels (ListArgs, last parameter likewise)
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_BVH) k_warpq_list(const DScene sc, const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                         unsigned long long* unit_head, const __grid_constant__ ListArgs ls) {
-    warpq_bvh_body<MEDIA, LEGACY, WqBvh, false, true>(sc, cam, a, buf, unit_head, nullptr, &ls);
-}
-template <bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat_list(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                               const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
-                                                                               const __grid_constant__ ListArgs ls) {
-    warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
-}
-template <bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media_list(const DScene sc, const __grid_constant__ FlatProgram flat,
-                                                                                      const DCamera cam, const RenderArgs a, const RenderBuffers buf,
-                                                                                      unsigned long long* unit_head, const __grid_constant__ ListArgs ls) {
-    warpq_flat_body<true, LEGACY, WqMedia, VKQ_K_MEDIA, false, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
-}
-#if !VK_SIMPLE
-template <bool MEDIA, bool LEGACY>
-__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid_list(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera cam,
-                                                                                 const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
-                                                                                 const __grid_constant__ ListArgs ls) {
-    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true, false, true>(sc, &flat, cam, a, buf, unit_head, nullptr, &ls);
+                                                                            const RenderArgs a, const RenderBuffers buf, unsigned long long* unit_head,
+                                                                            const __grid_constant__ D dom) {
+    warpq_flat_body<MEDIA, LEGACY, WqHyb, 1, true>(sc, &flat, cam, a, buf, unit_head, dom);
 }
 #endif
 
 // grid = sm_count * resident CTAs (persistent); *unit_head must be zero on the stream before the launch
-// fr != nullptr: a batch of frames, the *_frames kernels (the same choice of kernel, FrameArgs as one more argument)
-// ls != nullptr: a pass over a pixel list, the *_list kernels (likewise, ListArgs)
+template <class D>
 cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const FrameArgs* fr, const ListArgs* ls) {
+                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
-#define VKQ_LAUNCH_FLAT(KERNEL, WARP, ...)                                                                             \
+#define VKQ_LAUNCH_FLAT(KERNEL, WARP)                                                                                  \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WARP);                                                                  \
         if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
-        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, *flat, cam, a, b, unit_head __VA_ARGS__); \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, *flat, cam, a, b, unit_head, dom);    \
     }
-#define VKQ_LAUNCH_BVH(KERNEL, ...)                                                                                    \
+#define VKQ_LAUNCH_BVH(KERNEL)                                                                                         \
     {                                                                                                                  \
         const size_t smem = VKQ_WARPS * sizeof(WqBvh);                                                                 \
         if ((e = warpq_prepare(KERNEL, smem, &bps)) != cudaSuccess) return e;                                          \
-        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head __VA_ARGS__);   \
+        KERNEL<<<sm_count * (bps < 1 ? 1 : bps), 32 * VKQ_WARPS, smem, st>>>(sc, cam, a, b, unit_head, dom);           \
     }
 #if VK_SIMPLE
     (void)legacy; // the trimmed build exists for the HEAD integrator on flat scenes only
-#define VKQ_DISPATCH(FRAMES, ...)                                                                                      \
-    if (media) VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<false>, WqMedia, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<false>, WqFlat, __VA_ARGS__)
+    if (media) VKQ_LAUNCH_FLAT((k_warpq_flat_media<false, D>), WqMedia) else VKQ_LAUNCH_FLAT((k_warpq_flat<false, D>), WqFlat)
 #else
-#define VKQ_LAUNCH_HYB(M, G, FRAMES, ...) VKQ_LAUNCH_FLAT((k_warpq_hybrid##FRAMES<M, G>), WqHyb, __VA_ARGS__)
-#define VKQ_DISPATCH(FRAMES, ...)                                                                                      \
-    if (flat && flat->n && flat->n_bvh) {                                                                              \
-        if (media) { if (legacy) VKQ_LAUNCH_HYB(true, true, FRAMES, __VA_ARGS__) else VKQ_LAUNCH_HYB(true, false, FRAMES, __VA_ARGS__) } \
-        else { if (legacy) VKQ_LAUNCH_HYB(false, true, FRAMES, __VA_ARGS__) else VKQ_LAUNCH_HYB(false, false, FRAMES, __VA_ARGS__) } \
-    } else if (flat && flat->n) {                                                                                      \
-        if (media) { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<true>, WqMedia, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat_media##FRAMES<false>, WqMedia, __VA_ARGS__) } \
-        else { if (legacy) VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<true>, WqFlat, __VA_ARGS__) else VKQ_LAUNCH_FLAT(k_warpq_flat##FRAMES<false>, WqFlat, __VA_ARGS__) } \
-    } else {                                                                                                           \
-        if (media) { if (legacy) VKQ_LAUNCH_BVH((k_warpq##FRAMES<true, true>), __VA_ARGS__) else VKQ_LAUNCH_BVH((k_warpq##FRAMES<true, false>), __VA_ARGS__) } \
-        else { if (legacy) VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, true>), __VA_ARGS__) else VKQ_LAUNCH_BVH((k_warpq##FRAMES<false, false>), __VA_ARGS__) } \
+#define VKQ_LAUNCH_HYB(M, G) VKQ_LAUNCH_FLAT((k_warpq_hybrid<M, G, D>), WqHyb)
+    if (flat && flat->n && flat->n_bvh) {
+        if (media) { if (legacy) VKQ_LAUNCH_HYB(true, true) else VKQ_LAUNCH_HYB(true, false) }
+        else { if (legacy) VKQ_LAUNCH_HYB(false, true) else VKQ_LAUNCH_HYB(false, false) }
+    } else if (flat && flat->n) {
+        if (media) { if (legacy) VKQ_LAUNCH_FLAT((k_warpq_flat_media<true, D>), WqMedia) else VKQ_LAUNCH_FLAT((k_warpq_flat_media<false, D>), WqMedia) }
+        else { if (legacy) VKQ_LAUNCH_FLAT((k_warpq_flat<true, D>), WqFlat) else VKQ_LAUNCH_FLAT((k_warpq_flat<false, D>), WqFlat) }
+    } else {
+        if (media) { if (legacy) VKQ_LAUNCH_BVH((k_warpq<true, true, D>)) else VKQ_LAUNCH_BVH((k_warpq<true, false, D>)) }
+        else { if (legacy) VKQ_LAUNCH_BVH((k_warpq<false, true, D>)) else VKQ_LAUNCH_BVH((k_warpq<false, false, D>)) }
     }
-#endif
-    if (ls) { VKQ_DISPATCH(_list, , *ls) }
-    else if (fr) { VKQ_DISPATCH(_frames, , *fr) }
-    else { VKQ_DISPATCH(, ) }
-#undef VKQ_DISPATCH
 #undef VKQ_LAUNCH_HYB
+#endif
 #undef VKQ_LAUNCH_FLAT
 #undef VKQ_LAUNCH_BVH
     return cudaGetLastError();
 }
+#define VKQ_INSTANTIATE(D)                                                                                             \
+    template cudaError_t launch_warpq(const DScene&, const FlatProgram*, const DCamera&, const RenderArgs&, const RenderBuffers&, \
+                                      unsigned long long*, int, bool, cudaStream_t, const D&);
+VKQ_INSTANTIATE(OneFrame)
+VKQ_INSTANTIATE(FrameArgs)
+VKQ_INSTANTIATE(ListArgs)
+#undef VKQ_INSTANTIATE
 
 } // namespace VK_NS

@@ -103,22 +103,10 @@ VKD void wq_converge() {
     asm volatile("barrier.sync.aligned %0, 32;" ::"r"((threadIdx.x >> 5) + 1u) : "memory");
 #endif
 }
-// FR: a batch of frames (FrameArgs; separate instantiations, the single-frame code is untouched).  Its chunks are frame-major,
-// and the unit cursor's row is then the batch-wide row f * height + y.
-// LS: a pass over a list of active pixels (ListArgs); its chunks are VKQ_CHUNK consecutive list entries of one sample, and the
-// unit cursor's column is then a list index.  (Frame x list is not instantiated.)
-template <bool FR, bool LS = false>
-struct WqFrameRef {}; // (one frame: nothing, not even a null pointer -- the single-frame kernels stay as they were)
-template <>
-struct WqFrameRef<true, false> {
-    const FrameArgs* fr;
-};
-template <>
-struct WqFrameRef<false, true> {
-    const ListArgs* ls;
-};
-template <class W, bool FR = false, bool LS = false>
-struct WqCtx : WqFrameRef<FR, LS> {
+// (the work domain travels beside the context, as an argument of its own: as a reference member it changed the code of
+// the single-frame kernels, whose domain is empty)
+template <class W>
+struct WqCtx {
     const DCamera& cam;
     const RenderArgs& a;
     W& S;
@@ -127,6 +115,81 @@ struct WqCtx : WqFrameRef<FR, LS> {
     unsigned long long* unit_head;
     uint32_t lane, below;
 };
+
+// ---- the work domains' chunks (see vk_device.cuh) ---------------------------------------------------------------------
+// One frame: chunk c = (sample * height + row) * chunks_per_row + segment.  A batch: the same, frame-major, and the unit
+// cursor's row is then the batch-wide row f * height + y.  A list: VKQ_CHUNK consecutive entries of one sample (the list is
+// one row), and the cursor's column is then a list index.
+template <class D> VKD uint32_t wq_row_length(const D&, const RenderArgs& a) { return a.width; }
+VKD uint32_t wq_row_length(const ListArgs& ls, const RenderArgs&) { return ls.n; }
+template <class D> VKD uint32_t wq_rows(const D&, const RenderArgs& a) { return a.height; }
+VKD uint32_t wq_rows(const ListArgs&, const RenderArgs&) { return 1u; }
+template <class W, class D>
+VKD WqCtx<W> wq_ctx(const D& dom, const DCamera& cam, const RenderArgs& a, W& S, unsigned long long* unit_head, uint32_t lane) {
+    const uint32_t cpr = (wq_row_length(dom, a) + VKQ_CHUNK - 1u) / VKQ_CHUNK, cps = cpr * wq_rows(dom, a);
+    return WqCtx<W>{cam, a, S, cpr, cps, (unsigned long long)cps * a.spp_count * dom_frames(dom), unit_head, lane, (1u << lane) - 1u};
+}
+// chunk c -> the unit cursor of the warp (lane 0 only)
+template <class W>
+VKD void wq_chunk(const WqCtx<W>& C, const OneFrame&, unsigned long long c) {
+    W& S = C.S;
+    const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
+    const uint32_t r = (uint32_t)(c - (unsigned long long)sb * C.chunks_per_sample);
+    const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
+    S.left = min(VKQ_CHUNK, C.a.width - x0);
+    S.cur_s = sb;
+    S.cur_y = row;
+    S.cur_x = x0;
+}
+template <class W>
+VKD void wq_chunk(const WqCtx<W>& C, const FrameArgs&, unsigned long long c) {
+    // c = ((f * spp_count + sample) * height + row) * chunks_per_row + segment; f * spp_count + sample stays 64-bit until
+    // the frame is split off (it passes 2^32 long before the batch's pixel index does)
+    W& S = C.S;
+    const unsigned long long fs = c / C.chunks_per_sample;
+    const uint32_t f = (uint32_t)(fs / C.a.spp_count);
+    const uint32_t r = (uint32_t)(c - fs * C.chunks_per_sample);
+    const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
+    S.left = min(VKQ_CHUNK, C.a.width - x0);
+    S.cur_s = (uint32_t)(fs - (unsigned long long)f * C.a.spp_count);
+    S.cur_y = f * C.a.height + row;
+    S.cur_x = x0;
+}
+template <class W>
+VKD void wq_chunk(const WqCtx<W>& C, const ListArgs& ls, unsigned long long c) { // c = sample * chunks_per_sample + chunk of the list
+    W& S = C.S;
+    const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
+    const uint32_t x0 = ((uint32_t)c - sb * C.chunks_per_sample) * VKQ_CHUNK;
+    S.left = min(VKQ_CHUNK, ls.n - x0);
+    S.cur_s = sb;
+    S.cur_y = 0u;
+    S.cur_x = x0;
+}
+// The unit (x, y) of the cursor, rng.pixel = y * width + x: the camera ray of the pixel it stands for, with that pixel's
+// Philox counter pixel and key.  Returns the pixel the slot keeps: the accumulator index.
+template <class W>
+VKD uint32_t wq_camera_ray(const WqCtx<W>& C, const OneFrame&, uint32_t x, uint32_t y, PathRng& rng, float3& o, float3& d, float& time) {
+    camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
+    return rng.pixel;
+}
+template <class W>
+VKD uint32_t wq_camera_ray(const WqCtx<W>& C, const FrameArgs& fr, uint32_t x, uint32_t y, PathRng& rng, float3& o, float3& d, float& time) {
+    const uint32_t p = rng.pixel; // y is the batch-wide row, p the batch-wide pixel
+    const uint32_t f = y / C.a.height;
+    y -= f * C.a.height;
+    rng.pixel = y * C.a.width + x;
+    rng.key = frame_key(C.a, f);
+    camera_get_ray(fr.cams[f], rng, x, y, C.a.width, C.a.height, o, d, time);
+    return p;
+}
+template <class W>
+VKD uint32_t wq_camera_ray(const WqCtx<W>& C, const ListArgs& ls, uint32_t x, uint32_t y, PathRng& rng, float3& o, float3& d, float& time) {
+    rng.pixel = ls.list[x]; // x is a list index
+    y = rng.pixel / C.a.width;
+    x = rng.pixel - y * C.a.width;
+    camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
+    return rng.pixel;
+}
 
 // Append the lanes with cls != VKQ_NONE to the queue of their class: one match groups the lanes, the first
 // lane of each group moves that queue's counters (no other lane touches them: different groups, different queues).
@@ -151,8 +214,8 @@ VKD void wq_push(W& S, uint32_t cls, uint32_t slot, uint32_t lane, uint32_t belo
 // sample, so the lanes' units are (s, y, x0 + i) with nothing to wrap and nothing to divide; lane 0 splits the chunk
 // number into (sample, row, row segment) once per chunk.  Which warp renders which unit does not show in the image
 // (Philox is keyed by pixel and sample, the accumulators are integers).
-template <class W, bool FR, bool LS>
-VKD bool wq_regen(const WqCtx<W, FR, LS>& C, bool want, uint32_t slot) {
+template <class W, class D>
+VKD bool wq_regen(const WqCtx<W>& C, const D& dom, bool want, uint32_t slot) {
     W& S = C.S;
     const uint32_t m = __ballot_sync(0xFFFFFFFFu, want);
     if (m == 0u) return false;
@@ -170,33 +233,7 @@ VKD bool wq_regen(const WqCtx<W, FR, LS>& C, bool want, uint32_t slot) {
             if (C.lane == 0) {
                 const unsigned long long c = atomicAdd(C.unit_head, 1ull);
                 if (c >= C.n_chunks) S.exhausted = 1u;
-                else if constexpr (FR) {
-                    // c = ((f * spp_count + sample) * height + row) * chunks_per_row + segment; f * spp_count + sample stays
-                    // 64-bit until the frame is split off (it passes 2^32 long before the batch's pixel index does)
-                    const unsigned long long fs = c / C.chunks_per_sample;
-                    const uint32_t f = (uint32_t)(fs / C.a.spp_count);
-                    const uint32_t r = (uint32_t)(c - fs * C.chunks_per_sample);
-                    const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
-                    S.left = min(VKQ_CHUNK, C.a.width - x0);
-                    S.cur_s = (uint32_t)(fs - (unsigned long long)f * C.a.spp_count);
-                    S.cur_y = f * C.a.height + row;
-                    S.cur_x = x0;
-                } else if constexpr (LS) { // c = sample * chunks_per_sample + chunk of the list
-                    const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
-                    const uint32_t x0 = ((uint32_t)c - sb * C.chunks_per_sample) * VKQ_CHUNK;
-                    S.left = min(VKQ_CHUNK, C.ls->n - x0);
-                    S.cur_s = sb;
-                    S.cur_y = 0u;
-                    S.cur_x = x0;
-                } else {
-                    const uint32_t sb = (uint32_t)(c / C.chunks_per_sample);
-                    const uint32_t r = (uint32_t)(c - (unsigned long long)sb * C.chunks_per_sample);
-                    const uint32_t row = r / C.chunks_per_row, x0 = (r - row * C.chunks_per_row) * VKQ_CHUNK;
-                    S.left = min(VKQ_CHUNK, C.a.width - x0);
-                    S.cur_s = sb;
-                    S.cur_y = row;
-                    S.cur_x = x0;
-                }
+                else wq_chunk(C, dom, c);
             }
             __syncwarp();
             if (__any_sync(0xFFFFFFFFu, S.exhausted != 0u)) break;
@@ -219,56 +256,22 @@ VKD bool wq_regen(const WqCtx<W, FR, LS>& C, bool want, uint32_t slot) {
         served += take;
     }
     if (got) {
-        const uint32_t p = y * C.a.width + x; // i = y*width + x, row 0 = bottom (src/main.rs:182-183); FR: + f * n_pix
         PathRng rng;
-        rng.pixel = p;
+        rng.pixel = y * C.a.width + x; // i = y*width + x, row 0 = bottom (src/main.rs:182-183)
         rng.sample = C.a.spp_begin + s;
         rng.key = make_uint2(C.a.seed_lo, C.a.seed_hi);
         float3 o, d;
         float time;
-        if constexpr (FR) {
-            const uint32_t f = y / C.a.height;
-            y -= f * C.a.height;
-            rng.pixel = y * C.a.width + x;
-            rng.key = frame_key(C.a, f);
-            camera_get_ray(C.fr->cams[f], rng, x, y, C.a.width, C.a.height, o, d, time);
-        } else if constexpr (LS) { // x is a list index
-            rng.pixel = C.ls->list[x];
-            y = rng.pixel / C.a.width;
-            x = rng.pixel - y * C.a.width;
-            camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
-        } else {
-            camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
-        }
+        const uint32_t p = wq_camera_ray(C, dom, x, y, rng, o, d, time);
         S.ro[slot] = make_float4(o.x, o.y, o.z, time);
         S.rd[slot] = make_float4(d.x, d.y, d.z, __uint_as_float(1u)); // ray_color(ray, .., 1)
         S.bt[slot] = make_float4(1.0f, 1.0f, 1.0f, __uint_as_float(rng.sample));
-        S.px[slot] = LS ? rng.pixel : p;
+        S.px[slot] = p;
         S.mark_new(slot);
     }
     return got;
 }
 
-template <class W>
-VKD WqCtx<W> wq_ctx(const DCamera& cam, const RenderArgs& a, W& S, unsigned long long* unit_head, uint32_t lane) {
-    const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
-    return WqCtx<W>{{}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count, unit_head, lane, (1u << lane) - 1u};
-}
-// the context of a body instantiated for one frame (FR, LS false: wq_ctx, `fr` and `ls` unused), for a batch or for a list
-template <bool FR, bool LS = false, class W>
-VKD WqCtx<W, FR, LS> wq_ctx_fr(const DCamera& cam, const RenderArgs& a, const FrameArgs* fr, W& S, unsigned long long* unit_head, uint32_t lane,
-                               const ListArgs* ls = nullptr) {
-    if constexpr (LS) {
-        const uint32_t cps = (ls->n + VKQ_CHUNK - 1u) / VKQ_CHUNK;
-        return WqCtx<W, false, true>{{ls}, cam, a, S, cps, cps, (unsigned long long)cps * a.spp_count, unit_head, lane, (1u << lane) - 1u};
-    } else if constexpr (FR) {
-        const uint32_t cpr = (a.width + VKQ_CHUNK - 1u) / VKQ_CHUNK;
-        return WqCtx<W, true>{{fr}, cam, a, S, cpr, cpr * a.height, (unsigned long long)(cpr * a.height) * a.spp_count * fr->n_frames,
-                              unit_head, lane, (1u << lane) - 1u};
-    } else {
-        return wq_ctx(cam, a, S, unit_head, lane);
-    }
-}
 VKD bool wq_black_miss(const RenderArgs& a) {
     return !(a.flags & VK_FLAG_SKY_BACKGROUND) && a.background.x == 0.0f && a.background.y == 0.0f && a.background.z == 0.0f;
 }
@@ -341,8 +344,8 @@ VKD uint32_t wq_pop(W& S, uint32_t q, uint32_t n_q, uint32_t tail_q, uint32_t ca
 #ifndef VKQ_FAST_RESOLVE
 #define VKQ_FAST_RESOLVE 1 // (Cornell, 1000 spp: 37.9 against 40.0 ms per frame)
 #endif
-template <bool LEGACY, bool FLAT, class W, bool FR, bool LS>
-VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR, LS>& C, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
+template <bool LEGACY, bool FLAT, class W, class D>
+VKD void wq_shade_batch(const DScene& sc, const WqCtx<W>& C, const D& dom, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
     W& S = C.S;
     const RenderArgs& a = C.a;
     const uint32_t lane = C.lane;
@@ -365,7 +368,7 @@ VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR, LS>& C, const Rende
                 rng.pixel = pixel;
                 rng.sample = __float_as_uint(bt.w);
                 rng.key = make_uint2(a.seed_lo, a.seed_hi);
-                if constexpr (FR) frame_rng(rng, a, C.fr->n_pix, pixel); // (the slot's pixel is batch-wide, the accumulator index too)
+                dom_slot_rng(dom, a, rng); // (the slot's pixel is the accumulator index: batch-wide in a batch)
                 HitRecD rec;
                 bool direct = false;
                 uint32_t leaf = prim, hi = hp.z;
@@ -413,12 +416,8 @@ VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR, LS>& C, const Rende
                 S.bt[slot] = make_float4(beta.x, beta.y, beta.z, bt.w);
                 S.mark_new(slot);
             } else {
-                if (valid && finite3(L)) {
-                    accumulate_sample(buf, pixel, L);
-                    if constexpr (LS) accumulate_square(C.ls->sq, pixel, L);
-                } else {
-                    ++n_drop;
-                }
+                if (valid && finite3(L)) dom_accumulate(dom, buf, pixel, L);
+                else ++n_drop;
                 ended = true;
             }
         }
@@ -430,7 +429,7 @@ VKD void wq_shade_batch(const DScene& sc, const WqCtx<W, FR, LS>& C, const Rende
     // regenerated together, with full warps.
     const uint32_t m_end = __ballot_sync(0xFFFFFFFFu, ended);
     bool to_end = false;
-    if (q == VKQ_END || (uint32_t)__popc(m_end) >= VKQ_REGEN_MIN) alive = wq_regen(C, ended, slot) || alive;
+    if (q == VKQ_END || (uint32_t)__popc(m_end) >= VKQ_REGEN_MIN) alive = wq_regen(C, dom, ended, slot) || alive;
     else to_end = ended;
     // survivors (and regenerated samples) to the extend queue, queued regenerations to theirs: two ballots
     const uint32_t m_ext = __ballot_sync(0xFFFFFFFFu, alive), m_q = __ballot_sync(0xFFFFFFFFu, to_end);
