@@ -357,7 +357,8 @@ int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames,
  * out_rgb: the means sum / n_p in vk_render's layout; out_rgb8: to_color of the same means, top-down like vk_render_rgb8;
  * out_spp (nullable): n_p, W*H in the order of the image it accompanies.  stats: paths = sum of n_p; rays, dropped
  * samples, ms_kernels and launches are totals over all passes; variant is the kernel that ran.  Each pass costs one 4-byte
- * D2H of the active count and a stream synchronisation.  One frame on one device: no batches, no multi-GPU context.
+ * D2H of the active count and a stream synchronisation.  One frame on one device (a batch of frames:
+ * vk_render_frames_adaptive; no multi-GPU context).
  * Errors, before anything is launched: VK_ERR_INVALID for pass_spp == 0, max_error negative or NaN, spp_begin != 0,
  * spp_count not 0 or spp, spp > 65536, and every check of vk_render; VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED /
  * VK_VARIANT_WAVEFRONT; VK_ERR_NO_SCENE without a scene. */
@@ -367,6 +368,35 @@ int vk_render_adaptive(vk_ctx* ctx, const vk_camera* cam, const vk_render_params
 int vk_render_adaptive_rgb8(vk_ctx* ctx, const vk_camera* cam, const vk_render_params* params,
                             uint32_t pass_spp, float max_error,
                             uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats);
+
+/* Adaptive sampling of K cameras of one scene: vk_render_adaptive's passes and stopping rule over a batch, as
+ * vk_render_frames batches vk_render.  Frame f uses cams[f] and Philox key params->seed + f.  Pass k renders global samples
+ * [k*pass_spp, min((k+1)*pass_spp, spp)) of every pixel still active in ANY frame, in ONE launch over one list of the active
+ * pixels of all frames (the frames share the warps and one drain tail per pass); the rule is applied per pixel, unchanged,
+ * and a frame whose pixels have all stopped simply has no entries left.  The call ends when no pixel is active or spp is
+ * reached; each pass costs one 4-byte D2H and a stream synchronisation.
+ * Frame f's image AND counts equal, bit for bit, what vk_render_adaptive(_rgb8) returns for (cams[f], seed + f, pass_spp,
+ * max_error) ON THE SAME KERNEL (a pixel's decision depends on its own integer sums only).  The same-kernel caveat is
+ * vk_render_frames': VK_VARIANT_AUTO decides once, on the batch's pass-0 path count n_frames * W*H * min(pass_spp, spp), so a
+ * batch may run another kernel than its frames would one by one.  With VK_FLAG_STRICT_MATH the frames are equal whatever
+ * ran.  In the render build each compiled kernel contracts multiply-adds its own way and a batch runs kernels of its own, so
+ * there equality needs the same variant and is not bit for bit everywhere: the lane megakernel for flat scenes lit by one
+ * rect (Cornell box) gives the same counts but rounds some pixels differently.
+ * Like vk_render_adaptive's, the estimate is slightly BIASED: pixels that happen to look smooth stop early.
+ * out_rgb: n_frames planes of W*H*3 means, frame f at offset f * W*H*3, rows bottom-up (vk_render_frames' layout);
+ * out_rgb8: each frame top-down (vk_render_frames_rgb8's layout); out_spp (nullable): n_frames * W*H counts in the row order
+ * of the image they accompany.  stats: paths = sum of n_p over all frames; rays, dropped samples, ms_kernels and launches
+ * are totals over all passes; variant is the kernel that ran.  n_frames == 1 is vk_render_adaptive(_rgb8).
+ * Errors, before anything is launched: every error of vk_render_frames (n_frames == 0, a null pointer, a bad camera with
+ * the frame named, n_frames * W*H*3 >= 2^31, VK_ERR_OOM) and of vk_render_adaptive (pass_spp, max_error,
+ * spp_begin / spp_count, spp > 65536); VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED / VK_VARIANT_WAVEFRONT; VK_ERR_NO_SCENE
+ * without a scene. */
+int vk_render_frames_adaptive(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                              uint32_t pass_spp, float max_error,
+                              float* out_rgb, uint32_t* out_spp, vk_stats* stats);
+int vk_render_frames_adaptive_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                                   uint32_t pass_spp, float max_error,
+                                   uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats);
 
 /* Same loop, device-resident result: writes per-pixel SUMS (not means) of samples
  * [spp_begin, spp_begin+spp_count) to d_sum (and d_sumsq, nullable), both device

@@ -114,6 +114,12 @@ extern "C" {
                               out_rgb: *mut f32, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
     pub fn vk_render_adaptive_rgb8(ctx: *mut vk_ctx, cam: *const vk_camera, params: *const vk_render_params, pass_spp: u32,
                                    max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
+    // adaptive sampling of K cameras: every pass one launch over the active pixels of all frames; frame f (cams[f], seed + f)
+    // and its counts equal vk_render_adaptive of that camera (bit for bit with VK_FLAG_STRICT_MATH; the header states the render build)
+    pub fn vk_render_frames_adaptive(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                                     pass_spp: u32, max_error: f32, out_rgb: *mut f32, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
+    pub fn vk_render_frames_adaptive_rgb8(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                                          pass_spp: u32, max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
     // one context over several GPUs of the node (samples split by global index, peer-memory reduce on devices[0])
     pub fn vk_multi_create(devices: *const c_int, n_devices: c_int, out: *mut *mut vk_multi) -> c_int;
     pub fn vk_multi_destroy(m: *mut vk_multi);
@@ -319,6 +325,34 @@ impl Gpu {
         let mut n = vec![0u32; width * height];
         let mut st = vk_stats::default();
         self.check(unsafe { vk_render_adaptive_rgb8(self.ctx, cam, &p, pass_spp, max_error, out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
+    }
+    /// `render_adaptive` of K cameras, every pass one launch over the active pixels of all frames: frame f is
+    /// `render_adaptive(&cams[f], .., seed + f, ..)`, at offset f * W*H*3 of the means and f * W*H of the counts -- bit for
+    /// bit in the strict build; this (render) build may round some pixels differently (AUTO decides on the batch's pass-0 path count).
+    pub fn render_frames_adaptive(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                                  pass_spp: u32, max_error: f32) -> Result<(Vec<f32>, Vec<u32>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_frames_adaptive: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0f32; cams.len() * width * height * 3];
+        let mut n = vec![0u32; cams.len() * width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_frames_adaptive(self.ctx, cams.as_ptr(), cams.len() as u32, &p, pass_spp, max_error,
+                                                      out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
+    }
+    /// `render_frames_adaptive` with every frame as `render_adaptive_rgb8` returns it (image and counts top-down).
+    pub fn render_frames_adaptive_rgb8(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                                       pass_spp: u32, max_error: f32) -> Result<(Vec<u8>, Vec<u32>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_frames_adaptive_rgb8: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; cams.len() * width * height * 3];
+        let mut n = vec![0u32; cams.len() * width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_frames_adaptive_rgb8(self.ctx, cams.as_ptr(), cams.len() as u32, &p, pass_spp, max_error,
+                                                           out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
         Ok((out, n, st))
     }
     /// One spp slice [begin, begin+count) of the frame, already divided by the full `spp`: slices of disjoint

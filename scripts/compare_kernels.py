@@ -1,22 +1,26 @@
 #!/usr/bin/env python3
 """Kernel-by-kernel comparison of two builds of libvecchio_gpu.so (`make gpu` in each tree, no GPU needed).
 
-    python scripts/compare_kernels.py BASE_TREE HEAD_TREE
+    python scripts/compare_kernels.py BASE_TREE HEAD_TREE [--changed KERNEL ..]
 
 Reads each tree's vecchio_b200/csrc/ptxas_*.log (registers, stack frame, spill stores / loads) and the
 `cuobjdump -sass` of vecchio_b200/lib/libvecchio_gpu.so.  Kernels are matched by demangled name and template
-arguments, with the work domain (OneFrame / FrameArgs / ListArgs) as the last template argument; the older
+arguments, with the work domain (OneFrame / FrameArgs / ListArgs / FrameListArgs) as the last template argument; the older
 form of a domain kernel, `X_frames<a..>` / `X_list<a..>`, maps to `X<a.., FrameArgs>` / `X<a.., ListArgs>`,
 and any other kernel to itself with the domain OneFrame.  SASS verdicts:
     same          identical instructions
     local-slots   identical once the offsets of local loads / stores are masked (a different stack-slot assignment)
     same-ops      the same multiset of opcodes
     DIFF          anything else
-Exit status 0 when both builds have the same kernels, every kernel keeps its resources, every single-frame
-kernel is `same` and every other one `same` or `local-slots`."""
+A head kernel of a domain the base build has no kernel of at all is listed as NEW with its resources, beside those of
+its ListArgs twin (the same kernel over a pixel list of one frame) when the head build has one.
+Exit status 0 when every base kernel is in the head build and every head kernel either is in the base build or NEW,
+every matched kernel keeps its resources, every single-frame kernel is `same` and every other one `same` or
+`local-slots`.  A kernel named after --changed (its demangled name without namespace or arguments, e.g.
+k_to_color_adaptive) is one the change means to alter: it is listed with its verdict and does not fail the comparison."""
 import collections, glob, os, re, shutil, subprocess, sys
 
-DOMAINS = ("OneFrame", "FrameArgs", "ListArgs")
+DOMAINS = ("OneFrame", "FrameArgs", "ListArgs", "FrameListArgs")
 
 
 def demangle(names):
@@ -85,20 +89,32 @@ def verdict(a, b):
 
 
 def main():
-    if len(sys.argv) != 3:
+    args = sys.argv[1:]
+    if len(args) < 2 or (len(args) > 2 and args[2] != "--changed"):
         sys.exit(__doc__)
-    base, head = load(sys.argv[1]), load(sys.argv[2])
+    changed = set(args[3:])
+    base, head = load(args[0]), load(args[1])
     ok = True
-    for k in sorted(base.keys() - head.keys()) + sorted(head.keys() - base.keys()):
+    fmt = lambda r: "-" if r is None else f"{r['regs']}r {r['stack']}s {r['st']}/{r['ld']}"
+    base_domains = {d for _, d in base}
+    new = sorted(k for k in head.keys() - base.keys() if k[1] not in base_domains)
+    for k in sorted(base.keys() - head.keys()) + sorted(head.keys() - base.keys() - set(new)):
         print(f"UNMATCHED {'base' if k in base else 'head'}: {k[0]} [{k[1]}]")
         ok = False
     tally = collections.Counter()
-    fmt = lambda r: "-" if r is None else f"{r['regs']}r {r['stack']}s {r['st']}/{r['ld']}"
+    if new:
+        print(f"{'new kernel':<72} {'domain':<13} {'head':>16} {'ListArgs twin':>16}")
+    for k in new:
+        twin = head.get((k[0], "ListArgs"))
+        print(f"{k[0][:72]:<72} {k[1]:<13} {fmt(head[k][2]):>16} {fmt(twin[2]) if twin else '-':>16}  NEW")
+        tally[(k[1], "NEW")] += 1
     print(f"{'kernel':<72} {'domain':<9} {'base':>16} {'head':>16}  sass")
     for k in sorted(base.keys() & head.keys()):
         (_, ca, ra), (_, cb, rb) = base[k], head[k]
         v = verdict(ca, cb)
         bad = ra != rb or v in ("same-ops", "DIFF") or (k[1] == "OneFrame" and v != "same")
+        if bad and re.sub(r"<.*", "", k[0]).split("::")[-1] in changed:
+            v, bad = v + " (changed on purpose)", False
         ok &= not bad
         tally[(k[1], v)] += 1
         print(f"{k[0][:72]:<72} {k[1]:<9} {fmt(ra):>16} {fmt(rb):>16}  {v}{'  <--' if bad else ''}")

@@ -112,12 +112,17 @@ def gpu_lib():
                                          C.POINTER(_abi.vk_stats)]
         L.vk_render_adaptive_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), C.c_uint32, C.c_float, vp,
                                               vp, C.POINTER(_abi.vk_stats)]
+        L.vk_render_frames_adaptive.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32,
+                                                C.c_float, vp, vp, C.POINTER(_abi.vk_stats)]
+        L.vk_render_frames_adaptive_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32,
+                                                     C.c_float, vp, vp, C.POINTER(_abi.vk_stats)]
         for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
                   "vk_multi_render_frames_rgb8"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
                   "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
-                  "vk_render_frames", "vk_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8"):
+                  "vk_render_frames", "vk_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8",
+                  "vk_render_frames_adaptive", "vk_render_frames_adaptive_rgb8"):
             getattr(L, f).restype = C.c_int
         _gpu = L
     return _gpu
@@ -127,7 +132,8 @@ GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk
                "vk_finalize_device", "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks",
                "vk_device_info", "vk_multi_create", "vk_multi_destroy", "vk_multi_last_error", "vk_multi_device_count",
                "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8", "vk_render_frames", "vk_render_frames_rgb8",
-               "vk_multi_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8"]
+               "vk_multi_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8", "vk_render_frames_adaptive",
+               "vk_render_frames_adaptive_rgb8"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
                 "vkh_frame_filename", "vkh_last_error"]
@@ -356,6 +362,35 @@ class Context:
         self._check(self._L.vk_render_adaptive_rgb8(self._h, C.byref(cam), C.byref(params), int(pass_spp), float(max_error),
                                                     out.ctypes.data, spp.ctypes.data, C.byref(st)))
         return out.reshape(params.height, params.width, 3), spp.reshape(params.height, params.width), st
+
+    def render_frames_adaptive(self, cams, params, pass_spp, max_error):
+        """``vk_render_frames_adaptive``: render_adaptive over K cameras, every pass one launch over the active pixels of
+        all frames; frame f uses seed ``params.seed + f``.  Frame f's image and counts equal
+        ``render_adaptive(cams[f], params with seed + f, pass_spp, max_error)`` bit for bit with VK_FLAG_STRICT_MATH; AUTO decides
+        on the batch's pass-0 path count, and in the render build a batch kernel may round some pixels differently (the header).  Returns ((K, H, W, 3) float32 with row 0 = bottom,
+        (K, H, W) uint32 counts in the same order, stats of the batch)."""
+        _check_adaptive(pass_spp, max_error)
+        arr, k = _camera_array(cams)
+        n = k * params.width * params.height
+        rgb = np.empty(n * 3, dtype=np.float32)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_frames_adaptive(self._h, arr, k, C.byref(params), int(pass_spp), float(max_error),
+                                                      rgb.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return rgb.reshape(k, params.height, params.width, 3), spp.reshape(k, params.height, params.width), st
+
+    def render_frames_adaptive_rgb8(self, cams, params, pass_spp, max_error):
+        """``vk_render_frames_adaptive_rgb8``: render_frames_adaptive's frames as ``render_adaptive_rgb8`` returns each
+        (row 0 = top).  Returns ((K, H, W, 3) uint8, (K, H, W) uint32 counts with row 0 = top, stats of the batch)."""
+        _check_adaptive(pass_spp, max_error)
+        arr, k = _camera_array(cams)
+        n = k * params.width * params.height
+        out = np.empty(n * 3, dtype=np.uint8)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_render_frames_adaptive_rgb8(self._h, arr, k, C.byref(params), int(pass_spp), float(max_error),
+                                                           out.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return out.reshape(k, params.height, params.width, 3), spp.reshape(k, params.height, params.width), st
 
     def render_device(self, cam, params, d_sum_ptr, d_sumsq_ptr=None, want_stats=True):
         """``vk_render_device``: per-pixel SUMS of an spp slice into device memory.  With

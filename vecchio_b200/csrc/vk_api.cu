@@ -154,13 +154,15 @@ __global__ void k_finalize_adaptive(const unsigned long long* __restrict__ acc, 
     const float sum = (float)((double)(long long)acc[i] * VK_ACC_INV_SCALE);
     rgb[i] = sum / (float)nspp[i / 3];
 }
-// k_to_color of the same means, rows top-down; the counts follow the image's order
+// k_to_color of the same means over n_frames contiguous planes, each frame top-down on its own; the counts follow the
+// image's order
 __global__ void k_to_color_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, uint8_t* __restrict__ out,
-                                    uint32_t* __restrict__ spp_out, uint32_t width, uint32_t height) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, n = (size_t)width * height * 3;
-    if (i >= n) return;
-    const size_t row = i / ((size_t)width * 3), col = i - row * (size_t)width * 3;
-    const size_t j = (size_t)(height - 1 - row) * width * 3 + col;
+                                    uint32_t* __restrict__ spp_out, uint32_t width, uint32_t height, uint32_t n_frames) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, plane = (size_t)width * height * 3;
+    if (i >= plane * n_frames) return;
+    const size_t f = i / plane, k = i - f * plane;
+    const size_t row = k / ((size_t)width * 3), col = k - row * (size_t)width * 3;
+    const size_t j = f * plane + (size_t)(height - 1 - row) * width * 3 + col;
     const uint32_t np = nspp[j / 3];
     const float c = (float)((double)(long long)acc[j] * VK_ACC_INV_SCALE) / (float)np;
     float v = sqrtf(c);
@@ -668,10 +670,25 @@ static int plan_render(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, 
     return VK_OK;
 }
 
+// A batch's cameras go to the device with each launch over it (the kernels read them at regeneration only): c->cams.
+static int upload_cams(vk_ctx* c, const vk_camera* cams, uint32_t n_frames) {
+    if (c->cams_cap < n_frames) {
+        if (c->cams) cudaFree(c->cams);
+        c->cams = nullptr;
+        c->cams_cap = 0;
+        CU(c, cudaMalloc((void**)&c->cams, n_frames * sizeof(DCamera)));
+        c->cams_cap = n_frames;
+    }
+    c->cams_host.resize(n_frames);
+    for (uint32_t f = 0; f < n_frames; ++f) c->cams_host[f] = to_dcam(cams + f);
+    CU(c, cudaMemcpyAsync(c->cams, c->cams_host.data(), n_frames * sizeof(DCamera), cudaMemcpyHostToDevice, c->stream));
+    return VK_OK;
+}
+
 // One launch of the sample loop over global samples [spp_begin, spp_begin + count) into the accumulators of b (which the
 // caller has zeroed), on the kernel R names.  The work domain: n_frames > 1, cam points to n_frames cameras (FrameArgs);
-// ls != nullptr, only the listed pixels of one frame (ListArgs); otherwise one frame (OneFrame).  Adds the kernels it
-// launched to *launches.
+// ls != nullptr, only the listed pixels of one frame (ListArgs), or with n_frames > 1 of the batch (FrameListArgs: the
+// entries are batch-wide pixels); otherwise one frame (OneFrame).  Adds the kernels it launched to *launches.
 static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, const vk_render_params* P, uint32_t spp_begin, uint32_t count,
                        const RenderBuffers& b, uint32_t n_frames, const ListArgs* ls, uint32_t* launches) {
     const bool strict = R.strict, legacy = R.legacy, l0 = R.l0;
@@ -695,7 +712,8 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
     }
     // Lane megakernel: chunks of samples, sized for ~48 work items per resident warp (small items keep
     // the end-of-kernel tail short; an item costs one atomic).
-    const uint32_t n_tiles = a.tiles_x * a.tiles_y * n_frames; // (a batch: the items of all its frames share the warps)
+    // (a batch: the items of all its frames share the warps; a list across frames already spans them)
+    const uint32_t n_tiles = a.tiles_x * a.tiles_y * (ls ? 1u : n_frames);
     uint32_t n_chunks = (48u * R.resident_warps + n_tiles - 1) / n_tiles;
     if (n_chunks > count) n_chunks = count;
     if (n_chunks < 1) n_chunks = 1;
@@ -764,20 +782,11 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
         }
         return VK_OK;
     };
-    if (ls) return run(*ls);
-    if (n_frames == 1) return run(OneFrame{});
-    // a batch: its cameras go to the device with the call (read at regeneration only)
-    if (c->cams_cap < n_frames) {
-        if (c->cams) cudaFree(c->cams);
-        c->cams = nullptr;
-        c->cams_cap = 0;
-        CU(c, cudaMalloc((void**)&c->cams, n_frames * sizeof(DCamera)));
-        c->cams_cap = n_frames;
-    }
-    c->cams_host.resize(n_frames);
-    for (uint32_t f = 0; f < n_frames; ++f) c->cams_host[f] = to_dcam(cam + f);
-    CU(c, cudaMemcpyAsync(c->cams, c->cams_host.data(), n_frames * sizeof(DCamera), cudaMemcpyHostToDevice, c->stream));
-    return run(FrameArgs{c->cams, n_frames, P->width * P->height});
+    if (n_frames == 1) return ls ? run(*ls) : run(OneFrame{});
+    int rc = upload_cams(c, cam, n_frames);
+    if (rc != VK_OK) return rc;
+    const FrameArgs fr{c->cams, n_frames, P->width * P->height};
+    return ls ? run(FrameListArgs{fr, *ls}) : run(fr);
 }
 
 // shared body of vk_render / vk_render_device / vk_render_frames*
@@ -975,12 +984,16 @@ static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint
     return VK_OK;
 }
 
-// shared body of vk_render_adaptive / vk_render_adaptive_rgb8 (include/vecchio_gpu.h states the passes and the rule)
+// shared body of vk_render_adaptive* and vk_render_frames_adaptive* (include/vecchio_gpu.h states the passes and the rule).
+// n_frames > 1: cam points to n_frames cameras, every pass runs one launch over the active pixels of all frames (one list of
+// batch-wide pixels, FrameListArgs) and the result is n_frames contiguous planes.
 static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
-                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats, uint32_t n_frames = 1) {
     const std::string w(who);
     if (!cam || !P || (!out_rgb && !out_rgb8)) return fail(c, VK_ERR_INVALID, w + ": null argument");
-    int rc = check_render(c, cam, P);
+    int rc = n_frames > 1 ? check_frames(c, who, cam, n_frames, P) : VK_OK;
+    if (rc != VK_OK) return rc;
+    rc = check_render(c, cam, P);
     if (rc != VK_OK) return rc;
     if (pass_spp == 0) return fail(c, VK_ERR_INVALID, w + ": pass_spp must be >= 1");
     if (!(max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, w + ": max_error must be >= 0 (and not NaN)");
@@ -996,11 +1009,11 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
     vk_render_params Q = *P;
     Q.spp_count = pass_spp < P->spp ? pass_spp : P->spp;
     RenderPlan R;
-    if ((rc = plan_render(c, &Q, 1, &R)) != VK_OK) return rc;
+    if ((rc = plan_render(c, &Q, n_frames, &R)) != VK_OK) return rc;
     if (R.variant == VK_VARIANT_STAGED || R.variant == VK_VARIANT_WAVEFRONT)
         return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
 
-    const uint32_t n_pix = P->width * P->height;
+    const uint32_t n_pix = P->width * P->height * n_frames; // (all frames: a pixel index is batch-wide)
     const size_t plane = (size_t)n_pix * 3;
     // buffers: fixed-point sums (c->partial) | the adaptive block | the output staging (c->frame, pinned)
     if ((rc = ensure(c, &c->partial, &c->partial_floats, plane * 2)) != VK_OK) return rc;
@@ -1048,7 +1061,7 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
         const uint32_t cnt = P->spp - done < pass_spp ? P->spp - done : pass_spp;
         const ListArgs la{cur, n_active, sq};
         CU(c, cudaEventRecord(c->ev0, c->stream));
-        if ((rc = launch_pass(c, R, cam, P, done, cnt, b, 1, &la, &launches)) != VK_OK) return rc;
+        if ((rc = launch_pass(c, R, cam, P, done, cnt, b, n_frames, &la, &launches)) != VK_OK) return rc;
         paths += (uint64_t)n_active * cnt;
         done += cnt;
         k_adaptive_select<<<(n_active + 255) / 256, 256, 0, c->stream>>>(cur, n_active, b.acc, sq, done, P->spp, max_error, nspp, keep);
@@ -1077,7 +1090,7 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
         CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
         d_spp = nspp; // (vk_render's layout: the counts are already in pixel order)
     } else {
-        k_to_color_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, (uint8_t*)c->frame, d_spp, P->width, P->height);
+        k_to_color_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, (uint8_t*)c->frame, d_spp, P->width, P->height, n_frames);
         CU(c, cudaGetLastError());
         CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane, cudaMemcpyDeviceToHost, c->stream));
     }
@@ -1111,6 +1124,22 @@ int vk_render_adaptive_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_par
     if (!c) return VK_ERR_INVALID;
     if (!out_rgb8) return fail(c, VK_ERR_INVALID, "vk_render_adaptive_rgb8: null argument");
     return render_adaptive(c, "vk_render_adaptive_rgb8", cam, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats);
+}
+
+int vk_render_frames_adaptive(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                              float max_error, float* out_rgb, uint32_t* out_spp, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!cams || !P || !out_rgb || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_adaptive: null argument or no frames");
+    if (n_frames == 1) return vk_render_adaptive(c, cams, P, pass_spp, max_error, out_rgb, out_spp, stats);
+    return render_adaptive(c, "vk_render_frames_adaptive", cams, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats, n_frames);
+}
+
+int vk_render_frames_adaptive_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                                   float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!cams || !P || !out_rgb8 || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_adaptive_rgb8: null argument or no frames");
+    if (n_frames == 1) return vk_render_adaptive_rgb8(c, cams, P, pass_spp, max_error, out_rgb8, out_spp, stats);
+    return render_adaptive(c, "vk_render_frames_adaptive_rgb8", cams, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats, n_frames);
 }
 
 int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {

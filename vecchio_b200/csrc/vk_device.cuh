@@ -1749,8 +1749,10 @@ VKD uint32_t dom_frames(const FrameArgs& fr) { return fr.n_frames; }
 // the pixels a frame's units run over: W*H, or the list (a unit's "pixel" is then a list index, see dom_list_pixel)
 template <class D> VKD uint32_t dom_pixels(const D&, const RenderArgs& a) { return a.width * a.height; }
 VKD uint32_t dom_pixels(const ListArgs& ls, const RenderArgs&) { return ls.n; }
+VKD uint32_t dom_pixels(const FrameListArgs& fl, const RenderArgs&) { return fl.ls.n; }
 template <class D> VKD uint32_t dom_list_pixel(const D&, uint32_t i) { return i; }
 VKD uint32_t dom_list_pixel(const ListArgs& ls, uint32_t i) { return ls.list[i]; }
+VKD uint32_t dom_list_pixel(const FrameListArgs& fl, uint32_t i) { return fl.ls.list[i]; } // (batch-wide: see dom_unit_frame)
 // Frame-major units: u of `per` units per frame -> its frame, and u within that frame (one frame: 0, u unchanged)
 template <class D, class T> VKD uint32_t dom_split_frame(const D&, T&, T) { return 0u; }
 template <class T> VKD uint32_t dom_split_frame(const FrameArgs&, T& u, T per) {
@@ -1763,6 +1765,7 @@ template <class D> VKD uint32_t dom_plane(const D&, uint32_t) { return 0u; }
 VKD uint32_t dom_plane(const FrameArgs& fr, uint32_t f) { return f * fr.n_pix; }
 template <class D> VKD const DCamera& dom_camera(const D&, const DCamera& cam, uint32_t) { return cam; }
 VKD const DCamera& dom_camera(const FrameArgs& fr, const DCamera&, uint32_t f) { return fr.cams[f]; }
+VKD const DCamera& dom_camera(const FrameListArgs& fl, const DCamera&, uint32_t f) { return fl.fr.cams[f]; }
 template <class D> VKD void dom_frame_key(const D&, const RenderArgs&, uint32_t, PathRng&) {}
 VKD void dom_frame_key(const FrameArgs&, const RenderArgs& a, uint32_t f, PathRng& rng) { rng.key = frame_key(a, f); }
 // The pixel a warp-queue slot keeps (rng.pixel, the accumulator index: batch-wide in a batch) -> the Philox counter's
@@ -1773,12 +1776,24 @@ VKD void dom_slot_rng(const FrameArgs& fr, const RenderArgs& a, PathRng& rng) {
     rng.pixel = rng.pixel - f * fr.n_pix;
     rng.key = frame_key(a, f);
 }
+VKD void dom_slot_rng(const FrameListArgs& fl, const RenderArgs& a, PathRng& rng) { dom_slot_rng(fl.fr, a, rng); }
+// Only a list across frames has a frame per unit rather than per item (the lane megakernels ask this when a unit's
+// rng.pixel holds its list entry, the batch-wide pixel): rng.pixel becomes the frame's pixel, rng.key the frame's key, and
+// the frame is returned.  Its accumulator pixel is then plane + rng.pixel, its camera dom_camera(dom, cam, f).
+template <class D> struct dom_frame_per_unit { static constexpr bool value = false; };
+template <> struct dom_frame_per_unit<FrameListArgs> { static constexpr bool value = true; };
+VKD uint32_t dom_unit_frame(const FrameListArgs& fl, const RenderArgs& a, PathRng& rng) {
+    const uint32_t f = rng.pixel / fl.fr.n_pix;
+    dom_slot_rng(fl.fr, a, rng);
+    return f;
+}
 // a finished, finite sample into accumulator pixel `pixel`; an adaptive pass also keeps its squares
 template <class D> VKD void dom_accumulate(const D&, const RenderBuffers& buf, uint32_t pixel, float3 L) { accumulate_sample(buf, pixel, L); }
 VKD void dom_accumulate(const ListArgs& ls, const RenderBuffers& buf, uint32_t pixel, float3 L) {
     accumulate_sample(buf, pixel, L);
     accumulate_square(ls.sq, pixel, L);
 }
+VKD void dom_accumulate(const FrameListArgs& fl, const RenderBuffers& buf, uint32_t pixel, float3 L) { dom_accumulate(fl.ls, buf, pixel, L); }
 // Unit u of a lane-megakernel item: pixel (px0, py0) + (u & 7, u >> 3 & 3) of an 8x4 tile -> (px, py) and the frame pixel
 // index; false for a unit outside the image.  A list's "tile" is 32 consecutive entries, unit u takes entry u & 31.
 template <class D>
@@ -1796,6 +1811,17 @@ VKD bool mk_unit(const ListArgs& ls, const RenderArgs& a, uint32_t tile, uint32_
     pixel = ls.list[li];
     py = pixel / a.width;
     px = pixel - py * a.width;
+    return true;
+}
+// over a list across frames `pixel` is the batch-wide entry (the body resolves its frame with dom_unit_frame), (px, py) its frame's
+VKD bool mk_unit(const FrameListArgs& fl, const RenderArgs& a, uint32_t tile, uint32_t, uint32_t, uint32_t u, uint32_t& px, uint32_t& py,
+                 uint32_t& pixel) {
+    const uint32_t li = tile * 32u + (u & 31u);
+    if (!(li < fl.ls.n)) return false;
+    pixel = fl.ls.list[li];
+    const uint32_t p = pixel % fl.fr.n_pix;
+    py = p / a.width;
+    px = p - py * a.width;
     return true;
 }
 

@@ -195,6 +195,7 @@ struct RenderArgs {
 //   OneFrame   the W*H pixels of one frame (the single-frame kernels: the empty parameter adds nothing to their code)
 //   FrameArgs  a batch of frames
 //   ListArgs   a list of active pixels of one frame
+//   FrameListArgs  a list of active pixels across a batch of frames
 struct OneFrame {};
 
 // A batch of frames (vk_render_frames): frame f renders with cams[f] and Philox key seed + f (64-bit add) into the
@@ -217,6 +218,16 @@ struct ListArgs {
     const uint32_t* list;   // active pixels, ascending
     uint32_t n;             // list length
     unsigned long long* sq; // W*H*3 fixed-point sums of squares (VK_SQ_SCALE)
+};
+
+// A pass of an adaptive render of a batch of frames (vk_render_frames_adaptive): one list of active pixels across all the
+// frames.  An entry is the batch-wide pixel g = f * n_pix + y * width + x, ascending, so it is the index of the batch's
+// contiguous accumulator planes (and of the squares, ls.sq: n_frames * W*H*3) and what a warp-queue slot keeps in a batch.
+// Each unit resolves its own frame from g: the camera fr.cams[f], the key seed + f and the frame pixel g - f * n_pix, so every
+// frame equals its single-frame adaptive render.  The units run over the list alone (fr.n_frames does not multiply them).
+struct FrameListArgs {
+    FrameArgs fr;
+    ListArgs ls;
 };
 // Squares: VK_SQ_SCALE = 2^32 units per 1.0, each channel of a sample clamped to VK_SQ_CLAMP before it is squared (the clamp
 // touches the statistic only, never the image).  One sample adds at most 255^2 * 2^32 < 2^48 units, so VK_ADAPTIVE_MAX_SPP =
@@ -273,7 +284,7 @@ struct WfState {
     unsigned long long n_units;
 };
 
-// (the launchers that take a work domain D are instantiated for OneFrame, FrameArgs and ListArgs)
+// (the launchers that take a work domain D are instantiated for OneFrame, FrameArgs, ListArgs and FrameListArgs)
 #define VK_DECLARE_LAUNCHERS(NS)                                                                                       \
     namespace NS {                                                                                                     \
     template <class D>                                                                                                 \

@@ -33,7 +33,8 @@ namespace VK_NS {
 // A finished sample goes straight into its pixel's integer accumulators (accumulate_sample).
 // A batch of frames: item = frame x chunk x tile, frame outermost.  A list of pixels: a "tile" is 32 consecutive list
 // entries (the host sets tiles_x to their number, tiles_y to 1), unit u of an item is entry tile * 32 + (u & 31) x sample
-// c0 + (u >> 5).
+// c0 + (u >> 5).  A list across a batch of frames: the same, and each unit resolves its frame (camera, key, plane) from the
+// batch-wide entry it takes, since an item's 32 entries may belong to two frames.
 template <bool FLAT, bool MEDIA, bool LEGACY, class D>
 VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,
                          const RenderBuffers& buf, const D& dom) {
@@ -50,8 +51,8 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
         if (lane == 0) item = (uint32_t)atomicAdd(&buf.counters[2], 1ull);
         item = __shfl_sync(0xFFFFFFFFu, item, 0);
         if (item >= total) break;
-        const uint32_t f = dom_split_frame(dom, item, n_tiles * a.n_chunks); // frame of the item
-        const uint32_t pbase = dom_plane(dom, f);                            // its first pixel in the accumulators
+        uint32_t f = dom_split_frame(dom, item, n_tiles * a.n_chunks); // frame of the item (a list across frames: of the unit)
+        uint32_t pbase = dom_plane(dom, f);                            // its first pixel in the accumulators
         const uint32_t chunk = item / n_tiles, tile = item - chunk * n_tiles;
         const uint32_t px0 = (tile % a.tiles_x) * 8u, py0 = (tile / a.tiles_x) * 4u;
         const uint32_t c0 = a.spp_begin + chunk * a.chunk_spp;
@@ -83,6 +84,10 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
                     s_end = s + 1u;
                     rng.pixel = pixel;
                     has_unit = true;
+                    if constexpr (dom_frame_per_unit<D>::value) { // (an item's 32 entries may straddle a frame boundary)
+                        f = dom_unit_frame(dom, a, rng);
+                        pbase = f * dom.fr.n_pix;
+                    }
                 }
                 px = x;
                 py = y;
@@ -175,7 +180,7 @@ VKD void megakernel_body(const DScene& sc, const FlatProgram* flat, const DCamer
 #ifndef VK_DYN_NODE_STEPS
 #define VK_DYN_NODE_STEPS 4
 #endif
-// unit = frame x sample x pixel, frame outermost (a list of pixels: sample x list entry)
+// unit = frame x sample x pixel, frame outermost (a list of pixels: sample x list entry; across frames the entry names the frame)
 template <bool MEDIA, class D>
 VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
                              unsigned long long* unit_head, const D& dom) {
@@ -241,11 +246,15 @@ VKD void megakernel_dyn_body(const DScene& sc, const DCamera& cam, const RenderA
             if (need_unit) {
                 unsigned long long u = base + __popc(mu & lanes_below);
                 if (u < n_units) {
-                    const uint32_t f = dom_split_frame(dom, u, (unsigned long long)n_pixels * a.spp_count);
+                    uint32_t f = dom_split_frame(dom, u, (unsigned long long)n_pixels * a.spp_count);
                     pbase = f * n_pixels;
                     dom_frame_key(dom, a, f, rng);
                     const uint32_t sb = (uint32_t)(u / n_pixels);
                     rng.pixel = dom_list_pixel(dom, (uint32_t)(u - (unsigned long long)sb * n_pixels)); // i = y*width + x (src/main.rs:182-183)
+                    if constexpr (dom_frame_per_unit<D>::value) {
+                        f = dom_unit_frame(dom, a, rng);
+                        pbase = f * dom.fr.n_pix;
+                    }
                     rng.sample = a.spp_begin + sb;
                     camera_get_ray(dom_camera(dom, cam, f), rng, rng.pixel % a.width, rng.pixel / a.width, a.width, a.height, o, d, time);
                     beta = f3(1.0f, 1.0f, 1.0f);
@@ -469,6 +478,7 @@ cudaError_t launch_megakernel(const DScene& sc, const FlatProgram* flatp, const 
 VK_INSTANTIATE(OneFrame)
 VK_INSTANTIATE(FrameArgs)
 VK_INSTANTIATE(ListArgs)
+VK_INSTANTIATE(FrameListArgs)
 #undef VK_INSTANTIATE
 cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk_ray* rays, size_t n, const float* medium_xi,
                              vk_hit* out, cudaStream_t st) {

@@ -422,6 +422,7 @@ cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs&
 VKS_INSTANTIATE(OneFrame)
 VKS_INSTANTIATE(FrameArgs)
 VKS_INSTANTIATE(ListArgs)
+VKS_INSTANTIATE(FrameListArgs)
 #undef VKS_INSTANTIATE
 
 } // namespace VK_NS

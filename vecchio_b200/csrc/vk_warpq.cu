@@ -302,6 +302,7 @@ cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamer
 VKQ_INSTANTIATE(OneFrame)
 VKQ_INSTANTIATE(FrameArgs)
 VKQ_INSTANTIATE(ListArgs)
+VKQ_INSTANTIATE(FrameListArgs)
 #undef VKQ_INSTANTIATE
 
 } // namespace VK_NS

@@ -122,8 +122,10 @@ struct WqCtx {
 // one row), and the cursor's column is then a list index.
 template <class D> VKD uint32_t wq_row_length(const D&, const RenderArgs& a) { return a.width; }
 VKD uint32_t wq_row_length(const ListArgs& ls, const RenderArgs&) { return ls.n; }
+VKD uint32_t wq_row_length(const FrameListArgs& fl, const RenderArgs&) { return fl.ls.n; }
 template <class D> VKD uint32_t wq_rows(const D&, const RenderArgs& a) { return a.height; }
 VKD uint32_t wq_rows(const ListArgs&, const RenderArgs&) { return 1u; }
+VKD uint32_t wq_rows(const FrameListArgs&, const RenderArgs&) { return 1u; }
 template <class W, class D>
 VKD WqCtx<W> wq_ctx(const D& dom, const DCamera& cam, const RenderArgs& a, W& S, unsigned long long* unit_head, uint32_t lane) {
     const uint32_t cpr = (wq_row_length(dom, a) + VKQ_CHUNK - 1u) / VKQ_CHUNK, cps = cpr * wq_rows(dom, a);
@@ -165,6 +167,8 @@ VKD void wq_chunk(const WqCtx<W>& C, const ListArgs& ls, unsigned long long c) {
     S.cur_y = 0u;
     S.cur_x = x0;
 }
+template <class W>
+VKD void wq_chunk(const WqCtx<W>& C, const FrameListArgs& fl, unsigned long long c) { wq_chunk(C, fl.ls, c); } // (a list is a list)
 // The unit (x, y) of the cursor, rng.pixel = y * width + x: the camera ray of the pixel it stands for, with that pixel's
 // Philox counter pixel and key.  Returns the pixel the slot keeps: the accumulator index.
 template <class W>
@@ -189,6 +193,15 @@ VKD uint32_t wq_camera_ray(const WqCtx<W>& C, const ListArgs& ls, uint32_t x, ui
     x = rng.pixel - y * C.a.width;
     camera_get_ray(C.cam, rng, x, y, C.a.width, C.a.height, o, d, time);
     return rng.pixel;
+}
+template <class W>
+VKD uint32_t wq_camera_ray(const WqCtx<W>& C, const FrameListArgs& fl, uint32_t x, uint32_t, PathRng& rng, float3& o, float3& d, float& time) {
+    const uint32_t g = fl.ls.list[x]; // x is a list index, the entry a batch-wide pixel
+    rng.pixel = g;
+    const uint32_t f = dom_unit_frame(fl, C.a, rng);
+    const uint32_t y = rng.pixel / C.a.width;
+    camera_get_ray(fl.fr.cams[f], rng, rng.pixel - y * C.a.width, y, C.a.width, C.a.height, o, d, time);
+    return g;
 }
 
 // Append the lanes with cls != VKQ_NONE to the queue of their class: one match groups the lanes, the first
