@@ -398,6 +398,85 @@ int vk_render_frames_adaptive_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t 
                                    uint32_t pass_spp, float max_error,
                                    uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats);
 
+/* Adaptive render sessions: vk_render_frames_adaptive's passes and stopping rule, with the state kept between calls so a
+ * render can be tightened step by step (a preview at max_error 8 that becomes the final frame at 1 without repeating a
+ * sample), saved and resumed.  A session renders K >= 1 cameras of the context's scene: frame f uses cams[f] and Philox key
+ * params->seed + f, and every pass renders pass_spp = M samples (the last one up to the cap).  It is moved by targets: */
+typedef struct vk_adaptive_target {
+    uint32_t spp;     /* cap: no pixel renders more than spp samples                                */
+    uint32_t min_spp; /* floor: a pixel does not stop before n >= min_spp (the cap still wins)      */
+    float max_error;  /* the stopping rule's bound in 8-bit steps; 0 = never stop early            */
+} vk_adaptive_target;
+typedef struct vk_adaptive_session vk_adaptive_session;
+
+/* The rule, checked at pass boundaries only: a pixel at n samples stops when n == spp, or when n >= min_spp, n > 1 and the
+ * largest channel error e <= max_error (e as vk_render_adaptive states it).  With min_spp = 0 it is the one-shot calls'
+ * rule.  A pixel's count is therefore on the pass grid (a multiple of M) or equal to a cap.
+ * Tightening: a target T2 may follow the target T1 the session last reached only if
+ *     T2.max_error <= T1.max_error, where 0 is the tightest value (after 0 only 0 may follow);
+ *     T2.min_spp >= T1.min_spp;
+ *     T2.spp >= T1.spp, and T2.spp > T1.spp only when T1.spp is a multiple of M (pixels stopped at the old cap go on along
+ *     the pass grid);
+ *     T2.spp <= params->spp, the session's limit.
+ * A fresh session has reached no target and accepts any first target within its limit.
+ * Guarantee: after any sequence of tightening targets ending in T, the state (sums, squares, counts) is bit for bit the
+ * state of a fresh session refined once to T.  (A pixel that stopped at n1 under T1 went on at every earlier grid point b:
+ * b < T1.min_spp <= T2.min_spp or e(b) > T1.max_error >= T2.max_error, so a fresh T2 render also reaches n1 with the same
+ * integer sums; from n1 on both apply T2's rule to the same integers.)  A fresh session refined to {params->spp, 0, E}
+ * equals vk_render_adaptive(_rgb8) (K = 1) or vk_render_frames_adaptive(_rgb8) (K > 1) at max_error = E in image, counts and
+ * stats.paths, in both math builds: it runs the same kernels.
+ * Sessions borrow their context: destroy them before the context.  Other calls on the context (vk_render, the one-shot
+ * adaptive calls, other sessions) may run between a session's calls and do not touch its state.  No multi-GPU context.
+ * Errors are reported through vk_last_error of the context. */
+
+/* Begins a session: every check of vk_render_frames_adaptive (params->spp is the session's limit, <= 65536; spp_begin
+ * must be 0 and spp_count 0 or spp; pass_spp >= 1; VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED / VK_VARIANT_WAVEFRONT;
+ * VK_ERR_NO_SCENE without a scene), then the session's own device buffers (sums, squares, counts and pass lists for
+ * n_frames * W*H pixels, zeroed) and its kernel: VK_VARIANT_AUTO decides here, once, by the one-shot rule on
+ * n_frames * W*H * min(pass_spp, spp) paths.  The cameras and params are copied. */
+int vk_adaptive_begin(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                      uint32_t pass_spp, vk_adaptive_session** out);
+
+/* Renders until `target` is reached.  A pixel below the new cap that the new rule lets go on renders on from its count;
+ * the passes run level by level (a level is a count on the pass grid: 0, M, 2M, ..), each pass one launch over the pixels
+ * at that level, and a level without pixels costs nothing.  One small read-back per refine, plus one per pass as in the
+ * one-shot calls.  stats (nullable) are for this refine only: paths = samples added; rays, dropped samples, ms_kernels and
+ * launches as the one-shot calls count them.
+ * VK_ERR_INVALID, the state untouched: a null target; target.spp 0 or above the limit; max_error negative or NaN; a target
+ * that does not tighten the one reached (see above); the scene changed (re-uploaded) since the session began; an earlier
+ * refine or import that failed part way (the state is lost: read, export and refine refuse until a successful
+ * vk_adaptive_import replaces the whole state, e.g. from a checkpoint; otherwise only destroy is left). */
+int vk_adaptive_refine(vk_adaptive_session* session, const vk_adaptive_target* target, vk_stats* stats);
+
+/* The state's image, in the one-shot calls' layouts: vk_adaptive_read gives the means sum / n in vk_render_frames' layout
+ * (rows bottom-up), vk_adaptive_read_rgb8 to_color of them, each frame top-down.  out_spp (nullable): the counts and
+ * out_error (nullable): per pixel the largest channel e as the rule sees it, as float, +inf where n < 2; both
+ * n_frames * W*H in the row order of the image they accompany.  Reading does not change the state. */
+int vk_adaptive_read(vk_adaptive_session* session, float* out_rgb, uint32_t* out_spp, float* out_error);
+int vk_adaptive_read_rgb8(vk_adaptive_session* session, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error);
+
+/* The raw state, for checkpoints: sums (signed fixed point, 2^30 units per 1.0) and squares (unsigned fixed point, 2^32
+ * units per 1.0, each sample's channel clamped to 255 first), n_frames * W*H * 3 each, and counts,
+ * n_frames * W*H, all in the accumulators' order (frame by frame, rows bottom-up); reached (nullable) is the last target
+ * reached, all zero for a session that has reached none. */
+int vk_adaptive_export(vk_adaptive_session* session, int64_t* sums, uint64_t* squares, uint32_t* counts,
+                       vk_adaptive_target* reached);
+/* Replaces the state by exported arrays of a session with the same scene, cameras, params, pass_spp and kernel (the library
+ * cannot see those: the caller keeps them with the checkpoint).  VK_ERR_INVALID, the state untouched, unless reached.spp is
+ * within the limit, reached.max_error >= 0, and every count is <= reached.spp and on the grid (a multiple of pass_spp or
+ * reached.spp; a count of 0 with zero sums and squares).  reached.spp == 0 is a state that reached no target.  Because
+ * it replaces the whole state, a successful import is also how a session recovers after a refine or import that failed
+ * part way. */
+int vk_adaptive_import(vk_adaptive_session* session, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
+                       const vk_adaptive_target* reached);
+
+/* The kernel (VK_VARIANT_*) every pass of the session runs, fixed by vk_adaptive_begin: part of a checkpoint's identity,
+ * since the render build's kernels may round differently.  0 for a null session. */
+uint32_t vk_adaptive_variant(const vk_adaptive_session* session);
+
+/* Frees the session's buffers.  Before vk_destroy of its context. */
+void vk_adaptive_destroy(vk_adaptive_session* session);
+
 /* Same loop, device-resident result: writes per-pixel SUMS (not means) of samples
  * [spp_begin, spp_begin+spp_count) to d_sum (and d_sumsq, nullable), both device
  * pointers of W*H*3 floats, enqueued on the context stream; synchronised before return

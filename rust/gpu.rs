@@ -86,6 +86,9 @@ pub struct vk_render_params { pub width: u32, pub height: u32, pub spp: u32, pub
 pub struct vk_stats { pub paths: u64, pub rays: u64, pub dropped_samples: u64, pub ms_kernels: f32, pub ms_total: f32,
                       pub variant: u32, pub launches: u32, pub node_visits: u64, pub prim_tests: u64 }
 #[repr(C)] pub struct vk_ctx { _private: [u8; 0] }
+#[repr(C)] #[derive(Clone, Copy, Default, PartialEq)]
+pub struct vk_adaptive_target { pub spp: u32, pub min_spp: u32, pub max_error: f32 }
+#[repr(C)] pub struct vk_adaptive_session { _private: [u8; 0] }
 
 #[link(name = "vecchio_gpu")]
 extern "C" {
@@ -120,6 +123,19 @@ extern "C" {
                                      pass_spp: u32, max_error: f32, out_rgb: *mut f32, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
     pub fn vk_render_frames_adaptive_rgb8(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
                                           pass_spp: u32, max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
+    // adaptive sessions: the state of an adaptive render kept between calls, moved by tightening targets; each refine ends
+    // bit for bit where a fresh session refined once to that target would (the header states the rule and the refusals)
+    pub fn vk_adaptive_begin(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, pass_spp: u32,
+                             out: *mut *mut vk_adaptive_session) -> c_int;
+    pub fn vk_adaptive_refine(session: *mut vk_adaptive_session, target: *const vk_adaptive_target, stats: *mut vk_stats) -> c_int;
+    pub fn vk_adaptive_read(session: *mut vk_adaptive_session, out_rgb: *mut f32, out_spp: *mut u32, out_error: *mut f32) -> c_int;
+    pub fn vk_adaptive_read_rgb8(session: *mut vk_adaptive_session, out_rgb8: *mut u8, out_spp: *mut u32, out_error: *mut f32) -> c_int;
+    pub fn vk_adaptive_export(session: *mut vk_adaptive_session, sums: *mut i64, squares: *mut u64, counts: *mut u32,
+                              reached: *mut vk_adaptive_target) -> c_int;
+    pub fn vk_adaptive_import(session: *mut vk_adaptive_session, sums: *const i64, squares: *const u64, counts: *const u32,
+                              reached: *const vk_adaptive_target) -> c_int;
+    pub fn vk_adaptive_variant(session: *const vk_adaptive_session) -> u32;
+    pub fn vk_adaptive_destroy(session: *mut vk_adaptive_session);
     // one context over several GPUs of the node (samples split by global index, peer-memory reduce on devices[0])
     pub fn vk_multi_create(devices: *const c_int, n_devices: c_int, out: *mut *mut vk_multi) -> c_int;
     pub fn vk_multi_destroy(m: *mut vk_multi);
@@ -366,8 +382,58 @@ impl Gpu {
         self.check(unsafe { vk_render(self.ctx, cam, &p, out.as_mut_ptr(), std::ptr::null_mut(), &mut st) })?;
         Ok((out, st))
     }
+    /// An adaptive render whose state outlives a call (vk_adaptive_begin): `refine` tightens it step by step, each step
+    /// bit for bit a one-shot render at that target; `export` / `import` checkpoint it.  `spp` is the session's limit.
+    /// The session borrows the context, so it cannot outlive it.
+    pub fn adaptive_session(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                            pass_spp: u32) -> Result<AdaptiveSession<'_>, GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("adaptive_session: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut s = std::ptr::null_mut();
+        self.check(unsafe { vk_adaptive_begin(self.ctx, cams.as_ptr(), cams.len() as u32, &p, pass_spp, &mut s) })?;
+        Ok(AdaptiveSession { gpu: self, s, n_pix: cams.len() * width * height })
+    }
 }
 impl Drop for Gpu { fn drop(&mut self) { unsafe { vk_destroy(self.ctx) } } }
+
+/// A session of `Gpu::adaptive_session`; the lifetime ties it to its context.
+pub struct AdaptiveSession<'a> { gpu: &'a mut Gpu, s: *mut vk_adaptive_session, n_pix: usize }
+impl<'a> AdaptiveSession<'a> {
+    /// Renders until `target` is reached; an error (and an unchanged state) for one that does not tighten the last.
+    pub fn refine(&mut self, target: &vk_adaptive_target) -> Result<vk_stats, GpuError> {
+        let mut st = vk_stats::default();
+        self.gpu.check(unsafe { vk_adaptive_refine(self.s, target, &mut st) })?;
+        Ok(st)
+    }
+    /// Means (rows bottom-up), counts and each pixel's error as the rule sees it (+inf below two samples).
+    pub fn read(&mut self) -> Result<(Vec<f32>, Vec<u32>, Vec<f32>), GpuError> {
+        let (mut out, mut n, mut e) = (vec![0f32; self.n_pix * 3], vec![0u32; self.n_pix], vec![0f32; self.n_pix]);
+        self.gpu.check(unsafe { vk_adaptive_read(self.s, out.as_mut_ptr(), n.as_mut_ptr(), e.as_mut_ptr()) })?;
+        Ok((out, n, e))
+    }
+    /// `read` as the P3 file holds the image: to_color, rows top-down, counts and errors in the same order.
+    pub fn read_rgb8(&mut self) -> Result<(Vec<u8>, Vec<u32>, Vec<f32>), GpuError> {
+        let (mut out, mut n, mut e) = (vec![0u8; self.n_pix * 3], vec![0u32; self.n_pix], vec![0f32; self.n_pix]);
+        self.gpu.check(unsafe { vk_adaptive_read_rgb8(self.s, out.as_mut_ptr(), n.as_mut_ptr(), e.as_mut_ptr()) })?;
+        Ok((out, n, e))
+    }
+    /// The raw state: fixed-point sums and squares (3 per pixel), counts, and the target reached.
+    pub fn export(&mut self) -> Result<(Vec<i64>, Vec<u64>, Vec<u32>, vk_adaptive_target), GpuError> {
+        let (mut sums, mut sq, mut n) = (vec![0i64; self.n_pix * 3], vec![0u64; self.n_pix * 3], vec![0u32; self.n_pix]);
+        let mut t = vk_adaptive_target::default();
+        self.gpu.check(unsafe { vk_adaptive_export(self.s, sums.as_mut_ptr(), sq.as_mut_ptr(), n.as_mut_ptr(), &mut t) })?;
+        Ok((sums, sq, n, t))
+    }
+    /// Replaces the state by an exported one of a session with the same scene, cameras, params and pass_spp.
+    pub fn import(&mut self, sums: &[i64], squares: &[u64], counts: &[u32], reached: &vk_adaptive_target) -> Result<(), GpuError> {
+        if sums.len() != self.n_pix * 3 || squares.len() != self.n_pix * 3 || counts.len() != self.n_pix {
+            return Err(GpuError::Unsupported("AdaptiveSession::import: array lengths do not match the session"));
+        }
+        self.gpu.check(unsafe { vk_adaptive_import(self.s, sums.as_ptr(), squares.as_ptr(), counts.as_ptr(), reached) })
+    }
+}
+impl<'a> Drop for AdaptiveSession<'a> { fn drop(&mut self) { unsafe { vk_adaptive_destroy(self.s) } } }
 // A context is used by one thread at a time and owns its device: it may move between threads.
 unsafe impl Send for Gpu {}
 

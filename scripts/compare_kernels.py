@@ -17,7 +17,8 @@ its ListArgs twin (the same kernel over a pixel list of one frame) when the head
 Exit status 0 when every base kernel is in the head build and every head kernel either is in the base build or NEW,
 every matched kernel keeps its resources, every single-frame kernel is `same` and every other one `same` or
 `local-slots`.  A kernel named after --changed (its demangled name without namespace or arguments, e.g.
-k_to_color_adaptive) is one the change means to alter: it is listed with its verdict and does not fail the comparison."""
+k_to_color_adaptive) is one the change means to alter or add: it is listed with its verdict, or as NEW when the base build
+lacks it, and does not fail the comparison."""
 import collections, glob, os, re, shutil, subprocess, sys
 
 DOMAINS = ("OneFrame", "FrameArgs", "ListArgs", "FrameListArgs")
@@ -97,7 +98,8 @@ def main():
     ok = True
     fmt = lambda r: "-" if r is None else f"{r['regs']}r {r['stack']}s {r['st']}/{r['ld']}"
     base_domains = {d for _, d in base}
-    new = sorted(k for k in head.keys() - base.keys() if k[1] not in base_domains)
+    short = lambda k: re.sub(r"<.*", "", k[0]).split("::")[-1]
+    new = sorted(k for k in head.keys() - base.keys() if k[1] not in base_domains or short(k) in changed)
     for k in sorted(base.keys() - head.keys()) + sorted(head.keys() - base.keys() - set(new)):
         print(f"UNMATCHED {'base' if k in base else 'head'}: {k[0]} [{k[1]}]")
         ok = False
@@ -113,7 +115,7 @@ def main():
         (_, ca, ra), (_, cb, rb) = base[k], head[k]
         v = verdict(ca, cb)
         bad = ra != rb or v in ("same-ops", "DIFF") or (k[1] == "OneFrame" and v != "same")
-        if bad and re.sub(r"<.*", "", k[0]).split("::")[-1] in changed:
+        if bad and short(k) in changed:
             v, bad = v + " (changed on purpose)", False
         ok &= not bad
         tally[(k[1], v)] += 1

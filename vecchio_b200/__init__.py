@@ -9,6 +9,7 @@ There is no CPU fallback: :class:`Context` raises if the CUDA library is missing
 """
 import ctypes as C
 import os
+import weakref
 
 import numpy as np
 
@@ -116,13 +117,25 @@ def gpu_lib():
                                                 C.c_float, vp, vp, C.POINTER(_abi.vk_stats)]
         L.vk_render_frames_adaptive_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32,
                                                      C.c_float, vp, vp, C.POINTER(_abi.vk_stats)]
+        L.vk_adaptive_begin.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32,
+                                        C.POINTER(vp)]
+        L.vk_adaptive_refine.argtypes = [vp, C.POINTER(_abi.vk_adaptive_target), C.POINTER(_abi.vk_stats)]
+        L.vk_adaptive_read.argtypes = [vp, vp, vp, vp]
+        L.vk_adaptive_read_rgb8.argtypes = [vp, vp, vp, vp]
+        L.vk_adaptive_export.argtypes = [vp, vp, vp, vp, C.POINTER(_abi.vk_adaptive_target)]
+        L.vk_adaptive_import.argtypes = [vp, vp, vp, vp, C.POINTER(_abi.vk_adaptive_target)]
+        L.vk_adaptive_variant.argtypes = [vp]
+        L.vk_adaptive_variant.restype = C.c_uint32
+        L.vk_adaptive_destroy.argtypes = [vp]
+        L.vk_adaptive_destroy.restype = None
         for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
                   "vk_multi_render_frames_rgb8"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
                   "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
                   "vk_render_frames", "vk_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8",
-                  "vk_render_frames_adaptive", "vk_render_frames_adaptive_rgb8"):
+                  "vk_render_frames_adaptive", "vk_render_frames_adaptive_rgb8", "vk_adaptive_begin", "vk_adaptive_refine",
+                  "vk_adaptive_read", "vk_adaptive_read_rgb8", "vk_adaptive_export", "vk_adaptive_import"):
             getattr(L, f).restype = C.c_int
         _gpu = L
     return _gpu
@@ -133,7 +146,8 @@ GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk
                "vk_device_info", "vk_multi_create", "vk_multi_destroy", "vk_multi_last_error", "vk_multi_device_count",
                "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8", "vk_render_frames", "vk_render_frames_rgb8",
                "vk_multi_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8", "vk_render_frames_adaptive",
-               "vk_render_frames_adaptive_rgb8"]
+               "vk_render_frames_adaptive_rgb8", "vk_adaptive_begin", "vk_adaptive_refine", "vk_adaptive_read", "vk_adaptive_read_rgb8",
+               "vk_adaptive_export", "vk_adaptive_import", "vk_adaptive_variant", "vk_adaptive_destroy"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
                 "vkh_frame_filename", "vkh_last_error"]
@@ -278,6 +292,170 @@ def _check_adaptive(pass_spp, max_error):
         raise ValueError("render_adaptive: max_error must be >= 0 (and not NaN)")
 
 
+ADAPTIVE_MAX_SPP = 65536  # the limit of the fixed-point sums of squares (include/vecchio_gpu.h)
+
+
+def _adaptive_target(max_error, spp, min_spp):
+    """A session target as (spp, min_spp, max_error), max_error as the library holds it (float32); bad values are
+    refused here, before the library is called."""
+    if int(spp) < 1:
+        raise ValueError("adaptive target: spp must be >= 1")
+    if int(min_spp) < 0:
+        raise ValueError("adaptive target: min_spp must be >= 0")
+    if not float(max_error) >= 0.0:  # (NaN fails the comparison)
+        raise ValueError("adaptive target: max_error must be >= 0 (and not NaN)")
+    return int(spp), int(min_spp), float(np.float32(max_error))
+
+
+def _check_tightens(reached, target, limit, pass_spp):
+    """What vk_adaptive_refine refuses of a target after ``reached`` (None: a fresh session), refused here first:
+    the target must lie within the session's limit and tighten what was reached (include/vecchio_gpu.h)."""
+    spp, min_spp, max_error = target
+    if spp > limit:
+        raise ValueError(f"adaptive target: spp {spp} exceeds the session's limit params.spp = {limit}")
+    if reached is None:
+        return
+    r_spp, r_min, r_err = reached
+    if (max_error != 0.0) if r_err == 0.0 else (max_error != 0.0 and max_error > r_err):
+        raise ValueError(f"adaptive target: max_error {max_error} loosens {r_err} (0 is the tightest: after 0 only 0 may follow)")
+    if min_spp < r_min:
+        raise ValueError(f"adaptive target: min_spp {min_spp} is below the {r_min} already reached (it may only rise)")
+    if spp < r_spp:
+        raise ValueError(f"adaptive target: spp {spp} is below the {r_spp} already reached (it may only rise)")
+    if spp > r_spp and r_spp % pass_spp:
+        raise ValueError(f"adaptive target: spp may rise only from a cap on the pass grid; {r_spp} is not a multiple of pass_spp = {pass_spp}")
+
+
+class AdaptiveSession:
+    """``vk_adaptive_begin`` .. ``vk_adaptive_destroy``: an adaptive render whose state outlives a call.  ``refine`` moves
+    it to tighter targets, each step ending bit for bit where a fresh session refined once to that target would; a fresh
+    session refined to ``(max_error, params.spp)`` is ``render_adaptive`` / ``render_frames_adaptive``.  One camera gives
+    (H, W) shapes, a list of K cameras (K, H, W).  Made by ``Context.adaptive_session``; keeps its context alive."""
+
+    def __init__(self, ctx, cams, params, pass_spp):
+        if int(pass_spp) < 1:
+            raise ValueError("adaptive_session: pass_spp must be >= 1")
+        self.single = isinstance(cams, _abi.vk_camera)
+        cams = [cams] if self.single else list(cams)
+        if not cams:
+            raise ValueError("adaptive_session: at least one camera")
+        arr, k = _camera_array(cams)
+        self._h = None
+        h = C.c_void_p()
+        ctx._check(ctx._L.vk_adaptive_begin(ctx._h, arr, k, C.byref(params), int(pass_spp), C.byref(h)))
+        self._ctx, self._L, self._h = ctx, ctx._L, h
+        ctx._sessions.add(self)
+        self.cams = [_abi.vk_camera.from_buffer_copy(c) for c in cams]
+        self.params = _abi.vk_render_params.from_buffer_copy(params)
+        self.pass_spp, self.n_frames = int(pass_spp), k
+        self.variant = int(self._L.vk_adaptive_variant(h))
+        self.reached = None  # the last target reached, (spp, min_spp, max_error)
+
+    def _check(self, rc):
+        self._ctx._check(rc)
+
+    def _shape(self):
+        hw = (self.params.height, self.params.width)
+        return hw if self.single else (self.n_frames,) + hw
+
+    def target(self, max_error, spp=None, min_spp=0):
+        """The target (spp, min_spp, max_error) refine would move to; spp None = the session's limit."""
+        return _adaptive_target(max_error, self.params.spp if spp is None else spp, min_spp)
+
+    def refine(self, max_error, spp=None, min_spp=0):
+        """``vk_adaptive_refine``: render until every pixel meets the target; returns this refine's stats (paths =
+        samples added).  A target that loosens the one reached, or bad values, raise ValueError before the library."""
+        t = self.target(max_error, spp, min_spp)
+        _check_tightens(self.reached, t, self.params.spp, self.pass_spp)
+        T = _abi.vk_adaptive_target(*t)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_adaptive_refine(self._h, C.byref(T), C.byref(st)))
+        self.reached = t
+        return st
+
+    def _read(self, fn, dtype):
+        shape = self._shape()
+        n = int(np.prod(shape))
+        img = np.empty(n * 3, dtype=dtype)
+        cnt = np.empty(n, dtype=np.uint32)
+        err = np.empty(n, dtype=np.float32)
+        self._check(fn(self._h, img.ctypes.data, cnt.ctypes.data, err.ctypes.data))
+        return img.reshape(shape + (3,)), cnt.reshape(shape), err.reshape(shape)
+
+    def read(self):
+        """``vk_adaptive_read``: (means float32 with row 0 = bottom, counts, error map) in ``render_adaptive``'s layout;
+        the error map is the largest channel error the rule sees, +inf below two samples."""
+        return self._read(self._L.vk_adaptive_read, np.float32)
+
+    def read_rgb8(self):
+        """``vk_adaptive_read_rgb8``: read()'s image through to_color with row 0 = top, counts and errors in that order."""
+        return self._read(self._L.vk_adaptive_read_rgb8, np.uint8)
+
+    def export(self):
+        """``vk_adaptive_export``: (sums int64, squares uint64, both shape + (3,), counts uint32, reached), the raw
+        fixed-point state in the accumulators' order (rows bottom-up)."""
+        shape = self._shape()
+        sums = np.empty(shape + (3,), dtype=np.int64)
+        squares = np.empty(shape + (3,), dtype=np.uint64)
+        counts = np.empty(shape, dtype=np.uint32)
+        T = _abi.vk_adaptive_target()
+        self._check(self._L.vk_adaptive_export(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
+        return sums, squares, counts, (None if T.spp == 0 else (int(T.spp), int(T.min_spp), float(T.max_error)))
+
+    def import_(self, sums, squares, counts, reached):
+        """``vk_adaptive_import``: replace the state by an exported one (``reached`` None: a state that reached no
+        target).  The library refuses counts off the pass grid or above the cap reached."""
+        shape = self._shape()
+        sums = np.ascontiguousarray(sums, dtype=np.int64)
+        squares = np.ascontiguousarray(squares, dtype=np.uint64)
+        counts = np.ascontiguousarray(counts, dtype=np.uint32)
+        if sums.shape != shape + (3,) or squares.shape != shape + (3,) or counts.shape != shape:
+            raise ValueError(f"import_: the session's shape is {shape}, the state's {counts.shape}")
+        r = (0, 0, 0.0) if reached is None else _adaptive_target(reached[2], reached[0], reached[1])
+        T = _abi.vk_adaptive_target(*r)
+        self._check(self._L.vk_adaptive_import(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
+        self.reached = None if reached is None else r
+
+    def key(self, scene_name, scene_seed, scene_param=0):
+        """The identity a checkpoint of this session carries (``adaptive_checkpoint.session_key``)."""
+        from .adaptive_checkpoint import session_key
+        return session_key(scene_name, scene_seed, self.cams, self.params, self.pass_spp, self.variant, scene_param)
+
+    def _own_key(self, key):
+        """``key`` if it is this session's identity (its scene fields with the session's own cameras, params, pass_spp
+        and kernel); ValueError otherwise, so that a state is never saved under, or loaded into, another session."""
+        key = dict(key)
+        own = self.key(key.get("scene"), key.get("scene_seed", 0), key.get("scene_param", 0))
+        diff = sorted(k for k in set(own) | set(key) if own.get(k) != key.get(k))
+        if diff:
+            raise ValueError(f"the key is not this session's identity (differs in {', '.join(diff)})")
+        return own
+
+    def save(self, path, key):
+        """The exported state and ``key`` (this session's identity, ``key()``) in one ``.npz``, written by
+        write-and-rename."""
+        from .adaptive_checkpoint import save_state
+        save_state(path, self._own_key(key), *self.export())
+
+    def load(self, path, key):
+        """Imports a checkpoint written for ``key``.  ValueError, before the library is called, when ``key`` is not
+        this session's own identity (other cameras, params, pass_spp or kernel) or the file's identity differs."""
+        from .adaptive_checkpoint import load_state
+        self.import_(*load_state(path, self._own_key(key)))
+
+    def close(self):
+        if getattr(self, "_h", None):
+            self._L.vk_adaptive_destroy(self._h)
+            self._h = None
+            self._ctx._sessions.discard(self)
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Context:
     """One GPU context (``vk_create``).  Fails loudly without the CUDA library or a device."""
 
@@ -290,10 +468,16 @@ class Context:
         self._h = h
         self._L = L
         self.device = device
+        self._sessions = weakref.WeakSet()
 
     def _check(self, rc):
         if rc != 0:
             raise VecchioError(rc, (self._L.vk_last_error(self._h) or b"").decode())
+
+    def adaptive_session(self, cams, params, pass_spp):
+        """``vk_adaptive_begin``: an :class:`AdaptiveSession` over one camera ((H, W) shapes) or a list of K
+        ((K, H, W)); frame f uses seed ``params.seed + f`` and ``params.spp`` is the session's limit."""
+        return AdaptiveSession(self, cams, params, pass_spp)
 
     def upload(self, scene):
         self._check(self._L.vk_scene_upload(self._h, scene.desc_ptr))
@@ -442,6 +626,8 @@ class Context:
 
     def close(self):
         if getattr(self, "_h", None):
+            for s in list(getattr(self, "_sessions", ())):  # (sessions borrow the context: they go first)
+                s.close()
             self._L.vk_destroy(self._h)
             self._h = None
 

@@ -140,3 +140,7 @@ EVAL_DTYPE = _np.dtype([("op", "<u4"), ("index", "<u4"), ("ray_o", "<f4", 3), ("
                         ("alive", "<u4"), ("valid", "<u4"), ("out_o", "<f4", 3), ("out_d", "<f4", 3), ("out_time", "<f4"),
                         ("beta", "<f4", 3), ("L", "<f4", 3), ("value", "<f4")])
 assert RAY_DTYPE.itemsize == 36 and HIT_DTYPE.itemsize == 56 and EVAL_DTYPE.itemsize == 43 * 4
+
+
+class vk_adaptive_target(C.Structure):
+    _fields_ = [("spp", C.c_uint32), ("min_spp", C.c_uint32), ("max_error", C.c_float)]

@@ -9,6 +9,7 @@
 #include <vector>
 
 #include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 #include "vk_internal.h"
 #include "vk_relayout.h"
@@ -57,8 +58,8 @@ struct vk_ctx {
     DCamera* cams = nullptr; // vk_render_frames: the batch's cameras on the device (FrameArgs::cams)
     size_t cams_cap = 0;
     std::vector<DCamera> cams_host;
-    void* adapt = nullptr; // vk_render_adaptive: squares | per-pixel counts | two pixel lists | flags | count | compaction scratch
-    size_t adapt_bytes = 0;
+    vk_adaptive_session* oneshot = nullptr; // vk_render_adaptive*: the session each call begins, refines once and reads
+    uint64_t scene_gen = 0;                 // scene uploads so far: a session refines only on the scene it began with
     // wavefront variant: the slot pool (allocated on first use) and a pinned word block for the
     // host's termination checks
     WfState wf{};
@@ -67,6 +68,9 @@ struct vk_ctx {
 };
 
 static thread_local std::string g_create_err;
+extern "C" {
+static void adaptive_free(vk_adaptive_session* s); // (defined with the sessions, in the C ABI's block)
+}
 
 static int fail(vk_ctx* c, int code, const std::string& msg) {
     if (c) c->err = msg;
@@ -123,28 +127,68 @@ __global__ void k_iota(uint32_t* list, uint32_t n) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) list[i] = i;
 }
-// The stopping rule of vk_render_adaptive (include/vecchio_gpu.h) for every listed pixel after a pass that brought it to
-// n_done samples: records n_done as its count, keep[i] = 1 when it renders on.  Computed from the integer sums alone, so
-// the decision does not depend on the order the samples arrived in.
+// The largest channel error e of pixel p after n >= 2 samples (include/vecchio_gpu.h states it), from the integer sums
+// alone, so that it does not depend on the order the samples arrived in.
+__device__ __forceinline__ double adaptive_error(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
+                                                 uint32_t p, uint32_t n) {
+    double e = 0.0;
+    for (uint32_t ch = 0; ch < 3u; ++ch) {
+        const double m = (double)(long long)acc[3u * p + ch] * VK_ACC_INV_SCALE / n;
+        const double q = (double)sq[3u * p + ch] * VK_SQ_INV_SCALE / n;
+        const double se = sqrt(fmax(q - m * m, 0.0) / (double)(n - 1u));
+        e = fmax(e, 128.0 * (sqrt(fmax(m + se, 0.0)) - sqrt(fmax(m - se, 0.0))));
+    }
+    return e;
+}
+// The stopping rule, the one place it is written: a pixel at n samples stops at the cap spp, or once n >= min_spp, n > 1
+// (one sample has no standard error) and e <= max_error; max_error == 0 never stops early.
+__device__ __forceinline__ bool adaptive_stop(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
+                                              uint32_t p, uint32_t n, uint32_t spp, uint32_t min_spp, float max_error) {
+    bool stop = n >= spp;
+    if (!stop && max_error > 0.0f && n > 1u && n >= min_spp) stop = adaptive_error(acc, sq, p, n) <= (double)max_error;
+    return stop;
+}
+// The rule for every listed pixel after a pass that brought it to n_done samples: records n_done as its count,
+// keep[i] = 1 when it renders on.
 __global__ void k_adaptive_select(const uint32_t* __restrict__ list, uint32_t n, const unsigned long long* __restrict__ acc,
-                                  const unsigned long long* __restrict__ sq, uint32_t n_done, uint32_t spp, float max_error,
-                                  uint32_t* __restrict__ nspp, uint8_t* __restrict__ keep) {
+                                  const unsigned long long* __restrict__ sq, uint32_t n_done, uint32_t spp, uint32_t min_spp,
+                                  float max_error, uint32_t* __restrict__ nspp, uint8_t* __restrict__ keep) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const uint32_t p = list[i];
     nspp[p] = n_done;
-    bool stop = n_done >= spp;
-    if (!stop && max_error > 0.0f && n_done > 1u) { // (one sample has no standard error)
-        double e = 0.0;
-        for (uint32_t ch = 0; ch < 3u; ++ch) {
-            const double m = (double)(long long)acc[3u * p + ch] * VK_ACC_INV_SCALE / n_done;
-            const double q = (double)sq[3u * p + ch] * VK_SQ_INV_SCALE / n_done;
-            const double se = sqrt(fmax(q - m * m, 0.0) / (double)(n_done - 1u));
-            e = fmax(e, 128.0 * (sqrt(fmax(m + se, 0.0)) - sqrt(fmax(m - se, 0.0))));
-        }
-        stop = e <= (double)max_error;
+    keep[i] = adaptive_stop(acc, sq, p, n_done, spp, min_spp, max_error) ? 0u : 1u;
+}
+// A refine of a session that already holds samples: the rule of the new target for every pixel below its cap.  level[p] =
+// n_p / pass_spp + 1 for a pixel that renders on (its count is on the pass grid, see vk_adaptive_refine), 0 otherwise;
+// n_level[l] counts the pixels that render on from level l (one atomic per warp and level).
+__global__ void k_adaptive_levels(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
+                                  const uint32_t* __restrict__ nspp, uint32_t n_pix, uint32_t spp, uint32_t min_spp, float max_error,
+                                  uint32_t pass_spp, uint32_t* __restrict__ level, uint32_t* __restrict__ n_level) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    uint32_t lv = 0;
+    if (i < n_pix) {
+        const uint32_t n = nspp[i];
+        if (!adaptive_stop(acc, sq, i, n, spp, min_spp, max_error)) lv = n / pass_spp + 1u;
+        level[i] = lv;
     }
-    keep[i] = stop ? 0u : 1u;
+    const unsigned peers = __match_any_sync(0xFFFFFFFFu, lv);
+    if (lv && (uint32_t)(__ffs(peers) - 1) == (threadIdx.x & 31u)) atomicAdd(&n_level[lv - 1u], (uint32_t)__popc(peers));
+}
+// The error map of a session: e per pixel as the rule sees it, +inf below two samples; top_down: each frame's rows
+// top-down (the order of an rgb8 image), otherwise the accumulators' order
+__global__ void k_adaptive_error_map(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
+                                     const uint32_t* __restrict__ nspp, float* __restrict__ out, uint32_t width, uint32_t height,
+                                     uint32_t n_frames, bool top_down) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, frame = (size_t)width * height;
+    if (i >= frame * n_frames) return;
+    size_t p = i;
+    if (top_down) {
+        const size_t f = i / frame, k = i - f * frame, row = k / width;
+        p = f * frame + (height - 1 - row) * (size_t)width + (k - row * width);
+    }
+    const uint32_t n = nspp[p];
+    out[i] = n < 2u ? __int_as_float(0x7F800000) : (float)adaptive_error(acc, sq, (uint32_t)p, n);
 }
 // mean = sum / n_p with k_acc_to_sum's and k_finalize's operations, so a pixel that stopped at n equals vk_render(spp = n)
 __global__ void k_finalize_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, float* __restrict__ rgb,
@@ -326,7 +370,7 @@ void vk_destroy(vk_ctx* c) {
     if (c->frame) cudaFree(c->frame);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->cams) cudaFree(c->cams);
-    if (c->adapt) cudaFree(c->adapt);
+    adaptive_free(c->oneshot);
     if (c->counters) cudaFree(c->counters);
     if (c->debug) cudaFree(c->debug);
     if (c->ev0) cudaEventDestroy(c->ev0);
@@ -354,6 +398,7 @@ int vk_scene_upload(vk_ctx* c, const vk_scene_desc* d) {
     if (!v.run()) return fail(c, v.code, "vk_scene_upload: " + v.err);
     CU(c, cudaSetDevice(c->device));
     free_scene(c);
+    ++c->scene_gen;
     if (c->arena_need > c->arena_cap) { // the previous upload did not fit: grow (cudaFree waits for the work that reads the old block)
         if (c->arena) cudaFree(c->arena);
         c->arena = nullptr;
@@ -984,14 +1029,49 @@ static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint
     return VK_OK;
 }
 
-// shared body of vk_render_adaptive* and vk_render_frames_adaptive* (include/vecchio_gpu.h states the passes and the rule).
-// n_frames > 1: cam points to n_frames cameras, every pass runs one launch over the active pixels of all frames (one list of
-// batch-wide pixels, FrameListArgs) and the result is n_frames contiguous planes.
-static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
-                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats, uint32_t n_frames = 1) {
-    const std::string w(who);
-    if (!cam || !P || (!out_rgb && !out_rgb8)) return fail(c, VK_ERR_INVALID, w + ": null argument");
-    int rc = n_frames > 1 ? check_frames(c, who, cam, n_frames, P) : VK_OK;
+// ---- adaptive sessions (vk_adaptive_*; the one-shot vk_render_adaptive* calls run one on c->oneshot) ----
+// Device state of a session: fixed-point sums and squares and the counts of every pixel of its K frames, plus the pass
+// loop's scratch (two pixel lists, the select flags, the level of every pixel, the level counts, the compaction scratch).
+struct vk_adaptive_session {
+    vk_ctx* c = nullptr;
+    std::vector<vk_camera> cams;
+    vk_render_params P{}; // P.spp: the session's limit
+    uint32_t n_frames = 0, pass_spp = 0, n_pix = 0, max_levels = 0;
+    RenderPlan R{};
+    uint64_t scene_gen = 0;
+    bool reached_any = false; // a target has been reached (or imported); false: every count is 0
+    bool broken = false;      // a refine or import failed on the device part way: the state is lost
+    vk_adaptive_target reached{};
+    void* block = nullptr;
+    size_t bytes = 0, cub_bytes = 0;
+    unsigned long long *acc = nullptr, *sq = nullptr;
+    uint32_t *nspp = nullptr, *cur = nullptr, *nxt = nullptr, *level = nullptr, *n_level = nullptr;
+    uint8_t* keep = nullptr;
+    int* d_count = nullptr;
+    void* cub_tmp = nullptr;
+};
+
+static void adaptive_free(vk_adaptive_session* s) {
+    if (!s) return;
+    if (s->block && s->c) {
+        cudaSetDevice(s->c->device);
+        cudaFree(s->block);
+    }
+    delete s;
+}
+
+// The pixels that render on from level l of a refine: those k_adaptive_levels marked with l + 1, in ascending order.
+struct AtLevel {
+    const uint32_t* level;
+    uint32_t want;
+    __device__ bool operator()(uint32_t p) const { return level[p] == want; }
+};
+
+// What vk_render_adaptive*, vk_render_frames_adaptive* and vk_adaptive_begin refuse before anything is allocated or
+// launched (max_error: the one-shot calls' target; a session checks its targets in refine).
+static int check_adaptive(vk_ctx* c, const std::string& w, const vk_camera* cam, uint32_t n_frames, const vk_render_params* P,
+                          uint32_t pass_spp, float max_error) {
+    int rc = n_frames > 1 ? check_frames(c, w.c_str(), cam, n_frames, P) : VK_OK;
     if (rc != VK_OK) return rc;
     rc = check_render(c, cam, P);
     if (rc != VK_OK) return rc;
@@ -1004,8 +1084,17 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
                                            ", the limit of the fixed-point sums of squares (2^16 samples of at most 255^2 * 2^32 units)");
     if (P->variant == VK_VARIANT_STAGED || P->variant == VK_VARIANT_WAVEFRONT)
         return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
+    return VK_OK;
+}
+
+// Checks, plans the kernel, sizes s's buffers (a larger block than needed is reused) and zeroes its state.
+static int adaptive_begin(vk_ctx* c, const std::string& w, const vk_camera* cam, uint32_t n_frames, const vk_render_params* P,
+                          uint32_t pass_spp, float max_error, vk_adaptive_session* s) {
+    s->c = c;
+    int rc = check_adaptive(c, w, cam, n_frames, P, pass_spp, max_error);
+    if (rc != VK_OK) return rc;
     CU(c, cudaSetDevice(c->device));
-    // AUTO decides once, on pass 0's path count; every pass runs that kernel
+    // AUTO decides once, on pass 0's path count; every pass of every refine runs that kernel
     vk_render_params Q = *P;
     Q.spp_count = pass_spp < P->spp ? pass_spp : P->spp;
     RenderPlan R;
@@ -1015,99 +1104,228 @@ static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, con
 
     const uint32_t n_pix = P->width * P->height * n_frames; // (all frames: a pixel index is batch-wide)
     const size_t plane = (size_t)n_pix * 3;
-    // buffers: fixed-point sums (c->partial) | the adaptive block | the output staging (c->frame, pinned)
-    if ((rc = ensure(c, &c->partial, &c->partial_floats, plane * 2)) != VK_OK) return rc;
-    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane + n_pix)) != VK_OK) return rc; // rgb or rgb8 | counts in output order
+    const uint32_t max_levels = (P->spp - 1) / pass_spp + 1;
     auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    size_t cub_bytes = 0;
-    CU(c, cub::DeviceSelect::Flagged(nullptr, cub_bytes, (const uint32_t*)nullptr, (const uint8_t*)nullptr, (uint32_t*)nullptr, (int*)nullptr,
+    size_t sel_bytes = 0, lvl_bytes = 0;
+    CU(c, cub::DeviceSelect::Flagged(nullptr, sel_bytes, (const uint32_t*)nullptr, (const uint8_t*)nullptr, (uint32_t*)nullptr, (int*)nullptr,
                                      (int)n_pix, c->stream));
-    const size_t o_sq = 0, o_n = o_sq + al(plane * 8), o_l0 = o_n + al(n_pix * 4ull), o_l1 = o_l0 + al(n_pix * 4ull),
-                 o_keep = o_l1 + al(n_pix * 4ull), o_cnt = o_keep + al(n_pix), o_cub = o_cnt + 256, need = o_cub + al(cub_bytes);
-    if (c->adapt_bytes < need) {
-        if (c->adapt) cudaFree(c->adapt);
-        c->adapt = nullptr;
-        c->adapt_bytes = 0;
-        CU(c, cudaMalloc(&c->adapt, need));
-        c->adapt_bytes = need;
+    CU(c, cub::DeviceSelect::If(nullptr, lvl_bytes, thrust::counting_iterator<uint32_t>(0), (uint32_t*)nullptr, (int*)nullptr, (int)n_pix,
+                                AtLevel{nullptr, 0}, c->stream));
+    const size_t cub_bytes = sel_bytes > lvl_bytes ? sel_bytes : lvl_bytes;
+    const size_t o_acc = 0, o_sq = o_acc + al(plane * 8), o_n = o_sq + al(plane * 8), o_l0 = o_n + al(n_pix * 4ull),
+                 o_l1 = o_l0 + al(n_pix * 4ull), o_lv = o_l1 + al(n_pix * 4ull), o_nl = o_lv + al(n_pix * 4ull),
+                 o_keep = o_nl + al(max_levels * 4ull), o_cnt = o_keep + al(n_pix), o_cub = o_cnt + 256, need = o_cub + al(cub_bytes);
+    if (s->bytes < need) {
+        if (s->block) cudaFree(s->block);
+        s->block = nullptr;
+        s->bytes = 0;
+        CU(c, cudaMalloc(&s->block, need));
+        s->bytes = need;
     }
-    if ((rc = ensure_pinned(c, plane + n_pix + 1)) != VK_OK) return rc; // floats: rgb | counts | the active count
-    char* base = (char*)c->adapt;
-    unsigned long long* sq = (unsigned long long*)(base + o_sq);
-    uint32_t* nspp = (uint32_t*)(base + o_n);
-    uint32_t* cur = (uint32_t*)(base + o_l0);
-    uint32_t* nxt = (uint32_t*)(base + o_l1);
-    uint8_t* keep = (uint8_t*)(base + o_keep);
-    int* d_count = (int*)(base + o_cnt);
-    void* cub_tmp = base + o_cub;
-    uint32_t* h_count = (uint32_t*)(c->pinned + plane + n_pix);
+    char* base = (char*)s->block;
+    s->acc = (unsigned long long*)(base + o_acc);
+    s->sq = (unsigned long long*)(base + o_sq);
+    s->nspp = (uint32_t*)(base + o_n);
+    s->cur = (uint32_t*)(base + o_l0);
+    s->nxt = (uint32_t*)(base + o_l1);
+    s->level = (uint32_t*)(base + o_lv);
+    s->n_level = (uint32_t*)(base + o_nl);
+    s->keep = (uint8_t*)(base + o_keep);
+    s->d_count = (int*)(base + o_cnt);
+    s->cub_tmp = base + o_cub;
+    s->cub_bytes = cub_bytes;
+    // a session starts with no samples: zero sums, squares and counts (the pass loop adds samples [n_p, ..) to them)
+    CU(c, cudaMemsetAsync(base, 0, o_l0, c->stream));
+    s->cams.assign(cam, cam + n_frames);
+    s->P = *P;
+    s->n_frames = n_frames;
+    s->pass_spp = pass_spp;
+    s->n_pix = n_pix;
+    s->max_levels = max_levels;
+    s->R = R;
+    s->scene_gen = c->scene_gen;
+    s->reached_any = false;
+    s->broken = false;
+    s->reached = vk_adaptive_target{0, 0, 0.0f};
+    return VK_OK;
+}
 
+// Whether T may follow what s has reached (include/vecchio_gpu.h, vk_adaptive_refine); a message when not.
+static std::string adaptive_refusal(const vk_adaptive_session* s, const vk_adaptive_target& T) {
+    if (T.spp == 0) return "the target's spp must be >= 1";
+    if (T.spp > s->P.spp) return "the target's spp " + std::to_string(T.spp) + " exceeds the session's limit params->spp = " + std::to_string(s->P.spp);
+    if (!(T.max_error >= 0.0f)) return "max_error must be >= 0 (and not NaN)";
+    if (!s->reached_any) return "";
+    const vk_adaptive_target& A = s->reached;
+    if (A.max_error == 0.0f ? T.max_error != 0.0f : (T.max_error != 0.0f && T.max_error > A.max_error))
+        return "max_error may only tighten (0 is the tightest: after 0 only 0 may follow)";
+    if (T.min_spp < A.min_spp) return "min_spp may only rise";
+    if (T.spp < A.spp) return "spp may only rise";
+    if (T.spp > A.spp && A.spp % s->pass_spp != 0)
+        return "spp may rise only from a cap on the pass grid (a multiple of pass_spp): pixels stopped at " + std::to_string(A.spp) +
+               " would go on off the grid";
+    return "";
+}
+
+// The pass loop of every adaptive render: renders s until target T is reached (the caller has checked T).  A fresh state is
+// today's one-shot render: every pixel from level 0.  Otherwise k_adaptive_levels re-applies the rule of T to every pixel
+// and counts per level those that render on; from the lowest non-empty level upward, each pass covers the pixels reopened
+// at that level plus the survivors of the level below, and empty levels cost nothing.  Adds what it launched and the samples
+// it started to *launches / *paths and the passes' kernel time to *ms_kernels.
+static int adaptive_refine(vk_adaptive_session* s, const vk_adaptive_target& T, uint32_t* launches, uint64_t* paths, float* ms_kernels) {
+    vk_ctx* c = s->c;
+    const uint32_t M = s->pass_spp, n_pix = s->n_pix;
+    CU(c, cudaSetDevice(c->device));
+    int rc = ensure_pinned(c, (size_t)s->max_levels + 1);
+    if (rc != VK_OK) return rc;
+    uint32_t* h_count = (uint32_t*)c->pinned;
+    uint32_t* h_level = h_count + 1;
+    s->broken = true; // until the loop has run to its end
+    const bool fresh = !s->reached_any;
+    const uint32_t n_levels = (T.spp - 1) / M + 1; // levels 0 .. n_levels-1: pixels at l * M samples
+    uint32_t *cur = s->cur, *nxt = s->nxt;
+    // the list of level l's reopened pixels into `out` (their count is h_level[l])
+    auto level_list = [&](uint32_t l, uint32_t* out) -> int {
+        size_t bytes = s->cub_bytes;
+        CU(c, cub::DeviceSelect::If(s->cub_tmp, bytes, thrust::counting_iterator<uint32_t>(0), out, s->d_count, (int)n_pix,
+                                    AtLevel{s->level, l + 1u}, c->stream));
+        *launches += 2; // (its init and select kernels)
+        return VK_OK;
+    };
+    uint32_t lvl = 0, n_active = 0;
+    if (fresh) {
+        k_iota<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(cur, n_pix); // every pixel from level 0, ascending
+        *launches += 1;
+        n_active = n_pix;
+    } else {
+        CU(c, cudaMemsetAsync(s->n_level, 0, n_levels * sizeof(uint32_t), c->stream));
+        k_adaptive_levels<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(s->acc, s->sq, s->nspp, n_pix, T.spp, T.min_spp, T.max_error, M,
+                                                                      s->level, s->n_level);
+        *launches += 1;
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(h_level, s->n_level, n_levels * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaStreamSynchronize(c->stream)); // one read-back per refine: which levels have pixels
+        while (lvl < n_levels && h_level[lvl] == 0u) ++lvl;
+        if (lvl < n_levels) {
+            if ((rc = level_list(lvl, cur)) != VK_OK) return rc;
+            n_active = h_level[lvl];
+        }
+    }
+    apply_l2_window(c);
     RenderBuffers b{};
     b.counters = c->counters;
     b.debug = c->debug;
-    b.acc = (unsigned long long*)c->partial;
+    b.acc = s->acc;
     b.accsq = nullptr;
-    CU(c, cudaEventRecord(c->ev2, c->stream));
-    // the accumulators are zeroed once per call: pass k adds samples [k * pass_spp, ..) to what passes 0 .. k-1 left
-    CU(c, cudaMemsetAsync(c->partial, 0, plane * 2 * sizeof(float), c->stream));
-    CU(c, cudaMemsetAsync(sq, 0, plane * sizeof(unsigned long long), c->stream));
-    uint32_t launches = 1;
-    k_iota<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(cur, n_pix); // pass 0: every pixel, ascending
-    apply_l2_window(c);
-    uint32_t n_active = n_pix, done = 0;
-    uint64_t paths = 0;
-    float ms_kernels = 0.0f;
-    for (;;) {
-        const uint32_t cnt = P->spp - done < pass_spp ? P->spp - done : pass_spp;
-        const ListArgs la{cur, n_active, sq};
+    while (n_active) {
+        const uint32_t done = lvl * M, cnt = T.spp - done < M ? T.spp - done : M;
+        const ListArgs la{cur, n_active, s->sq};
         CU(c, cudaEventRecord(c->ev0, c->stream));
-        if ((rc = launch_pass(c, R, cam, P, done, cnt, b, n_frames, &la, &launches)) != VK_OK) return rc;
-        paths += (uint64_t)n_active * cnt;
-        done += cnt;
-        k_adaptive_select<<<(n_active + 255) / 256, 256, 0, c->stream>>>(cur, n_active, b.acc, sq, done, P->spp, max_error, nspp, keep);
-        ++launches;
-        const bool last = done == P->spp;
-        if (!last) { // the next list: the kept entries, compacted in their (ascending) order
-            CU(c, cub::DeviceSelect::Flagged(cub_tmp, cub_bytes, cur, keep, nxt, d_count, (int)n_active, c->stream));
-            launches += 2; // (its init and select kernels)
+        if ((rc = launch_pass(c, s->R, s->cams.data(), &s->P, done, cnt, b, s->n_frames, &la, launches)) != VK_OK) return rc;
+        *paths += (uint64_t)n_active * cnt;
+        k_adaptive_select<<<(n_active + 255) / 256, 256, 0, c->stream>>>(cur, n_active, s->acc, s->sq, done + cnt, T.spp, T.min_spp,
+                                                                         T.max_error, s->nspp, s->keep);
+        ++*launches;
+        const bool last = done + cnt == T.spp;
+        // the next list: level lvl + 1's reopened pixels, then the kept entries, compacted in their (ascending) order
+        const uint32_t reopened = !fresh && lvl + 1 < n_levels ? h_level[lvl + 1] : 0u;
+        if (!last) {
+            if (reopened && (rc = level_list(lvl + 1, nxt)) != VK_OK) return rc;
+            CU(c, cub::DeviceSelect::Flagged(s->cub_tmp, s->cub_bytes, cur, s->keep, nxt + reopened, s->d_count, (int)n_active, c->stream));
+            *launches += 2;
         }
         CU(c, cudaGetLastError());
         CU(c, cudaEventRecord(c->ev1, c->stream));
         // one 4-byte D2H and a stream synchronisation per pass: the host sizes the next pass's work from the count
-        if (!last) CU(c, cudaMemcpyAsync(h_count, d_count, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        if (!last) CU(c, cudaMemcpyAsync(h_count, s->d_count, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
         CU(c, cudaStreamSynchronize(c->stream));
         float ms = 0.0f;
         CU(c, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-        ms_kernels += ms;
-        if (last || *h_count == 0u) break;
-        n_active = *h_count;
+        *ms_kernels += ms;
+        if (last) break;
+        n_active = *h_count + reopened;
+        ++lvl;
         std::swap(cur, nxt);
+        if (n_active == 0 && !fresh) { // nothing left at this level: on to the next level with reopened pixels
+            ++lvl;
+            while (lvl < n_levels && h_level[lvl] == 0u) ++lvl;
+            if (lvl < n_levels) {
+                if ((rc = level_list(lvl, cur)) != VK_OK) return rc;
+                n_active = h_level[lvl];
+            }
+        }
     }
+    s->reached = T;
+    s->reached_any = true;
+    s->broken = false;
+    return VK_OK;
+}
+
+// The state's image into the caller's buffers (the one-shot calls' layouts), its counts and (nullable) error map.
+static int adaptive_read(vk_adaptive_session* s, float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error, uint32_t* launches) {
+    vk_ctx* c = s->c;
+    const size_t n_pix = s->n_pix, plane = n_pix * 3;
+    CU(c, cudaSetDevice(c->device));
+    int rc;
+    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane + 2 * n_pix)) != VK_OK) return rc; // rgb or rgb8 | counts | errors
+    if ((rc = ensure_pinned(c, plane + 2 * n_pix)) != VK_OK) return rc;
     uint32_t* d_spp = (uint32_t*)(c->frame + plane);
+    float* d_err = c->frame + plane + n_pix;
+    const unsigned blocks = (unsigned)((plane + 255) / 256);
     if (out_rgb) {
-        k_finalize_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, c->frame, plane);
+        k_finalize_adaptive<<<blocks, 256, 0, c->stream>>>(s->acc, s->nspp, c->frame, plane);
         CU(c, cudaGetLastError());
         CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        d_spp = nspp; // (vk_render's layout: the counts are already in pixel order)
+        d_spp = s->nspp; // (vk_render's layout: the counts are already in pixel order)
     } else {
-        k_to_color_adaptive<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(b.acc, nspp, (uint8_t*)c->frame, d_spp, P->width, P->height, n_frames);
+        k_to_color_adaptive<<<blocks, 256, 0, c->stream>>>(s->acc, s->nspp, (uint8_t*)c->frame, d_spp, s->P.width, s->P.height, s->n_frames);
         CU(c, cudaGetLastError());
         CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane, cudaMemcpyDeviceToHost, c->stream));
     }
-    ++launches;
+    ++*launches;
     if (out_spp) CU(c, cudaMemcpyAsync(c->pinned + plane, d_spp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (out_error) {
+        k_adaptive_error_map<<<(unsigned)((n_pix + 255) / 256), 256, 0, c->stream>>>(s->acc, s->sq, s->nspp, d_err, s->P.width, s->P.height,
+                                                                                     s->n_frames, out_rgb8 != nullptr);
+        ++*launches;
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned + plane + n_pix, d_err, n_pix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    }
     CU(c, cudaEventRecord(c->ev1, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     if (out_rgb) std::memcpy(out_rgb, c->pinned, plane * sizeof(float));
     else std::memcpy(out_rgb8, c->pinned, plane);
     if (out_spp) std::memcpy(out_spp, c->pinned + plane, n_pix * sizeof(uint32_t));
+    if (out_error) std::memcpy(out_error, c->pinned + plane + n_pix, n_pix * sizeof(float));
+    return VK_OK;
+}
+
+// shared body of vk_render_adaptive* and vk_render_frames_adaptive* (include/vecchio_gpu.h states the passes and the rule):
+// begin, one refine to {spp, 0, max_error} and read, on the context's own session.
+// n_frames > 1: cam points to n_frames cameras, every pass runs one launch over the active pixels of all frames (one list of
+// batch-wide pixels, FrameListArgs) and the result is n_frames contiguous planes.
+static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
+                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats, uint32_t n_frames = 1) {
+    const std::string w(who);
+    if (!cam || !P || (!out_rgb && !out_rgb8)) return fail(c, VK_ERR_INVALID, w + ": null argument");
+    if (!c->oneshot) c->oneshot = new vk_adaptive_session;
+    vk_adaptive_session* s = c->oneshot;
+    CU(c, cudaSetDevice(c->device));
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    int rc = adaptive_begin(c, w, cam, n_frames, P, pass_spp, max_error, s);
+    if (rc != VK_OK) return rc;
+    uint32_t launches = 0;
+    uint64_t paths = 0;
+    float ms_kernels = 0.0f;
+    if ((rc = adaptive_refine(s, vk_adaptive_target{P->spp, 0u, max_error}, &launches, &paths, &ms_kernels)) != VK_OK) return rc;
+    if ((rc = adaptive_read(s, out_rgb, out_rgb8, out_spp, nullptr, &launches)) != VK_OK) return rc;
     c->launches += launches;
     c->paths += paths;
     vk_stats st{};
     if ((rc = vk_flush_stats(c, &st)) != VK_OK) return rc;
     st.ms_kernels = ms_kernels;
     CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
-    st.variant = R.variant;
+    st.variant = s->R.variant;
     if (stats) *stats = st;
     return VK_OK;
 }
@@ -1141,6 +1359,117 @@ int vk_render_frames_adaptive_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_
     if (n_frames == 1) return vk_render_adaptive_rgb8(c, cams, P, pass_spp, max_error, out_rgb8, out_spp, stats);
     return render_adaptive(c, "vk_render_frames_adaptive_rgb8", cams, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats, n_frames);
 }
+
+int vk_adaptive_begin(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                      vk_adaptive_session** out) {
+    if (!c) return VK_ERR_INVALID;
+    if (!out || !cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_adaptive_begin: null argument or no frames");
+    *out = nullptr;
+    vk_adaptive_session* s = new vk_adaptive_session;
+    s->c = c;
+    const int rc = adaptive_begin(c, "vk_adaptive_begin", cams, n_frames, P, pass_spp, 0.0f, s);
+    if (rc != VK_OK) {
+        adaptive_free(s);
+        return rc;
+    }
+    *out = s;
+    return VK_OK;
+}
+
+int vk_adaptive_refine(vk_adaptive_session* s, const vk_adaptive_target* T, vk_stats* stats) {
+    if (!s) return VK_ERR_INVALID;
+    vk_ctx* c = s->c;
+    if (!T) return fail(c, VK_ERR_INVALID, "vk_adaptive_refine: null target");
+    if (s->broken) return fail(c, VK_ERR_INVALID, "vk_adaptive_refine: an earlier refine or import failed part way; the session's state is lost");
+    if (!c->has_scene || c->scene_gen != s->scene_gen)
+        return fail(c, VK_ERR_INVALID, "vk_adaptive_refine: the scene changed since the session began");
+    const std::string why = adaptive_refusal(s, *T);
+    if (!why.empty()) return fail(c, VK_ERR_INVALID, "vk_adaptive_refine: " + why);
+    CU(c, cudaSetDevice(c->device));
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    uint32_t launches = 0;
+    uint64_t paths = 0;
+    float ms_kernels = 0.0f;
+    int rc = adaptive_refine(s, *T, &launches, &paths, &ms_kernels);
+    if (rc != VK_OK) return rc;
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    c->launches += launches;
+    c->paths += paths;
+    vk_stats st{};
+    if ((rc = vk_flush_stats(c, &st)) != VK_OK) return rc;
+    st.ms_kernels = ms_kernels;
+    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
+    st.variant = s->R.variant;
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+static int adaptive_read_call(vk_adaptive_session* s, const char* who, float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error) {
+    if (!s) return VK_ERR_INVALID;
+    vk_ctx* c = s->c;
+    if (!out_rgb && !out_rgb8) return fail(c, VK_ERR_INVALID, std::string(who) + ": null argument");
+    if (s->broken) return fail(c, VK_ERR_INVALID, std::string(who) + ": an earlier refine or import failed part way; the session's state is lost");
+    uint32_t launches = 0; // (a read is not part of any refine's stats)
+    return adaptive_read(s, out_rgb, out_rgb8, out_spp, out_error, &launches);
+}
+
+int vk_adaptive_read(vk_adaptive_session* s, float* out_rgb, uint32_t* out_spp, float* out_error) {
+    return adaptive_read_call(s, "vk_adaptive_read", out_rgb, nullptr, out_spp, out_error);
+}
+
+int vk_adaptive_read_rgb8(vk_adaptive_session* s, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error) {
+    return adaptive_read_call(s, "vk_adaptive_read_rgb8", nullptr, out_rgb8, out_spp, out_error);
+}
+
+int vk_adaptive_export(vk_adaptive_session* s, int64_t* sums, uint64_t* squares, uint32_t* counts, vk_adaptive_target* reached) {
+    if (!s) return VK_ERR_INVALID;
+    vk_ctx* c = s->c;
+    if (!sums || !squares || !counts) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: null argument");
+    if (s->broken) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: an earlier refine or import failed part way; the session's state is lost");
+    const size_t n_pix = s->n_pix;
+    CU(c, cudaSetDevice(c->device));
+    CU(c, cudaMemcpyAsync(sums, s->acc, n_pix * 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(squares, s->sq, n_pix * 3 * sizeof(uint64_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(counts, s->nspp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (reached) *reached = s->reached;
+    return VK_OK;
+}
+
+int vk_adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
+                       const vk_adaptive_target* reached) {
+    if (!s) return VK_ERR_INVALID;
+    vk_ctx* c = s->c;
+    if (!sums || !squares || !counts || !reached) return fail(c, VK_ERR_INVALID, "vk_adaptive_import: null argument");
+    const vk_adaptive_target& A = *reached;
+    const std::string w = "vk_adaptive_import: ";
+    if (A.spp > s->P.spp) return fail(c, VK_ERR_INVALID, w + "the reached spp exceeds the session's limit params->spp");
+    if (!(A.max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, w + "the reached max_error must be >= 0 (and not NaN)");
+    if (A.spp == 0 && (A.min_spp != 0 || A.max_error != 0.0f)) return fail(c, VK_ERR_INVALID, w + "a state that reached no target has spp, min_spp and max_error 0");
+    for (size_t p = 0; p < s->n_pix; ++p) {
+        const uint32_t n = counts[p];
+        if (n > A.spp) return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has more samples than the reached spp");
+        if (n % s->pass_spp != 0 && n != A.spp)
+            return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has a count off the pass grid (neither a multiple of pass_spp nor the reached spp)");
+        if (n == 0 && (sums[3 * p] | sums[3 * p + 1] | sums[3 * p + 2] | (int64_t)(squares[3 * p] | squares[3 * p + 1] | squares[3 * p + 2])) != 0)
+            return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has no samples but non-zero sums");
+    }
+    const size_t n_pix = s->n_pix;
+    CU(c, cudaSetDevice(c->device));
+    s->broken = true; // until every array has arrived
+    CU(c, cudaMemcpyAsync(s->acc, sums, n_pix * 3 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    CU(c, cudaMemcpyAsync(s->sq, squares, n_pix * 3 * sizeof(uint64_t), cudaMemcpyHostToDevice, c->stream));
+    CU(c, cudaMemcpyAsync(s->nspp, counts, n_pix * sizeof(uint32_t), cudaMemcpyHostToDevice, c->stream));
+    CU(c, cudaStreamSynchronize(c->stream));
+    s->reached = A;
+    s->reached_any = A.spp != 0;
+    s->broken = false;
+    return VK_OK;
+}
+
+uint32_t vk_adaptive_variant(const vk_adaptive_session* s) { return s ? s->R.variant : 0u; }
+
+void vk_adaptive_destroy(vk_adaptive_session* s) { adaptive_free(s); }
 
 int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {
     if (!c) return VK_ERR_INVALID;
