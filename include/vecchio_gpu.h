@@ -349,8 +349,14 @@ int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames,
  * the pixel stops when the largest e of its three channels is <= max_error, or when n == spp.  max_error == 0 never stops
  * early; a pixel with one sample (pass_spp == 1, pass 0) has no standard error and renders on.
  * The squares behind the rule are 64-bit fixed-point sums (2^32 units per 1.0, the sample's channel clamped to 255 first:
- * the clamp touches the statistic only, never the image), exact and order independent, and the decision is deterministic;
- * this bounds spp to 65536.
+ * the clamp touches the statistic only, never the image), exact and order independent; this bounds spp to 65536.
+ * The decision is a stated function of the integer state (sum S: int64 at 2^30 units per 1.0, Q: uint64, n), every step
+ * an IEEE double operation rounded to nearest:
+ *     m = (double)S * 2^-30 / n,  q = (double)Q * 2^-32 / n   (the conversions round to nearest),
+ *     v = fma(-m, m, q)   (q - m^2 with ONE rounding),
+ *     se = sqrt(max(v, 0) / (n - 1)),  e_c = (sqrt(max(m + se, 0)) - sqrt(max(m - se, 0))) * 128,
+ *     e = max(0, e_R, e_G, e_B), and the test is e <= (double)max_error;
+ * out_error maps hold (float)e.  tests/adaptive_model.py restates it on the host, bit for bit.
  * The rule looks at the samples, so the estimate is slightly BIASED: pixels that happen to look smooth stop early.
  * Kernel: VK_VARIANT_AUTO decides once, by vk_render's rule on pass 0's path count W*H*pass_spp, and every pass runs that
  * kernel, so a pass boundary never changes rounding (render build included).

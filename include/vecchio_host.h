@@ -21,7 +21,8 @@ typedef struct vkh_scene vkh_scene;
  *       api_surface_demo (SpecDiffuse, sphere and box lights) |
  *       random_spheres_cover (random_spheres_demo without its light: sky-lit, legacy integrator only) |
  *       book1_cover (the book-1 final scene of sample/inoneweekend.png: grey ground, fixed camera; legacy only) |
- *       furnace_demo (param = 0 Lambertian | 1 Metal | 2 Dielectric | 3 white-medium sphere inside an emitting shell; closed form)
+ *       furnace_demo (param = 0 Lambertian | 1 Metal | 2 Dielectric | 3 white-medium sphere inside an emitting shell; closed form |
+ *                     4 the Lambertian one in a shell 1000x as bright, samples above adaptive sampling's 255 clamp)
  * seed: seeds the host RNG standing in for rand::thread_rng() (scene + BVH axis choices).
  * assets_dir: directory holding earthmap.png etc. (NULL => "assets"). */
 int vkh_scene_build(const char* name, uint64_t seed, const char* assets_dir, uint32_t param, vkh_scene** out);

@@ -128,14 +128,18 @@ __global__ void k_iota(uint32_t* list, uint32_t n) {
     if (i < n) list[i] = i;
 }
 // The largest channel error e of pixel p after n >= 2 samples (include/vecchio_gpu.h states it), from the integer sums
-// alone, so that it does not depend on the order the samples arrived in.
+// alone, so that it does not depend on the order the samples arrived in.  Every operation is IEEE double, rounded to
+// nearest (this file is built without -prec-div / -prec-sqrt = false), and q - m^2 is written as the one fused
+// multiply-add it is: left to the compiler, each inlined copy could be contracted or not, and the one-shot kernel
+// (k_adaptive_select) and a refine's (k_adaptive_levels) could then decide differently within an ulp of max_error.
+// tests/adaptive_model.py restates the sequence on the host, bit for bit.
 __device__ __forceinline__ double adaptive_error(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
                                                  uint32_t p, uint32_t n) {
     double e = 0.0;
     for (uint32_t ch = 0; ch < 3u; ++ch) {
         const double m = (double)(long long)acc[3u * p + ch] * VK_ACC_INV_SCALE / n;
         const double q = (double)sq[3u * p + ch] * VK_SQ_INV_SCALE / n;
-        const double se = sqrt(fmax(q - m * m, 0.0) / (double)(n - 1u));
+        const double se = sqrt(fmax(fma(-m, m, q), 0.0) / (double)(n - 1u));
         e = fmax(e, 128.0 * (sqrt(fmax(m + se, 0.0)) - sqrt(fmax(m - se, 0.0))));
     }
     return e;

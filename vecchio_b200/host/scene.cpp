@@ -182,13 +182,15 @@ SceneConfig api_surface_demo() {
 // other object's box.  Every direction leaving the object ends on the room, so the object's radiance is exactly
 // albedo * E for a Lambertian (`kind` 0) whatever the sampling strategy, albedo * E for a fuzz-0 Metal (1), and E
 // for a Dielectric (2, up to the depth cap) and, in expectation, for a white ConstantMedium (3); pixels beside
-// the object show E.  The light list holds a rect OUTSIDE
+// the object show E.  Kind 4 is kind 0 with the room 1000 times as bright, E = (800, 600, 400): the samples beside the
+// sphere lie above 255, where the squares behind adaptive sampling's stopping rule clamp, and the sphere's straddle it
+// in R and B.  The light list holds a rect OUTSIDE
 // the room and not in the world -- the reference keeps lights in their own list (src/main.rs:169) and
 // `pdf_value` tests only the light's own geometry -- so the mixture estimator must weight light-sampled
 // directions correctly although they never reach that rect.
 SceneConfig furnace_demo(uint32_t kind) {
     SceneConfig s;
-    auto glow = arc<DiffuseLight>(solid(0.8f, 0.6f, 0.4f));
+    auto glow = arc<DiffuseLight>(kind == 4 ? solid(800.0f, 600.0f, 400.0f) : solid(0.8f, 0.6f, 0.4f));
     const float L = 40.0f;
     s.world.push_back(rect(Rect::XYRect(-L, L, -L, L, -L, glow)));
     s.world.push_back(flip(rect(Rect::XYRect(-L, L, -L, L, L, glow))));

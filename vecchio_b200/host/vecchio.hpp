@@ -376,7 +376,7 @@ SceneConfig final_scene();
 SceneConfig cornell_smoke();
 SceneConfig stress_spheres(uint32_t grid_side);
 SceneConfig api_surface_demo();     // SpecDiffuse + sphere and box lights (API surface no shipped scene uses)
-SceneConfig furnace_demo(uint32_t kind); // one object (0 Lambertian, 1 Metal, 2 Dielectric, 3 white medium) inside an emitting shell: closed-form radiance
+SceneConfig furnace_demo(uint32_t kind); // one object (0 Lambertian, 1 Metal, 2 Dielectric, 3 white medium, 4 Lambertian in a 1000x brighter shell) inside an emitting shell: closed-form radiance
 SceneConfig book1_cover();          // the book-1 final scene as sample/inoneweekend.png shows it (grey ground, brown sphere, fixed camera; legacy integrator)
 SceneConfig random_spheres_cover(); // random_spheres_demo without its light: the sky-lit book-1 cover (legacy integrator)
 
