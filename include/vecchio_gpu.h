@@ -364,7 +364,7 @@ int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames,
  * out_spp (nullable): n_p, W*H in the order of the image it accompanies.  stats: paths = sum of n_p; rays, dropped
  * samples, ms_kernels and launches are totals over all passes; variant is the kernel that ran.  Each pass costs one 4-byte
  * D2H of the active count and a stream synchronisation.  One frame on one device (a batch of frames:
- * vk_render_frames_adaptive; no multi-GPU context).
+ * vk_render_frames_adaptive; several devices: vk_multi_render_adaptive_rgb8).
  * Errors, before anything is launched: VK_ERR_INVALID for pass_spp == 0, max_error negative or NaN, spp_begin != 0,
  * spp_count not 0 or spp, spp > 65536, and every check of vk_render; VK_ERR_UNSUPPORTED for VK_VARIANT_STAGED /
  * VK_VARIANT_WAVEFRONT; VK_ERR_NO_SCENE without a scene. */
@@ -432,7 +432,8 @@ typedef struct vk_adaptive_session vk_adaptive_session;
  * equals vk_render_adaptive(_rgb8) (K = 1) or vk_render_frames_adaptive(_rgb8) (K > 1) at max_error = E in image, counts and
  * stats.paths, in both math builds: it runs the same kernels.
  * Sessions borrow their context: destroy them before the context.  Other calls on the context (vk_render, the one-shot
- * adaptive calls, other sessions) may run between a session's calls and do not touch its state.  No multi-GPU context.
+ * adaptive calls, other sessions) may run between a session's calls and do not touch its state.  Several GPUs:
+ * vk_adaptive_begin_shard on each, or vk_multi_adaptive_begin over a vk_multi.
  * Errors are reported through vk_last_error of the context. */
 
 /* Begins a session: every check of vk_render_frames_adaptive (params->spp is the session's limit, <= 65536; spp_begin
@@ -442,6 +443,28 @@ typedef struct vk_adaptive_session vk_adaptive_session;
  * n_frames * W*H * min(pass_spp, spp) paths.  The cameras and params are copied. */
 int vk_adaptive_begin(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
                       uint32_t pass_spp, vk_adaptive_session** out);
+
+/* Shard sessions: a session that renders only the pixels shard `shard` of n_shards owns, so that n_shards devices (or
+ * processes) can split one adaptive render between them without any traffic until the image is read.
+ * Ownership: with g the batch-wide pixel index f*W*H + y*W + x, pixel g belongs to shard (g / VK_SHARD_RUN) mod n_shards.
+ * A run of VK_SHARD_RUN = 32 pixels is one warp's list entries and one lane-megakernel item, so a shard's lists keep the
+ * alignment and the camera-ray coherence of the unsharded lists, and the fine interleaving spreads noisy regions evenly.
+ * The session is an ordinary vk_adaptive_session: refine, read, read_rgb8, export, import, variant and destroy take it.
+ * Its buffers are full size (n_frames * W*H) and indices stay batch-wide.  Pixels it does not own are never rendered:
+ * their sums, squares and counts stay 0 and read like any pixel without samples (count 0, mean 0/0 = NaN, rgb8 0, error
+ * +inf).  Its kernel is the unsharded session's: VK_VARIANT_AUTO decides on the whole batch's
+ * n_frames * W*H * min(pass_spp, spp) paths, not on the shard's share.
+ * A shard that owns no pixel (n_frames * W*H <= 32 * shard) is legal: its refines render nothing, add 0 paths and still
+ * reach their target.  vk_adaptive_import also refuses (VK_ERR_INVALID, the state untouched) any non-zero sum, square or
+ * count on a pixel the shard does not own.
+ * Guarantee: a pixel's decisions depend on its own integer state only and Philox is keyed by (pixel, global sample), so an
+ * owned pixel ends every refine with the integers it has in the unsharded session.  For any sequence of tightening targets,
+ * the sum over shards k = 0 .. n_shards-1 of their exports equals the unsharded session's export bit for bit (and paths add
+ * up likewise).  Shard 0 of 1 is vk_adaptive_begin.
+ * Errors: those of vk_adaptive_begin, and VK_ERR_INVALID for n_shards == 0 or shard >= n_shards. */
+#define VK_SHARD_RUN 32
+int vk_adaptive_begin_shard(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                            uint32_t pass_spp, uint32_t shard, uint32_t n_shards, vk_adaptive_session** out);
 
 /* Renders until `target` is reached.  A pixel below the new cap that the new rule lets go on renders on from its count;
  * the passes run level by level (a level is a count on the pass grid: 0, M, 2M, ..), each pass one launch over the pixels
@@ -524,6 +547,41 @@ int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_para
                          vk_stats* stats);                                      /* vk_render_rgb8 over all devices         */
 int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
                                 uint8_t* out_rgb8, vk_stats* stats);            /* vk_render_frames_rgb8 over all devices  */
+
+/* Adaptive sessions over all devices of a vk_multi: the vk_adaptive_* calls with the same meaning and arguments.  Adaptive
+ * sampling splits PIXELS, not samples (a pixel's decision after each pass needs the sums of all its samples): device k
+ * runs shard k of N (vk_adaptive_begin_shard), the existing pass loop over the pixels it owns.  A refine runs the devices'
+ * pass loops at once, one host thread per device inside the call, all joined before it returns.  stats: paths, rays,
+ * dropped samples and launches summed over the devices, ms_kernels the slowest device's, variant the shared kernel.
+ * A read or an export after a refine or an import first gathers every pixel's sums, squares and count from the device
+ * that owns it into one state on devices[0] (one kernel reading the peers' memory over NVLink, 52 bytes a pixel), then
+ * reads it as vk_adaptive_read* / vk_adaptive_export do.  An import checks the whole state as vk_adaptive_import does and
+ * gives each device the pixels it owns; a refused import changes nothing.  After a refine or import that failed part way
+ * on any device the session refuses everything but import and destroy.  Errors: vk_multi_last_error of the vk_multi.
+ * Guarantee: the image, counts, error map, export and stats.paths equal those of a one-GPU session with the same
+ * arguments, bit for bit, in both math builds: every device runs the one-GPU session's kernel on the same integers.  So an
+ * export of either resumes in the other.  Destroy the session before the vk_multi.
+ * The balance is static: the slowest shard sets the time of every refine. */
+typedef struct vk_multi_adaptive_session vk_multi_adaptive_session;
+int vk_multi_adaptive_begin(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                            uint32_t pass_spp, vk_multi_adaptive_session** out);
+int vk_multi_adaptive_refine(vk_multi_adaptive_session* session, const vk_adaptive_target* target, vk_stats* stats);
+int vk_multi_adaptive_read(vk_multi_adaptive_session* session, float* out_rgb, uint32_t* out_spp, float* out_error);
+int vk_multi_adaptive_read_rgb8(vk_multi_adaptive_session* session, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error);
+int vk_multi_adaptive_export(vk_multi_adaptive_session* session, int64_t* sums, uint64_t* squares, uint32_t* counts,
+                             vk_adaptive_target* reached);
+int vk_multi_adaptive_import(vk_multi_adaptive_session* session, const int64_t* sums, const uint64_t* squares,
+                             const uint32_t* counts, const vk_adaptive_target* reached);
+uint32_t vk_multi_adaptive_variant(const vk_multi_adaptive_session* session);
+void vk_multi_adaptive_destroy(vk_multi_adaptive_session* session);
+/* vk_render_adaptive_rgb8 / vk_render_frames_adaptive_rgb8 over all devices: begin, one refine to {spp, 0, max_error} and
+ * read_rgb8 on a session the vk_multi keeps; the same bytes, counts and stats.paths as on one GPU.  (Float means, error
+ * maps and exports: through a session.)  stats.ms_total: the call's wall time. */
+int vk_multi_render_adaptive_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* params, uint32_t pass_spp,
+                                  float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats);
+int vk_multi_render_frames_adaptive_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
+                                         uint32_t pass_spp, float max_error, uint8_t* out_rgb8, uint32_t* out_spp,
+                                         vk_stats* stats);
 
 /* Parity hook: closest hit of `world.hit(&r, tmin, tmax)` (src/accel.rs:58-83) for
  * a batch of rays.  medium_xi (nullable): n * VK_MEDIUM_XI_SLOTS uniform variates

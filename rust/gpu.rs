@@ -136,6 +136,10 @@ extern "C" {
                               reached: *const vk_adaptive_target) -> c_int;
     pub fn vk_adaptive_variant(session: *const vk_adaptive_session) -> u32;
     pub fn vk_adaptive_destroy(session: *mut vk_adaptive_session);
+    // a session over the pixels shard `shard` of n_shards owns ((g / VK_SHARD_RUN) mod n_shards == shard); the shards' exports
+    // add up to the unsharded session's bit for bit
+    pub fn vk_adaptive_begin_shard(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, pass_spp: u32,
+                                   shard: u32, n_shards: u32, out: *mut *mut vk_adaptive_session) -> c_int;
     // one context over several GPUs of the node (samples split by global index, peer-memory reduce on devices[0])
     pub fn vk_multi_create(devices: *const c_int, n_devices: c_int, out: *mut *mut vk_multi) -> c_int;
     pub fn vk_multi_destroy(m: *mut vk_multi);
@@ -147,8 +151,26 @@ extern "C" {
                                 out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
     pub fn vk_multi_render_frames_rgb8(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
                                        out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
+    // adaptive sampling over several GPUs: device k renders shard k's pixels; every result equals the one-GPU call's bit for bit
+    pub fn vk_multi_adaptive_begin(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, pass_spp: u32,
+                                   out: *mut *mut vk_multi_adaptive_session) -> c_int;
+    pub fn vk_multi_adaptive_refine(session: *mut vk_multi_adaptive_session, target: *const vk_adaptive_target, stats: *mut vk_stats) -> c_int;
+    pub fn vk_multi_adaptive_read(session: *mut vk_multi_adaptive_session, out_rgb: *mut f32, out_spp: *mut u32, out_error: *mut f32) -> c_int;
+    pub fn vk_multi_adaptive_read_rgb8(session: *mut vk_multi_adaptive_session, out_rgb8: *mut u8, out_spp: *mut u32, out_error: *mut f32) -> c_int;
+    pub fn vk_multi_adaptive_export(session: *mut vk_multi_adaptive_session, sums: *mut i64, squares: *mut u64, counts: *mut u32,
+                                    reached: *mut vk_adaptive_target) -> c_int;
+    pub fn vk_multi_adaptive_import(session: *mut vk_multi_adaptive_session, sums: *const i64, squares: *const u64, counts: *const u32,
+                                    reached: *const vk_adaptive_target) -> c_int;
+    pub fn vk_multi_adaptive_variant(session: *const vk_multi_adaptive_session) -> u32;
+    pub fn vk_multi_adaptive_destroy(session: *mut vk_multi_adaptive_session);
+    pub fn vk_multi_render_adaptive_rgb8(m: *mut vk_multi, cam: *const vk_camera, params: *const vk_render_params, pass_spp: u32,
+                                         max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
+    pub fn vk_multi_render_frames_adaptive_rgb8(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
+                                                pass_spp: u32, max_error: f32, out_rgb8: *mut u8, out_spp: *mut u32, stats: *mut vk_stats) -> c_int;
 }
 #[repr(C)] pub struct vk_multi { _private: [u8; 0] }
+#[repr(C)] pub struct vk_multi_adaptive_session { _private: [u8; 0] }
+pub const VK_SHARD_RUN: u32 = 32;
 
 #[derive(Debug)]
 pub enum GpuError { Unsupported(&'static str), Library(i32, String) }
@@ -476,8 +498,76 @@ impl MultiGpu {
         self.check(unsafe { vk_multi_render_frames_rgb8(self.m, cams.as_ptr(), cams.len() as u32, &p, out.as_mut_ptr(), &mut st) })?;
         Ok((out, st))
     }
+    /// `Gpu::render_adaptive_rgb8` over all devices (device k renders the pixels of shard k): the same bytes and counts.
+    pub fn render_adaptive_rgb8(&mut self, cam: &vk_camera, width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                                pass_spp: u32, max_error: f32) -> Result<(Vec<u8>, Vec<u32>, vk_stats), GpuError> {
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; width * height * 3];
+        let mut n = vec![0u32; width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_multi_render_adaptive_rgb8(self.m, cam, &p, pass_spp, max_error, out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
+    }
+    /// `Gpu::render_frames_adaptive_rgb8` over all devices: the same bytes and counts as one GPU's batch.
+    pub fn render_frames_adaptive_rgb8(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                                       pass_spp: u32, max_error: f32) -> Result<(Vec<u8>, Vec<u32>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_frames_adaptive_rgb8: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut out = vec![0u8; cams.len() * width * height * 3];
+        let mut n = vec![0u32; cams.len() * width * height];
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_multi_render_frames_adaptive_rgb8(self.m, cams.as_ptr(), cams.len() as u32, &p, pass_spp, max_error,
+                                                                 out.as_mut_ptr(), n.as_mut_ptr(), &mut st) })?;
+        Ok((out, n, st))
+    }
+    /// `Gpu::adaptive_session` over all devices (vk_multi_adaptive_begin): the same results, and checkpoints that move
+    /// between one GPU and several.  The session borrows the MultiGpu.
+    pub fn adaptive_session(&mut self, cams: &[vk_camera], width: usize, height: usize, spp: u32, max_depth: u32, seed: u64,
+                            pass_spp: u32) -> Result<MultiAdaptiveSession<'_>, GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("adaptive_session: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp, spp_begin: 0, spp_count: 0, max_depth, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let mut s = std::ptr::null_mut();
+        self.check(unsafe { vk_multi_adaptive_begin(self.m, cams.as_ptr(), cams.len() as u32, &p, pass_spp, &mut s) })?;
+        Ok(MultiAdaptiveSession { multi: self, s, n_pix: cams.len() * width * height })
+    }
 }
 impl Drop for MultiGpu { fn drop(&mut self) { unsafe { vk_multi_destroy(self.m) } } }
+
+/// A session of `MultiGpu::adaptive_session`: `AdaptiveSession`'s methods over all devices.
+pub struct MultiAdaptiveSession<'a> { multi: &'a mut MultiGpu, s: *mut vk_multi_adaptive_session, n_pix: usize }
+impl<'a> MultiAdaptiveSession<'a> {
+    pub fn refine(&mut self, target: &vk_adaptive_target) -> Result<vk_stats, GpuError> {
+        let mut st = vk_stats::default();
+        self.multi.check(unsafe { vk_multi_adaptive_refine(self.s, target, &mut st) })?;
+        Ok(st)
+    }
+    pub fn read(&mut self) -> Result<(Vec<f32>, Vec<u32>, Vec<f32>), GpuError> {
+        let (mut out, mut n, mut e) = (vec![0f32; self.n_pix * 3], vec![0u32; self.n_pix], vec![0f32; self.n_pix]);
+        self.multi.check(unsafe { vk_multi_adaptive_read(self.s, out.as_mut_ptr(), n.as_mut_ptr(), e.as_mut_ptr()) })?;
+        Ok((out, n, e))
+    }
+    pub fn read_rgb8(&mut self) -> Result<(Vec<u8>, Vec<u32>, Vec<f32>), GpuError> {
+        let (mut out, mut n, mut e) = (vec![0u8; self.n_pix * 3], vec![0u32; self.n_pix], vec![0f32; self.n_pix]);
+        self.multi.check(unsafe { vk_multi_adaptive_read_rgb8(self.s, out.as_mut_ptr(), n.as_mut_ptr(), e.as_mut_ptr()) })?;
+        Ok((out, n, e))
+    }
+    pub fn export(&mut self) -> Result<(Vec<i64>, Vec<u64>, Vec<u32>, vk_adaptive_target), GpuError> {
+        let (mut sums, mut sq, mut n) = (vec![0i64; self.n_pix * 3], vec![0u64; self.n_pix * 3], vec![0u32; self.n_pix]);
+        let mut t = vk_adaptive_target::default();
+        self.multi.check(unsafe { vk_multi_adaptive_export(self.s, sums.as_mut_ptr(), sq.as_mut_ptr(), n.as_mut_ptr(), &mut t) })?;
+        Ok((sums, sq, n, t))
+    }
+    pub fn import(&mut self, sums: &[i64], squares: &[u64], counts: &[u32], reached: &vk_adaptive_target) -> Result<(), GpuError> {
+        if sums.len() != self.n_pix * 3 || squares.len() != self.n_pix * 3 || counts.len() != self.n_pix {
+            return Err(GpuError::Unsupported("MultiAdaptiveSession::import: array lengths do not match the session"));
+        }
+        self.multi.check(unsafe { vk_multi_adaptive_import(self.s, sums.as_ptr(), squares.as_ptr(), counts.as_ptr(), reached) })
+    }
+}
+impl<'a> Drop for MultiAdaptiveSession<'a> { fn drop(&mut self) { unsafe { vk_multi_adaptive_destroy(self.s) } } }
 unsafe impl Send for MultiGpu {}
 fn multi_error(m: *const vk_multi) -> String {
     unsafe { let p = vk_multi_last_error(m); if p.is_null() { String::new() } else { CStr::from_ptr(p).to_string_lossy().into_owned() } }

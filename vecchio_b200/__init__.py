@@ -128,8 +128,16 @@ def gpu_lib():
         L.vk_adaptive_variant.restype = C.c_uint32
         L.vk_adaptive_destroy.argtypes = [vp]
         L.vk_adaptive_destroy.restype = None
+        L.vk_adaptive_begin_shard.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32,
+                                              C.c_uint32, C.c_uint32, C.POINTER(vp)]
+        for f in ("begin", "refine", "read", "read_rgb8", "export", "import", "variant", "destroy"):  # the same arguments over a vk_multi
+            getattr(L, "vk_multi_adaptive_" + f).argtypes = getattr(L, "vk_adaptive_" + f).argtypes
+            getattr(L, "vk_multi_adaptive_" + f).restype = getattr(L, "vk_adaptive_" + f).restype
+        L.vk_multi_render_adaptive_rgb8.argtypes = L.vk_render_adaptive_rgb8.argtypes
+        L.vk_multi_render_frames_adaptive_rgb8.argtypes = L.vk_render_frames_adaptive_rgb8.argtypes
         for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
-                  "vk_multi_render_frames_rgb8"):
+                  "vk_multi_render_frames_rgb8", "vk_multi_render_adaptive_rgb8", "vk_multi_render_frames_adaptive_rgb8",
+                  "vk_adaptive_begin_shard"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
                   "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
@@ -147,7 +155,10 @@ GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk
                "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8", "vk_render_frames", "vk_render_frames_rgb8",
                "vk_multi_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8", "vk_render_frames_adaptive",
                "vk_render_frames_adaptive_rgb8", "vk_adaptive_begin", "vk_adaptive_refine", "vk_adaptive_read", "vk_adaptive_read_rgb8",
-               "vk_adaptive_export", "vk_adaptive_import", "vk_adaptive_variant", "vk_adaptive_destroy"]
+               "vk_adaptive_export", "vk_adaptive_import", "vk_adaptive_variant", "vk_adaptive_destroy", "vk_adaptive_begin_shard",
+               "vk_multi_adaptive_begin", "vk_multi_adaptive_refine", "vk_multi_adaptive_read", "vk_multi_adaptive_read_rgb8",
+               "vk_multi_adaptive_export", "vk_multi_adaptive_import", "vk_multi_adaptive_variant", "vk_multi_adaptive_destroy",
+               "vk_multi_render_adaptive_rgb8", "vk_multi_render_frames_adaptive_rgb8"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
                 "vkh_frame_filename", "vkh_last_error"]
@@ -326,30 +337,57 @@ def _check_tightens(reached, target, limit, pass_spp):
         raise ValueError(f"adaptive target: spp may rise only from a cap on the pass grid; {r_spp} is not a multiple of pass_spp = {pass_spp}")
 
 
+def _check_shard(shard):
+    """``shard`` as (k, n) ints, or None; what vk_adaptive_begin_shard refuses, refused here first."""
+    if shard is None:
+        return None
+    k, n = (int(x) for x in shard)
+    if n < 1 or not 0 <= k < n:
+        raise ValueError(f"adaptive_session: shard (k, n) needs 0 <= k < n, got ({k}, {n})")
+    return k, n
+
+
 class AdaptiveSession:
     """``vk_adaptive_begin`` .. ``vk_adaptive_destroy``: an adaptive render whose state outlives a call.  ``refine`` moves
     it to tighter targets, each step ending bit for bit where a fresh session refined once to that target would; a fresh
     session refined to ``(max_error, params.spp)`` is ``render_adaptive`` / ``render_frames_adaptive``.  One camera gives
-    (H, W) shapes, a list of K cameras (K, H, W).  Made by ``Context.adaptive_session``; keeps its context alive."""
+    (H, W) shapes, a list of K cameras (K, H, W).  Made by ``Context.adaptive_session``; keeps its context alive.
 
-    def __init__(self, ctx, cams, params, pass_spp):
+    ``shard=(k, n)`` (``vk_adaptive_begin_shard``) renders only the pixels shard k of n owns (batch-wide pixel g belongs to
+    shard (g // 32) % n); the others stay 0, and the n shards' exports add up to the unsharded export bit for bit.  Over a
+    :class:`MultiContext` the same methods call ``vk_multi_adaptive_*``: device k runs shard k, and every result equals a
+    one-GPU session's."""
+
+    shard = None  # (k, n) of a shard session
+    _api = "vk_adaptive_"  # the C calls: vk_adaptive_* on a Context, vk_multi_adaptive_* on a MultiContext
+
+    def __init__(self, ctx, cams, params, pass_spp, shard=None):
         if int(pass_spp) < 1:
             raise ValueError("adaptive_session: pass_spp must be >= 1")
+        shard = _check_shard(shard)
         self.single = isinstance(cams, _abi.vk_camera)
         cams = [cams] if self.single else list(cams)
         if not cams:
             raise ValueError("adaptive_session: at least one camera")
         arr, k = _camera_array(cams)
         self._h = None
+        self._api = ctx._adaptive_api
         h = C.c_void_p()
-        ctx._check(ctx._L.vk_adaptive_begin(ctx._h, arr, k, C.byref(params), int(pass_spp), C.byref(h)))
+        if shard is None:
+            ctx._check(getattr(ctx._L, self._api + "begin")(ctx._h, arr, k, C.byref(params), int(pass_spp), C.byref(h)))
+        else:
+            ctx._check(ctx._L.vk_adaptive_begin_shard(ctx._h, arr, k, C.byref(params), int(pass_spp), shard[0], shard[1], C.byref(h)))
+            self.shard = shard
         self._ctx, self._L, self._h = ctx, ctx._L, h
         ctx._sessions.add(self)
         self.cams = [_abi.vk_camera.from_buffer_copy(c) for c in cams]
         self.params = _abi.vk_render_params.from_buffer_copy(params)
         self.pass_spp, self.n_frames = int(pass_spp), k
-        self.variant = int(self._L.vk_adaptive_variant(h))
+        self.variant = int(self._fn("variant")(h))
         self.reached = None  # the last target reached, (spp, min_spp, max_error)
+
+    def _fn(self, name):
+        return getattr(self._L, self._api + name)
 
     def _check(self, rc):
         self._ctx._check(rc)
@@ -369,7 +407,7 @@ class AdaptiveSession:
         _check_tightens(self.reached, t, self.params.spp, self.pass_spp)
         T = _abi.vk_adaptive_target(*t)
         st = _abi.vk_stats()
-        self._check(self._L.vk_adaptive_refine(self._h, C.byref(T), C.byref(st)))
+        self._check(self._fn("refine")(self._h, C.byref(T), C.byref(st)))
         self.reached = t
         return st
 
@@ -385,11 +423,11 @@ class AdaptiveSession:
     def read(self):
         """``vk_adaptive_read``: (means float32 with row 0 = bottom, counts, error map) in ``render_adaptive``'s layout;
         the error map is the largest channel error the rule sees, +inf below two samples."""
-        return self._read(self._L.vk_adaptive_read, np.float32)
+        return self._read(self._fn("read"), np.float32)
 
     def read_rgb8(self):
         """``vk_adaptive_read_rgb8``: read()'s image through to_color with row 0 = top, counts and errors in that order."""
-        return self._read(self._L.vk_adaptive_read_rgb8, np.uint8)
+        return self._read(self._fn("read_rgb8"), np.uint8)
 
     def export(self):
         """``vk_adaptive_export``: (sums int64, squares uint64, both shape + (3,), counts uint32, reached), the raw
@@ -399,7 +437,7 @@ class AdaptiveSession:
         squares = np.empty(shape + (3,), dtype=np.uint64)
         counts = np.empty(shape, dtype=np.uint32)
         T = _abi.vk_adaptive_target()
-        self._check(self._L.vk_adaptive_export(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
+        self._check(self._fn("export")(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
         return sums, squares, counts, (None if T.spp == 0 else (int(T.spp), int(T.min_spp), float(T.max_error)))
 
     def import_(self, sums, squares, counts, reached):
@@ -413,13 +451,13 @@ class AdaptiveSession:
             raise ValueError(f"import_: the session's shape is {shape}, the state's {counts.shape}")
         r = (0, 0, 0.0) if reached is None else _adaptive_target(reached[2], reached[0], reached[1])
         T = _abi.vk_adaptive_target(*r)
-        self._check(self._L.vk_adaptive_import(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
+        self._check(self._fn("import")(self._h, sums.ctypes.data, squares.ctypes.data, counts.ctypes.data, C.byref(T)))
         self.reached = None if reached is None else r
 
     def key(self, scene_name, scene_seed, scene_param=0):
         """The identity a checkpoint of this session carries (``adaptive_checkpoint.session_key``)."""
         from .adaptive_checkpoint import session_key
-        return session_key(scene_name, scene_seed, self.cams, self.params, self.pass_spp, self.variant, scene_param)
+        return session_key(scene_name, scene_seed, self.cams, self.params, self.pass_spp, self.variant, scene_param, self.shard)
 
     def _own_key(self, key):
         """``key`` if it is this session's identity (its scene fields with the session's own cameras, params, pass_spp
@@ -445,7 +483,7 @@ class AdaptiveSession:
 
     def close(self):
         if getattr(self, "_h", None):
-            self._L.vk_adaptive_destroy(self._h)
+            self._fn("destroy")(self._h)
             self._h = None
             self._ctx._sessions.discard(self)
 
@@ -458,6 +496,8 @@ class AdaptiveSession:
 
 class Context:
     """One GPU context (``vk_create``).  Fails loudly without the CUDA library or a device."""
+
+    _adaptive_api = "vk_adaptive_"
 
     def __init__(self, device=0):
         L = gpu_lib()
@@ -474,10 +514,11 @@ class Context:
         if rc != 0:
             raise VecchioError(rc, (self._L.vk_last_error(self._h) or b"").decode())
 
-    def adaptive_session(self, cams, params, pass_spp):
+    def adaptive_session(self, cams, params, pass_spp, shard=None):
         """``vk_adaptive_begin``: an :class:`AdaptiveSession` over one camera ((H, W) shapes) or a list of K
-        ((K, H, W)); frame f uses seed ``params.seed + f`` and ``params.spp`` is the session's limit."""
-        return AdaptiveSession(self, cams, params, pass_spp)
+        ((K, H, W)); frame f uses seed ``params.seed + f`` and ``params.spp`` is the session's limit.  ``shard=(k, n)``:
+        ``vk_adaptive_begin_shard``, only the pixels shard k of n owns."""
+        return AdaptiveSession(self, cams, params, pass_spp, shard)
 
     def upload(self, scene):
         self._check(self._L.vk_scene_upload(self._h, scene.desc_ptr))
@@ -640,7 +681,11 @@ class Context:
 
 class MultiContext:
     """``vk_multi_create``: one context over several GPUs of the node (spp slices per device, the peers' integer
-    accumulators added on the first device over NVLink).  Same frame as one GPU, bit for bit."""
+    accumulators added on the first device over NVLink).  Same frame as one GPU, bit for bit.  Adaptive sampling splits
+    pixels instead: device k renders shard k of N (``adaptive_session``, ``render_adaptive_rgb8``), again the one-GPU
+    result bit for bit."""
+
+    _adaptive_api = "vk_multi_adaptive_"
 
     def __init__(self, devices):
         L = gpu_lib()
@@ -650,6 +695,38 @@ class MultiContext:
         if rc != 0:
             raise VecchioError(rc, (L.vk_multi_last_error(None) or b"").decode())
         self._h, self._L, self.devices = h, L, list(devices)
+        self._sessions = weakref.WeakSet()
+
+    def adaptive_session(self, cams, params, pass_spp):
+        """``vk_multi_adaptive_begin``: :class:`AdaptiveSession`'s methods over all devices (device k renders the pixels
+        shard k of N owns); image, counts, error map, export and paths equal ``Context.adaptive_session``'s, and its
+        checkpoints are interchangeable with a one-GPU session's."""
+        return AdaptiveSession(self, cams, params, pass_spp)
+
+    def render_adaptive_rgb8(self, cam, params, pass_spp, max_error):
+        """``vk_multi_render_adaptive_rgb8``: ``Context.render_adaptive_rgb8`` over all devices, the same bytes and counts.
+        Returns (rgb8 (H, W, 3) uint8, spp (H, W) uint32 with row 0 = top, stats)."""
+        _check_adaptive(pass_spp, max_error)
+        n = params.width * params.height
+        out = np.empty(n * 3, dtype=np.uint8)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_multi_render_adaptive_rgb8(self._h, C.byref(cam), C.byref(params), int(pass_spp), float(max_error),
+                                                          out.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return out.reshape(params.height, params.width, 3), spp.reshape(params.height, params.width), st
+
+    def render_frames_adaptive_rgb8(self, cams, params, pass_spp, max_error):
+        """``vk_multi_render_frames_adaptive_rgb8``: ``Context.render_frames_adaptive_rgb8`` over all devices, the same
+        bytes and counts.  Returns ((K, H, W, 3) uint8, (K, H, W) uint32 counts with row 0 = top, stats of the batch)."""
+        _check_adaptive(pass_spp, max_error)
+        arr, k = _camera_array(cams)
+        n = k * params.width * params.height
+        out = np.empty(n * 3, dtype=np.uint8)
+        spp = np.empty(n, dtype=np.uint32)
+        st = _abi.vk_stats()
+        self._check(self._L.vk_multi_render_frames_adaptive_rgb8(self._h, arr, k, C.byref(params), int(pass_spp), float(max_error),
+                                                                 out.ctypes.data, spp.ctypes.data, C.byref(st)))
+        return out.reshape(k, params.height, params.width, 3), spp.reshape(k, params.height, params.width), st
 
     def _check(self, rc):
         if rc != 0:
@@ -684,6 +761,8 @@ class MultiContext:
 
     def close(self):
         if getattr(self, "_h", None):
+            for s in list(getattr(self, "_sessions", ())):  # (sessions borrow the devices: they go first)
+                s.close()
             self._L.vk_multi_destroy(self._h)
             self._h = None
 

@@ -18,10 +18,11 @@ from .accumulate import frame_key
 _FORMAT = 1
 
 
-def session_key(scene_name, scene_seed, cams, params, pass_spp, variant, scene_param=0):
+def session_key(scene_name, scene_seed, cams, params, pass_spp, variant, scene_param=0, shard=None):
     """Identity of a session's state: ``frame_key`` of its first camera with the hashes of ALL its cameras, plus
     ``pass_spp`` (the pass grid the counts lie on) and the kernel that ran (``variant``: the render build's kernels may
-    round differently).  ``params.spp`` in it is the session's limit."""
+    round differently).  ``params.spp`` in it is the session's limit.  A shard session's key adds ``"shard": [k, n]``, so
+    its partial state never loads into a whole session; a whole state's key (one GPU or several) has no such entry."""
     cams = list(cams)
     if not cams:
         raise ValueError("session_key: at least one camera")
@@ -30,6 +31,8 @@ def session_key(scene_name, scene_seed, cams, params, pass_spp, variant, scene_p
     key["camera"] = [k["camera"] for k in keys]
     key["pass_spp"] = int(pass_spp)
     key["variant"] = int(variant)
+    if shard is not None:
+        key["shard"] = [int(shard[0]), int(shard[1])]
     return key
 
 

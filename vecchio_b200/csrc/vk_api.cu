@@ -1,11 +1,13 @@
 // vk_api.cu -- the C ABI of include/vecchio_gpu.h: context, scene validation + upload (with the
 // GPU-side re-layout), render orchestration, the parity hook and the roofline microbenchmarks.
 // No CPU fallback anywhere: every entry point either runs CUDA kernels or returns an error.
+#include <chrono>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <functional>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include <cub/device/device_select.cuh>
@@ -123,9 +125,15 @@ __global__ void k_to_color_frames(const float* __restrict__ sum, uint8_t* __rest
     out[i] = (uint8_t)__float2uint_rz(256.0f * v);
 }
 // ---- adaptive sampling (vk_render_adaptive) ----
-__global__ void k_iota(uint32_t* list, uint32_t n) {
+// The pixels shard `shard` of n_shards owns (include/vecchio_gpu.h, vk_adaptive_begin_shard): pixel g belongs to shard
+// (g / VK_SHARD_RUN) mod n_shards.  A fresh refine's pass-0 list: the n_owned owned pixels of n_pix, ascending (entry i
+// lies in the shard's run i / VK_SHARD_RUN); with one shard, every pixel.
+__device__ __forceinline__ bool shard_owns(uint32_t p, uint32_t shard, uint32_t n_shards) {
+    return (p / VK_SHARD_RUN) % n_shards == shard;
+}
+__global__ void k_shard_list(uint32_t* list, uint32_t n_owned, uint32_t shard, uint32_t n_shards) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) list[i] = i;
+    if (i < n_owned) list[i] = ((i / VK_SHARD_RUN) * n_shards + shard) * VK_SHARD_RUN + i % VK_SHARD_RUN;
 }
 // The largest channel error e of pixel p after n >= 2 samples (include/vecchio_gpu.h states it), from the integer sums
 // alone, so that it does not depend on the order the samples arrived in.  Every operation is IEEE double, rounded to
@@ -165,15 +173,17 @@ __global__ void k_adaptive_select(const uint32_t* __restrict__ list, uint32_t n,
 }
 // A refine of a session that already holds samples: the rule of the new target for every pixel below its cap.  level[p] =
 // n_p / pass_spp + 1 for a pixel that renders on (its count is on the pass grid, see vk_adaptive_refine), 0 otherwise;
-// n_level[l] counts the pixels that render on from level l (one atomic per warp and level).
+// n_level[l] counts the pixels that render on from level l (one atomic per warp and level).  A shard's pixels it does not
+// own stay at level 0: they are never listed.
 __global__ void k_adaptive_levels(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
                                   const uint32_t* __restrict__ nspp, uint32_t n_pix, uint32_t spp, uint32_t min_spp, float max_error,
-                                  uint32_t pass_spp, uint32_t* __restrict__ level, uint32_t* __restrict__ n_level) {
+                                  uint32_t pass_spp, uint32_t shard, uint32_t n_shards, uint32_t* __restrict__ level,
+                                  uint32_t* __restrict__ n_level) {
     const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     uint32_t lv = 0;
     if (i < n_pix) {
         const uint32_t n = nspp[i];
-        if (!adaptive_stop(acc, sq, i, n, spp, min_spp, max_error)) lv = n / pass_spp + 1u;
+        if (shard_owns(i, shard, n_shards) && !adaptive_stop(acc, sq, i, n, spp, min_spp, max_error)) lv = n / pass_spp + 1u;
         level[i] = lv;
     }
     const unsigned peers = __match_any_sync(0xFFFFFFFFu, lv);
@@ -1041,6 +1051,7 @@ struct vk_adaptive_session {
     std::vector<vk_camera> cams;
     vk_render_params P{}; // P.spp: the session's limit
     uint32_t n_frames = 0, pass_spp = 0, n_pix = 0, max_levels = 0;
+    uint32_t shard = 0, n_shards = 1, n_owned = 0; // the pixels the pass loop renders: shard_owns(p, shard, n_shards), n_owned of them
     RenderPlan R{};
     uint64_t scene_gen = 0;
     bool reached_any = false; // a target has been reached (or imported); false: every count is 0
@@ -1091,9 +1102,20 @@ static int check_adaptive(vk_ctx* c, const std::string& w, const vk_camera* cam,
     return VK_OK;
 }
 
-// Checks, plans the kernel, sizes s's buffers (a larger block than needed is reused) and zeroes its state.
+// How many of n_pix pixels shard `shard` of n_shards owns (k_shard_list's rule): whole runs, less the missing tail of the
+// last run when the shard owns it.
+static uint32_t shard_pixels(uint32_t n_pix, uint32_t shard, uint32_t n_shards) {
+    const uint32_t runs = (n_pix + VK_SHARD_RUN - 1) / VK_SHARD_RUN;
+    if (runs <= shard) return 0u;
+    const uint32_t owned_runs = (runs - 1u - shard) / n_shards + 1u;
+    const uint32_t tail = (runs - 1u) % n_shards == shard ? runs * VK_SHARD_RUN - n_pix : 0u;
+    return owned_runs * VK_SHARD_RUN - tail;
+}
+
+// Checks, plans the kernel, sizes s's buffers (a larger block than needed is reused) and zeroes its state.  The kernel is
+// planned on the whole batch whatever the shard, so every shard runs the kernel the unsharded session runs.
 static int adaptive_begin(vk_ctx* c, const std::string& w, const vk_camera* cam, uint32_t n_frames, const vk_render_params* P,
-                          uint32_t pass_spp, float max_error, vk_adaptive_session* s) {
+                          uint32_t pass_spp, float max_error, vk_adaptive_session* s, uint32_t shard = 0, uint32_t n_shards = 1) {
     s->c = c;
     int rc = check_adaptive(c, w, cam, n_frames, P, pass_spp, max_error);
     if (rc != VK_OK) return rc;
@@ -1145,6 +1167,9 @@ static int adaptive_begin(vk_ctx* c, const std::string& w, const vk_camera* cam,
     s->n_frames = n_frames;
     s->pass_spp = pass_spp;
     s->n_pix = n_pix;
+    s->shard = shard;
+    s->n_shards = n_shards;
+    s->n_owned = shard_pixels(n_pix, shard, n_shards);
     s->max_levels = max_levels;
     s->R = R;
     s->scene_gen = c->scene_gen;
@@ -1197,14 +1222,15 @@ static int adaptive_refine(vk_adaptive_session* s, const vk_adaptive_target& T, 
         return VK_OK;
     };
     uint32_t lvl = 0, n_active = 0;
-    if (fresh) {
-        k_iota<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(cur, n_pix); // every pixel from level 0, ascending
+    if (s->n_owned == 0) { // a shard without pixels: nothing to render, and the target is reached
+    } else if (fresh) {
+        n_active = s->n_owned; // every owned pixel from level 0, ascending
+        k_shard_list<<<(n_active + 255) / 256, 256, 0, c->stream>>>(cur, n_active, s->shard, s->n_shards);
         *launches += 1;
-        n_active = n_pix;
     } else {
         CU(c, cudaMemsetAsync(s->n_level, 0, n_levels * sizeof(uint32_t), c->stream));
         k_adaptive_levels<<<(n_pix + 255) / 256, 256, 0, c->stream>>>(s->acc, s->sq, s->nspp, n_pix, T.spp, T.min_spp, T.max_error, M,
-                                                                      s->level, s->n_level);
+                                                                      s->shard, s->n_shards, s->level, s->n_level);
         *launches += 1;
         CU(c, cudaGetLastError());
         CU(c, cudaMemcpyAsync(h_level, s->n_level, n_levels * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1364,20 +1390,32 @@ int vk_render_frames_adaptive_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_
     return render_adaptive(c, "vk_render_frames_adaptive_rgb8", cams, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats, n_frames);
 }
 
-int vk_adaptive_begin(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
-                      vk_adaptive_session** out) {
+// shared body of vk_adaptive_begin and vk_adaptive_begin_shard
+static int begin_session(vk_ctx* c, const std::string& w, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
+                         uint32_t pass_spp, uint32_t shard, uint32_t n_shards, vk_adaptive_session** out) {
     if (!c) return VK_ERR_INVALID;
-    if (!out || !cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_adaptive_begin: null argument or no frames");
+    if (!out || !cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, w + ": null argument or no frames");
     *out = nullptr;
+    if (n_shards == 0 || shard >= n_shards) return fail(c, VK_ERR_INVALID, w + ": shard must be < n_shards (and n_shards >= 1)");
     vk_adaptive_session* s = new vk_adaptive_session;
     s->c = c;
-    const int rc = adaptive_begin(c, "vk_adaptive_begin", cams, n_frames, P, pass_spp, 0.0f, s);
+    const int rc = adaptive_begin(c, w, cams, n_frames, P, pass_spp, 0.0f, s, shard, n_shards);
     if (rc != VK_OK) {
         adaptive_free(s);
         return rc;
     }
     *out = s;
     return VK_OK;
+}
+
+int vk_adaptive_begin(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                      vk_adaptive_session** out) {
+    return begin_session(c, "vk_adaptive_begin", cams, n_frames, P, pass_spp, 0, 1, out);
+}
+
+int vk_adaptive_begin_shard(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                            uint32_t shard, uint32_t n_shards, vk_adaptive_session** out) {
+    return begin_session(c, "vk_adaptive_begin_shard", cams, n_frames, P, pass_spp, shard, n_shards, out);
 }
 
 int vk_adaptive_refine(vk_adaptive_session* s, const vk_adaptive_target* T, vk_stats* stats) {
@@ -1425,11 +1463,9 @@ int vk_adaptive_read_rgb8(vk_adaptive_session* s, uint8_t* out_rgb8, uint32_t* o
     return adaptive_read_call(s, "vk_adaptive_read_rgb8", nullptr, out_rgb8, out_spp, out_error);
 }
 
-int vk_adaptive_export(vk_adaptive_session* s, int64_t* sums, uint64_t* squares, uint32_t* counts, vk_adaptive_target* reached) {
-    if (!s) return VK_ERR_INVALID;
+// The state into host arrays (vk_adaptive_export's layout).
+static int adaptive_export(vk_adaptive_session* s, int64_t* sums, uint64_t* squares, uint32_t* counts, vk_adaptive_target* reached) {
     vk_ctx* c = s->c;
-    if (!sums || !squares || !counts) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: null argument");
-    if (s->broken) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: an earlier refine or import failed part way; the session's state is lost");
     const size_t n_pix = s->n_pix;
     CU(c, cudaSetDevice(c->device));
     CU(c, cudaMemcpyAsync(sums, s->acc, n_pix * 3 * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1440,24 +1476,39 @@ int vk_adaptive_export(vk_adaptive_session* s, int64_t* sums, uint64_t* squares,
     return VK_OK;
 }
 
-int vk_adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
-                       const vk_adaptive_target* reached) {
+int vk_adaptive_export(vk_adaptive_session* s, int64_t* sums, uint64_t* squares, uint32_t* counts, vk_adaptive_target* reached) {
     if (!s) return VK_ERR_INVALID;
     vk_ctx* c = s->c;
-    if (!sums || !squares || !counts || !reached) return fail(c, VK_ERR_INVALID, "vk_adaptive_import: null argument");
-    const vk_adaptive_target& A = *reached;
-    const std::string w = "vk_adaptive_import: ";
+    if (!sums || !squares || !counts) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: null argument");
+    if (s->broken) return fail(c, VK_ERR_INVALID, "vk_adaptive_export: an earlier refine or import failed part way; the session's state is lost");
+    return adaptive_export(s, sums, squares, counts, reached);
+}
+
+// What vk_adaptive_import refuses of a state for s (`w` prefixes the message); VK_OK when s may take it.
+static int adaptive_import_check(vk_adaptive_session* s, const std::string& w, const int64_t* sums, const uint64_t* squares,
+                                 const uint32_t* counts, const vk_adaptive_target& A) {
+    vk_ctx* c = s->c;
     if (A.spp > s->P.spp) return fail(c, VK_ERR_INVALID, w + "the reached spp exceeds the session's limit params->spp");
     if (!(A.max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, w + "the reached max_error must be >= 0 (and not NaN)");
     if (A.spp == 0 && (A.min_spp != 0 || A.max_error != 0.0f)) return fail(c, VK_ERR_INVALID, w + "a state that reached no target has spp, min_spp and max_error 0");
     for (size_t p = 0; p < s->n_pix; ++p) {
         const uint32_t n = counts[p];
+        const bool nonzero = (sums[3 * p] | sums[3 * p + 1] | sums[3 * p + 2] | (int64_t)(squares[3 * p] | squares[3 * p + 1] | squares[3 * p + 2])) != 0;
+        if (s->n_shards > 1 && (p / VK_SHARD_RUN) % s->n_shards != s->shard && (n != 0 || nonzero))
+            return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " is not this shard's but has samples or non-zero sums");
         if (n > A.spp) return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has more samples than the reached spp");
         if (n % s->pass_spp != 0 && n != A.spp)
             return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has a count off the pass grid (neither a multiple of pass_spp nor the reached spp)");
-        if (n == 0 && (sums[3 * p] | sums[3 * p + 1] | sums[3 * p + 2] | (int64_t)(squares[3 * p] | squares[3 * p + 1] | squares[3 * p + 2])) != 0)
+        if (n == 0 && nonzero)
             return fail(c, VK_ERR_INVALID, w + "pixel " + std::to_string(p) + " has no samples but non-zero sums");
     }
+    return VK_OK;
+}
+
+// Replaces s's state by the checked arrays.
+static int adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
+                           const vk_adaptive_target& A) {
+    vk_ctx* c = s->c;
     const size_t n_pix = s->n_pix;
     CU(c, cudaSetDevice(c->device));
     s->broken = true; // until every array has arrived
@@ -1469,6 +1520,14 @@ int vk_adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64
     s->reached_any = A.spp != 0;
     s->broken = false;
     return VK_OK;
+}
+
+int vk_adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
+                       const vk_adaptive_target* reached) {
+    if (!s) return VK_ERR_INVALID;
+    if (!sums || !squares || !counts || !reached) return fail(s->c, VK_ERR_INVALID, "vk_adaptive_import: null argument");
+    const int rc = adaptive_import_check(s, "vk_adaptive_import: ", sums, squares, counts, *reached);
+    return rc != VK_OK ? rc : adaptive_import(s, sums, squares, counts, *reached);
 }
 
 uint32_t vk_adaptive_variant(const vk_adaptive_session* s) { return s ? s->R.variant : 0u; }
@@ -1548,10 +1607,48 @@ __global__ void k_reduce_peers(PeerAcc pa, size_t n, float* __restrict__ sum, fl
         sumsq[i] = (float)q;
     }
 }
+// An adaptive session over the devices of a vk_multi (vk_multi_adaptive_*): device k holds shard k of n, an ordinary
+// shard session (vk_adaptive_begin_shard's pixels) whose pass loop runs on its own thread during a refine.  A read or an
+// export first gathers the owners' states into `comp`, an unsharded session's buffers on device 0, and then runs the
+// single-context code on it.
+struct vk_multi_adaptive_session {
+    vk_multi* m = nullptr;
+    std::vector<vk_adaptive_session*> shard; // shard k on device k
+    vk_adaptive_session* comp = nullptr;     // device 0: the whole state, gathered from the shards
+    bool comp_current = false;               // comp holds the shards' present state
+    bool broken = false;                     // a refine or import failed part way on some shard: the state is lost
+};
+static void multi_adaptive_free(vk_multi_adaptive_session* ms) {
+    if (!ms) return;
+    for (vk_adaptive_session* s : ms->shard) adaptive_free(s);
+    adaptive_free(ms->comp);
+    delete ms;
+}
+// every pixel's sums, squares and count from the shard that owns it; the shards of devices 1.. are read over NVLink
+// (vk_multi_create maps their memory on device 0)
+struct ShardState {
+    const unsigned long long* acc[VK_MULTI_MAX];
+    const unsigned long long* sq[VK_MULTI_MAX];
+    const uint32_t* nspp[VK_MULTI_MAX];
+    uint32_t n;
+};
+__global__ void k_gather_shards(ShardState st, uint32_t n_pix, unsigned long long* __restrict__ acc, unsigned long long* __restrict__ sq,
+                                uint32_t* __restrict__ nspp) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_pix) return;
+    const uint32_t k = (i / VK_SHARD_RUN) % st.n;
+    for (uint32_t ch = 0; ch < 3u; ++ch) {
+        acc[3u * i + ch] = st.acc[k][3u * i + ch];
+        sq[3u * i + ch] = st.sq[k][3u * i + ch];
+    }
+    nspp[i] = st.nspp[k][i];
+}
+
 struct vk_multi {
     std::vector<vk_ctx*> ctx;
     std::vector<cudaEvent_t> done; // device k's slice has finished (recorded on its stream)
     std::string err;
+    vk_multi_adaptive_session* oneshot = nullptr; // vk_multi_render_*adaptive_rgb8: the session each call begins, refines and reads
 };
 static thread_local std::string g_multi_err;
 static int mfail(vk_multi* m, int code, const std::string& msg) {
@@ -1606,6 +1703,7 @@ int vk_multi_create(const int* devices, int n, vk_multi** out) {
 }
 void vk_multi_destroy(vk_multi* m) {
     if (!m) return;
+    multi_adaptive_free(m->oneshot);
     for (size_t i = 0; i < m->ctx.size(); ++i) {
         if (i < m->done.size() && m->done[i]) {
             cudaSetDevice(m->ctx[i]->device);
@@ -1765,6 +1863,237 @@ int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_f
     if (stats) *stats = st;
     return VK_OK;
 }
+
+// ---- adaptive sessions over several GPUs (include/vecchio_gpu.h, vk_multi_adaptive_begin) ----
+static const char* const k_multi_lost = ": an earlier refine or import failed part way; the session's state is lost";
+
+// Checks and begins shard k of n on device k, and the composite on device 0, all with zero state.
+static int multi_adaptive_begin(vk_multi* m, const std::string& w, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
+                                uint32_t pass_spp, float max_error, vk_multi_adaptive_session* ms) {
+    const uint32_t n = (uint32_t)m->ctx.size();
+    ms->m = m;
+    ms->shard.resize(n, nullptr);
+    for (uint32_t k = 0; k < n; ++k) {
+        if (!ms->shard[k]) ms->shard[k] = new vk_adaptive_session;
+        const int rc = adaptive_begin(m->ctx[k], w, cams, n_frames, P, pass_spp, max_error, ms->shard[k], k, n);
+        if (rc != VK_OK) return mfail(m, rc, m->ctx[k]->err);
+    }
+    if (!ms->comp) ms->comp = new vk_adaptive_session;
+    const int rc = adaptive_begin(m->ctx[0], w, cams, n_frames, P, pass_spp, max_error, ms->comp);
+    if (rc != VK_OK) return mfail(m, rc, m->ctx[0]->err);
+    ms->comp_current = true; // (zero, like every shard)
+    ms->broken = false;
+    return VK_OK;
+}
+
+// Every shard's refine to T at once, one host thread per device (each pass of a shard ends in a host synchronisation of its
+// device), all joined before the stats are summed: paths, rays, dropped samples and launches over all devices, ms_kernels
+// the slowest device's.
+static int multi_adaptive_refine(vk_multi_adaptive_session* ms, const std::string& w, const vk_adaptive_target& T, vk_stats* out) {
+    vk_multi* m = ms->m;
+    const size_t n = ms->shard.size();
+    for (size_t k = 0; k < n; ++k) {
+        vk_ctx* c = m->ctx[k];
+        if (!c->has_scene || c->scene_gen != ms->shard[k]->scene_gen) return mfail(m, VK_ERR_INVALID, w + ": the scene changed since the session began");
+    }
+    const std::string why = adaptive_refusal(ms->shard[0], T);
+    if (!why.empty()) return mfail(m, VK_ERR_INVALID, w + ": " + why);
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<int> rc(n, VK_OK);
+    std::vector<uint32_t> launches(n, 0u);
+    std::vector<uint64_t> paths(n, 0u);
+    std::vector<float> ms_k(n, 0.0f);
+    auto run = [&](size_t k) { rc[k] = adaptive_refine(ms->shard[k], T, &launches[k], &paths[k], &ms_k[k]); };
+    ms->comp_current = false;
+    ms->broken = true; // until every shard has reached T
+    {
+        std::vector<std::thread> threads;
+        for (size_t k = 1; k < n; ++k) {
+            try {
+                threads.emplace_back(run, k);
+            } catch (...) { // no thread to be had: this shard runs on the calling thread after shard 0
+                threads.emplace_back();
+            }
+        }
+        run(0);
+        for (size_t k = 1; k < n; ++k) {
+            if (threads[k - 1].joinable()) threads[k - 1].join();
+            else run(k);
+        }
+    }
+    vk_stats total{};
+    for (size_t k = 0; k < n; ++k) {
+        vk_ctx* c = m->ctx[k];
+        if (rc[k] != VK_OK) return mfail(m, rc[k], w + ": device " + std::to_string(c->device) + ": " + c->err);
+        c->launches += launches[k];
+        c->paths += paths[k];
+        vk_stats s{};
+        const int r = vk_flush_stats(c, &s);
+        if (r != VK_OK) return mfail(m, r, w + ": " + c->err);
+        total.paths += s.paths; total.rays += s.rays; total.dropped_samples += s.dropped_samples;
+        total.node_visits += s.node_visits; total.prim_tests += s.prim_tests; total.launches += s.launches;
+        total.ms_kernels = ms_k[k] > total.ms_kernels ? ms_k[k] : total.ms_kernels;
+    }
+    total.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    total.variant = ms->shard[0]->R.variant;
+    ms->broken = false;
+    if (out) *out = total;
+    return VK_OK;
+}
+
+// The composite on device 0 after a refine: one launch of k_gather_shards (a read or an export synchronises device 0
+// before it returns, so no shard is written while the gather reads it).
+static int multi_adaptive_composite(vk_multi_adaptive_session* ms, const std::string& w) {
+    if (ms->comp_current) return VK_OK;
+    vk_multi* m = ms->m;
+    vk_adaptive_session* cs = ms->comp;
+    ShardState st{};
+    st.n = (uint32_t)ms->shard.size();
+    for (uint32_t k = 0; k < st.n; ++k) {
+        st.acc[k] = ms->shard[k]->acc;
+        st.sq[k] = ms->shard[k]->sq;
+        st.nspp[k] = ms->shard[k]->nspp;
+    }
+    vk_ctx* c0 = m->ctx[0];
+    cudaError_t e = cudaSetDevice(c0->device);
+    if (e == cudaSuccess) {
+        k_gather_shards<<<(cs->n_pix + 255) / 256, 256, 0, c0->stream>>>(st, cs->n_pix, cs->acc, cs->sq, cs->nspp);
+        e = cudaGetLastError();
+    }
+    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, w + ": k_gather_shards: " + cudaGetErrorString(e));
+    cs->reached = ms->shard[0]->reached;
+    cs->reached_any = ms->shard[0]->reached_any;
+    ms->comp_current = true;
+    return VK_OK;
+}
+
+static int multi_adaptive_read_call(vk_multi_adaptive_session* ms, const std::string& w, float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp,
+                                    float* out_error) {
+    if (!ms) return VK_ERR_INVALID;
+    vk_multi* m = ms->m;
+    if (!out_rgb && !out_rgb8) return mfail(m, VK_ERR_INVALID, w + ": null argument");
+    if (ms->broken) return mfail(m, VK_ERR_INVALID, w + k_multi_lost);
+    int rc = multi_adaptive_composite(ms, w);
+    if (rc != VK_OK) return rc;
+    uint32_t launches = 0;
+    rc = adaptive_read(ms->comp, out_rgb, out_rgb8, out_spp, out_error, &launches);
+    return rc == VK_OK ? VK_OK : mfail(m, rc, w + ": " + m->ctx[0]->err);
+}
+
+// shared body of vk_multi_render_adaptive_rgb8 and vk_multi_render_frames_adaptive_rgb8: begin, one refine to
+// {spp, 0, max_error} and read, on the vk_multi's own session
+static int multi_render_adaptive(vk_multi* m, const std::string& w, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
+                                 uint32_t pass_spp, float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    const auto t0 = std::chrono::steady_clock::now();
+    if (!m->oneshot) m->oneshot = new vk_multi_adaptive_session;
+    vk_multi_adaptive_session* ms = m->oneshot;
+    int rc = multi_adaptive_begin(m, w, cams, n_frames, P, pass_spp, max_error, ms);
+    if (rc != VK_OK) return rc;
+    vk_stats st{};
+    if ((rc = multi_adaptive_refine(ms, w, vk_adaptive_target{P->spp, 0u, max_error}, &st)) != VK_OK) return rc;
+    if ((rc = multi_adaptive_read_call(ms, w, nullptr, out_rgb8, out_spp, nullptr)) != VK_OK) return rc;
+    st.launches += 2; // (the gather and the readout)
+    st.ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+int vk_multi_render_adaptive_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
+                                  uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!m) return VK_ERR_INVALID;
+    if (!cam || !P || !out_rgb8) return mfail(m, VK_ERR_INVALID, "vk_multi_render_adaptive_rgb8: null argument");
+    return multi_render_adaptive(m, "vk_multi_render_adaptive_rgb8", cam, 1, P, pass_spp, max_error, out_rgb8, out_spp, stats);
+}
+
+int vk_multi_render_frames_adaptive_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                                         float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!m) return VK_ERR_INVALID;
+    if (!cams || !P || !out_rgb8 || n_frames == 0)
+        return mfail(m, VK_ERR_INVALID, "vk_multi_render_frames_adaptive_rgb8: null argument or no frames");
+    return multi_render_adaptive(m, "vk_multi_render_frames_adaptive_rgb8", cams, n_frames, P, pass_spp, max_error, out_rgb8, out_spp, stats);
+}
+
+int vk_multi_adaptive_begin(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                            vk_multi_adaptive_session** out) {
+    if (!m) return VK_ERR_INVALID;
+    if (!out || !cams || !P || n_frames == 0) return mfail(m, VK_ERR_INVALID, "vk_multi_adaptive_begin: null argument or no frames");
+    *out = nullptr;
+    vk_multi_adaptive_session* ms = new vk_multi_adaptive_session;
+    const int rc = multi_adaptive_begin(m, "vk_multi_adaptive_begin", cams, n_frames, P, pass_spp, 0.0f, ms);
+    if (rc != VK_OK) {
+        multi_adaptive_free(ms);
+        return rc;
+    }
+    *out = ms;
+    return VK_OK;
+}
+
+int vk_multi_adaptive_refine(vk_multi_adaptive_session* ms, const vk_adaptive_target* T, vk_stats* stats) {
+    if (!ms) return VK_ERR_INVALID;
+    if (!T) return mfail(ms->m, VK_ERR_INVALID, "vk_multi_adaptive_refine: null target");
+    if (ms->broken) return mfail(ms->m, VK_ERR_INVALID, std::string("vk_multi_adaptive_refine") + k_multi_lost);
+    return multi_adaptive_refine(ms, "vk_multi_adaptive_refine", *T, stats);
+}
+
+int vk_multi_adaptive_read(vk_multi_adaptive_session* ms, float* out_rgb, uint32_t* out_spp, float* out_error) {
+    return multi_adaptive_read_call(ms, "vk_multi_adaptive_read", out_rgb, nullptr, out_spp, out_error);
+}
+
+int vk_multi_adaptive_read_rgb8(vk_multi_adaptive_session* ms, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error) {
+    return multi_adaptive_read_call(ms, "vk_multi_adaptive_read_rgb8", nullptr, out_rgb8, out_spp, out_error);
+}
+
+int vk_multi_adaptive_export(vk_multi_adaptive_session* ms, int64_t* sums, uint64_t* squares, uint32_t* counts, vk_adaptive_target* reached) {
+    if (!ms) return VK_ERR_INVALID;
+    vk_multi* m = ms->m;
+    const std::string w = "vk_multi_adaptive_export";
+    if (!sums || !squares || !counts) return mfail(m, VK_ERR_INVALID, w + ": null argument");
+    if (ms->broken) return mfail(m, VK_ERR_INVALID, w + k_multi_lost);
+    int rc = multi_adaptive_composite(ms, w);
+    if (rc != VK_OK) return rc;
+    rc = adaptive_export(ms->comp, sums, squares, counts, reached);
+    return rc == VK_OK ? VK_OK : mfail(m, rc, w + ": " + m->ctx[0]->err);
+}
+
+// The whole state is checked as vk_adaptive_import checks it (which is what every shard's check of its part adds up to:
+// the parts carry zeros on the pixels a shard does not own), then each shard takes its owned pixels and the composite
+// takes the whole.
+int vk_multi_adaptive_import(vk_multi_adaptive_session* ms, const int64_t* sums, const uint64_t* squares, const uint32_t* counts,
+                             const vk_adaptive_target* reached) {
+    if (!ms) return VK_ERR_INVALID;
+    vk_multi* m = ms->m;
+    const std::string w = "vk_multi_adaptive_import: ";
+    if (!sums || !squares || !counts || !reached) return mfail(m, VK_ERR_INVALID, w + "null argument");
+    vk_adaptive_session* cs = ms->comp;
+    int rc = adaptive_import_check(cs, w, sums, squares, counts, *reached);
+    if (rc != VK_OK) return mfail(m, rc, m->ctx[0]->err);
+    const size_t n_pix = cs->n_pix, n = ms->shard.size();
+    ms->broken = true; // until every shard has its part
+    ms->comp_current = false;
+    std::vector<int64_t> s_part(n_pix * 3);
+    std::vector<uint64_t> q_part(n_pix * 3);
+    std::vector<uint32_t> n_part(n_pix);
+    for (size_t k = 0; k < n; ++k) {
+        for (size_t p = 0; p < n_pix; ++p) {
+            const bool own = (p / VK_SHARD_RUN) % n == k;
+            for (size_t ch = 0; ch < 3; ++ch) {
+                s_part[3 * p + ch] = own ? sums[3 * p + ch] : 0;
+                q_part[3 * p + ch] = own ? squares[3 * p + ch] : 0u;
+            }
+            n_part[p] = own ? counts[p] : 0u;
+        }
+        if ((rc = adaptive_import(ms->shard[k], s_part.data(), q_part.data(), n_part.data(), *reached)) != VK_OK)
+            return mfail(m, rc, w + m->ctx[k]->err);
+    }
+    if ((rc = adaptive_import(cs, sums, squares, counts, *reached)) != VK_OK) return mfail(m, rc, w + m->ctx[0]->err);
+    ms->comp_current = true;
+    ms->broken = false;
+    return VK_OK;
+}
+
+uint32_t vk_multi_adaptive_variant(const vk_multi_adaptive_session* ms) { return ms && !ms->shard.empty() ? ms->shard[0]->R.variant : 0u; }
+
+void vk_multi_adaptive_destroy(vk_multi_adaptive_session* ms) { multi_adaptive_free(ms); }
 
 int vk_eval_batch(vk_ctx* c, vk_eval* recs, size_t n, uint32_t flags) {
     if (!c) return VK_ERR_INVALID;
