@@ -17,8 +17,8 @@ its ListArgs twin (the same kernel over a pixel list of one frame) when the head
 Exit status 0 when every base kernel is in the head build and every head kernel either is in the base build or NEW,
 every matched kernel keeps its resources, every single-frame kernel is `same` and every other one `same` or
 `local-slots`.  A kernel named after --changed (its demangled name without namespace or arguments, e.g.
-k_to_color_adaptive) is one the change means to alter or add: it is listed with its verdict, or as NEW when the base build
-lacks it, and does not fail the comparison."""
+k_to_color) is one the change means to alter, add or remove: it is listed with its verdict, as NEW when the base
+build lacks it or as REMOVED when the head build does, and does not fail the comparison."""
 import collections, glob, os, re, shutil, subprocess, sys
 
 DOMAINS = ("OneFrame", "FrameArgs", "ListArgs", "FrameListArgs")
@@ -100,10 +100,14 @@ def main():
     base_domains = {d for _, d in base}
     short = lambda k: re.sub(r"<.*", "", k[0]).split("::")[-1]
     new = sorted(k for k in head.keys() - base.keys() if k[1] not in base_domains or short(k) in changed)
-    for k in sorted(base.keys() - head.keys()) + sorted(head.keys() - base.keys() - set(new)):
+    removed = sorted(k for k in base.keys() - head.keys() if short(k) in changed)
+    for k in sorted(base.keys() - head.keys() - set(removed)) + sorted(head.keys() - base.keys() - set(new)):
         print(f"UNMATCHED {'base' if k in base else 'head'}: {k[0]} [{k[1]}]")
         ok = False
     tally = collections.Counter()
+    for k in removed:
+        print(f"{k[0][:72]:<72} {k[1]:<13} {fmt(base[k][2]):>16}  REMOVED")
+        tally[(k[1], "REMOVED")] += 1
     if new:
         print(f"{'new kernel':<72} {'domain':<13} {'head':>16} {'ListArgs twin':>16}")
     for k in new:

@@ -85,8 +85,8 @@ def stops(e, counts, target):
 
 
 def means(sums, counts):
-    """k_finalize_adaptive: (float)((double)S * 2^-30) / (float)n per channel (0 / 0 = NaN for a pixel without
-    samples)."""
+    """k_finalize over an adaptive state (AccOverCount): (float)((double)S * 2^-30) / (float)n per channel (0 / 0 = NaN
+    for a pixel without samples)."""
     s = int64_to_double(sums) * 2.0 ** -30
     with np.errstate(divide="ignore", invalid="ignore"):
         return s.astype(np.float32) / np.asarray(counts, dtype=np.uint32).astype(np.float32)[..., None]

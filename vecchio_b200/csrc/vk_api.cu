@@ -35,7 +35,7 @@ struct vk_ctx {
     // do not fit fall back to their own allocation (scene_allocs) and the block grows before the next upload.
     char* arena = nullptr;
     size_t arena_cap = 0, arena_used = 0, arena_need = 0;
-    cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr}; // vk_render: D2H in chunks, copy-out of one while the next arrives
+    cudaEvent_t ev_chunk[4] = {nullptr, nullptr, nullptr, nullptr}; // readout: D2H in chunks, copy-out of one while the next arrives
     DScene scene{};
     FlatProgram flat{}; // flat.n == 0: scene too large, BVH traversal
     bool has_scene = false;
@@ -53,9 +53,9 @@ struct vk_ctx {
     float* sq_stack = nullptr; // step-queue kernel: overflow of the traversal stacks (allocated on first use)
     size_t sq_stack_floats = 0;
     uint32_t stack_need = 0, levels_sub = 0; // of the uploaded scene (vk_scene_info)
-    float* frame = nullptr; // vk_render staging: sum | sumsq | rgb
+    float* frame = nullptr; // device staging of a render call's results (Staging)
     size_t frame_floats = 0;
-    float* pinned = nullptr; // pinned host staging for the D2H of vk_render
+    float* pinned = nullptr; // pinned host staging of the results' copy back (Staging), and of the adaptive pass loop's counts
     size_t pinned_floats = 0;
     DCamera* cams = nullptr; // vk_render_frames: the batch's cameras on the device (FrameArgs::cams)
     size_t cams_cap = 0;
@@ -98,31 +98,45 @@ __global__ void k_acc_to_sum(const unsigned long long* __restrict__ acc, const d
     sum[i] = (float)((double)(long long)acc[i] * VK_ACC_INV_SCALE);
     if (sumsq) sumsq[i] = (float)accsq[i];
 }
-__global__ void k_finalize(const float* __restrict__ sum, float* __restrict__ rgb, size_t n, float spp) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) rgb[i] = sum[i] / spp; // c /= SAMPLES_PER_PIXEL as f32 (src/main.rs:196)
+// Where the readout kernels take a pixel's mean from (k_finalize, k_to_color).  SumsOverSpp: float sums (k_acc_to_sum's or
+// k_reduce_peers') over a constant spp, c /= SAMPLES_PER_PIXEL as f32 (src/main.rs:196).  AccOverCount: an adaptive state's
+// fixed-point sums over each pixel's own count; it forms k_acc_to_sum's float sum, (float)((double)(long long)acc *
+// VK_ACC_INV_SCALE), in a register and divides it by the float count as SumsOverSpp does, so a pixel that stopped at n
+// samples reads out as vk_render(spp = n) does, bit for bit.
+struct SumsOverSpp {
+    static constexpr bool counted = false;
+    const float* __restrict__ sum;
+    float spp;
+    __device__ float mean(size_t j) const { return sum[j] / spp; }
+};
+struct AccOverCount {
+    static constexpr bool counted = true;
+    const unsigned long long* __restrict__ acc;
+    const uint32_t* __restrict__ nspp;
+    __device__ float mean(size_t j) const { return (float)((double)(long long)acc[j] * VK_ACC_INV_SCALE) / (float)nspp[j / 3]; }
+};
+// The element of n_frames contiguous planes, in the accumulators' order (each frame's rows bottom-up), that element i of the
+// same planes top-down holds (the order of an rgb8 image and of the PPM, src/main.rs:209); a row is width * per elements.
+__device__ __forceinline__ size_t flip_rows(size_t i, uint32_t width, uint32_t height, uint32_t per) {
+    const size_t row_len = (size_t)width * per, frame = row_len * height, f = i / frame, k = i - f * frame, row = k / row_len;
+    return f * frame + (height - 1 - row) * row_len + (k - row * row_len);
 }
-// Vec3::to_color (src/vec3.rs:54-61) of sum / spp, rows flipped to the PPM's top-down order (src/main.rs:209)
-__global__ void k_to_color(const float* __restrict__ sum, uint8_t* __restrict__ out, uint32_t width, uint32_t height, float spp) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, n = (size_t)width * height * 3;
-    if (i >= n) return;
-    const size_t row = i / ((size_t)width * 3), col = i - row * (size_t)width * 3;
-    const float c = sum[(size_t)(height - 1 - row) * width * 3 + col] / spp; // c /= SAMPLES_PER_PIXEL (main.rs:196)
-    float v = sqrtf(c);
+template <class Src> __global__ void k_finalize(Src src, float* __restrict__ rgb, size_t n) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) rgb[i] = src.mean(i);
+}
+// Vec3::to_color (src/vec3.rs:54-61) of the means of n_frames frames, each frame top-down on its own; spp_out (AccOverCount,
+// nullable): the counts in the image's order
+template <class Src>
+__global__ void k_to_color(Src src, uint8_t* __restrict__ out, uint32_t* __restrict__ spp_out, uint32_t width, uint32_t height, uint32_t n_frames) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)width * height * 3 * n_frames) return;
+    const size_t j = flip_rows(i, width, height, 3);
+    float v = sqrtf(src.mean(j));
     v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v); // Vec3::clamp keeps NaN
     out[i] = (uint8_t)__float2uint_rz(256.0f * v);   // `as u32`: NaN -> 0
-}
-// k_to_color over n_frames frames of a batch (contiguous planes), each frame top-down on its own
-__global__ void k_to_color_frames(const float* __restrict__ sum, uint8_t* __restrict__ out, uint32_t width, uint32_t height, uint32_t n_frames,
-                                  float spp) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, plane = (size_t)width * height * 3;
-    if (i >= plane * n_frames) return;
-    const size_t f = i / plane, j = i - f * plane;
-    const size_t row = j / ((size_t)width * 3), col = j - row * (size_t)width * 3;
-    const float c = sum[f * plane + (size_t)(height - 1 - row) * width * 3 + col] / spp;
-    float v = sqrtf(c);
-    v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v);
-    out[i] = (uint8_t)__float2uint_rz(256.0f * v);
+    if constexpr (Src::counted)
+        if (spp_out && i % 3 == 0) spp_out[i / 3] = src.nspp[j / 3];
 }
 // ---- adaptive sampling (vk_render_adaptive) ----
 // The pixels shard `shard` of n_shards owns (include/vecchio_gpu.h, vk_adaptive_begin_shard): pixel g belongs to shard
@@ -194,39 +208,11 @@ __global__ void k_adaptive_levels(const unsigned long long* __restrict__ acc, co
 __global__ void k_adaptive_error_map(const unsigned long long* __restrict__ acc, const unsigned long long* __restrict__ sq,
                                      const uint32_t* __restrict__ nspp, float* __restrict__ out, uint32_t width, uint32_t height,
                                      uint32_t n_frames, bool top_down) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, frame = (size_t)width * height;
-    if (i >= frame * n_frames) return;
-    size_t p = i;
-    if (top_down) {
-        const size_t f = i / frame, k = i - f * frame, row = k / width;
-        p = f * frame + (height - 1 - row) * (size_t)width + (k - row * width);
-    }
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (size_t)width * height * n_frames) return;
+    const size_t p = top_down ? flip_rows(i, width, height, 1) : i;
     const uint32_t n = nspp[p];
     out[i] = n < 2u ? __int_as_float(0x7F800000) : (float)adaptive_error(acc, sq, (uint32_t)p, n);
-}
-// mean = sum / n_p with k_acc_to_sum's and k_finalize's operations, so a pixel that stopped at n equals vk_render(spp = n)
-__global__ void k_finalize_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, float* __restrict__ rgb,
-                                    size_t n) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float sum = (float)((double)(long long)acc[i] * VK_ACC_INV_SCALE);
-    rgb[i] = sum / (float)nspp[i / 3];
-}
-// k_to_color of the same means over n_frames contiguous planes, each frame top-down on its own; the counts follow the
-// image's order
-__global__ void k_to_color_adaptive(const unsigned long long* __restrict__ acc, const uint32_t* __restrict__ nspp, uint8_t* __restrict__ out,
-                                    uint32_t* __restrict__ spp_out, uint32_t width, uint32_t height, uint32_t n_frames) {
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x, plane = (size_t)width * height * 3;
-    if (i >= plane * n_frames) return;
-    const size_t f = i / plane, k = i - f * plane;
-    const size_t row = k / ((size_t)width * 3), col = k - row * (size_t)width * 3;
-    const size_t j = f * plane + (size_t)(height - 1 - row) * width * 3 + col;
-    const uint32_t np = nspp[j / 3];
-    const float c = (float)((double)(long long)acc[j] * VK_ACC_INV_SCALE) / (float)np;
-    float v = sqrtf(c);
-    v = v < 0.0f ? 0.0f : (v > 0.999f ? 0.999f : v);
-    out[i] = (uint8_t)__float2uint_rz(256.0f * v);
-    if (col % 3 == 0) spp_out[i / 3] = np;
 }
 // FP32 peak: 8 independent FFMA chains per thread, no memory traffic
 __global__ void k_ffma_peak(float* out, int iters) {
@@ -659,33 +645,43 @@ static void apply_l2_window(vk_ctx* c) {
     cudaGetLastError();
 }
 
-// What vk_render_frames* reject before anything is allocated or launched (`who` names the call in the message).
-static int check_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P) {
-    if (!cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, std::string(who) + ": null argument or no frames");
-    if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, std::string(who) + ": no scene uploaded");
-    for (uint32_t f = 0; f < n_frames; ++f)
-        if (!(cams[f].time0 < cams[f].time1))
-            return fail(c, VK_ERR_INVALID, std::string(who) + ": frame " + std::to_string(f) + ": camera time0 >= time1 (gen_range panics, src/main.rs:118)");
-    // the kernels index the accumulators of the whole batch with 32-bit pixels: render_into's bound for one frame, on the batch
-    if ((uint64_t)P->width * P->height * n_frames > 0x7FFFFFFFull / 3)
-        return fail(c, VK_ERR_INVALID, std::string(who) + ": batch too large (n_frames * width * height * 3 exceeds 2^31 - 1)");
-    if (n_frames > 1 && (P->variant == VK_VARIANT_STAGED || P->variant == VK_VARIANT_WAVEFRONT))
-        return fail(c, VK_ERR_UNSUPPORTED, std::string(who) + ": the staged and wavefront kernels render one frame per call");
+// The staged and wavefront kernels render one whole frame per launch: no batches of frames, no pixel lists (list: an
+// adaptive render's passes).  `variant`: the one asked for, or the one AUTO chose.
+static int check_variant(vk_ctx* c, const std::string& who, uint32_t variant, uint32_t n_frames, bool list) {
+    if (variant != VK_VARIANT_STAGED && variant != VK_VARIANT_WAVEFRONT) return VK_OK;
+    if (list) return fail(c, VK_ERR_UNSUPPORTED, who + ": the staged and wavefront kernels have no pixel-list passes");
+    if (n_frames > 1) return fail(c, VK_ERR_UNSUPPORTED, who + ": the staged and wavefront kernels render one frame per call");
     return VK_OK;
 }
 
-// What every render call checks of its camera and parameters before anything is launched.
-static int check_render(vk_ctx* c, const vk_camera* cam, const vk_render_params* P) {
-    if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, "render: no scene uploaded");
-    if (!cam || !P) return fail(c, VK_ERR_INVALID, "render: null argument");
-    if (P->width < 2 || P->height < 2) return fail(c, VK_ERR_INVALID, "render: width/height must be >= 2 ((width-1) divides, src/main.rs:187)");
-    if (P->spp == 0 || P->spp_begin >= P->spp) return fail(c, VK_ERR_INVALID, "render: bad spp / spp_begin");
+// What every render call refuses of its cameras and parameters before anything is allocated or launched (`who` names the
+// call in the message).  adaptive: a render in passes over pixel lists (vk_render_adaptive*, vk_adaptive_begin*), with its
+// pass_spp and the one-shot calls' max_error (a session checks its targets in refine).
+static int check_render(vk_ctx* c, const std::string& who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
+                        bool adaptive = false, uint32_t pass_spp = 0, float max_error = 0.0f) {
+    if (!cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, who + ": null argument or no frames");
+    if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, who + ": no scene uploaded");
+    if (P->width < 2 || P->height < 2) return fail(c, VK_ERR_INVALID, who + ": width/height must be >= 2 ((width-1) divides, src/main.rs:187)");
+    if (P->spp == 0 || P->spp_begin >= P->spp) return fail(c, VK_ERR_INVALID, who + ": bad spp / spp_begin");
     const uint32_t count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
-    if ((uint64_t)P->spp_begin + count > P->spp) return fail(c, VK_ERR_INVALID, "render: sample slice exceeds spp");
-    if ((uint64_t)P->width * P->height > 0x7FFFFFFFull / 3) return fail(c, VK_ERR_INVALID, "render: image too large");
-    if (P->variant > VK_VARIANT_STEPQ) return fail(c, VK_ERR_INVALID, "render: unknown variant");
-    if (!(cam->time0 < cam->time1)) return fail(c, VK_ERR_INVALID, "render: camera time0 >= time1 (gen_range panics, src/main.rs:118)");
-    return VK_OK;
+    if ((uint64_t)P->spp_begin + count > P->spp) return fail(c, VK_ERR_INVALID, who + ": sample slice exceeds spp");
+    // the kernels index the accumulators of the whole batch with 32-bit element indices
+    if ((uint64_t)P->width * P->height * n_frames > 0x7FFFFFFFull / 3)
+        return fail(c, VK_ERR_INVALID, who + ": image too large (n_frames * width * height * 3 exceeds 2^31 - 1)");
+    if (P->variant > VK_VARIANT_STEPQ) return fail(c, VK_ERR_INVALID, who + ": unknown variant");
+    for (uint32_t f = 0; f < n_frames; ++f)
+        if (!(cams[f].time0 < cams[f].time1))
+            return fail(c, VK_ERR_INVALID, who + ": frame " + std::to_string(f) + ": camera time0 >= time1 (gen_range panics, src/main.rs:118)");
+    if (adaptive) {
+        if (pass_spp == 0) return fail(c, VK_ERR_INVALID, who + ": pass_spp must be >= 1");
+        if (!(max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, who + ": max_error must be >= 0 (and not NaN)");
+        if (P->spp_begin != 0 || (P->spp_count != 0 && P->spp_count != P->spp))
+            return fail(c, VK_ERR_INVALID, who + ": an adaptive render draws samples [0, n_p) of every pixel: spp_begin must be 0, spp_count 0 or spp");
+        if (P->spp > VK_ADAPTIVE_MAX_SPP)
+            return fail(c, VK_ERR_INVALID, who + ": spp above " + std::to_string(VK_ADAPTIVE_MAX_SPP) +
+                                               ", the limit of the fixed-point sums of squares (2^16 samples of at most 255^2 * 2^32 units)");
+    }
+    return check_variant(c, who, P->variant, n_frames, adaptive);
 }
 
 // The kernel a call runs and how it is launched, decided once per call (an adaptive render runs every pass on it).
@@ -696,7 +692,8 @@ struct RenderPlan {
     int grid;
     uint32_t resident_warps;
 };
-static int plan_render(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, RenderPlan* R) {
+// (check_render has passed; list: the passes of an adaptive render)
+static int plan_render(vk_ctx* c, const std::string& who, const vk_render_params* P, uint32_t n_frames, bool list, RenderPlan* R) {
     R->strict = (P->flags & VK_FLAG_STRICT_MATH) != 0;
     const bool strict = R->strict;
     const FlatProgram* flat = (c->flat.n && !(P->flags & VK_FLAG_FORCE_BVH)) ? &c->flat : nullptr;
@@ -708,11 +705,10 @@ static int plan_render(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, 
     // (lane megakernel on it: 51.5 against 46.1 ms on the final scene, profiles/r2_sweep_12.log)
     if (flat && flat->n_bvh && variant != VK_VARIANT_WARPQ && !std::getenv("VECCHIO_HYBRID_ALL")) flat = nullptr;
     if (legacy && c->has_specdiffuse)
-        return fail(c, VK_ERR_UNSUPPORTED, "render: SpecDiffuse has no legacy scatter (the reference's default unwraps a missing specular ray and panics, src/material.rs:21-28)");
+        return fail(c, VK_ERR_UNSUPPORTED, who + ": SpecDiffuse has no legacy scatter (the reference's default unwraps a missing specular ray and panics, src/material.rs:21-28)");
     if (!legacy && c->scene.n_lights == 0)
-        return fail(c, VK_ERR_INVALID, "render: empty light list (the reference panics: choose().unwrap(), src/hittable.rs:431); only VK_FLAG_LEGACY_SCATTER renders without lights");
-    if (n_frames > 1 && (variant == VK_VARIANT_STAGED || variant == VK_VARIANT_WAVEFRONT))
-        return fail(c, VK_ERR_UNSUPPORTED, "render: the staged and wavefront kernels render one frame per call");
+        return fail(c, VK_ERR_INVALID, who + ": empty light list (the reference panics: choose().unwrap(), src/hittable.rs:431); only VK_FLAG_LEGACY_SCATTER renders without lights");
+    if (const int rc = check_variant(c, who, variant, n_frames, list); rc != VK_OK) return rc;
     // the render build compiled for a light list of one unflipped Rect (VK_LIGHT0, see vk_device.cuh)
     const bool l0 = !strict && !legacy && c->one_rect_light && !c->has_specdiffuse && !std::getenv("VECCHIO_NO_LIGHT0");
     CU(c, strict ? vkstrict::megakernel_occupancy(flat != nullptr, c->scene.has_media, legacy, &bps, &bt)
@@ -781,8 +777,8 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
 
     CU(c, cudaMemsetAsync(c->counters + 2, 0, sizeof(unsigned long long), c->stream)); // work-queue head only
     const DCamera dc = to_dcam(cam);
-    // the variant switch, for the work domain `dom` (staged and wavefront have none: plan_render and render_adaptive keep
-    // batches and pixel lists away from them)
+    // the variant switch, for the work domain `dom` (staged and wavefront have none: check_variant keeps batches and pixel
+    // lists away from them)
     auto run = [&](const auto& dom) -> int {
         if (variant == VK_VARIANT_STEPQ) {
             const bool inst = c->levels_sub != 0u;
@@ -851,19 +847,19 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
 // shared body of vk_render / vk_render_device / vk_render_frames*
 // acc_only: leave the result in the context's integer accumulators (c->partial) and skip the conversion to fp32 sums
 // (the multi-GPU context reduces the accumulators of all its devices itself); want_sq then says whether squares are kept
-// n_frames > 1: cam points to n_frames cameras and the result is n_frames contiguous planes (check_frames has passed; the
-// batch kernels take FrameArgs, everything else is the single-frame path)
+// n_frames > 1: cam points to n_frames cameras and the result is n_frames contiguous planes (the batch kernels take
+// FrameArgs, everything else is the single-frame path)
 static int render_into(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* d_sum, float* d_sumsq, vk_stats* stats,
                        bool acc_only = false, bool want_sq = false, uint32_t n_frames = 1) {
     if (!c) return VK_ERR_INVALID;
-    int rc = check_render(c, cam, P);
+    int rc = check_render(c, "render", cam, n_frames, P);
     if (rc != VK_OK) return rc;
     if (!d_sum && !acc_only) return fail(c, VK_ERR_INVALID, "render: null argument");
     if (!acc_only) want_sq = d_sumsq != nullptr;
     const uint32_t count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
     CU(c, cudaSetDevice(c->device));
     RenderPlan R;
-    if ((rc = plan_render(c, P, n_frames, &R)) != VK_OK) return rc;
+    if ((rc = plan_render(c, "render", P, n_frames, false, &R)) != VK_OK) return rc;
 
     // Accumulators (see RenderBuffers): u64 fixed-point sums, plus double sums of squares when asked for.
     const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
@@ -906,7 +902,7 @@ int vk_render_device(vk_ctx* c, const vk_camera* cam, const vk_render_params* P,
 int vk_finalize_device(vk_ctx* c, const float* d_sum, float* d_rgb, size_t n, uint32_t spp) {
     if (!c || !d_sum || !d_rgb || spp == 0) return fail(c, VK_ERR_INVALID, "vk_finalize_device: bad argument");
     CU(c, cudaSetDevice(c->device));
-    if (n) k_finalize<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d_sum, d_rgb, n, (float)spp);
+    if (n) k_finalize<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(SumsOverSpp{d_sum, (float)spp}, d_rgb, n);
     c->launches += n ? 1 : 0;
     CU(c, cudaGetLastError());
     return VK_OK;
@@ -941,109 +937,6 @@ int vk_flush_stats(vk_ctx* c, vk_stats* stats) {
     return VK_OK;
 }
 
-int vk_render(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* out_rgb, float* out_sumsq, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!P || !out_rgb) return fail(c, VK_ERR_INVALID, "vk_render: null argument");
-    const size_t plane = (size_t)P->width * P->height * 3;
-    CU(c, cudaSetDevice(c->device));
-    int rc = ensure(c, &c->frame, &c->frame_floats, plane * 3);
-    if (rc != VK_OK) return rc;
-    if ((rc = ensure_pinned(c, plane * 2)) != VK_OK) return rc;
-    float *d_sum = c->frame, *d_sq = out_sumsq ? c->frame + plane : nullptr, *d_rgb = c->frame + 2 * plane;
-    CU(c, cudaEventRecord(c->ev2, c->stream));
-    vk_stats st{};
-    rc = render_into(c, cam, P, d_sum, d_sq, &st);
-    if (rc != VK_OK) return rc;
-    k_finalize<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, d_rgb, plane, (float)P->spp);
-    CU(c, cudaGetLastError());
-    // the frame comes back in four chunks: the caller's (pageable) buffer is filled from the pinned staging chunk by chunk
-    // while the later chunks are still on the bus
-    constexpr int NCH = 4;
-    size_t off[NCH + 1];
-    for (int i = 0; i <= NCH; ++i) off[i] = plane * (size_t)i / NCH;
-    for (int i = 0; i < NCH; ++i) {
-        if (!c->ev_chunk[i]) CU(c, cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
-        CU(c, cudaMemcpyAsync(c->pinned + off[i], d_rgb + off[i], (off[i + 1] - off[i]) * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        CU(c, cudaEventRecord(c->ev_chunk[i], c->stream));
-    }
-    if (out_sumsq) CU(c, cudaMemcpyAsync(c->pinned + plane, d_sq, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    CU(c, cudaEventRecord(c->ev1, c->stream));
-    for (int i = 0; i < NCH; ++i) {
-        CU(c, cudaEventSynchronize(c->ev_chunk[i]));
-        std::memcpy(out_rgb + off[i], c->pinned + off[i], (off[i + 1] - off[i]) * sizeof(float));
-    }
-    CU(c, cudaStreamSynchronize(c->stream));
-    if (out_sumsq) std::memcpy(out_sumsq, c->pinned + plane, plane * sizeof(float));
-    st.launches += 1;
-    c->launches = 0;
-    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
-    if (stats) *stats = st;
-    return VK_OK;
-}
-
-int vk_render_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!P || !out_rgb8) return fail(c, VK_ERR_INVALID, "vk_render_rgb8: null argument");
-    const size_t plane = (size_t)P->width * P->height * 3;
-    CU(c, cudaSetDevice(c->device));
-    int rc = ensure(c, &c->frame, &c->frame_floats, plane * 3);
-    if (rc != VK_OK) return rc;
-    if ((rc = ensure_pinned(c, plane * 2)) != VK_OK) return rc;
-    float* d_sum = c->frame;
-    uint8_t* d_rgb8 = (uint8_t*)(c->frame + 2 * plane);
-    CU(c, cudaEventRecord(c->ev2, c->stream));
-    vk_stats st{};
-    rc = render_into(c, cam, P, d_sum, nullptr, &st);
-    if (rc != VK_OK) return rc;
-    k_to_color<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, d_rgb8, P->width, P->height, (float)P->spp);
-    CU(c, cudaGetLastError());
-    CU(c, cudaMemcpyAsync(c->pinned, d_rgb8, plane, cudaMemcpyDeviceToHost, c->stream));
-    CU(c, cudaEventRecord(c->ev1, c->stream));
-    CU(c, cudaStreamSynchronize(c->stream));
-    std::memcpy(out_rgb8, c->pinned, plane);
-    st.launches += 1;
-    c->launches = 0;
-    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
-    if (stats) *stats = st;
-    return VK_OK;
-}
-
-// shared body of vk_render_frames / vk_render_frames_rgb8 (n_frames > 1; one frame is vk_render / vk_render_rgb8): one
-// launch over every frame's units, then the conversion of all planes and one copy back through the pinned staging
-static int render_frames(vk_ctx* c, const char* who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb,
-                         uint8_t* out_rgb8, vk_stats* stats) {
-    int rc = check_frames(c, who, cams, n_frames, P);
-    if (rc != VK_OK) return rc;
-    const size_t plane = (size_t)P->width * P->height * 3 * n_frames; // all frames
-    CU(c, cudaSetDevice(c->device));
-    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane * 2)) != VK_OK) return rc; // sums | rgb
-    if ((rc = ensure_pinned(c, out_rgb ? plane : (plane + 3) / 4)) != VK_OK) return rc;
-    float *d_sum = c->frame, *d_rgb = c->frame + plane;
-    CU(c, cudaEventRecord(c->ev2, c->stream));
-    vk_stats st{};
-    rc = render_into(c, cams, P, d_sum, nullptr, &st, false, false, n_frames);
-    if (rc != VK_OK) return rc;
-    if (out_rgb) {
-        k_finalize<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, d_rgb, plane, (float)P->spp);
-        CU(c, cudaGetLastError());
-        CU(c, cudaMemcpyAsync(c->pinned, d_rgb, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    } else {
-        k_to_color_frames<<<(unsigned)((plane + 255) / 256), 256, 0, c->stream>>>(d_sum, (uint8_t*)d_rgb, P->width, P->height, n_frames, (float)P->spp);
-        CU(c, cudaGetLastError());
-        CU(c, cudaMemcpyAsync(c->pinned, d_rgb, plane, cudaMemcpyDeviceToHost, c->stream));
-    }
-    CU(c, cudaEventRecord(c->ev1, c->stream));
-    CU(c, cudaStreamSynchronize(c->stream));
-    if (out_rgb) std::memcpy(out_rgb, c->pinned, plane * sizeof(float));
-    else std::memcpy(out_rgb8, c->pinned, plane);
-    st.launches += 1;
-    c->launches = 0;
-    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
-    if (stats) *stats = st;
-    return VK_OK;
-}
-
-// ---- adaptive sessions (vk_adaptive_*; the one-shot vk_render_adaptive* calls run one on c->oneshot) ----
 // Device state of a session: fixed-point sums and squares and the counts of every pixel of its K frames, plus the pass
 // loop's scratch (two pixel lists, the select flags, the level of every pixel, the level counts, the compaction scratch).
 struct vk_adaptive_session {
@@ -1066,6 +959,127 @@ struct vk_adaptive_session {
     void* cub_tmp = nullptr;
 };
 
+// What a render call hands back to host buffers (null: not asked for): the image as floats or as rgb8 bytes, a fixed
+// render's sums of squares, an adaptive read's counts and error map.
+struct Outputs {
+    float* rgb;
+    uint8_t* rgb8;
+    float* sumsq;
+    uint32_t* spp;
+    float* error;
+};
+
+// Where a call's results lie in c->frame and c->pinned, in floats from the start of each: the image, the squares, the counts
+// and the error map at the same offsets on both sides, then on the device only the float sums of a fixed render (`fixed`).
+// A fixed render stages before its sums are written, so that the readout's own call finds the buffers large enough and
+// moves nothing.
+struct Staging {
+    size_t sumsq, counts, error, sum;
+};
+static int stage(vk_ctx* c, size_t plane, bool fixed, const Outputs& o, Staging* S) {
+    const size_t n_pix = plane / 3;
+    S->sumsq = o.rgb ? plane : (plane + 3) / 4;
+    S->counts = S->sumsq + (o.sumsq ? plane : 0);
+    S->error = S->counts + (o.spp ? n_pix : 0);
+    S->sum = S->error + (o.error ? n_pix : 0);
+    const int rc = ensure(c, &c->frame, &c->frame_floats, S->sum + (fixed ? plane : 0));
+    return rc != VK_OK ? rc : ensure_pinned(c, S->sum);
+}
+
+// The end of every render call into host buffers, given its result on c's device: the float sums over P->spp of a fixed
+// render (s == nullptr) in c->frame where stage() puts them, or session s's state.  Converts the means of the n_frames
+// frames into c->frame (k_finalize, or k_to_color with the counts in the image's order), copies the image back through
+// c->pinned in four chunks -- the caller's buffer fills from each chunk while the later ones are still on the bus -- and the
+// extras whole, records ev1 and synchronises.  With stats, adds the readout's launches and ends ms_total at ev1 (it began
+// at ev2).
+static int readout(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, const vk_adaptive_session* s, const Outputs& o, vk_stats* stats) {
+    const size_t plane = (size_t)P->width * P->height * 3 * n_frames, n_pix = plane / 3;
+    CU(c, cudaSetDevice(c->device));
+    Staging S;
+    int rc = stage(c, plane, !s, o, &S);
+    if (rc != VK_OK) return rc;
+    float* d = c->frame;
+    uint32_t* d_spp = o.spp && o.rgb8 ? (uint32_t*)(d + S.counts) : nullptr; // (a float image's counts: the session's own, in pixel order)
+    auto convert = [&](auto src) {
+        const unsigned blocks = (unsigned)((plane + 255) / 256);
+        if (o.rgb) k_finalize<<<blocks, 256, 0, c->stream>>>(src, d, plane);
+        else k_to_color<<<blocks, 256, 0, c->stream>>>(src, (uint8_t*)d, d_spp, P->width, P->height, n_frames);
+    };
+    if (s) convert(AccOverCount{s->acc, s->nspp});
+    else convert(SumsOverSpp{d + S.sum, (float)P->spp});
+    CU(c, cudaGetLastError());
+    constexpr int NCH = 4;
+    const size_t elem = o.rgb ? sizeof(float) : 1;
+    size_t off[NCH + 1]; // in bytes
+    for (int i = 0; i <= NCH; ++i) off[i] = plane * (size_t)i / NCH * elem;
+    for (int i = 0; i < NCH; ++i) {
+        if (!c->ev_chunk[i]) CU(c, cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
+        CU(c, cudaMemcpyAsync((char*)c->pinned + off[i], (const char*)d + off[i], off[i + 1] - off[i], cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaEventRecord(c->ev_chunk[i], c->stream));
+    }
+    if (o.sumsq) CU(c, cudaMemcpyAsync(c->pinned + S.sumsq, d + S.sumsq, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    if (o.spp) CU(c, cudaMemcpyAsync(c->pinned + S.counts, d_spp ? d_spp : s->nspp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (o.error) {
+        k_adaptive_error_map<<<(unsigned)((n_pix + 255) / 256), 256, 0, c->stream>>>(s->acc, s->sq, s->nspp, d + S.error, P->width, P->height,
+                                                                                     n_frames, o.rgb8 != nullptr);
+        CU(c, cudaGetLastError());
+        CU(c, cudaMemcpyAsync(c->pinned + S.error, d + S.error, n_pix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    }
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    char* image = o.rgb ? (char*)o.rgb : (char*)o.rgb8;
+    for (int i = 0; i < NCH; ++i) {
+        CU(c, cudaEventSynchronize(c->ev_chunk[i]));
+        std::memcpy(image + off[i], (const char*)c->pinned + off[i], off[i + 1] - off[i]);
+    }
+    CU(c, cudaStreamSynchronize(c->stream));
+    if (o.sumsq) std::memcpy(o.sumsq, c->pinned + S.sumsq, plane * sizeof(float));
+    if (o.spp) std::memcpy(o.spp, c->pinned + S.counts, n_pix * sizeof(uint32_t));
+    if (o.error) std::memcpy(o.error, c->pinned + S.error, n_pix * sizeof(float));
+    if (stats) {
+        stats->launches += o.error ? 2 : 1;
+        c->launches = 0;
+        CU(c, cudaEventElapsedTime(&stats->ms_total, c->ev2, c->ev1));
+    }
+    return VK_OK;
+}
+
+// shared body of vk_render, vk_render_rgb8, vk_render_frames and vk_render_frames_rgb8: one launch over every frame's units
+// into float sums (and squares) in c->frame, then the readout
+static int render_host(vk_ctx* c, const std::string& who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb,
+                       uint8_t* out_rgb8, float* out_sumsq, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!out_rgb && !out_rgb8) return fail(c, VK_ERR_INVALID, who + ": null argument");
+    int rc = check_render(c, who, cams, n_frames, P);
+    if (rc != VK_OK) return rc;
+    const Outputs o{out_rgb, out_rgb8, out_sumsq, nullptr, nullptr};
+    CU(c, cudaSetDevice(c->device));
+    Staging S;
+    if ((rc = stage(c, (size_t)P->width * P->height * 3 * n_frames, true, o, &S)) != VK_OK) return rc;
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    vk_stats st{};
+    rc = render_into(c, cams, P, c->frame + S.sum, out_sumsq ? c->frame + S.sumsq : nullptr, &st, false, false, n_frames);
+    if (rc == VK_OK) rc = readout(c, P, n_frames, nullptr, o, &st);
+    if (rc == VK_OK && stats) *stats = st;
+    return rc;
+}
+
+int vk_render(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, float* out_rgb, float* out_sumsq, vk_stats* stats) {
+    return render_host(c, "vk_render", cam, 1, P, out_rgb, nullptr, out_sumsq, stats);
+}
+
+int vk_render_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
+    return render_host(c, "vk_render_rgb8", cam, 1, P, nullptr, out_rgb8, nullptr, stats);
+}
+
+int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {
+    return render_host(c, "vk_render_frames", cams, n_frames, P, out_rgb, nullptr, nullptr, stats);
+}
+
+int vk_render_frames_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
+    return render_host(c, "vk_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, nullptr, stats);
+}
+
+// ---- adaptive sessions (vk_adaptive_*; the one-shot vk_render_adaptive* calls run one on c->oneshot) ----
 static void adaptive_free(vk_adaptive_session* s) {
     if (!s) return;
     if (s->block && s->c) {
@@ -1082,26 +1096,6 @@ struct AtLevel {
     __device__ bool operator()(uint32_t p) const { return level[p] == want; }
 };
 
-// What vk_render_adaptive*, vk_render_frames_adaptive* and vk_adaptive_begin refuse before anything is allocated or
-// launched (max_error: the one-shot calls' target; a session checks its targets in refine).
-static int check_adaptive(vk_ctx* c, const std::string& w, const vk_camera* cam, uint32_t n_frames, const vk_render_params* P,
-                          uint32_t pass_spp, float max_error) {
-    int rc = n_frames > 1 ? check_frames(c, w.c_str(), cam, n_frames, P) : VK_OK;
-    if (rc != VK_OK) return rc;
-    rc = check_render(c, cam, P);
-    if (rc != VK_OK) return rc;
-    if (pass_spp == 0) return fail(c, VK_ERR_INVALID, w + ": pass_spp must be >= 1");
-    if (!(max_error >= 0.0f)) return fail(c, VK_ERR_INVALID, w + ": max_error must be >= 0 (and not NaN)");
-    if (P->spp_begin != 0 || (P->spp_count != 0 && P->spp_count != P->spp))
-        return fail(c, VK_ERR_INVALID, w + ": an adaptive render draws samples [0, n_p) of every pixel: spp_begin must be 0, spp_count 0 or spp");
-    if (P->spp > VK_ADAPTIVE_MAX_SPP)
-        return fail(c, VK_ERR_INVALID, w + ": spp above " + std::to_string(VK_ADAPTIVE_MAX_SPP) +
-                                           ", the limit of the fixed-point sums of squares (2^16 samples of at most 255^2 * 2^32 units)");
-    if (P->variant == VK_VARIANT_STAGED || P->variant == VK_VARIANT_WAVEFRONT)
-        return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
-    return VK_OK;
-}
-
 // How many of n_pix pixels shard `shard` of n_shards owns (k_shard_list's rule): whole runs, less the missing tail of the
 // last run when the shard owns it.
 static uint32_t shard_pixels(uint32_t n_pix, uint32_t shard, uint32_t n_shards) {
@@ -1117,16 +1111,14 @@ static uint32_t shard_pixels(uint32_t n_pix, uint32_t shard, uint32_t n_shards) 
 static int adaptive_begin(vk_ctx* c, const std::string& w, const vk_camera* cam, uint32_t n_frames, const vk_render_params* P,
                           uint32_t pass_spp, float max_error, vk_adaptive_session* s, uint32_t shard = 0, uint32_t n_shards = 1) {
     s->c = c;
-    int rc = check_adaptive(c, w, cam, n_frames, P, pass_spp, max_error);
+    int rc = check_render(c, w, cam, n_frames, P, true, pass_spp, max_error);
     if (rc != VK_OK) return rc;
     CU(c, cudaSetDevice(c->device));
     // AUTO decides once, on pass 0's path count; every pass of every refine runs that kernel
     vk_render_params Q = *P;
     Q.spp_count = pass_spp < P->spp ? pass_spp : P->spp;
     RenderPlan R;
-    if ((rc = plan_render(c, &Q, n_frames, &R)) != VK_OK) return rc;
-    if (R.variant == VK_VARIANT_STAGED || R.variant == VK_VARIANT_WAVEFRONT)
-        return fail(c, VK_ERR_UNSUPPORTED, w + ": the staged and wavefront kernels have no pixel-list passes");
+    if ((rc = plan_render(c, w, &Q, n_frames, true, &R)) != VK_OK) return rc;
 
     const uint32_t n_pix = P->width * P->height * n_frames; // (all frames: a pixel index is batch-wide)
     const size_t plane = (size_t)n_pix * 3;
@@ -1291,110 +1283,60 @@ static int adaptive_refine(vk_adaptive_session* s, const vk_adaptive_target& T, 
     return VK_OK;
 }
 
-// The state's image into the caller's buffers (the one-shot calls' layouts), its counts and (nullable) error map.
-static int adaptive_read(vk_adaptive_session* s, float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, float* out_error, uint32_t* launches) {
-    vk_ctx* c = s->c;
-    const size_t n_pix = s->n_pix, plane = n_pix * 3;
-    CU(c, cudaSetDevice(c->device));
-    int rc;
-    if ((rc = ensure(c, &c->frame, &c->frame_floats, plane + 2 * n_pix)) != VK_OK) return rc; // rgb or rgb8 | counts | errors
-    if ((rc = ensure_pinned(c, plane + 2 * n_pix)) != VK_OK) return rc;
-    uint32_t* d_spp = (uint32_t*)(c->frame + plane);
-    float* d_err = c->frame + plane + n_pix;
-    const unsigned blocks = (unsigned)((plane + 255) / 256);
-    if (out_rgb) {
-        k_finalize_adaptive<<<blocks, 256, 0, c->stream>>>(s->acc, s->nspp, c->frame, plane);
-        CU(c, cudaGetLastError());
-        CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        d_spp = s->nspp; // (vk_render's layout: the counts are already in pixel order)
-    } else {
-        k_to_color_adaptive<<<blocks, 256, 0, c->stream>>>(s->acc, s->nspp, (uint8_t*)c->frame, d_spp, s->P.width, s->P.height, s->n_frames);
-        CU(c, cudaGetLastError());
-        CU(c, cudaMemcpyAsync(c->pinned, c->frame, plane, cudaMemcpyDeviceToHost, c->stream));
-    }
-    ++*launches;
-    if (out_spp) CU(c, cudaMemcpyAsync(c->pinned + plane, d_spp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
-    if (out_error) {
-        k_adaptive_error_map<<<(unsigned)((n_pix + 255) / 256), 256, 0, c->stream>>>(s->acc, s->sq, s->nspp, d_err, s->P.width, s->P.height,
-                                                                                     s->n_frames, out_rgb8 != nullptr);
-        ++*launches;
-        CU(c, cudaGetLastError());
-        CU(c, cudaMemcpyAsync(c->pinned + plane + n_pix, d_err, n_pix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    }
-    CU(c, cudaEventRecord(c->ev1, c->stream));
-    CU(c, cudaStreamSynchronize(c->stream));
-    if (out_rgb) std::memcpy(out_rgb, c->pinned, plane * sizeof(float));
-    else std::memcpy(out_rgb8, c->pinned, plane);
-    if (out_spp) std::memcpy(out_spp, c->pinned + plane, n_pix * sizeof(uint32_t));
-    if (out_error) std::memcpy(out_error, c->pinned + plane + n_pix, n_pix * sizeof(float));
-    return VK_OK;
-}
-
 // shared body of vk_render_adaptive* and vk_render_frames_adaptive* (include/vecchio_gpu.h states the passes and the rule):
 // begin, one refine to {spp, 0, max_error} and read, on the context's own session.
-// n_frames > 1: cam points to n_frames cameras, every pass runs one launch over the active pixels of all frames (one list of
+// n_frames > 1: cams points to n_frames cameras, every pass runs one launch over the active pixels of all frames (one list of
 // batch-wide pixels, FrameListArgs) and the result is n_frames contiguous planes.
-static int render_adaptive(vk_ctx* c, const char* who, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
-                           float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats, uint32_t n_frames = 1) {
-    const std::string w(who);
-    if (!cam || !P || (!out_rgb && !out_rgb8)) return fail(c, VK_ERR_INVALID, w + ": null argument");
+static int render_adaptive(vk_ctx* c, const std::string& who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
+                           float max_error, float* out_rgb, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    if (!out_rgb && !out_rgb8) return fail(c, VK_ERR_INVALID, who + ": null argument");
     if (!c->oneshot) c->oneshot = new vk_adaptive_session;
     vk_adaptive_session* s = c->oneshot;
     CU(c, cudaSetDevice(c->device));
     CU(c, cudaEventRecord(c->ev2, c->stream));
-    int rc = adaptive_begin(c, w, cam, n_frames, P, pass_spp, max_error, s);
+    int rc = adaptive_begin(c, who, cams, n_frames, P, pass_spp, max_error, s);
     if (rc != VK_OK) return rc;
     uint32_t launches = 0;
     uint64_t paths = 0;
     float ms_kernels = 0.0f;
     if ((rc = adaptive_refine(s, vk_adaptive_target{P->spp, 0u, max_error}, &launches, &paths, &ms_kernels)) != VK_OK) return rc;
-    if ((rc = adaptive_read(s, out_rgb, out_rgb8, out_spp, nullptr, &launches)) != VK_OK) return rc;
     c->launches += launches;
     c->paths += paths;
     vk_stats st{};
     if ((rc = vk_flush_stats(c, &st)) != VK_OK) return rc;
     st.ms_kernels = ms_kernels;
-    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
     st.variant = s->R.variant;
+    if ((rc = readout(c, P, n_frames, s, Outputs{out_rgb, out_rgb8, nullptr, out_spp, nullptr}, &st)) != VK_OK) return rc;
     if (stats) *stats = st;
     return VK_OK;
 }
 
 int vk_render_adaptive(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error, float* out_rgb,
                        uint32_t* out_spp, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!out_rgb) return fail(c, VK_ERR_INVALID, "vk_render_adaptive: null argument");
-    return render_adaptive(c, "vk_render_adaptive", cam, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats);
+    return render_adaptive(c, "vk_render_adaptive", cam, 1, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats);
 }
 
 int vk_render_adaptive_rgb8(vk_ctx* c, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
                             uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!out_rgb8) return fail(c, VK_ERR_INVALID, "vk_render_adaptive_rgb8: null argument");
-    return render_adaptive(c, "vk_render_adaptive_rgb8", cam, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats);
+    return render_adaptive(c, "vk_render_adaptive_rgb8", cam, 1, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats);
 }
 
 int vk_render_frames_adaptive(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
                               float max_error, float* out_rgb, uint32_t* out_spp, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!cams || !P || !out_rgb || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_adaptive: null argument or no frames");
-    if (n_frames == 1) return vk_render_adaptive(c, cams, P, pass_spp, max_error, out_rgb, out_spp, stats);
-    return render_adaptive(c, "vk_render_frames_adaptive", cams, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats, n_frames);
+    return render_adaptive(c, "vk_render_frames_adaptive", cams, n_frames, P, pass_spp, max_error, out_rgb, nullptr, out_spp, stats);
 }
 
 int vk_render_frames_adaptive_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
                                    float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!cams || !P || !out_rgb8 || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_adaptive_rgb8: null argument or no frames");
-    if (n_frames == 1) return vk_render_adaptive_rgb8(c, cams, P, pass_spp, max_error, out_rgb8, out_spp, stats);
-    return render_adaptive(c, "vk_render_frames_adaptive_rgb8", cams, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats, n_frames);
+    return render_adaptive(c, "vk_render_frames_adaptive_rgb8", cams, n_frames, P, pass_spp, max_error, nullptr, out_rgb8, out_spp, stats);
 }
 
 // shared body of vk_adaptive_begin and vk_adaptive_begin_shard
 static int begin_session(vk_ctx* c, const std::string& w, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
                          uint32_t pass_spp, uint32_t shard, uint32_t n_shards, vk_adaptive_session** out) {
     if (!c) return VK_ERR_INVALID;
-    if (!out || !cams || !P || n_frames == 0) return fail(c, VK_ERR_INVALID, w + ": null argument or no frames");
+    if (!out) return fail(c, VK_ERR_INVALID, w + ": null argument");
     *out = nullptr;
     if (n_shards == 0 || shard >= n_shards) return fail(c, VK_ERR_INVALID, w + ": shard must be < n_shards (and n_shards >= 1)");
     vk_adaptive_session* s = new vk_adaptive_session;
@@ -1451,8 +1393,7 @@ static int adaptive_read_call(vk_adaptive_session* s, const char* who, float* ou
     vk_ctx* c = s->c;
     if (!out_rgb && !out_rgb8) return fail(c, VK_ERR_INVALID, std::string(who) + ": null argument");
     if (s->broken) return fail(c, VK_ERR_INVALID, std::string(who) + ": an earlier refine or import failed part way; the session's state is lost");
-    uint32_t launches = 0; // (a read is not part of any refine's stats)
-    return adaptive_read(s, out_rgb, out_rgb8, out_spp, out_error, &launches);
+    return readout(c, &s->P, s->n_frames, s, Outputs{out_rgb, out_rgb8, nullptr, out_spp, out_error}, nullptr); // (no refine's stats)
 }
 
 int vk_adaptive_read(vk_adaptive_session* s, float* out_rgb, uint32_t* out_spp, float* out_error) {
@@ -1533,20 +1474,6 @@ int vk_adaptive_import(vk_adaptive_session* s, const int64_t* sums, const uint64
 uint32_t vk_adaptive_variant(const vk_adaptive_session* s) { return s ? s->R.variant : 0u; }
 
 void vk_adaptive_destroy(vk_adaptive_session* s) { adaptive_free(s); }
-
-int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!cams || !P || !out_rgb || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames: null argument or no frames");
-    if (n_frames == 1) return vk_render(c, cams, P, out_rgb, nullptr, stats);
-    return render_frames(c, "vk_render_frames", cams, n_frames, P, out_rgb, nullptr, stats);
-}
-
-int vk_render_frames_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
-    if (!c) return VK_ERR_INVALID;
-    if (!cams || !P || !out_rgb8 || n_frames == 0) return fail(c, VK_ERR_INVALID, "vk_render_frames_rgb8: null argument or no frames");
-    if (n_frames == 1) return vk_render_rgb8(c, cams, P, out_rgb8, stats);
-    return render_frames(c, "vk_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, stats);
-}
 
 int vk_intersect(vk_ctx* c, const vk_ray* rays, size_t n, const float* medium_xi, uint32_t flags, vk_hit* out) {
     if (!c) return VK_ERR_INVALID;
@@ -1725,18 +1652,35 @@ int vk_multi_scene_upload(vk_multi* m, const vk_scene_desc* scene) {
     return VK_OK;
 }
 
-// shared body of vk_multi_render / vk_multi_render_rgb8: every device accumulates its slice, device 0 reduces
-// (n_frames > 1: a batch, every device renders its sample slice of every frame; check_frames has passed on every device)
-static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_params* P, bool want_sq, float** d_sum, float** d_sq, vk_stats* st,
-                             uint32_t n_frames = 1) {
-    if (!m || !cam || !P) return mfail(m, VK_ERR_INVALID, "vk_multi_render: null argument");
+// a CUDA call made for a vk_multi: its error is the vk_multi's
+#define CUM(m, call)                                                                                                   \
+    do {                                                                                                               \
+        cudaError_t e_ = (call);                                                                                       \
+        if (e_ != cudaSuccess)                                                                                         \
+            return mfail(m, e_ == cudaErrorMemoryAllocation ? VK_ERR_OOM : VK_ERR_CUDA,                                \
+                         std::string(#call) + ": " + cudaGetErrorString(e_));                                          \
+    } while (0)
+
+// shared body of vk_multi_render, vk_multi_render_rgb8 and vk_multi_render_frames_rgb8: every device accumulates its sample
+// slice of every frame, device 0 adds the slices up into its staging (k_reduce_peers) and runs the readout
+static int multi_render(vk_multi* m, const std::string& who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, float* out_rgb,
+                        uint8_t* out_rgb8, float* out_sumsq, vk_stats* stats) {
+    if (!m) return VK_ERR_INVALID;
+    if (!out_rgb && !out_rgb8) return mfail(m, VK_ERR_INVALID, who + ": null argument");
+    for (vk_ctx* c : m->ctx) { // every device, before any of them launches
+        const int rc = check_render(c, who, cams, n_frames, P);
+        if (rc != VK_OK) return mfail(m, rc, c->err);
+    }
     const int n = (int)m->ctx.size();
-    const uint32_t begin = P->spp_begin, count = P->spp_count ? P->spp_count : (P->spp > P->spp_begin ? P->spp - P->spp_begin : 0u);
-    if (P->spp == 0 || count == 0 || (uint64_t)begin + count > P->spp) return mfail(m, VK_ERR_INVALID, "vk_multi_render: bad spp range");
-    vk_ctx* c0 = m->ctx[0];
+    const uint32_t begin = P->spp_begin, count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
     const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
-    cudaSetDevice(c0->device);
-    cudaEventRecord(c0->ev2, c0->stream);
+    const Outputs o{out_rgb, out_rgb8, out_sumsq, nullptr, nullptr};
+    vk_ctx* c0 = m->ctx[0];
+    CUM(m, cudaSetDevice(c0->device));
+    Staging S;
+    int rc = stage(c0, plane, true, o, &S);
+    if (rc != VK_OK) return mfail(m, rc, c0->err);
+    CUM(m, cudaEventRecord(c0->ev2, c0->stream));
     int active = 0;
     PeerAcc pa{};
     for (int k = 0; k < n; ++k) { // global samples [begin + k * count / n, begin + (k + 1) * count / n)
@@ -1746,122 +1690,51 @@ static int multi_render_sums(vk_multi* m, const vk_camera* cam, const vk_render_
         q.spp_begin = s0;
         q.spp_count = s1 - s0;
         vk_ctx* c = m->ctx[k];
-        const int rc = render_into(c, cam, &q, nullptr, nullptr, nullptr, true, want_sq, n_frames);
-        if (rc != VK_OK) return mfail(m, rc, c->err);
-        cudaSetDevice(c->device);
-        cudaEventRecord(m->done[k], c->stream);
+        if ((rc = render_into(c, cams, &q, nullptr, nullptr, nullptr, true, out_sumsq != nullptr, n_frames)) != VK_OK) return mfail(m, rc, c->err);
+        CUM(m, cudaSetDevice(c->device));
+        CUM(m, cudaEventRecord(m->done[k], c->stream));
         pa.acc[active] = (const unsigned long long*)c->partial;
-        pa.accsq[active] = want_sq ? (const double*)(c->partial + plane * 2) : nullptr;
+        pa.accsq[active] = out_sumsq ? (const double*)(c->partial + plane * 2) : nullptr;
         ++active;
     }
     // device 0's stream waits for every slice, then reads the peers' accumulators
-    cudaSetDevice(c0->device);
-    for (int k = 0; k < n; ++k) cudaStreamWaitEvent(c0->stream, m->done[k], 0);
-    int rc = ensure(c0, &c0->frame, &c0->frame_floats, plane * 3);
-    if (rc != VK_OK) return mfail(m, rc, c0->err);
-    *d_sum = c0->frame;
-    *d_sq = want_sq ? c0->frame + plane : nullptr;
+    CUM(m, cudaSetDevice(c0->device));
+    for (int k = 0; k < n; ++k) CUM(m, cudaStreamWaitEvent(c0->stream, m->done[k], 0));
     pa.n = active;
-    k_reduce_peers<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(pa, plane, *d_sum, *d_sq);
-    const cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("k_reduce_peers: ") + cudaGetErrorString(e));
+    k_reduce_peers<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(pa, plane, c0->frame + S.sum, out_sumsq ? c0->frame + S.sumsq : nullptr);
+    CUM(m, cudaGetLastError());
     c0->launches += 1;
     // counters of all devices (synchronises each)
-    vk_stats total{};
+    vk_stats st{};
     float ms_max = 0.0f;
     for (int k = 0; k < n; ++k) {
         vk_stats s{};
         vk_ctx* c = m->ctx[k];
         if ((rc = vk_flush_stats(c, &s)) != VK_OK) return mfail(m, rc, c->err);
         float ms = 0.0f;
-        if (s.paths) cudaEventElapsedTime(&ms, c->ev0, c->ev1);
+        if (s.paths) CUM(m, cudaEventElapsedTime(&ms, c->ev0, c->ev1));
         ms_max = ms > ms_max ? ms : ms_max;
-        total.paths += s.paths; total.rays += s.rays; total.dropped_samples += s.dropped_samples;
-        total.node_visits += s.node_visits; total.prim_tests += s.prim_tests; total.launches += s.launches;
+        st.paths += s.paths; st.rays += s.rays; st.dropped_samples += s.dropped_samples;
+        st.node_visits += s.node_visits; st.prim_tests += s.prim_tests; st.launches += s.launches;
     }
-    total.ms_kernels = ms_max; // the slowest device's render kernels
-    total.variant = VK_VARIANT_AUTO;
-    *st = total;
-    return VK_OK;
-}
-static int multi_pinned(vk_multi* m, vk_ctx* c0, size_t floats) {
-    if (ensure_pinned(c0, floats) != VK_OK) return mfail(m, VK_ERR_OOM, "vk_multi_render: pinned staging");
-    return VK_OK;
-}
-int vk_multi_render(vk_multi* m, const vk_camera* cam, const vk_render_params* P, float* out_rgb, float* out_sumsq, vk_stats* stats) {
-    if (!m || !P || !out_rgb) return mfail(m, VK_ERR_INVALID, "vk_multi_render: null argument");
-    float *d_sum = nullptr, *d_sq = nullptr;
-    vk_stats st{};
-    int rc = multi_render_sums(m, cam, P, out_sumsq != nullptr, &d_sum, &d_sq, &st);
-    if (rc != VK_OK) return rc;
-    vk_ctx* c0 = m->ctx[0];
-    const size_t plane = (size_t)P->width * P->height * 3;
-    if ((rc = multi_pinned(m, c0, plane * 2)) != VK_OK) return rc;
-    cudaSetDevice(c0->device);
-    float* d_rgb = c0->frame + 2 * plane;
-    k_finalize<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(d_sum, d_rgb, plane, (float)P->spp);
-    cudaMemcpyAsync(c0->pinned, d_rgb, plane * sizeof(float), cudaMemcpyDeviceToHost, c0->stream);
-    if (out_sumsq) cudaMemcpyAsync(c0->pinned + plane, d_sq, plane * sizeof(float), cudaMemcpyDeviceToHost, c0->stream);
-    cudaEventRecord(c0->ev1, c0->stream);
-    cudaError_t e = cudaStreamSynchronize(c0->stream);
-    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("vk_multi_render: ") + cudaGetErrorString(e));
-    std::memcpy(out_rgb, c0->pinned, plane * sizeof(float));
-    if (out_sumsq) std::memcpy(out_sumsq, c0->pinned + plane, plane * sizeof(float));
-    cudaEventElapsedTime(&st.ms_total, c0->ev2, c0->ev1);
-    st.launches += 1;
-    if (stats) *stats = st;
-    return VK_OK;
-}
-int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
-    if (!m || !P || !out_rgb8) return mfail(m, VK_ERR_INVALID, "vk_multi_render_rgb8: null argument");
-    float *d_sum = nullptr, *d_sq = nullptr;
-    vk_stats st{};
-    int rc = multi_render_sums(m, cam, P, false, &d_sum, &d_sq, &st);
-    if (rc != VK_OK) return rc;
-    vk_ctx* c0 = m->ctx[0];
-    const size_t plane = (size_t)P->width * P->height * 3;
-    if ((rc = multi_pinned(m, c0, plane)) != VK_OK) return rc;
-    cudaSetDevice(c0->device);
-    uint8_t* d_rgb8 = (uint8_t*)(c0->frame + 2 * plane);
-    k_to_color<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(d_sum, d_rgb8, P->width, P->height, (float)P->spp);
-    cudaMemcpyAsync(c0->pinned, d_rgb8, plane, cudaMemcpyDeviceToHost, c0->stream);
-    cudaEventRecord(c0->ev1, c0->stream);
-    cudaError_t e = cudaStreamSynchronize(c0->stream);
-    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("vk_multi_render_rgb8: ") + cudaGetErrorString(e));
-    std::memcpy(out_rgb8, c0->pinned, plane);
-    cudaEventElapsedTime(&st.ms_total, c0->ev2, c0->ev1);
-    st.launches += 1;
+    st.ms_kernels = ms_max; // the slowest device's render kernels
+    st.variant = VK_VARIANT_AUTO;
+    if ((rc = readout(c0, P, n_frames, nullptr, o, &st)) != VK_OK) return mfail(m, rc, c0->err);
     if (stats) *stats = st;
     return VK_OK;
 }
 
+int vk_multi_render(vk_multi* m, const vk_camera* cam, const vk_render_params* P, float* out_rgb, float* out_sumsq, vk_stats* stats) {
+    return multi_render(m, "vk_multi_render", cam, 1, P, out_rgb, nullptr, out_sumsq, stats);
+}
+
+int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
+    return multi_render(m, "vk_multi_render_rgb8", cam, 1, P, nullptr, out_rgb8, nullptr, stats);
+}
+
 int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8,
                                 vk_stats* stats) {
-    if (!m || !cams || !P || !out_rgb8 || n_frames == 0) return mfail(m, VK_ERR_INVALID, "vk_multi_render_frames_rgb8: null argument or no frames");
-    if (n_frames == 1) return vk_multi_render_rgb8(m, cams, P, out_rgb8, stats);
-    for (vk_ctx* c : m->ctx) { // every device, before any of them launches
-        const int rc = check_frames(c, "vk_multi_render_frames_rgb8", cams, n_frames, P);
-        if (rc != VK_OK) return mfail(m, rc, c->err);
-    }
-    float *d_sum = nullptr, *d_sq = nullptr;
-    vk_stats st{};
-    int rc = multi_render_sums(m, cams, P, false, &d_sum, &d_sq, &st, n_frames);
-    if (rc != VK_OK) return rc;
-    vk_ctx* c0 = m->ctx[0];
-    const size_t plane = (size_t)P->width * P->height * 3 * n_frames;
-    if ((rc = multi_pinned(m, c0, (plane + 3) / 4)) != VK_OK) return rc;
-    cudaSetDevice(c0->device);
-    uint8_t* d_rgb8 = (uint8_t*)(c0->frame + 2 * plane);
-    k_to_color_frames<<<(unsigned)((plane + 255) / 256), 256, 0, c0->stream>>>(d_sum, d_rgb8, P->width, P->height, n_frames, (float)P->spp);
-    cudaMemcpyAsync(c0->pinned, d_rgb8, plane, cudaMemcpyDeviceToHost, c0->stream);
-    cudaEventRecord(c0->ev1, c0->stream);
-    cudaError_t e = cudaStreamSynchronize(c0->stream);
-    if (e != cudaSuccess) return mfail(m, VK_ERR_CUDA, std::string("vk_multi_render_frames_rgb8: ") + cudaGetErrorString(e));
-    std::memcpy(out_rgb8, c0->pinned, plane);
-    cudaEventElapsedTime(&st.ms_total, c0->ev2, c0->ev1);
-    st.launches += 1;
-    if (stats) *stats = st;
-    return VK_OK;
+    return multi_render(m, "vk_multi_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, nullptr, stats);
 }
 
 // ---- adaptive sessions over several GPUs (include/vecchio_gpu.h, vk_multi_adaptive_begin) ----
@@ -1975,8 +1848,7 @@ static int multi_adaptive_read_call(vk_multi_adaptive_session* ms, const std::st
     if (ms->broken) return mfail(m, VK_ERR_INVALID, w + k_multi_lost);
     int rc = multi_adaptive_composite(ms, w);
     if (rc != VK_OK) return rc;
-    uint32_t launches = 0;
-    rc = adaptive_read(ms->comp, out_rgb, out_rgb8, out_spp, out_error, &launches);
+    rc = readout(m->ctx[0], &ms->comp->P, ms->comp->n_frames, ms->comp, Outputs{out_rgb, out_rgb8, nullptr, out_spp, out_error}, nullptr);
     return rc == VK_OK ? VK_OK : mfail(m, rc, w + ": " + m->ctx[0]->err);
 }
 
@@ -1984,6 +1856,8 @@ static int multi_adaptive_read_call(vk_multi_adaptive_session* ms, const std::st
 // {spp, 0, max_error} and read, on the vk_multi's own session
 static int multi_render_adaptive(vk_multi* m, const std::string& w, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P,
                                  uint32_t pass_spp, float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
+    if (!m) return VK_ERR_INVALID;
+    if (!out_rgb8) return mfail(m, VK_ERR_INVALID, w + ": null argument");
     const auto t0 = std::chrono::steady_clock::now();
     if (!m->oneshot) m->oneshot = new vk_multi_adaptive_session;
     vk_multi_adaptive_session* ms = m->oneshot;
@@ -2000,23 +1874,18 @@ static int multi_render_adaptive(vk_multi* m, const std::string& w, const vk_cam
 
 int vk_multi_render_adaptive_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_params* P, uint32_t pass_spp, float max_error,
                                   uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
-    if (!m) return VK_ERR_INVALID;
-    if (!cam || !P || !out_rgb8) return mfail(m, VK_ERR_INVALID, "vk_multi_render_adaptive_rgb8: null argument");
     return multi_render_adaptive(m, "vk_multi_render_adaptive_rgb8", cam, 1, P, pass_spp, max_error, out_rgb8, out_spp, stats);
 }
 
 int vk_multi_render_frames_adaptive_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
                                          float max_error, uint8_t* out_rgb8, uint32_t* out_spp, vk_stats* stats) {
-    if (!m) return VK_ERR_INVALID;
-    if (!cams || !P || !out_rgb8 || n_frames == 0)
-        return mfail(m, VK_ERR_INVALID, "vk_multi_render_frames_adaptive_rgb8: null argument or no frames");
     return multi_render_adaptive(m, "vk_multi_render_frames_adaptive_rgb8", cams, n_frames, P, pass_spp, max_error, out_rgb8, out_spp, stats);
 }
 
 int vk_multi_adaptive_begin(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t pass_spp,
                             vk_multi_adaptive_session** out) {
     if (!m) return VK_ERR_INVALID;
-    if (!out || !cams || !P || n_frames == 0) return mfail(m, VK_ERR_INVALID, "vk_multi_adaptive_begin: null argument or no frames");
+    if (!out) return mfail(m, VK_ERR_INVALID, "vk_multi_adaptive_begin: null argument");
     *out = nullptr;
     vk_multi_adaptive_session* ms = new vk_multi_adaptive_session;
     const int rc = multi_adaptive_begin(m, "vk_multi_adaptive_begin", cams, n_frames, P, pass_spp, 0.0f, ms);
