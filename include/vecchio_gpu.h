@@ -301,6 +301,7 @@ typedef struct vk_scene_info {
     uint32_t dynamic_megakernel;   /* 1 = BVH large enough for the dynamic re-fill megakernel               */
     uint32_t flat_boxes;           /* Boxy entries of the flat program (render build: one slab test each)   */
     uint32_t flat_direct;          /* hit-table entries whose HitRec the shade stage writes down directly   */
+    uint32_t flat_shape;           /* 0, or the flat program's shape the warp-queue kernel is compiled for  */
 } vk_scene_info;
 int vk_scene_check(const vk_scene_desc* scene, vk_scene_info* info, char* err, size_t err_len);
 

@@ -108,7 +108,7 @@ class vk_stats(C.Structure):
 
 class vk_scene_info(C.Structure):
     _fields_ = [(n, C.c_uint32) for n in ("flat_entries", "flat_segments", "flat_subtrees", "simple", "wide_nodes", "wide_levels_world",
-                                          "wide_levels_instance", "stack_need", "dynamic_megakernel", "flat_boxes", "flat_direct")]
+                                          "wide_levels_instance", "stack_need", "dynamic_megakernel", "flat_boxes", "flat_direct", "flat_shape")]
 
 
 class vk_ray(C.Structure):

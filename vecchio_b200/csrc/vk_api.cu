@@ -46,6 +46,7 @@ struct vk_ctx {
     bool has_specdiffuse = false;
     bool simple_scene = false; // only what the VK_SIMPLE build of the staged kernel keeps (see vk_device.cuh)
     bool one_rect_light = false; // the light list is exactly one unflipped Rect: the VK_LIGHT0 builds apply
+    uint32_t flat_shape = VKF_SHAPE_NONE; // the flat program's shape, if the trimmed warp-queue kernel is compiled for it
     unsigned long long* debug = nullptr;    // per-CTA diagnostics of the staged kernel (VK_DEBUG_CTAS x 4 words)
     unsigned long long* counters = nullptr; // [0] rays [1] dropped [2] work head
     float* partial = nullptr;               // accumulators: W*H*3 x u64 fixed-point sums | W*H*3 x double sums of squares
@@ -498,6 +499,7 @@ int vk_scene_upload(vk_ctx* c, const vk_scene_desc* d) {
     c->wnodes_bytes = wnodes.size() * sizeof(float4);
     c->has_specdiffuse = R.has_specdiffuse;
     c->simple_scene = R.simple;
+    c->flat_shape = R.flat_shape;
     c->one_rect_light = d->n_lights == 1 && VK_REF_TYPE(d->lights[0]) == VK_T_RECT && !(d->rects[VK_REF_INDEX(d->lights[0])].axes & VK_RECT_FLIP);
     c->stack_need = R.stack_need;
     c->levels_sub = R.levels_sub;
@@ -801,10 +803,12 @@ static int launch_pass(vk_ctx* c, const RenderPlan& R, const vk_camera* cam, con
             // (a hybrid program -- flat top, homogeneous subtrees walked inside extend -- runs k_warpq_hybrid)
             const FlatProgram* sflat = flat;
             const bool simple = !strict && !legacy && sflat && sflat->n_bvh == 0 && c->simple_scene && !std::getenv("VECCHIO_NO_SIMPLE");
-            CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
-                  : simple ? vkfast_simple::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
-                  : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
-                           : vkfast::launch_warpq(c->scene, sflat, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom));
+            // the trimmed build's kernel compiled for the program's shape, if there is one (VECCHIO_NO_STATIC_FLAT: the generic one)
+            const uint32_t shape = std::getenv("VECCHIO_NO_STATIC_FLAT") ? (uint32_t)VKF_SHAPE_NONE : c->flat_shape;
+            CU(c, strict   ? vkstrict::launch_warpq(c->scene, sflat, VKF_SHAPE_NONE, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                  : simple ? vkfast_simple::launch_warpq(c->scene, sflat, shape, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                  : l0     ? vkfast_l0::launch_warpq(c->scene, sflat, VKF_SHAPE_NONE, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom)
+                           : vkfast::launch_warpq(c->scene, sflat, VKF_SHAPE_NONE, dc, a, b, c->counters + 2, c->sm_count, legacy, c->stream, dom));
             *launches += 1;
         } else if (variant == VK_VARIANT_WAVEFRONT) {
             uint32_t n = 0;

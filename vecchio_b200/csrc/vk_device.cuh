@@ -718,30 +718,32 @@ VKD void flat_rects(const FlatProgram& P, uint32_t i0, uint32_t i1, float3 co, f
 // exact t = 0 it has in the six-rect form (see the rejected experiment in flat_rects_k).  ~40 instructions per ray
 // instead of six rect tests of ~15.  The winning side's entry of the hit table: sides 0|1, 2|3, 4|5 are consecutive.
 template <int K>
+VKD void flat_box_k(const FlatBox& bx, const float3 (&co)[K], const float3 (&ci)[K], float tmin, float (&best_t)[K], uint32_t (&best_hit)[K]) {
+    const float4 mn = bx.mn, mx = bx.mx;
+    const uint32_t hz = __float_as_uint(mn.w), hy = __float_as_uint(mx.w) & 0xFFFFu, hx = __float_as_uint(mx.w) >> 16;
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        const float x0 = (mn.x - co[q].x) * ci[q].x, x1 = (mx.x - co[q].x) * ci[q].x;
+        const float y0 = (mn.y - co[q].y) * ci[q].y, y1 = (mx.y - co[q].y) * ci[q].y;
+        const float z0 = (mn.z - co[q].z) * ci[q].z, z1 = (mx.z - co[q].z) * ci[q].z;
+        const float nx = fminf(x0, x1), ny = fminf(y0, y1), nz = fminf(z0, z1);
+        const float fx = fmaxf(x0, x1), fy = fmaxf(y0, y1), fz = fmaxf(z0, z1);
+        const float t_near = fmaxf(fmaxf(nx, ny), nz), t_far = fminf(fminf(fx, fy), fz);
+        const bool enter = t_near >= tmin;
+        const float t = enter ? t_near : t_far;
+        const bool hit = (t_near <= t_far) & (t >= tmin) & (t < best_t[q]);
+        const bool on_z = (enter ? nz : fz) == t, on_y = (enter ? ny : fy) == t;
+        const float at_max = on_z ? z1 : (on_y ? y1 : x1); // distance of the axis' box_max plane: sides 0, 2, 4
+        const uint32_t id = (on_z ? hz : (on_y ? hy : hx)) + (at_max == t ? 0u : 1u);
+        best_t[q] = hit ? t : best_t[q];
+        best_hit[q] = hit ? id : best_hit[q];
+    }
+}
+template <int K>
 VKD void flat_boxes_k(const FlatProgram& P, uint32_t i0, uint32_t i1, const float3 (&co)[K], const float3 (&ci)[K], float tmin,
                       float (&best_t)[K], uint32_t (&best_hit)[K]) {
 #pragma unroll 1
-    for (uint32_t i = i0; i < i1; ++i) {
-        const float4 mn = P.boxes[i].mn, mx = P.boxes[i].mx;
-        const uint32_t hz = __float_as_uint(mn.w), hy = __float_as_uint(mx.w) & 0xFFFFu, hx = __float_as_uint(mx.w) >> 16;
-#pragma unroll
-        for (int q = 0; q < K; ++q) {
-            const float x0 = (mn.x - co[q].x) * ci[q].x, x1 = (mx.x - co[q].x) * ci[q].x;
-            const float y0 = (mn.y - co[q].y) * ci[q].y, y1 = (mx.y - co[q].y) * ci[q].y;
-            const float z0 = (mn.z - co[q].z) * ci[q].z, z1 = (mx.z - co[q].z) * ci[q].z;
-            const float nx = fminf(x0, x1), ny = fminf(y0, y1), nz = fminf(z0, z1);
-            const float fx = fmaxf(x0, x1), fy = fmaxf(y0, y1), fz = fmaxf(z0, z1);
-            const float t_near = fmaxf(fmaxf(nx, ny), nz), t_far = fminf(fminf(fx, fy), fz);
-            const bool enter = t_near >= tmin;
-            const float t = enter ? t_near : t_far;
-            const bool hit = (t_near <= t_far) & (t >= tmin) & (t < best_t[q]);
-            const bool on_z = (enter ? nz : fz) == t, on_y = (enter ? ny : fy) == t;
-            const float at_max = on_z ? z1 : (on_y ? y1 : x1); // distance of the axis' box_max plane: sides 0, 2, 4
-            const uint32_t id = (on_z ? hz : (on_y ? hy : hx)) + (at_max == t ? 0u : 1u);
-            best_t[q] = hit ? t : best_t[q];
-            best_hit[q] = hit ? id : best_hit[q];
-        }
-    }
+    for (uint32_t i = i0; i < i1; ++i) flat_box_k<K>(P.boxes[i], co, ci, tmin, best_t, best_hit);
 }
 #endif
 template <bool MEDIA>
@@ -859,6 +861,42 @@ VKD TraceHit trace_flat(const DScene& sc, const FlatProgram& P, float3 o, float3
 // K rays per thread through the flat program (the staged kernel traces all the slots a thread owns
 // together): an entry's operands are fetched once for the K rays and the K closest-hit chains are
 // independent, which is the instruction-level parallelism a warp-per-SM-quarter schedule lacks.
+// One rect entry for K rays (flat_rects_k walks a range of them, trace_flat_static names each one).
+template <int K, int AX, bool BOX_SIDE>
+VKD void flat_rect_k(const FlatRect& r, const float3 (&co)[K], const float3 (&cd)[K], const float3 (&ci)[K], float tmin, float (&best_t)[K],
+                     uint32_t (&best_hit)[K]) {
+    const float4 bd = r.bounds;
+    const float k = r.k;
+    const uint32_t id = r.hitc;
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        float tt, a, b;
+        if (AX == 0) {
+            tt = VKF_PLANE_T(k, co[q].z, cd[q].z, ci[q].z);
+            a = co[q].x + tt * cd[q].x;
+            b = co[q].y + tt * cd[q].y;
+        } else if (AX == 1) {
+            tt = VKF_PLANE_T(k, co[q].y, cd[q].y, ci[q].y);
+            a = co[q].x + tt * cd[q].x;
+            b = co[q].z + tt * cd[q].z;
+        } else {
+            tt = VKF_PLANE_T(k, co[q].x, cd[q].x, ci[q].x);
+            a = co[q].y + tt * cd[q].y;
+            b = co[q].z + tt * cd[q].z;
+        }
+        // same predicate as Rect::hit, evaluated without branches (bitwise on the comparison results).
+        // (Measured and rejected in round 2: the plane distance as one fma, k * (1/d) - o * (1/d), and the bounds as
+        // |a - centre| <= half extent.  0.6 % faster, but a ray that STARTS on the plane -- every scattered ray --
+        // no longer gets t = 0 exactly: the two products cancel to rounding noise of either sign, scaled by 1/d.
+        // Dropped samples rose from 26 to 1503 per 3.6e8 paths and light leaked around the box.)
+        // (the comparison with the closest hit so far comes last: it is the only link between one entry and the next)
+        bool miss = (a < bd.x) | (a > bd.y) | (b < bd.z) | (b > bd.w) | (tt < tmin);
+        miss = miss | (tt > best_t[q]);
+        if (BOX_SIDE) miss = miss | !(tt < best_t[q]);
+        best_t[q] = miss ? best_t[q] : tt;
+        best_hit[q] = miss ? best_hit[q] : id;
+    }
+}
 template <int K, int AX, bool BOX_SIDE>
 VKD void flat_rects_k(const FlatProgram& P, uint32_t i0, uint32_t i1, const float3 (&co)[K], const float3 (&cd)[K], const float3 (&ci)[K],
                       float tmin, float (&best_t)[K], uint32_t (&best_hit)[K]) {
@@ -866,39 +904,7 @@ VKD void flat_rects_k(const FlatProgram& P, uint32_t i0, uint32_t i1, const floa
     // compares of a ray as three independent two-compare chains joined by one PLOP3 -- depth 3 instead of 6, one more
     // instruction -- is 1 % slower: the loop is bound by what it issues, not by the predicate chain, profiles/r2_sweep_15.log)
 #pragma unroll 1
-    for (uint32_t i = i0; i < i1; ++i) {
-        const float4 bd = P.rects[i].bounds;
-        const float k = P.rects[i].k;
-        const uint32_t id = P.rects[i].hitc;
-#pragma unroll
-        for (int q = 0; q < K; ++q) {
-            float tt, a, b;
-            if (AX == 0) {
-                tt = VKF_PLANE_T(k, co[q].z, cd[q].z, ci[q].z);
-                a = co[q].x + tt * cd[q].x;
-                b = co[q].y + tt * cd[q].y;
-            } else if (AX == 1) {
-                tt = VKF_PLANE_T(k, co[q].y, cd[q].y, ci[q].y);
-                a = co[q].x + tt * cd[q].x;
-                b = co[q].z + tt * cd[q].z;
-            } else {
-                tt = VKF_PLANE_T(k, co[q].x, cd[q].x, ci[q].x);
-                a = co[q].y + tt * cd[q].y;
-                b = co[q].z + tt * cd[q].z;
-            }
-            // same predicate as Rect::hit, evaluated without branches (bitwise on the comparison results).
-            // (Measured and rejected in round 2: the plane distance as one fma, k * (1/d) - o * (1/d), and the bounds as
-            // |a - centre| <= half extent.  0.6 % faster, but a ray that STARTS on the plane -- every scattered ray --
-            // no longer gets t = 0 exactly: the two products cancel to rounding noise of either sign, scaled by 1/d.
-            // Dropped samples rose from 26 to 1503 per 3.6e8 paths and light leaked around the box.)
-            // (the comparison with the closest hit so far comes last: it is the only link between one entry and the next)
-            bool miss = (a < bd.x) | (a > bd.y) | (b < bd.z) | (b > bd.w) | (tt < tmin);
-            miss = miss | (tt > best_t[q]);
-            if (BOX_SIDE) miss = miss | !(tt < best_t[q]);
-            best_t[q] = miss ? best_t[q] : tt;
-            best_hit[q] = miss ? best_hit[q] : id;
-        }
-    }
+    for (uint32_t i = i0; i < i1; ++i) flat_rect_k<K, AX, BOX_SIDE>(P.rects[i], co, cd, ci, tmin, best_t, best_hit);
 }
 // `live` masks the rays that exist (an idle slot's ray is traced as a dummy and ignored); best_hit
 // is 0xFFFFFFFF or the class-tagged id of the entry (VKF_HITC: index into P.hits | queue class << 8).
@@ -945,6 +951,34 @@ VKD bool flat_medium_box(const FlatMedium& fm, uint32_t ref, float3 o, float3 d,
     return true;
 }
 #endif
+// One static sphere entry for K rays.
+template <int K>
+VKD void flat_sphere_k(const FlatSphere& s, const float3 (&co)[K], const float3 (&cd)[K], float tmin, float (&best_t)[K], uint32_t (&best_hit)[K]) {
+    const float4 sp = s.a;
+    const uint32_t id = s.hitc;
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        float tt;
+        if (sphere_t(f3(sp), sp.w, co[q], cd[q], tmin, best_t[q], tt)) {
+            best_t[q] = tt;
+            best_hit[q] = id;
+        }
+    }
+}
+// The world rays (wo, wd) into a segment's frame through its chain composed into one affine map m (render build).
+template <int K>
+VKD void flat_affine_k(const float* m, const float3 (&wo)[K], const float3 (&wd)[K], float3 (&co)[K], float3 (&cd)[K]) {
+    const float r00 = m[0], r01 = m[1], r02 = m[2], r10 = m[3], r11 = m[4], r12 = m[5], r20 = m[6], r21 = m[7], r22 = m[8];
+    const float t0 = m[9], t1 = m[10], t2 = m[11];
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        const float3 o = wo[q], d = wd[q];
+        co[q] = f3(fmaf(r00, o.x, fmaf(r01, o.y, fmaf(r02, o.z, t0))), fmaf(r10, o.x, fmaf(r11, o.y, fmaf(r12, o.z, t1))),
+                   fmaf(r20, o.x, fmaf(r21, o.y, fmaf(r22, o.z, t2))));
+        cd[q] = f3(fmaf(r00, d.x, fmaf(r01, d.y, r02 * d.z)), fmaf(r10, d.x, fmaf(r11, d.y, r12 * d.z)),
+                   fmaf(r20, d.x, fmaf(r21, d.y, r22 * d.z)));
+    }
+}
 // One segment of the program: (co, cd) is the ray in the segment's frame, (o, d) the world ray.
 template <int K, bool MEDIA, bool HYBRID>
 VKD void flat_segment_k(const DScene& sc, const FlatProgram& P, const FlatSeg& g, uint32_t s, const float3 (&o)[K], const float3 (&d)[K],
@@ -964,18 +998,7 @@ VKD void flat_segment_k(const DScene& sc, const FlatProgram& P, const FlatSeg& g
     flat_boxes_k<K>(P, g.box0, g.box1, co, ci, tmin, best_t, best_hit);
 #endif
 #pragma unroll 1
-    for (uint32_t i = g.sph0; i < g.sph1; ++i) {
-        const float4 sp = P.spheres[i].a;
-        const uint32_t id = P.spheres[i].hitc;
-#pragma unroll
-        for (int q = 0; q < K; ++q) {
-            float tt;
-            if (sphere_t(f3(sp), sp.w, co[q], cd[q], tmin, best_t[q], tt)) {
-                best_t[q] = tt;
-                best_hit[q] = id;
-            }
-        }
-    }
+    for (uint32_t i = g.sph0; i < g.sph1; ++i) flat_sphere_k<K>(P.spheres[i], co, cd, tmin, best_t, best_hit);
 #if !VK_SIMPLE
 #pragma unroll 1
     for (uint32_t i = g.msph0; i < g.msph1; ++i) {
@@ -1070,19 +1093,7 @@ VKD void trace_flat_k(const DScene& sc, const FlatProgram& P, const float3 (&o)[
     for (uint32_t s = 1; s < n_segs; ++s) {
         const FlatSeg& g = P.segs[s];
         float3 co[K], cd[K];
-        {   // the chain as one affine map (composed at upload): no loop, no switch on the wrapper kind
-            const float* m = P.seg_affine[s];
-            const float r00 = m[0], r01 = m[1], r02 = m[2], r10 = m[3], r11 = m[4], r12 = m[5], r20 = m[6], r21 = m[7], r22 = m[8];
-            const float t0 = m[9], t1 = m[10], t2 = m[11];
-#pragma unroll
-            for (int q = 0; q < K; ++q) {
-                const float3 wo = o[q], wd = d[q];
-                co[q] = f3(fmaf(r00, wo.x, fmaf(r01, wo.y, fmaf(r02, wo.z, t0))), fmaf(r10, wo.x, fmaf(r11, wo.y, fmaf(r12, wo.z, t1))),
-                           fmaf(r20, wo.x, fmaf(r21, wo.y, fmaf(r22, wo.z, t2))));
-                cd[q] = f3(fmaf(r00, wd.x, fmaf(r01, wd.y, r02 * wd.z)), fmaf(r10, wd.x, fmaf(r11, wd.y, r12 * wd.z)),
-                           fmaf(r20, wd.x, fmaf(r21, wd.y, r22 * wd.z)));
-            }
-        }
+        flat_affine_k<K>(P.seg_affine[s], o, d, co, cd); // the chain as one affine map (composed at upload): no loop, no switch on the wrapper kind
         flat_segment_k<K, MEDIA, HYBRID>(sc, P, g, s, o, d, co, cd, time, live, tmin, xi, best_t, best_hit, sub, tc);
     }
     return;
@@ -1113,24 +1124,57 @@ VKD void trace_flat_k(const DScene& sc, const FlatProgram& P, const float3 (&o)[
             }
         }
 #else
-        if (g.op1 != g.op0) { // the chain as one affine map (composed at upload): no loop, no switch on the wrapper kind
-            const float* m = P.seg_affine[s];
-            const float r00 = m[0], r01 = m[1], r02 = m[2], r10 = m[3], r11 = m[4], r12 = m[5], r20 = m[6], r21 = m[7], r22 = m[8];
-            const float t0 = m[9], t1 = m[10], t2 = m[11];
-#pragma unroll
-            for (int q = 0; q < K; ++q) {
-                const float3 wo = co[q], wd = cd[q];
-                co[q] = f3(fmaf(r00, wo.x, fmaf(r01, wo.y, fmaf(r02, wo.z, t0))), fmaf(r10, wo.x, fmaf(r11, wo.y, fmaf(r12, wo.z, t1))),
-                           fmaf(r20, wo.x, fmaf(r21, wo.y, fmaf(r22, wo.z, t2))));
-                cd[q] = f3(fmaf(r00, wd.x, fmaf(r01, wd.y, r02 * wd.z)), fmaf(r10, wd.x, fmaf(r11, wd.y, r12 * wd.z)),
-                           fmaf(r20, wd.x, fmaf(r21, wd.y, r22 * wd.z)));
-            }
-        }
+        if (g.op1 != g.op0) flat_affine_k<K>(P.seg_affine[s], o, d, co, cd); // the chain as one affine map (composed at upload)
 #endif
         flat_segment_k<K, MEDIA, HYBRID>(sc, P, g, s, o, d, co, cd, time, live, tmin, xi, best_t, best_hit, sub, tc);
     }
     }
 }
+
+#if !VK_STRICT
+// trace_flat_k without media or subtrees, for a program of a shape compiled in (FlatShape, vk_internal.h): the same
+// entries in the same order with the same arithmetic, but every loop unrolled over the shape's counts, so each operand
+// is a constant-bank load at a constant offset -- no walk over FlatSeg's byte ranges, no loop counters or branches.
+template <class G, int K>
+VKD void flat_segment_static(const FlatProgram& P, const float3 (&co)[K], const float3 (&cd)[K], float tmin, float (&best_t)[K],
+                             uint32_t (&best_hit)[K]) {
+    float3 ci[K];
+#pragma unroll
+    for (int q = 0; q < K; ++q) ci[q] = rcp3(cd[q]);
+#pragma unroll
+    for (int i = G::x0; i < G::x1; ++i) flat_rect_k<K, 0, false>(P.rects[i], co, cd, ci, tmin, best_t, best_hit);
+#pragma unroll
+    for (int i = G::y0; i < G::y1; ++i) flat_rect_k<K, 1, false>(P.rects[i], co, cd, ci, tmin, best_t, best_hit);
+#pragma unroll
+    for (int i = G::z0; i < G::z1; ++i) flat_rect_k<K, 2, false>(P.rects[i], co, cd, ci, tmin, best_t, best_hit);
+#pragma unroll
+    for (int i = G::b0; i < G::b1; ++i) flat_box_k<K>(P.boxes[i], co, ci, tmin, best_t, best_hit);
+#pragma unroll
+    for (int i = G::s0; i < G::s1; ++i) flat_sphere_k<K>(P.spheres[i], co, cd, tmin, best_t, best_hit);
+}
+template <int K, int S, class G, class... Rest>
+VKD void flat_segments_static(const FlatProgram& P, const float3 (&o)[K], const float3 (&d)[K], float tmin, float (&best_t)[K],
+                              uint32_t (&best_hit)[K]) {
+    if constexpr (S == 0) { // the world frame: the ray as it is
+        flat_segment_static<G, K>(P, o, d, tmin, best_t, best_hit);
+    } else {
+        float3 co[K], cd[K];
+        flat_affine_k<K>(P.seg_affine[S], o, d, co, cd);
+        flat_segment_static<G, K>(P, co, cd, tmin, best_t, best_hit);
+    }
+    if constexpr (sizeof...(Rest) > 0) flat_segments_static<K, S + 1, Rest...>(P, o, d, tmin, best_t, best_hit);
+}
+template <int K, class... Seg>
+VKD void trace_flat_static(const FlatProgram& P, FlatShape<Seg...>, const float3 (&o)[K], const float3 (&d)[K], float tmin, float (&best_t)[K],
+                           uint32_t (&best_hit)[K]) {
+#pragma unroll
+    for (int q = 0; q < K; ++q) {
+        best_t[q] = CUDART_INF_F;
+        best_hit[q] = 0xFFFFFFFFu;
+    }
+    flat_segments_static<K, 0, Seg...>(P, o, d, tmin, best_t, best_hit);
+}
+#endif
 
 // ---------------------------------------------------------------------------------------------
 // HitRec (src/hittable.rs:11-31) of the winning primitive, built once per segment.
@@ -1604,55 +1648,35 @@ struct BounceXiTable {
     VKD uint4 block0() const { return r; }
     VKD uint32_t spec() const { return s; }
 };
-// One bounce of ray_color's loop body after world.hit() returned `rec` (src/main.rs:131-149).
-// Returns false when the path ends.  `valid` is cleared when the reference's value would be
-// non-finite (the whole sample is then dropped, src/main.rs:191-194).
-template <class XI>
-VKD bool shade_xi(const DScene& sc, const HitRecD& rec, const XI& xi, float3& o, float3& d, float& time,
-                  float3& beta, float3& L, bool& valid) {
-    uint4 m = rec.m;
-    uint32_t type = m.x;
-    uint32_t spdf_type = type; // whose scattering_pdf applies
+// One bounce of ray_color's loop body after world.hit() returned `rec` (src/main.rs:131-149), one body per material
+// class: shade_xi dispatches on the material; a warp-queue shade batch whose queue fixes the class calls its body
+// directly (wq_shade_batch), so that it carries no code of the other classes.
+// DiffuseLight (src/material.rs:218-225; scatter_with_pdf -> None; src/main.rs:147-149): the path ends.
+VKD bool shade_emitter(const DScene& sc, const HitRecD& rec, const uint4& m, const float3& beta, float3& L) {
     float3 emitted = f3(0.0f, 0.0f, 0.0f);
-    if (!VK_SIMPLE && !VK_LIGHT0 && type == VK_M_SPECDIFFUSE) { // src/material.rs:474-488: emitted() is the trait default (0)
-        const uint32_t diffuse = m.w & ~VKD_MAT_NEEDS_UV;
-        spdf_type = __ldg(&sc.materials[diffuse]).x;
-        m = __ldg(&sc.materials[u01(xi.spec()) < __uint_as_float(m.z) ? m.y : diffuse]);
-        type = m.x;
-    } else if (type == VK_M_DIFFUSE_LIGHT) { // src/material.rs:218-225; scatter_with_pdf -> None
-        if (rec.front) emitted = tex_value(sc, m.y, rec.u, rec.v, rec.p);
-    }
-    if (type == VK_M_DIFFUSE_LIGHT) { // src/main.rs:147-149
-        L = L + beta * emitted;
-        return false;
-    }
-    const uint4 r = xi.block0();
-    if (type == VK_M_DIELECTRIC) { // src/material.rs:177-206, attenuation (1,1,1)
-        const float ref_idx = __uint_as_float(m.z);
-        const float etai_over_etat = rec.front ? 1.0f / ref_idx : ref_idx;
-        const float3 unit_direction = unit_vector(d);
-        const float cos_theta = fminf(dot3(-unit_direction, rec.normal), 1.0f);
-        const float sin_theta = sqrtf(1.0f - cos_theta * cos_theta);
-        float3 nd;
-        if (etai_over_etat * sin_theta > 1.0f) nd = reflect(unit_direction, rec.normal);
-        else if (u01(r.x) < schlick(cos_theta, etai_over_etat)) nd = reflect(unit_direction, rec.normal);
-        else nd = refract(unit_direction, rec.normal, etai_over_etat);
-        o = rec.p;
-        d = nd; // keeps r.time
-        return true;
-    }
-    if (!VK_SIMPLE && type == VK_M_METAL) { // src/material.rs:134-141: Ray::new -> time 0 (Q6), never absorbed
-        const float fuzz = __uint_as_float(m.z);
-        float3 nd = reflect(unit_vector(d), rec.normal);
-        if (fuzz != 0.0f) nd = nd + random_in_unit_sphere(u01(r.x), u01(r.y), u01(r.z)) * fuzz;
-        beta = beta * tex_value(sc, m.y, rec.u, rec.v, rec.p);
-        o = rec.p;
-        d = nd;
-        time = 0.0f;
-        return true;
-    }
-    // Lambertian / Isotropic (src/material.rs:92-108, :448-464): cosine lobe about rec.normal,
-    // mixed 50/50 with light sampling (src/main.rs:139-146).
+    if (rec.front) emitted = tex_value(sc, m.y, rec.u, rec.v, rec.p);
+    L = L + beta * emitted;
+    return false;
+}
+// Dielectric (src/material.rs:177-206), attenuation (1,1,1).
+VKD bool shade_dielectric(const HitRecD& rec, const uint4& m, const uint4& r, float3& o, float3& d) {
+    const float ref_idx = __uint_as_float(m.z);
+    const float etai_over_etat = rec.front ? 1.0f / ref_idx : ref_idx;
+    const float3 unit_direction = unit_vector(d);
+    const float cos_theta = fminf(dot3(-unit_direction, rec.normal), 1.0f);
+    const float sin_theta = sqrtf(1.0f - cos_theta * cos_theta);
+    float3 nd;
+    if (etai_over_etat * sin_theta > 1.0f) nd = reflect(unit_direction, rec.normal);
+    else if (u01(r.x) < schlick(cos_theta, etai_over_etat)) nd = reflect(unit_direction, rec.normal);
+    else nd = refract(unit_direction, rec.normal, etai_over_etat);
+    o = rec.p;
+    d = nd; // keeps r.time
+    return true;
+}
+// Lambertian / Isotropic (src/material.rs:92-108, :448-464): cosine lobe about rec.normal,
+// mixed 50/50 with light sampling (src/main.rs:139-146).  spdf_type: whose scattering_pdf applies.
+VKD bool shade_diffuse(const DScene& sc, const HitRecD& rec, const uint4& m, uint32_t spdf_type, const uint4& r, float3& o, float3& d,
+                       float3& beta, bool& valid) {
     const float3 attenuation = tex_value(sc, m.y, rec.u, rec.v, rec.p);
 #if VK_STRICT
     const Onb uvw = onb_from_w(rec.normal);
@@ -1698,6 +1722,40 @@ VKD bool shade_xi(const DScene& sc, const HitRecD& rec, const XI& xi, float3& o,
     o = rec.p;
     d = nd; // Ray::new_with_time(c.p, dir, r.time): keeps the camera-sampled time
     return true;
+}
+// Returns false when the path ends.  `valid` is cleared when the reference's value would be
+// non-finite (the whole sample is then dropped, src/main.rs:191-194).
+template <class XI>
+VKD bool shade_xi(const DScene& sc, const HitRecD& rec, const XI& xi, float3& o, float3& d, float& time,
+                  float3& beta, float3& L, bool& valid) {
+    uint4 m = rec.m;
+    uint32_t type = m.x;
+    uint32_t spdf_type = type; // whose scattering_pdf applies
+    if (!VK_SIMPLE && !VK_LIGHT0 && type == VK_M_SPECDIFFUSE) { // src/material.rs:474-488: emitted() is the trait default (0)
+        const uint32_t diffuse = m.w & ~VKD_MAT_NEEDS_UV;
+        spdf_type = __ldg(&sc.materials[diffuse]).x;
+        m = __ldg(&sc.materials[u01(xi.spec()) < __uint_as_float(m.z) ? m.y : diffuse]);
+        type = m.x;
+        if (type == VK_M_DIFFUSE_LIGHT) { // emitted() of the SpecDiffuse is 0 (src/main.rs:147-149)
+            L = L + beta * f3(0.0f, 0.0f, 0.0f);
+            return false;
+        }
+    } else if (type == VK_M_DIFFUSE_LIGHT) {
+        return shade_emitter(sc, rec, m, beta, L);
+    }
+    const uint4 r = xi.block0();
+    if (type == VK_M_DIELECTRIC) return shade_dielectric(rec, m, r, o, d);
+    if (!VK_SIMPLE && type == VK_M_METAL) { // src/material.rs:134-141: Ray::new -> time 0 (Q6), never absorbed
+        const float fuzz = __uint_as_float(m.z);
+        float3 nd = reflect(unit_vector(d), rec.normal);
+        if (fuzz != 0.0f) nd = nd + random_in_unit_sphere(u01(r.x), u01(r.y), u01(r.z)) * fuzz;
+        beta = beta * tex_value(sc, m.y, rec.u, rec.v, rec.p);
+        o = rec.p;
+        d = nd;
+        time = 0.0f;
+        return true;
+    }
+    return shade_diffuse(sc, rec, m, spdf_type, r, o, d, beta, valid);
 }
 VKD bool shade(const DScene& sc, const HitRecD& rec, const PathRng& rng, uint32_t depth, float3& o, float3& d, float& time,
                float3& beta, float3& L, bool& valid) {

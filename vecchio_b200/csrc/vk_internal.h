@@ -172,6 +172,35 @@ struct FlatProgram {
                                    // which costs the Cornell kernel 0.5 % (31.15 -> 31.32 ms, profiles/r2_sweep_21.log)
 };
 
+// A flat program's SHAPE compiled into the warp-queue kernel (trace_flat_static, vk_device.cuh): per segment, the entry
+// ranges the render build's trace reads -- rects per axis, static spheres, boxes -- as [begin, end) of FlatProgram's
+// arrays.  The entries stay where the builder put them; the kernel reads them at constant offsets with every loop
+// unrolled, instead of walking FlatSeg's byte ranges.  Every segment after the first is an instance frame with its affine
+// map, as in trace_flat_k.  A program matches a shape when its segments read exactly these entries and nothing else (no
+// moving sphere, medium or subtree).
+template <int X0, int X1, int Y0, int Y1, int Z0, int Z1, int S0, int S1, int B0, int B1>
+struct FlatSegShape {
+    static constexpr int x0 = X0, x1 = X1, y0 = Y0, y1 = Y1, z0 = Z0, z1 = Z1, s0 = S0, s1 = S1, b0 = B0, b1 = B1;
+    static bool matches(const FlatSeg& g) {
+        auto same = [](uint32_t a0, uint32_t a1, int w0, int w1) { return a1 - a0 == (uint32_t)(w1 - w0) && (w1 == w0 || a0 == (uint32_t)w0); };
+        return same(g.rect0[0], g.rect1[0], X0, X1) && same(g.rect0[1], g.rect1[1], Y0, Y1) && same(g.rect0[2], g.rect1[2], Z0, Z1) &&
+               same(g.sph0, g.sph1, S0, S1) && same(g.box0, g.box1, B0, B1) && g.msph0 == g.msph1 && g.med0 == g.med1 && g.bvh0 == g.bvh1;
+    }
+};
+template <class... Seg>
+struct FlatShape {
+    static constexpr uint32_t n_segs = sizeof...(Seg); // 0: no shape, the generic trace
+    static bool matches(const FlatProgram& P) {
+        uint32_t s = 0;
+        return n_segs != 0 && P.n != 0 && P.n_segs == n_segs && P.n_bvh == 0 && (Seg::matches(P.segs[s++]) && ...);
+    }
+};
+// The shapes the kernel is compiled for (vk_warpq.cu, namespace vkfast_simple), and the number naming each.
+// cornell_box: the world frame (1 XY, 3 XZ, 2 YZ rects, the glass sphere), the rotated box's instance frame (one box)
+using FlatShapeCornell = FlatShape<FlatSegShape<0, 1, 1, 4, 4, 6, 0, 1, 0, 0>, FlatSegShape<0, 0, 0, 0, 0, 0, 0, 0, 0, 1>>;
+enum { VKF_SHAPE_NONE = 0, VKF_SHAPE_CORNELL = 1 };
+inline uint32_t flat_static_shape(const FlatProgram& P) { return FlatShapeCornell::matches(P) ? (uint32_t)VKF_SHAPE_CORNELL : (uint32_t)VKF_SHAPE_NONE; }
+
 struct DCamera {
     float3 origin, lower_left_corner, horizontal, vertical, u, v;
     float lens_radius, time0, time1;
@@ -302,9 +331,9 @@ struct WfState {
     cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,      \
                               const RenderBuffers& b, unsigned long long* unit_head, int sm_count, cudaStream_t st);   \
     template <class D>                                                                                                 \
-    cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a,       \
-                             const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy,         \
-                             cudaStream_t st, const D& dom);                                                           \
+    cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, uint32_t flat_shape, const DCamera& cam,       \
+                             const RenderArgs& a, const RenderBuffers& b, unsigned long long* unit_head, int sm_count, \
+                             bool legacy, cudaStream_t st, const D& dom);                                              \
     size_t stepq_stack_words(uint32_t stack_need, bool inst, int sm_count, uint32_t* levels);                          \
     template <class D>                                                                                                 \
     cudaError_t launch_stepq(const DScene& sc, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,        \
@@ -323,6 +352,6 @@ namespace vkfast_simple { // vk_staged.cu / vk_warpq.cu compiled with VK_SIMPLE=
 cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
                           unsigned long long* unit_head, int sm_count, cudaStream_t st);
 template <class D>
-cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom);
+cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, uint32_t flat_shape, const DCamera& cam, const RenderArgs& a,
+                         const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom);
 }

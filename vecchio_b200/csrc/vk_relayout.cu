@@ -32,6 +32,7 @@ int vk_scene_check(const vk_scene_desc* d, vk_scene_info* info, char* err, size_
         info->dynamic_megakernel = d->n_nodes >= 65536u ? 1u : 0u;
         info->flat_boxes = 0;
         for (uint32_t s = 0; R.flat.n && s < R.flat.n_segs; ++s) info->flat_boxes += R.flat.segs[s].box1 - R.flat.segs[s].box0;
+        info->flat_shape = R.flat_shape;
         info->flat_direct = 0;
         for (size_t h = 0; 2 * h + 1 < R.flat_shade.size(); ++h) info->flat_direct += __float_as_uint_host(R.flat_shade[2 * h].w) & 1u;
     }

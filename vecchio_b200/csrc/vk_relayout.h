@@ -519,6 +519,7 @@ struct Relayout {
     FlatProgram flat{};
     uint32_t levels_world = 0, levels_sub = 0, n_wide = 0, stack_need = 0;
     bool simple = false, has_specdiffuse = false;
+    uint32_t flat_shape = VKF_SHAPE_NONE; // the compiled shape the program has (flat_static_shape), if any
     // Per entry of the flat program's hit table, for the render build's shade stage: {world-space outward normal,
     // flags} {material index, -, -, -}.  flags bit 0: the HitRec of this entry can be written down directly --
     // p = o + t d, normal = the constant normal turned against the ray -- instead of walking its wrapper chain; bit 1:
@@ -696,6 +697,7 @@ struct Relayout {
                 flat_shade[2 * h + 1].x = __uint_as_float_host(mat);
             }
         }
+        flat_shape = flat_static_shape(flat);
         has_specdiffuse = false;
         for (uint32_t i = 0; i < d->n_materials; ++i) has_specdiffuse |= d->materials[i].type == VK_M_SPECDIFFUSE;
         // simple: solid textures only; Lambertian / Dielectric / DiffuseLight / Isotropic only; no moving sphere;

@@ -34,7 +34,16 @@ namespace VK_NS {
 // cluster) are traversed inside the extend stage, every lane for its own ray; what differs between the lanes of a batch is
 // then only how long a walk through ONE kind of tree takes -- the heterogeneous top of the scene (loose spheres, media,
 // rects) is typed batches, and the shading runs on whole batches of a class.
-template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID, class D>
+// SHAPE: FlatShape<> walks the program as it comes (trace_flat_k); a compiled shape traces it with trace_flat_static.
+// The kernel of a compiled shape also shades each batch with the body of its queue's class (wq_shade_batch's SPLIT): the
+// queue number is warp-uniform, so the choice is one uniform branch per batch, and the shading code of a batch has no test
+// on the material's type.  (The generic kernel keeps one shading body: with the split it LOST 6 % on Cornell, 32.96
+// against 30.96 ms per frame -- a larger kernel around the same rolled trace; with the static trace the two together run
+// 26.98 ms, profiles/r3_static_flat_split_b200.jsonl.)
+#ifndef VKQ_CLASS_SHADE
+#define VKQ_CLASS_SHADE 1
+#endif
+template <bool MEDIA, bool LEGACY, class W, int K, bool HYBRID, class D, class SHAPE = FlatShape<>>
 VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& buf,
                          unsigned long long* unit_head, const D& dom) {
     extern __shared__ __align__(16) unsigned char vkq_raw[];
@@ -54,7 +63,8 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
         if (!wq_pick(S, wq_counts(S), EXT_CAP, q, n_q, tail_q)) break; // every queue is empty: all slots have retired
         const uint32_t n = wq_pop(S, q, n_q, tail_q, q == VKQ_EXT ? EXT_CAP : 32u, lane, head);
         if (q != VKQ_EXT) {
-            wq_shade_batch<LEGACY, !HYBRID>(sc, C, dom, buf, q, n, head, n_drop); // (no shading records for subtree hits)
+            constexpr bool SPLIT = VKQ_CLASS_SHADE && SHAPE::n_segs != 0;
+            wq_shade_batch<LEGACY, !HYBRID, SPLIT>(sc, C, dom, buf, q, n, head, n_drop); // (no shading records for subtree hits)
             continue;
         }
         // ---- extend: world.hit() (src/main.rs:130) for up to EXT_CAP rays, K per lane --------------------------------
@@ -81,7 +91,13 @@ VKD void warpq_flat_body(const DScene& sc, const FlatProgram* flat, const DCamer
             if (MEDIA) dom_slot_rng(dom, a, xi[k].rng);
         }
         TraceHit sub[K];
-        trace_flat_k<K, MEDIA, HYBRID>(sc, *flat, o, d, tm, live, 0.001f, xi, best_t, best_hit, sub, &tc);
+#if !VK_STRICT
+        if constexpr (SHAPE::n_segs != 0) {
+            static_assert(!MEDIA && !HYBRID, "a compiled shape has no media and no subtrees");
+            trace_flat_static<K>(*flat, SHAPE{}, o, d, 0.001f, best_t, best_hit);
+        } else
+#endif
+            trace_flat_k<K, MEDIA, HYBRID>(sc, *flat, o, d, tm, live, 0.001f, xi, best_t, best_hit, sub, &tc);
 #pragma unroll
         for (int k = 0; k < K; ++k) {
             uint32_t cls = VKQ_NONE;
@@ -241,6 +257,15 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat(co
                                                                           const __grid_constant__ D dom) {
     warpq_flat_body<false, LEGACY, WqFlat, VKQ_K_FLAT, false>(sc, &flat, cam, a, buf, unit_head, dom);
 }
+#if VK_SIMPLE
+// k_warpq_flat for a program of a compiled shape (FlatShape, vk_internal.h; chosen at upload)
+template <class SHAPE, class D>
+__global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_FLAT) k_warpq_flat_static(const DScene sc, const __grid_constant__ FlatProgram flat,
+                                                                                 const DCamera cam, const RenderArgs a, const RenderBuffers buf,
+                                                                                 unsigned long long* unit_head, const __grid_constant__ D dom) {
+    warpq_flat_body<false, false, WqFlat, VKQ_K_FLAT, false, D, SHAPE>(sc, &flat, cam, a, buf, unit_head, dom);
+}
+#endif
 template <bool LEGACY, class D>
 __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_MEDIA) k_warpq_flat_media(const DScene sc, const __grid_constant__ FlatProgram flat,
                                                                                  const DCamera cam, const RenderArgs a, const RenderBuffers buf,
@@ -257,9 +282,10 @@ __global__ void __launch_bounds__(32 * VKQ_WARPS, VKQ_MINB_HYB) k_warpq_hybrid(c
 #endif
 
 // grid = sm_count * resident CTAs (persistent); *unit_head must be zero on the stream before the launch
+// flat_shape: the program's compiled shape (VKF_SHAPE_*, found at upload), or VKF_SHAPE_NONE
 template <class D>
-cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
-                         unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom) {
+cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, uint32_t flat_shape, const DCamera& cam, const RenderArgs& a,
+                         const RenderBuffers& b, unsigned long long* unit_head, int sm_count, bool legacy, cudaStream_t st, const D& dom) {
     int bps = 0;
     cudaError_t e;
     const bool media = sc.has_media != 0u;
@@ -277,8 +303,11 @@ cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamer
     }
 #if VK_SIMPLE
     (void)legacy; // the trimmed build exists for the HEAD integrator on flat scenes only
-    if (media) VKQ_LAUNCH_FLAT((k_warpq_flat_media<false, D>), WqMedia) else VKQ_LAUNCH_FLAT((k_warpq_flat<false, D>), WqFlat)
+    if (media) VKQ_LAUNCH_FLAT((k_warpq_flat_media<false, D>), WqMedia)
+    else if (flat_shape == VKF_SHAPE_CORNELL) VKQ_LAUNCH_FLAT((k_warpq_flat_static<FlatShapeCornell, D>), WqFlat)
+    else VKQ_LAUNCH_FLAT((k_warpq_flat<false, D>), WqFlat)
 #else
+    (void)flat_shape; // (shapes are compiled into the trimmed build only)
 #define VKQ_LAUNCH_HYB(M, G) VKQ_LAUNCH_FLAT((k_warpq_hybrid<M, G, D>), WqHyb)
     if (flat && flat->n && flat->n_bvh) {
         if (media) { if (legacy) VKQ_LAUNCH_HYB(true, true) else VKQ_LAUNCH_HYB(true, false) }
@@ -297,8 +326,8 @@ cudaError_t launch_warpq(const DScene& sc, const FlatProgram* flat, const DCamer
     return cudaGetLastError();
 }
 #define VKQ_INSTANTIATE(D)                                                                                             \
-    template cudaError_t launch_warpq(const DScene&, const FlatProgram*, const DCamera&, const RenderArgs&, const RenderBuffers&, \
-                                      unsigned long long*, int, bool, cudaStream_t, const D&);
+    template cudaError_t launch_warpq(const DScene&, const FlatProgram*, uint32_t, const DCamera&, const RenderArgs&,         \
+                                      const RenderBuffers&, unsigned long long*, int, bool, cudaStream_t, const D&);
 VKQ_INSTANTIATE(OneFrame)
 VKQ_INSTANTIATE(FrameArgs)
 VKQ_INSTANTIATE(ListArgs)

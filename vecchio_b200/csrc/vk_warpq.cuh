@@ -357,86 +357,120 @@ VKD uint32_t wq_pop(W& S, uint32_t q, uint32_t n_q, uint32_t tail_q, uint32_t ca
 #ifndef VKQ_FAST_RESOLVE
 #define VKQ_FAST_RESOLVE 1 // (Cornell, 1000 spp: 37.9 against 40.0 ms per frame)
 #endif
-template <bool LEGACY, bool FLAT, class W, class D>
-VKD void wq_shade_batch(const DScene& sc, const WqCtx<W>& C, const D& dom, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
+// The shading of one lane's slot (act: the lane holds one), in the batch of a class.  CLS: the class every slot of the
+// batch has -- VKQ_EMIT (emitters and misses), VKQ_DIEL, VKQ_DIFF (Lambertian / Isotropic, the DIFF and DIFFI queues
+// alike) -- so that the code is that class's shading body alone; VKQ_NQ: any class, shade_xi's dispatch on the material.
+// The queue a slot sits in comes from its material at upload (VKF_HITC), so a slot of another class cannot occur: the
+// VKQ_SELFCHECK build counts one as a violation.
+template <bool LEGACY, bool FLAT, int CLS, class W, class D>
+VKD void wq_shade_slot(const DScene& sc, const WqCtx<W>& C, const D& dom, const RenderBuffers& buf, bool act, uint32_t slot, bool& alive,
+                       bool& ended, uint32_t& n_drop) {
+    static_assert(CLS == VKQ_NQ || (!LEGACY && (CLS == VKQ_EMIT || CLS == VKQ_DIEL || CLS == VKQ_DIFF)),
+                  "class bodies: the HEAD integrator's emitter, dielectric and diffuse");
     W& S = C.S;
     const RenderArgs& a = C.a;
+    if (act) {
+        const float4 ro = S.ro[slot], rd = S.rd[slot], bt = S.bt[slot];
+        const uint4 hp = S.hp[slot];
+        float3 o = f3(ro), d = f3(rd), beta = f3(bt), L = f3(0.0f, 0.0f, 0.0f);
+        float time = ro.w;
+        uint32_t depth = __float_as_uint(rd.w);
+        const uint32_t pixel = S.px[slot], prim = hp.y;
+        bool valid = true;
+#if VKQ_SELFCHECK
+        if (CLS != VKQ_NQ && CLS != VKQ_EMIT && prim == VK_REF_NONE) atomicAdd(&buf.counters[5], 1ull); // (a miss files as an emitter)
+#endif
+        if ((CLS == VKQ_NQ || CLS == VKQ_EMIT) && prim == VK_REF_NONE) {
+            L = beta * miss_color(a, d); // src/main.rs:151
+        } else {
+            PathRng rng;
+            rng.pixel = pixel;
+            rng.sample = __float_as_uint(bt.w);
+            rng.key = make_uint2(a.seed_lo, a.seed_hi);
+            dom_slot_rng(dom, a, rng); // (the slot's pixel is the accumulator index: batch-wide in a batch)
+            HitRecD rec;
+            bool direct = false;
+            uint32_t leaf = prim, hi = hp.z;
+            if (FLAT) { // a flat program's slot keeps the distance and the hit-table entry; the rest hangs under the entry
+                const float4 fs1 = __ldg(&sc.flat_shade[2u * hp.w + 1u]);
+                leaf = __float_as_uint(fs1.y);
+                hi = __float_as_uint(fs1.z);
+#if VKQ_FAST_RESOLVE && !VK_STRICT
+                const float4 fs = __ldg(&sc.flat_shade[2u * hp.w]);
+                const uint32_t fl = __float_as_uint(fs.w);
+                if (fl & 1u) {
+                    direct = true;
+                    const float3 nw = f3(fs);
+                    const bool toward = dot3(d, nw) < 0.0f;
+                    rec.t = __uint_as_float(hp.x);
+                    rec.p = at(o, d, rec.t);
+                    rec.normal = toward ? nw : -nw;
+                    rec.front = (toward ? 1u : 0u) ^ ((fl >> 1) & 1u);
+                    rec.u = 0.0f;
+                    rec.v = 0.0f;
+                    rec.mat = __float_as_uint(fs1.x);
+                    rec.m = __ldg(&sc.materials[rec.mat]);
+                }
+#endif
+            }
+            if (!direct) {
+                TraceHit h;
+                h.t = __uint_as_float(hp.x);
+                h.prim = leaf;
+                h.inst = (hi & 0x80000000u) ? (((uint32_t)VK_T_XFORM << 28) | (hi & 0x07FFFFFFu)) : 0u;
+                h.face = (hi >> 28) & 7u;
+                resolve_hit(sc, h, o, d, time, false, rec);
+            }
+            if constexpr (CLS == VKQ_NQ) {
+                alive = LEGACY ? shade_legacy(sc, rec, rng, depth, o, d, time, beta, L, valid)
+                               : shade(sc, rec, rng, depth, o, d, time, beta, L, valid);
+            } else {
+#if VKQ_SELFCHECK
+                const uint32_t t = rec.m.x;
+                const uint32_t mc = t == VK_M_DIFFUSE_LIGHT ? VKQ_EMIT : t == VK_M_DIELECTRIC ? VKQ_DIEL
+                                  : (t == VK_M_LAMBERTIAN || t == VK_M_ISOTROPIC) ? VKQ_DIFF : VKQ_NONE;
+                if (mc != (uint32_t)CLS) atomicAdd(&buf.counters[5], 1ull);
+#endif
+                if constexpr (CLS == VKQ_EMIT) {
+                    alive = shade_emitter(sc, rec, rec.m, beta, L);
+                } else {
+                    const uint4 r = rng.block(depth, 0u); // (BounceXiPhilox::block0)
+                    if constexpr (CLS == VKQ_DIEL) alive = shade_dielectric(rec, rec.m, r, o, d);
+                    else alive = shade_diffuse(sc, rec, rec.m, rec.m.x, r, o, d, beta, valid);
+                }
+            }
+            if (alive && ++depth > a.max_depth) alive = false; // `depth > MAX_DEPTH` -> 0 (src/main.rs:126)
+            if (alive && !(finite3(d) && finite3(o))) {          // the reference's sample is NaN here (see vk_kernels.cu)
+                valid = false;
+                alive = false;
+            }
+        }
+        if (alive) {
+            S.ro[slot] = make_float4(o.x, o.y, o.z, time);
+            S.rd[slot] = make_float4(d.x, d.y, d.z, __uint_as_float(depth));
+            S.bt[slot] = make_float4(beta.x, beta.y, beta.z, bt.w);
+            S.mark_new(slot);
+        } else {
+            if (valid && finite3(L)) dom_accumulate(dom, buf, pixel, L);
+            else ++n_drop;
+            ended = true;
+        }
+    }
+}
+// One batch of queue q: SPLIT (the trimmed build's flat kernels without media) runs the shading body of the queue's class,
+// chosen by one uniform branch per batch; the regeneration and the queue pushes after it are the same for every class.
+template <bool LEGACY, bool FLAT, bool SPLIT = false, class W, class D>
+VKD void wq_shade_batch(const DScene& sc, const WqCtx<W>& C, const D& dom, const RenderBuffers& buf, uint32_t q, uint32_t n, uint32_t head, uint32_t& n_drop) {
+    W& S = C.S;
     const uint32_t lane = C.lane;
     const bool act = lane < n;
     const uint32_t slot = S.ring[q][(head + (act ? lane : 0u)) & W::RMASK];
     bool alive = false, ended = false;
-    if (q != VKQ_END) {
-        if (act) {
-            const float4 ro = S.ro[slot], rd = S.rd[slot], bt = S.bt[slot];
-            const uint4 hp = S.hp[slot];
-            float3 o = f3(ro), d = f3(rd), beta = f3(bt), L = f3(0.0f, 0.0f, 0.0f);
-            float time = ro.w;
-            uint32_t depth = __float_as_uint(rd.w);
-            const uint32_t pixel = S.px[slot], prim = hp.y;
-            bool valid = true;
-            if (prim == VK_REF_NONE) {
-                L = beta * miss_color(a, d); // src/main.rs:151
-            } else {
-                PathRng rng;
-                rng.pixel = pixel;
-                rng.sample = __float_as_uint(bt.w);
-                rng.key = make_uint2(a.seed_lo, a.seed_hi);
-                dom_slot_rng(dom, a, rng); // (the slot's pixel is the accumulator index: batch-wide in a batch)
-                HitRecD rec;
-                bool direct = false;
-                uint32_t leaf = prim, hi = hp.z;
-                if (FLAT) { // a flat program's slot keeps the distance and the hit-table entry; the rest hangs under the entry
-                    const float4 fs1 = __ldg(&sc.flat_shade[2u * hp.w + 1u]);
-                    leaf = __float_as_uint(fs1.y);
-                    hi = __float_as_uint(fs1.z);
-#if VKQ_FAST_RESOLVE && !VK_STRICT
-                    const float4 fs = __ldg(&sc.flat_shade[2u * hp.w]);
-                    const uint32_t fl = __float_as_uint(fs.w);
-                    if (fl & 1u) {
-                        direct = true;
-                        const float3 nw = f3(fs);
-                        const bool toward = dot3(d, nw) < 0.0f;
-                        rec.t = __uint_as_float(hp.x);
-                        rec.p = at(o, d, rec.t);
-                        rec.normal = toward ? nw : -nw;
-                        rec.front = (toward ? 1u : 0u) ^ ((fl >> 1) & 1u);
-                        rec.u = 0.0f;
-                        rec.v = 0.0f;
-                        rec.mat = __float_as_uint(fs1.x);
-                        rec.m = __ldg(&sc.materials[rec.mat]);
-                    }
-#endif
-                }
-                if (!direct) {
-                    TraceHit h;
-                    h.t = __uint_as_float(hp.x);
-                    h.prim = leaf;
-                    h.inst = (hi & 0x80000000u) ? (((uint32_t)VK_T_XFORM << 28) | (hi & 0x07FFFFFFu)) : 0u;
-                    h.face = (hi >> 28) & 7u;
-                    resolve_hit(sc, h, o, d, time, false, rec);
-                }
-                alive = LEGACY ? shade_legacy(sc, rec, rng, depth, o, d, time, beta, L, valid)
-                               : shade(sc, rec, rng, depth, o, d, time, beta, L, valid);
-                if (alive && ++depth > a.max_depth) alive = false; // `depth > MAX_DEPTH` -> 0 (src/main.rs:126)
-                if (alive && !(finite3(d) && finite3(o))) {          // the reference's sample is NaN here (see vk_kernels.cu)
-                    valid = false;
-                    alive = false;
-                }
-            }
-            if (alive) {
-                S.ro[slot] = make_float4(o.x, o.y, o.z, time);
-                S.rd[slot] = make_float4(d.x, d.y, d.z, __uint_as_float(depth));
-                S.bt[slot] = make_float4(beta.x, beta.y, beta.z, bt.w);
-                S.mark_new(slot);
-            } else {
-                if (valid && finite3(L)) dom_accumulate(dom, buf, pixel, L);
-                else ++n_drop;
-                ended = true;
-            }
-        }
-    } else {
-        ended = act; // queued regenerations
-    }
+    if (q == VKQ_END) ended = act; // queued regenerations
+    else if constexpr (!SPLIT) wq_shade_slot<LEGACY, FLAT, VKQ_NQ>(sc, C, dom, buf, act, slot, alive, ended, n_drop);
+    else if (q == VKQ_DIFF || q == VKQ_DIFFI) wq_shade_slot<LEGACY, FLAT, VKQ_DIFF>(sc, C, dom, buf, act, slot, alive, ended, n_drop);
+    else if (q == VKQ_EMIT) wq_shade_slot<LEGACY, FLAT, VKQ_EMIT>(sc, C, dom, buf, act, slot, alive, ended, n_drop);
+    else wq_shade_slot<LEGACY, FLAT, VKQ_DIEL>(sc, C, dom, buf, act, slot, alive, ended, n_drop); // (no simple scene has Metal)
     // Regenerate in place when enough lanes ended -- the emitter / miss class does, every lane; in the other classes
     // only a few lanes end (a light-sampled direction below the surface has weight 0): those are queued and
     // regenerated together, with full warps.
