@@ -230,7 +230,10 @@ typedef struct vk_render_params {
     uint32_t spp;       /* SAMPLES_PER_PIXEL: the divisor of the mean (main.rs:196)     */
     uint32_t spp_begin; /* this call renders global samples [spp_begin, spp_begin+spp_count) */
     uint32_t spp_count; /* 0 == all of them (spp - spp_begin)                            */
-    uint32_t max_depth; /* MAX_DEPTH, `depth > MAX_DEPTH` semantics (main.rs:126)        */
+    uint32_t max_depth; /* MAX_DEPTH, `depth > MAX_DEPTH` semantics (main.rs:126): a path
+                         * traces at most max_depth segments.  Must be >= 1: ray_color starts
+                         * at depth 1, so 0 is a black frame with no rays, and every render
+                         * call refuses it with VK_ERR_INVALID.                          */
     uint64_t seed;      /* Philox4x32-10 key                                             */
     float background[3];/* src/main.rs:124 (always 0 at HEAD)                            */
     uint32_t variant;   /* VK_VARIANT_*                                                  */

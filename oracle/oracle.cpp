@@ -831,10 +831,14 @@ struct RayTap { // optional recorder of every traced segment (orc_harvest_rays)
 };
 static thread_local RayTap* tl_tap = nullptr;
 
+static Vec3 sky_color(const Ray& r);
+
 // `live` is instrumentation only: false once the path's accumulated weight is exactly zero or
 // non-finite, i.e. for segments the reference still traces although they cannot change the pixel.
+// `sky`: a miss returns the book-1 sky of the ray that missed (as ray_color_legacy and the GPU's miss_color do), not
+// the constant background.
 static Vec3 ray_color(const Ray& r, const Arc<Hittable>& world, const Arc<Hittable>& lights, uint32_t depth,
-                      uint32_t max_depth, Vec3 background, bool live = true) { // :123-153
+                      uint32_t max_depth, Vec3 background, bool sky, bool live = true) { // :123-153
     if (depth > max_depth) return Vec3::new_const(0.0f);
     tl_cnt.rays++;
     if (live) tl_cnt.rays_live++;
@@ -848,7 +852,7 @@ static Vec3 ray_color(const Ray& r, const Arc<Hittable>& world, const Arc<Hittab
         Vec3 emitted = c->material->emitted(*c, c->u, c->v, c->p);
         if (auto srec = c->material->scatter_with_pdf(r, *c)) {
             if (srec->specular_ray) // Specular!  (emitted is dropped, Q2)
-                return srec->attenuation * ray_color(*srec->specular_ray, world, lights, depth + 1, max_depth, background,
+                return srec->attenuation * ray_color(*srec->specular_ray, world, lights, depth + 1, max_depth, background, sky,
                                                      live && !(srec->attenuation.x == 0.0f && srec->attenuation.y == 0.0f && srec->attenuation.z == 0.0f));
             auto p_important = std::make_shared<HittablePDF>(lights, c->p);
             MixturePDF p(p_important, 0.5f, srec->pdf, 0.5f);
@@ -857,13 +861,13 @@ static Vec3 ray_color(const Ray& r, const Arc<Hittable>& world, const Arc<Hittab
             Vec3 w = srec->attenuation * c->material->scattering_pdf(r, *c, scattered) / pdf; // instrumentation
             bool child_live = live && w.is_finite() && !(w.x == 0.0f && w.y == 0.0f && w.z == 0.0f);
             return emitted + srec->attenuation * c->material->scattering_pdf(r, *c, scattered) *
-                                 ray_color(scattered, world, lights, depth + 1, max_depth, background, child_live) / pdf;
+                                 ray_color(scattered, world, lights, depth + 1, max_depth, background, sky, child_live) / pdf;
         }
         tl_cnt.n_emit_or_miss++;
         return emitted;
     }
     tl_cnt.n_emit_or_miss++;
-    return background;
+    return sky ? sky_color(r) : background;
 }
 
 // The book-1/2 integrator the legacy Material::scatter methods (still in the reference's API at HEAD,
@@ -1183,8 +1187,8 @@ int orc_render(const orc_scene* s, const vk_camera* cam_, const vk_render_params
                 Ray ray = cam.get_ray(u, v);
                 Vec3 color = (P->flags & VK_FLAG_LEGACY_SCATTER)
                                  ? ray_color_legacy(ray, s->s.world, 1, P->max_depth, background, (P->flags & VK_FLAG_SKY_BACKGROUND) != 0)
-                                 : ray_color(ray, s->s.world, s->s.lights, 1, P->max_depth,
-                                             (P->flags & VK_FLAG_SKY_BACKGROUND) ? sky_color(ray) : background);
+                                 : ray_color(ray, s->s.world, s->s.lights, 1, P->max_depth, background,
+                                             (P->flags & VK_FLAG_SKY_BACKGROUND) != 0);
                 if (color.is_finite()) { // :192-194
                     c = c + color;
                     c2 = c2 + color * color;
@@ -1248,7 +1252,7 @@ size_t orc_harvest_rays(const orc_scene* s, const vk_camera* cam_, uint32_t widt
                 rng.seed(seed, (uint64_t)y * width + x, sample);
                 float u = ((float)x + rng.gen_f32()) / (float)(width - 1);
                 float v = ((float)y + rng.gen_f32()) / (float)(height - 1);
-                ray_color(cam.get_ray(u, v), s->s.world, s->s.lights, 1, max_depth, Vec3::new_const(0.0f));
+                ray_color(cam.get_ray(u, v), s->s.world, s->s.lights, 1, max_depth, Vec3::new_const(0.0f), false);
             }
         ++sample;
         if (tap.n == before) break;

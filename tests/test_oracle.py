@@ -654,6 +654,34 @@ def test_legacy_integrator_agrees_with_head_in_expectation(vb, po):
     assert abs(a.mean() - b.mean()) <= 5 * se + 0.01 * b.mean(), (a.mean(), b.mean(), se)
 
 
+def mean_and_se(rgb, sumsq, spp):
+    """Per-channel image mean and its standard error from a render's sums of squares (pixels are independent)."""
+    m = rgb.astype(np.float64)
+    var = np.maximum(sumsq / spp - m * m, 0.0) * spp / (spp - 1)  # per-sample variance of each pixel-channel
+    n_pix = m.shape[0] * m.shape[1]
+    return m.mean(axis=(0, 1)), np.sqrt((var / spp).sum(axis=(0, 1))) / n_pix
+
+
+@pytest.mark.parametrize("name,W,spp_a,spp_b,depth", [("cornell_box", 40, 256, 64, 50), ("random_spheres_demo", 64, 256, 256, 20)],
+                         ids=["cornell_box", "random_spheres_demo"])
+def test_legacy_integrator_agrees_with_head_under_the_sky(vb, po, name, W, spp_a, spp_b, depth):
+    """The same agreement under the book-1 sky (VK_FLAG_SKY_BACKGROUND), channel by channel: both integrators return the
+    sky colour of the ray that misses, whatever its depth (a miss after a bounce sees another part of the sky than the
+    camera ray did; the sky's blue is 1 everywhere, so red and green are where a wrong direction shows)."""
+    s = vb.Scene(name)
+    cam = s.next_camera()
+    H = s.height_for(W)
+    o = po.OracleScene(s)
+    f = vb.VK_FLAG_SKY_BACKGROUND
+    a, qa, _ = o.render(cam, vb.render_params(W, H, spp_a, depth, seed=3, flags=f | vb.VK_FLAG_LEGACY_SCATTER), want_sumsq=True)
+    b, qb, _ = o.render(cam, vb.render_params(W, H, spp_b, depth, seed=4, flags=f), want_sumsq=True)
+    ma, ea = mean_and_se(a, qa, spp_a)
+    mb, eb = mean_and_se(b, qb, spp_b)
+    z = (ma - mb) / np.sqrt(ea ** 2 + eb ** 2)
+    print(f"{name} under the sky: legacy {ma}, HEAD {mb}, ratio HEAD/legacy {mb / ma}, z {z}")
+    assert np.all(np.abs(z) <= 4.0), (name, ma, mb, z)
+
+
 def test_legacy_refuses_what_the_reference_panics_on(vb, po):
     scene = vb.Scene("api_surface_demo")  # holds a SpecDiffuse: its default `scatter` unwraps None
     cam = scene.next_camera()

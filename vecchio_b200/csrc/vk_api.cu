@@ -560,7 +560,7 @@ static int wf_render(vk_ctx* c, bool strict, const FlatProgram* flat, const DCam
     // no sample ends before its first segment: at least spp_count * n_pixels / n_slots iterations
     const unsigned long long min_iters = ((unsigned long long)w.n_pixels * a.spp_count + w.n_slots - 1) / w.n_slots;
     unsigned long long next_check = min_iters > 8 ? min_iters : 8;
-    const unsigned long long max_iters = (min_iters + 2) * (unsigned long long)(a.max_depth ? a.max_depth : 1) + 64; // every path is <= max_depth segments
+    const unsigned long long max_iters = (min_iters + 2) * (unsigned long long)a.max_depth + 64; // every path is <= max_depth segments
     for (unsigned long long it = 0;; ++it) {
         if (it > max_iters) {
             cudaStreamSynchronize(c->stream); // the kernels already launched still use the accumulators
@@ -665,6 +665,8 @@ static int check_render(vk_ctx* c, const std::string& who, const vk_camera* cams
     if (!c->has_scene) return fail(c, VK_ERR_NO_SCENE, who + ": no scene uploaded");
     if (P->width < 2 || P->height < 2) return fail(c, VK_ERR_INVALID, who + ": width/height must be >= 2 ((width-1) divides, src/main.rs:187)");
     if (P->spp == 0 || P->spp_begin >= P->spp) return fail(c, VK_ERR_INVALID, who + ": bad spp / spp_begin");
+    // the kernels trace a path's first segment before they test its depth; depth 0 is a black frame with no rays
+    if (P->max_depth == 0) return fail(c, VK_ERR_INVALID, who + ": max_depth must be >= 1 (ray_color starts at depth 1, src/main.rs:126)");
     const uint32_t count = P->spp_count ? P->spp_count : P->spp - P->spp_begin;
     if ((uint64_t)P->spp_begin + count > P->spp) return fail(c, VK_ERR_INVALID, who + ": sample slice exceeds spp");
     // the kernels index the accumulators of the whole batch with 32-bit element indices

@@ -56,7 +56,7 @@ void usage(FILE* f) {
         "  --param K          scene parameter (stress_spheres: grid side)\n"
         "  --width W          image width, height = (W / aspect_ratio) as usize (default 900)\n"
         "  --spp S            SAMPLES_PER_PIXEL (default 1000)\n"
-        "  --depth D          MAX_DEPTH (default 100)\n"
+        "  --depth D          MAX_DEPTH (default 100, at least 1)\n"
         "  --frames K         stop after K frames (default: the whole camera iterator)\n"
         "  --first-frame F    skip the first F cameras (file numbering is kept)\n"
         "  --seed S           Philox key of the render (default 1); frame f uses S + f\n"
