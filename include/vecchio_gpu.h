@@ -342,6 +342,37 @@ int vk_render_frames(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, cons
 int vk_render_frames_rgb8(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
                           uint8_t* out_rgb8, vk_stats* stats);
 
+/* Feature buffers for a denoiser: the first-hit albedo, normal, depth and coverage of the render's own camera rays.
+ * Definition, for frame f of n_frames (frame f uses cams[f] and Philox key params->seed + f, as in vk_render_frames):
+ *   - pixel p, samples s = 0 .. aov_spp-1: the camera ray vk_render traces first for sample s of p (Philox blocks 0 and 1 of
+ *     depth 0, so a thin lens and the shutter time are the render's), traced by world.hit(r, 0.001, inf) through the scene's
+ *     traversal: the flat program, or the BVH with VK_FLAG_FORCE_BVH (vk_intersect's choice).  A ConstantMedium's free flight
+ *     draws the render's own variate: depth 1, block 1, the counter's fourth word counting groups of four.
+ *   - one sample contributes, on a hit: albedo A(material), the hit record's normal (it faces the ray; 0 for a
+ *     ConstantMedium), depth t * sqrtf(d.x*d.x + d.y*d.y + d.z*d.z) (the distance from the ray origin, lens offset included),
+ *     hit 1.  On a miss: albedo = the miss colour (params->background, or the sky with VK_FLAG_SKY_BACKGROUND) clamped to
+ *     [0, 1], normal 0, no depth, hit 0.
+ *   - A: the texture value at the hit for Lambertian, Metal and Isotropic; (1,1,1) for Dielectric; for DiffuseLight
+ *     min(emitted, 1) per channel on the front face and 0 on the back face (it emits from the front only); for SpecDiffuse
+ *     pct * A(specular) + (1.0f - pct) * A(diffuse) per channel.
+ *   - planes of a pixel with n = aov_spp samples, h of them hits: albedo and normal are float sums in sample order divided
+ *     by (float)n (normals are not renormalised); depth is the sum over the hits in sample order divided by (float)h, +inf
+ *     when h == 0; coverage is (float)h / (float)n.
+ * The planes depend on the cameras, width, height, seed, background and the flags VK_FLAG_STRICT_MATH, VK_FLAG_FORCE_BVH
+ * and VK_FLAG_SKY_BACKGROUND only; spp, spp_begin, spp_count, max_depth, variant and VK_FLAG_LEGACY_SCATTER do not
+ * change them.  With VK_FLAG_STRICT_MATH every operation is the IEEE single-precision one written above.
+ * Outputs (host buffers, each nullable, at least one non-null) in vk_render_frames' layout: frame f at offset f * W*H*c,
+ * pixel i = y*W + x, row 0 = bottom; c = 3 for out_albedo and out_normal, 1 for out_depth and out_coverage.
+ * One kernel that traces the n_frames * W*H * aov_spp camera rays and nothing else: stats.paths = stats.rays = that number,
+ * node_visits and prim_tests of those rays, launches, ms_kernels and ms_total as vk_render_frames reports them, variant 0.
+ * Errors, before anything is launched: those of vk_render_frames but its variant rule (VK_ERR_INVALID for n_frames == 0, a
+ * null pointer, a camera with time0 >= time1, width or height below 2, bad spp / spp_begin / spp_count, max_depth == 0,
+ * n_frames * W*H*3 >= 2^31; VK_ERR_NO_SCENE without a scene), and VK_ERR_INVALID for aov_spp == 0 or above
+ * VK_AOV_MAX_SPP and for all four outputs null. */
+#define VK_AOV_MAX_SPP 65536u
+int vk_render_aov(vk_ctx* ctx, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params, uint32_t aov_spp,
+                  float* out_albedo, float* out_normal, float* out_depth, float* out_coverage, vk_stats* stats);
+
 /* Adaptive sampling: every pixel renders until its displayed noise is below max_error, or until params->spp samples.
  * Passes: pass 0 renders global samples [0, pass_spp) of every pixel; pass k renders [k*pass_spp, min((k+1)*pass_spp, spp))
  * of every pixel still active.  A pixel therefore ends with n_p in {pass_spp, 2*pass_spp, ..} or n_p = spp samples, and
@@ -551,6 +582,9 @@ int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_para
                          vk_stats* stats);                                      /* vk_render_rgb8 over all devices         */
 int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params,
                                 uint8_t* out_rgb8, vk_stats* stats);            /* vk_render_frames_rgb8 over all devices  */
+/* vk_render_aov on the vk_multi's first device: the planes cost a fraction of a render, and they are the one-GPU bytes */
+int vk_multi_render_aov(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* params, uint32_t aov_spp,
+                        float* out_albedo, float* out_normal, float* out_depth, float* out_coverage, vk_stats* stats);
 
 /* Adaptive sessions over all devices of a vk_multi: the vk_adaptive_* calls with the same meaning and arguments.  Adaptive
  * sampling splits PIXELS, not samples (a pixel's decision after each pass needs the sums of all its samples): device k

@@ -48,6 +48,11 @@ void vkh_frame_to_rgb8(const float* frame, uint32_t width, uint32_t height, uint
  * of rgb8 (file order, as vk_render_rgb8 / vkh_frame_to_rgb8 produce it).  0 = OK, VK_ERR_INVALID on an I/O
  * failure (message in vkh_last_error) where the reference unwraps File::create. */
 int vkh_write_ppm(const char* path, const uint8_t* rgb8, uint32_t width, uint32_t height);
+/* A little-endian PFM of one frame plane: "PF" (channels 3) or "Pf" (channels 1), "W H", scale "-1.0" (the sign
+ * says little-endian), then the W*H*channels floats row 0 first -- PFM stores rows bottom-to-top, the order of
+ * vk_render's and vk_render_aov's planes, so nothing is flipped.  0 = OK, VK_ERR_INVALID for channels other than
+ * 1 or 3, a null argument or an I/O failure (message in vkh_last_error). */
+int vkh_write_pfm(const char* path, const float* data, uint32_t width, uint32_t height, uint32_t channels);
 /* "output_{:04}.ppm" (src/main.rs:201) under dir (NULL or "" = current directory) into buf; returns the length
  * or -1 if buf is too small. */
 int vkh_frame_filename(const char* dir, uint32_t file_idx, char* buf, size_t buf_len);

@@ -111,6 +111,11 @@ extern "C" {
                             out_rgb: *mut f32, stats: *mut vk_stats) -> c_int;
     pub fn vk_render_frames_rgb8(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
                                  out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
+    // feature buffers for a denoiser: first-hit albedo, normal, depth and coverage of the render's own camera rays for samples
+    // 0 .. aov_spp-1 (the header states each plane); every output nullable, at least one non-null
+    pub fn vk_render_aov(ctx: *mut vk_ctx, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, aov_spp: u32,
+                         out_albedo: *mut f32, out_normal: *mut f32, out_depth: *mut f32, out_coverage: *mut f32,
+                         stats: *mut vk_stats) -> c_int;
     // adaptive sampling: passes of pass_spp samples until a pixel's displayed noise is <= max_error (8-bit steps) or spp;
     // a pixel that stopped at n samples equals vk_render with spp = n on the same kernel (the header states the rule)
     pub fn vk_render_adaptive(ctx: *mut vk_ctx, cam: *const vk_camera, params: *const vk_render_params, pass_spp: u32, max_error: f32,
@@ -151,6 +156,9 @@ extern "C" {
                                 out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
     pub fn vk_multi_render_frames_rgb8(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params,
                                        out_rgb8: *mut u8, stats: *mut vk_stats) -> c_int;
+    pub fn vk_multi_render_aov(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, aov_spp: u32,
+                               out_albedo: *mut f32, out_normal: *mut f32, out_depth: *mut f32, out_coverage: *mut f32,
+                               stats: *mut vk_stats) -> c_int;
     // adaptive sampling over several GPUs: device k renders shard k's pixels; every result equals the one-GPU call's bit for bit
     pub fn vk_multi_adaptive_begin(m: *mut vk_multi, cams: *const vk_camera, n_frames: u32, params: *const vk_render_params, pass_spp: u32,
                                    out: *mut *mut vk_multi_adaptive_session) -> c_int;
@@ -339,6 +347,21 @@ impl Gpu {
         let mut st = vk_stats::default();
         self.check(unsafe { vk_render_frames_rgb8(self.ctx, cams.as_ptr(), cams.len() as u32, &p, out.as_mut_ptr(), &mut st) })?;
         Ok((out, st))
+    }
+    /// Feature buffers of K cameras for a denoiser (vk_render_aov in vecchio_gpu.h): first-hit albedo and normal (3 floats
+    /// per pixel), depth and coverage (1 float), each frame in `render`'s layout, from the camera rays of samples
+    /// 0 .. aov_spp-1 that `render_frames(.., seed, ..)` traces first.  Returns (albedo, normal, depth, coverage, stats).
+    pub fn render_aov(&mut self, cams: &[vk_camera], width: usize, height: usize, seed: u64, aov_spp: u32)
+                      -> Result<(Vec<f32>, Vec<f32>, Vec<f32>, Vec<f32>, vk_stats), GpuError> {
+        if cams.is_empty() { return Err(GpuError::Unsupported("render_aov: at least one camera")); }
+        let p = vk_render_params { width: width as u32, height: height as u32, spp: 1, spp_begin: 0, spp_count: 0, max_depth: 1, seed,
+                                   background: [0.0; 3], variant: 0, flags: 0 };
+        let n = cams.len() * width * height;
+        let (mut albedo, mut normal, mut depth, mut coverage) = (vec![0f32; n * 3], vec![0f32; n * 3], vec![0f32; n], vec![0f32; n]);
+        let mut st = vk_stats::default();
+        self.check(unsafe { vk_render_aov(self.ctx, cams.as_ptr(), cams.len() as u32, &p, aov_spp, albedo.as_mut_ptr(), normal.as_mut_ptr(),
+                                          depth.as_mut_ptr(), coverage.as_mut_ptr(), &mut st) })?;
+        Ok((albedo, normal, depth, coverage, st))
     }
     /// Adaptive sampling with `spp` as the cap: every pixel renders passes of `pass_spp` samples until half the width of
     /// sqrt(mean +- standard error) is <= `max_error` 8-bit steps in every channel (vk_render_adaptive in vecchio_gpu.h).

@@ -58,6 +58,8 @@ def host_lib():
         L.vkh_frame_to_rgb8.restype = None
         L.vkh_write_ppm.argtypes = [C.c_char_p, C.c_void_p, C.c_uint32, C.c_uint32]
         L.vkh_write_ppm.restype = C.c_int
+        L.vkh_write_pfm.argtypes = [C.c_char_p, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]
+        L.vkh_write_pfm.restype = C.c_int
         L.vkh_frame_filename.argtypes = [C.c_char_p, C.c_uint32, C.c_char_p, C.c_size_t]
         L.vkh_frame_filename.restype = C.c_int
         L.vkh_last_error.restype = C.c_char_p
@@ -109,6 +111,9 @@ def gpu_lib():
                                             C.POINTER(_abi.vk_stats)]
         L.vk_multi_render_frames_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), vp,
                                                   C.POINTER(_abi.vk_stats)]
+        L.vk_render_aov.argtypes = [vp, C.POINTER(_abi.vk_camera), C.c_uint32, C.POINTER(_abi.vk_render_params), C.c_uint32, vp, vp, vp, vp,
+                                    C.POINTER(_abi.vk_stats)]
+        L.vk_multi_render_aov.argtypes = L.vk_render_aov.argtypes
         L.vk_render_adaptive.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), C.c_uint32, C.c_float, vp, vp,
                                          C.POINTER(_abi.vk_stats)]
         L.vk_render_adaptive_rgb8.argtypes = [vp, C.POINTER(_abi.vk_camera), C.POINTER(_abi.vk_render_params), C.c_uint32, C.c_float, vp,
@@ -137,13 +142,13 @@ def gpu_lib():
         L.vk_multi_render_frames_adaptive_rgb8.argtypes = L.vk_render_frames_adaptive_rgb8.argtypes
         for f in ("vk_multi_create", "vk_multi_device_count", "vk_multi_scene_upload", "vk_multi_render", "vk_multi_render_rgb8",
                   "vk_multi_render_frames_rgb8", "vk_multi_render_adaptive_rgb8", "vk_multi_render_frames_adaptive_rgb8",
-                  "vk_adaptive_begin_shard"):
+                  "vk_adaptive_begin_shard", "vk_multi_render_aov"):
             getattr(L, f).restype = C.c_int
         for f in ("vk_create", "vk_scene_upload", "vk_render", "vk_render_rgb8", "vk_render_device", "vk_finalize_device",
                   "vk_set_stream", "vk_flush_stats", "vk_intersect", "vk_eval_batch", "vk_measure_peaks", "vk_device_info",
                   "vk_render_frames", "vk_render_frames_rgb8", "vk_render_adaptive", "vk_render_adaptive_rgb8",
                   "vk_render_frames_adaptive", "vk_render_frames_adaptive_rgb8", "vk_adaptive_begin", "vk_adaptive_refine",
-                  "vk_adaptive_read", "vk_adaptive_read_rgb8", "vk_adaptive_export", "vk_adaptive_import"):
+                  "vk_adaptive_read", "vk_adaptive_read_rgb8", "vk_adaptive_export", "vk_adaptive_import", "vk_render_aov"):
             getattr(L, f).restype = C.c_int
         _gpu = L
     return _gpu
@@ -158,10 +163,10 @@ GPU_SYMBOLS = ["vk_create", "vk_destroy", "vk_last_error", "vk_scene_check", "vk
                "vk_adaptive_export", "vk_adaptive_import", "vk_adaptive_variant", "vk_adaptive_destroy", "vk_adaptive_begin_shard",
                "vk_multi_adaptive_begin", "vk_multi_adaptive_refine", "vk_multi_adaptive_read", "vk_multi_adaptive_read_rgb8",
                "vk_multi_adaptive_export", "vk_multi_adaptive_import", "vk_multi_adaptive_variant", "vk_multi_adaptive_destroy",
-               "vk_multi_render_adaptive_rgb8", "vk_multi_render_frames_adaptive_rgb8"]
+               "vk_multi_render_adaptive_rgb8", "vk_multi_render_frames_adaptive_rgb8", "vk_render_aov", "vk_multi_render_aov"]
 HOST_SYMBOLS = ["vkh_scene_build", "vkh_scene_free", "vkh_scene_desc", "vkh_scene_aspect_ratio",
                 "vkh_scene_next_camera", "vkh_camera_new", "vkh_decode_png", "vkh_frame_to_rgb8", "vkh_write_ppm",
-                "vkh_frame_filename", "vkh_last_error"]
+                "vkh_frame_filename", "vkh_last_error", "vkh_write_pfm"]
 
 
 class Scene:
@@ -276,6 +281,17 @@ def write_ppm(path, rgb8):
         raise VecchioError(-1, L.vkh_last_error().decode())
 
 
+def write_pfm(path, plane):
+    """``vkh_write_pfm``: an (H, W, 3) or (H, W) float plane with row 0 = bottom (what render_aov returns) as a
+    little-endian PFM file."""
+    a = np.ascontiguousarray(plane, dtype=np.float32)
+    if a.ndim not in (2, 3) or (a.ndim == 3 and a.shape[2] != 3):
+        raise ValueError("write_pfm: an (H, W, 3) or (H, W) plane")
+    L = host_lib()
+    if L.vkh_write_pfm(os.fsencode(path), a.ctypes.data, a.shape[1], a.shape[0], 3 if a.ndim == 3 else 1) != 0:
+        raise VecchioError(-1, L.vkh_last_error().decode())
+
+
 def render_params(width, height, spp, max_depth=100, seed=1, spp_begin=0, spp_count=0, variant=0, flags=0,
                   background=(0.0, 0.0, 0.0)):
     p = _abi.vk_render_params()
@@ -293,6 +309,21 @@ def _camera_array(cams):
     if not cams:
         raise ValueError("render_frames: at least one camera")
     return (_abi.vk_camera * len(cams))(*cams), len(cams)
+
+
+AOV_PLANES = (("albedo", 3), ("normal", 3), ("depth", 1), ("coverage", 1))
+
+
+def _render_aov(fn, handle, check, cams, params, aov_spp):
+    """``vk_render_aov`` / ``vk_multi_render_aov`` of the (non-empty) list ``cams`` into the four planes, each (K, H, W, c)
+    with rows bottom-up, c = 1 squeezed.  Returns (planes, stats)."""
+    arr, k = _camera_array(cams)
+    n = k * params.width * params.height
+    out = {name: np.empty(n * c, dtype=np.float32) for name, c in AOV_PLANES}
+    st = _abi.vk_stats()
+    check(fn(handle, arr, k, C.byref(params), int(aov_spp), *(out[name].ctypes.data for name, _ in AOV_PLANES), C.byref(st)))
+    return {name: out[name].reshape((k, params.height, params.width, c) if c > 1 else (k, params.height, params.width))
+            for name, c in AOV_PLANES}, st
 
 
 def _check_adaptive(pass_spp, max_error):
@@ -561,6 +592,19 @@ class Context:
         self._check(self._L.vk_render_frames_rgb8(self._h, arr, k, C.byref(params), out.ctypes.data, C.byref(st)))
         return out.reshape(k, params.height, params.width, 3), st
 
+    def render_aov(self, cam, params, aov_spp):
+        """``vk_render_aov`` of one camera: the first-hit feature planes of the camera rays ``render(cam, params)`` traces
+        first for samples 0 .. aov_spp-1 (the header states each plane; the planes depend on the cameras, size, seed,
+        background and the flags STRICT_MATH, FORCE_BVH and SKY_BACKGROUND only).  Returns ({"albedo": (H, W, 3),
+        "normal": (H, W, 3), "depth": (H, W), "coverage": (H, W)} float32 with row 0 = bottom, stats)."""
+        planes, st = self.render_frames_aov([cam], params, aov_spp)
+        return {name: v[0] for name, v in planes.items()}, st
+
+    def render_frames_aov(self, cams, params, aov_spp):
+        """``vk_render_aov`` of K cameras in one launch, frame f with seed ``params.seed + f``: frame f equals
+        ``render_aov(cams[f], params with seed + f)`` bit for bit.  Returns (the planes with (K, ...) shapes, stats)."""
+        return _render_aov(self._L.vk_render_aov, self._h, self._check, cams, params, aov_spp)
+
     def render_adaptive(self, cam, params, pass_spp, max_error):
         """``vk_render_adaptive``: each pixel renders passes of ``pass_spp`` samples until its displayed noise (half the
         width of sqrt(mean +- standard error) in 8-bit steps) is <= ``max_error``, or until ``params.spp`` samples
@@ -750,6 +794,19 @@ class MultiContext:
         st = _abi.vk_stats()
         self._check(self._L.vk_multi_render_rgb8(self._h, C.byref(cam), C.byref(params), out.ctypes.data, C.byref(st)))
         return out.reshape(params.height, params.width, 3), st
+
+    def render_aov(self, cam, params, aov_spp):
+        """``vk_multi_render_aov`` of one camera, on the first device (the one-GPU planes): the first-hit feature planes of the camera rays ``render(cam, params)`` traces
+        first for samples 0 .. aov_spp-1 (the header states each plane; the planes depend on the cameras, size, seed,
+        background and the flags STRICT_MATH, FORCE_BVH and SKY_BACKGROUND only).  Returns ({"albedo": (H, W, 3),
+        "normal": (H, W, 3), "depth": (H, W), "coverage": (H, W)} float32 with row 0 = bottom, stats)."""
+        planes, st = self.render_frames_aov([cam], params, aov_spp)
+        return {name: v[0] for name, v in planes.items()}, st
+
+    def render_frames_aov(self, cams, params, aov_spp):
+        """``vk_multi_render_aov`` of K cameras in one launch, frame f with seed ``params.seed + f``: frame f equals
+        ``render_aov(cams[f], params with seed + f)`` bit for bit.  Returns (the planes with (K, ...) shapes, stats)."""
+        return _render_aov(self._L.vk_multi_render_aov, self._h, self._check, cams, params, aov_spp)
 
     def render_frames_rgb8(self, cams, params):
         """``vk_multi_render_frames_rgb8``: Context.render_frames_rgb8 over all devices, the same frames bit for bit as one GPU's batch."""

@@ -992,6 +992,35 @@ static int stage(vk_ctx* c, size_t plane, bool fixed, const Outputs& o, Staging*
     return rc != VK_OK ? rc : ensure_pinned(c, S->sum);
 }
 
+// The chunked copy-out every call into host buffers ends with: n elements of elem bytes from the start of c->frame go to the
+// host through c->pinned in VK_CHUNKS chunks.  chunks_begin enqueues the copies (off: the chunks' byte offsets); chunks_end
+// waits for each chunk in turn and hands its bytes to the caller's buffers it covers, so that they fill from one chunk while
+// the later ones are still on the bus.
+#define VK_CHUNKS 4
+struct HostSpan { // bytes [begin, end) of the staged result are host[0 .. end - begin)
+    char* host;
+    size_t begin, end;
+};
+static int chunks_begin(vk_ctx* c, size_t n, size_t elem, size_t off[VK_CHUNKS + 1]) {
+    for (int i = 0; i <= VK_CHUNKS; ++i) off[i] = n * (size_t)i / VK_CHUNKS * elem;
+    for (int i = 0; i < VK_CHUNKS; ++i) {
+        if (!c->ev_chunk[i]) CU(c, cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
+        CU(c, cudaMemcpyAsync((char*)c->pinned + off[i], (const char*)c->frame + off[i], off[i + 1] - off[i], cudaMemcpyDeviceToHost, c->stream));
+        CU(c, cudaEventRecord(c->ev_chunk[i], c->stream));
+    }
+    return VK_OK;
+}
+static int chunks_end(vk_ctx* c, const size_t off[VK_CHUNKS + 1], const HostSpan* spans, int n_spans) {
+    for (int i = 0; i < VK_CHUNKS; ++i) {
+        CU(c, cudaEventSynchronize(c->ev_chunk[i]));
+        for (int k = 0; k < n_spans; ++k) {
+            const size_t b = off[i] > spans[k].begin ? off[i] : spans[k].begin, e = off[i + 1] < spans[k].end ? off[i + 1] : spans[k].end;
+            if (b < e) std::memcpy(spans[k].host + (b - spans[k].begin), (const char*)c->pinned + b, e - b);
+        }
+    }
+    return VK_OK;
+}
+
 // The end of every render call into host buffers, given its result on c's device: the float sums over P->spp of a fixed
 // render (s == nullptr) in c->frame where stage() puts them, or session s's state.  Converts the means of the n_frames
 // frames into c->frame (k_finalize, or k_to_color with the counts in the image's order), copies the image back through
@@ -1014,15 +1043,8 @@ static int readout(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, cons
     if (s) convert(AccOverCount{s->acc, s->nspp});
     else convert(SumsOverSpp{d + S.sum, (float)P->spp});
     CU(c, cudaGetLastError());
-    constexpr int NCH = 4;
-    const size_t elem = o.rgb ? sizeof(float) : 1;
-    size_t off[NCH + 1]; // in bytes
-    for (int i = 0; i <= NCH; ++i) off[i] = plane * (size_t)i / NCH * elem;
-    for (int i = 0; i < NCH; ++i) {
-        if (!c->ev_chunk[i]) CU(c, cudaEventCreateWithFlags(&c->ev_chunk[i], cudaEventDisableTiming));
-        CU(c, cudaMemcpyAsync((char*)c->pinned + off[i], (const char*)d + off[i], off[i + 1] - off[i], cudaMemcpyDeviceToHost, c->stream));
-        CU(c, cudaEventRecord(c->ev_chunk[i], c->stream));
-    }
+    size_t off[VK_CHUNKS + 1];
+    if ((rc = chunks_begin(c, plane, o.rgb ? sizeof(float) : 1, off)) != VK_OK) return rc;
     if (o.sumsq) CU(c, cudaMemcpyAsync(c->pinned + S.sumsq, d + S.sumsq, plane * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     if (o.spp) CU(c, cudaMemcpyAsync(c->pinned + S.counts, d_spp ? d_spp : s->nspp, n_pix * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
     if (o.error) {
@@ -1032,11 +1054,8 @@ static int readout(vk_ctx* c, const vk_render_params* P, uint32_t n_frames, cons
         CU(c, cudaMemcpyAsync(c->pinned + S.error, d + S.error, n_pix * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     }
     CU(c, cudaEventRecord(c->ev1, c->stream));
-    char* image = o.rgb ? (char*)o.rgb : (char*)o.rgb8;
-    for (int i = 0; i < NCH; ++i) {
-        CU(c, cudaEventSynchronize(c->ev_chunk[i]));
-        std::memcpy(image + off[i], (const char*)c->pinned + off[i], off[i + 1] - off[i]);
-    }
+    const HostSpan image{o.rgb ? (char*)o.rgb : (char*)o.rgb8, 0, off[VK_CHUNKS]};
+    if ((rc = chunks_end(c, off, &image, 1)) != VK_OK) return rc;
     CU(c, cudaStreamSynchronize(c->stream));
     if (o.sumsq) std::memcpy(o.sumsq, c->pinned + S.sumsq, plane * sizeof(float));
     if (o.spp) std::memcpy(o.spp, c->pinned + S.counts, n_pix * sizeof(uint32_t));
@@ -1083,6 +1102,81 @@ int vk_render_frames(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const 
 
 int vk_render_frames_rgb8(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8, vk_stats* stats) {
     return render_host(c, "vk_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, nullptr, stats);
+}
+
+// The traversal vk_intersect and vk_render_aov run: the flat program, unless it holds subtrees (a hybrid program is the
+// warp-queue kernel's) or the flags force the BVH; nullptr: the BVH
+static const FlatProgram* hit_program(const vk_ctx* c, uint32_t flags) {
+    return (c->flat.n && (c->flat.n_bvh == 0 || std::getenv("VECCHIO_HYBRID_ALL")) && !(flags & VK_FLAG_FORCE_BVH)) ? &c->flat : nullptr;
+}
+
+// shared body of vk_render_aov and vk_multi_render_aov: one k_aov launch writes the planes asked for, packed in the order
+// albedo, normal, depth, coverage, into c->frame (staged as one float image), then the chunked copy-out hands each to its buffer
+static int render_aov(vk_ctx* c, const std::string& who, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t aov_spp,
+                      float* out_albedo, float* out_normal, float* out_depth, float* out_coverage, vk_stats* stats) {
+    if (!c) return VK_ERR_INVALID;
+    vk_render_params q{}; // every check of vk_render_frames but the variant's: no render kernel runs
+    if (P) {
+        q = *P;
+        q.variant = VK_VARIANT_AUTO;
+    }
+    int rc = check_render(c, who, cams, n_frames, P ? &q : nullptr);
+    if (rc != VK_OK) return rc;
+    if (aov_spp == 0 || aov_spp > VK_AOV_MAX_SPP) return fail(c, VK_ERR_INVALID, who + ": aov_spp must be 1 .. " + std::to_string(VK_AOV_MAX_SPP));
+    float* const outs[4] = {out_albedo, out_normal, out_depth, out_coverage};
+    const size_t n_pix = (size_t)P->width * P->height * n_frames, per[4] = {3, 3, 1, 1};
+    size_t at[4], total = 0;
+    float* first = nullptr;
+    for (int k = 0; k < 4; ++k) {
+        at[k] = total;
+        total += outs[k] ? per[k] * n_pix : 0;
+        if (!first) first = outs[k];
+    }
+    if (!first) return fail(c, VK_ERR_INVALID, who + ": every output is null");
+    CU(c, cudaSetDevice(c->device));
+    Staging S;
+    if ((rc = stage(c, total, false, Outputs{first, nullptr, nullptr, nullptr, nullptr}, &S)) != VK_OK) return rc;
+    float* dev[4];
+    for (int k = 0; k < 4; ++k) dev[k] = outs[k] ? c->frame + at[k] : nullptr;
+    RenderArgs a{};
+    a.width = P->width;
+    a.height = P->height;
+    a.seed_lo = (uint32_t)P->seed;
+    a.seed_hi = (uint32_t)(P->seed >> 32);
+    a.background = make_float3(P->background[0], P->background[1], P->background[2]);
+    a.flags = P->flags;
+    a.tiles_x = (P->width + 7) / 8;
+    a.tiles_y = (P->height + 3) / 4;
+    const FlatProgram* flat = hit_program(c, P->flags);
+    CU(c, cudaEventRecord(c->ev2, c->stream));
+    CU(c, cudaEventRecord(c->ev0, c->stream));
+    if ((rc = upload_cams(c, cams, n_frames)) != VK_OK) return rc;
+    CU(c, (P->flags & VK_FLAG_STRICT_MATH ? vkstrict::launch_aov : vkfast::launch_aov)(c->scene, c->flat, flat != nullptr, c->cams, n_frames, a, aov_spp,
+                                                                                     dev[0], dev[1], dev[2], dev[3], c->counters, c->stream));
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    c->launches += 1;
+    c->paths += n_pix * aov_spp;
+    vk_stats st{};
+    if ((rc = vk_flush_stats(c, &st)) != VK_OK) return rc;
+    CU(c, cudaEventElapsedTime(&st.ms_kernels, c->ev0, c->ev1));
+    st.variant = VK_VARIANT_AUTO;
+    size_t off[VK_CHUNKS + 1];
+    if ((rc = chunks_begin(c, total, sizeof(float), off)) != VK_OK) return rc;
+    CU(c, cudaEventRecord(c->ev1, c->stream));
+    HostSpan spans[4];
+    int n_spans = 0;
+    for (int k = 0; k < 4; ++k)
+        if (outs[k]) spans[n_spans++] = HostSpan{(char*)outs[k], at[k] * sizeof(float), (at[k] + per[k] * n_pix) * sizeof(float)};
+    if ((rc = chunks_end(c, off, spans, n_spans)) != VK_OK) return rc;
+    CU(c, cudaStreamSynchronize(c->stream));
+    CU(c, cudaEventElapsedTime(&st.ms_total, c->ev2, c->ev1));
+    if (stats) *stats = st;
+    return VK_OK;
+}
+
+int vk_render_aov(vk_ctx* c, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t aov_spp, float* out_albedo,
+                  float* out_normal, float* out_depth, float* out_coverage, vk_stats* stats) {
+    return render_aov(c, "vk_render_aov", cams, n_frames, P, aov_spp, out_albedo, out_normal, out_depth, out_coverage, stats);
 }
 
 // ---- adaptive sessions (vk_adaptive_*; the one-shot vk_render_adaptive* calls run one on c->oneshot) ----
@@ -1503,7 +1597,7 @@ int vk_intersect(vk_ctx* c, const vk_ray* rays, size_t n, const float* medium_xi
         STEP(cudaMemcpyAsync(d_xi, medium_xi, n * VK_MEDIUM_XI_SLOTS * sizeof(float), cudaMemcpyHostToDevice, c->stream))
     }
     STEP(cudaMemcpyAsync(d_rays, rays, n * sizeof(vk_ray), cudaMemcpyHostToDevice, c->stream))
-    const FlatProgram* flat = (c->flat.n && (c->flat.n_bvh == 0 || std::getenv("VECCHIO_HYBRID_ALL")) && !(flags & VK_FLAG_FORCE_BVH)) ? &c->flat : nullptr;
+    const FlatProgram* flat = hit_program(c, flags);
     STEP((flags & VK_FLAG_STRICT_MATH) ? vkstrict::launch_intersect(c->scene, flat, d_rays, n, d_xi, d_hits, c->stream)
                                        : vkfast::launch_intersect(c->scene, flat, d_rays, n, d_xi, d_hits, c->stream))
     STEP(cudaMemcpyAsync(out, d_hits, n * sizeof(vk_hit), cudaMemcpyDeviceToHost, c->stream))
@@ -1741,6 +1835,15 @@ int vk_multi_render_rgb8(vk_multi* m, const vk_camera* cam, const vk_render_para
 int vk_multi_render_frames_rgb8(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint8_t* out_rgb8,
                                 vk_stats* stats) {
     return multi_render(m, "vk_multi_render_frames_rgb8", cams, n_frames, P, nullptr, out_rgb8, nullptr, stats);
+}
+
+// the planes are small next to a render: device 0 computes them all, the bytes of a one-GPU call
+int vk_multi_render_aov(vk_multi* m, const vk_camera* cams, uint32_t n_frames, const vk_render_params* P, uint32_t aov_spp, float* out_albedo,
+                        float* out_normal, float* out_depth, float* out_coverage, vk_stats* stats) {
+    if (!m) return VK_ERR_INVALID;
+    vk_ctx* c0 = m->ctx[0];
+    const int rc = render_aov(c0, "vk_multi_render_aov", cams, n_frames, P, aov_spp, out_albedo, out_normal, out_depth, out_coverage, stats);
+    return rc == VK_OK ? rc : mfail(m, rc, c0->err);
 }
 
 // ---- adaptive sessions over several GPUs (include/vecchio_gpu.h, vk_multi_adaptive_begin) ----

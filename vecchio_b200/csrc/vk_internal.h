@@ -348,6 +348,17 @@ struct WfState {
 VK_DECLARE_LAUNCHERS(vkfast)
 VK_DECLARE_LAUNCHERS(vkstrict)
 VK_DECLARE_LAUNCHERS(vkfast_l0) // (vk_kernels.cu, vk_warpq.cu, vk_stepq.cu with VK_LIGHT0=1: the megakernel, warp-queue and step-queue launchers only)
+// vk_render_aov's kernel (vk_kernels.cu), in the render and strict builds: the feature planes of n_frames frames (cams: device
+// array; a.tiles_x x a.tiles_y: one frame's 8x4 tiles) written whole into the nullable device planes; use_flat: traverse
+// `flat`, otherwise the BVH.  counters[0] / [3] / [4]: rays, node visits, primitive tests.
+#define VK_DECLARE_AOV(NS)                                                                                             \
+    namespace NS {                                                                                                     \
+    cudaError_t launch_aov(const DScene& sc, const FlatProgram& flat, bool use_flat, const DCamera* cams, uint32_t n_frames, \
+                           const RenderArgs& a, uint32_t aov_spp, float* albedo, float* normal, float* depth, float* coverage, \
+                           unsigned long long* counters, cudaStream_t st);                                             \
+    }
+VK_DECLARE_AOV(vkfast)
+VK_DECLARE_AOV(vkstrict)
 namespace vkfast_simple { // vk_staged.cu / vk_warpq.cu compiled with VK_SIMPLE=1: kernels for "simple" flat scenes (see vk_device.cuh)
 cudaError_t launch_staged(const DScene& sc, const FlatProgram* flat, const DCamera& cam, const RenderArgs& a, const RenderBuffers& b,
                           unsigned long long* unit_head, int sm_count, cudaStream_t st);

@@ -376,6 +376,106 @@ __global__ void __launch_bounds__(VK_BLOCK) k_intersect_flat(const DScene sc, co
     intersect_body<true>(sc, &flat, rays, n, medium_xi, out);
 }
 
+#if !VK_LIGHT0
+// vk_render_aov: the first-hit feature planes of the render's own camera rays (include/vecchio_gpu.h states the
+// definition).  Albedo of one material record at a hit: the texture of Lambertian, Metal and Isotropic, (1,1,1) for a
+// Dielectric, a DiffuseLight's emission clamped to 1 on its front face and 0 behind it (it emits from the front only).
+VKD float3 aov_material_albedo(const DScene& sc, const uint4& m, const HitRecD& rec) {
+    if (m.x == VK_M_DIELECTRIC) return f3(1.0f, 1.0f, 1.0f);
+    if (m.x == VK_M_DIFFUSE_LIGHT) {
+        if (!rec.front) return f3(0.0f, 0.0f, 0.0f);
+        const float3 e = tex_value(sc, m.y, rec.u, rec.v, rec.p);
+        return f3(fminf(e.x, 1.0f), fminf(e.y, 1.0f), fminf(e.z, 1.0f));
+    }
+    return tex_value(sc, m.y, rec.u, rec.v, rec.p);
+}
+// a SpecDiffuse mixes its two components by its specular fraction (the upload refuses a SpecDiffuse component)
+VKD float3 aov_albedo(const DScene& sc, const HitRecD& rec) {
+    if (rec.m.x != VK_M_SPECDIFFUSE) return aov_material_albedo(sc, rec.m, rec);
+    const float pct = __uint_as_float(rec.m.z);
+    const float3 a = aov_material_albedo(sc, __ldg(&sc.materials[rec.m.y]), rec);
+    const float3 b = aov_material_albedo(sc, __ldg(&sc.materials[rec.m.w & ~VKD_MAT_NEEDS_UV]), rec);
+    return f3(pct * a.x + (1.0f - pct) * b.x, pct * a.y + (1.0f - pct) * b.y, pct * a.z + (1.0f - pct) * b.z);
+}
+// One lane per pixel, looping over samples 0 .. aov_spp-1 in order; a warp covers an 8x4 tile of one frame (the lane
+// megakernel's item shape), so its camera rays stay coherent.  Frame f: cams[f], key seed + f.  Every plane is nullable.
+// (FLAT: traverse `flat`; otherwise the BVH, and `flat` is not read)
+template <bool FLAT, bool MEDIA>
+__global__ void __launch_bounds__(VK_BLOCK) k_aov(const DScene sc, const __grid_constant__ FlatProgram flat, const DCamera* __restrict__ cams,
+                                                  uint32_t n_frames, const RenderArgs a, uint32_t aov_spp, float* __restrict__ albedo,
+                                                  float* __restrict__ normal, float* __restrict__ depth, float* __restrict__ coverage,
+                                                  unsigned long long* counters) {
+    const uint32_t lane = threadIdx.x & 31u;
+    const uint32_t warp = (uint32_t)(((size_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    const uint32_t n_tiles = a.tiles_x * a.tiles_y;
+    const uint32_t f = warp / n_tiles, tile = warp - f * n_tiles;
+    const uint32_t px = (tile % a.tiles_x) * 8u + (lane & 7u), py = (tile / a.tiles_x) * 4u + (lane >> 3);
+    uint32_t n_rays = 0;
+    TraceCounters tc = {0u, 0u};
+    if (f < n_frames && px < a.width && py < a.height) { // (ragged tiles: a lane outside the image only joins the counter sum)
+        const DCamera& cam = cams[f];
+        PathRng rng;
+        rng.pixel = py * a.width + px; // i = y*width + x, row 0 = bottom (src/main.rs:182-183)
+        rng.sample = 0;
+        rng.key = frame_key(a, f);
+        float3 alb = f3(0.0f, 0.0f, 0.0f), nrm = alb;
+        float dsum = 0.0f;
+        uint32_t hits = 0;
+#pragma unroll 1
+        for (uint32_t s = 0; s < aov_spp; ++s) {
+            rng.sample = s;
+            float3 o, d;
+            float time;
+            camera_get_ray(cam, rng, px, py, a.width, a.height, o, d, time);
+            MediumXi xi;
+            xi.table = nullptr;
+            xi.rng = rng;
+            xi.depth = 1u; // the camera ray is the path's segment 1 (ray_color(ray, .., 1), src/main.rs:190)
+            ++n_rays;
+            const TraceHit h = FLAT ? trace_flat<MEDIA>(sc, flat, o, d, time, 0.001f, CUDART_INF_F, xi, tc)
+                                    : trace<MEDIA>(sc, o, d, time, 0.001f, CUDART_INF_F, xi, tc);
+            if (h.prim == VK_REF_NONE) {
+                const float3 c = miss_color(a, d);
+                alb = alb + f3(fminf(fmaxf(c.x, 0.0f), 1.0f), fminf(fmaxf(c.y, 0.0f), 1.0f), fminf(fmaxf(c.z, 0.0f), 1.0f));
+            } else {
+                HitRecD rec;
+                resolve_hit(sc, h, o, d, time, true, rec);
+                alb = alb + aov_albedo(sc, rec);
+                if (VKD_TYPE(h.prim) != VK_T_MEDIUM) nrm = nrm + rec.normal; // a ConstantMedium's normal is arbitrary: 0
+                dsum += h.t * sqrtf(d.x * d.x + d.y * d.y + d.z * d.z);
+                ++hits;
+            }
+        }
+        const float n = (float)aov_spp;
+        const size_t p = (size_t)f * a.width * a.height + rng.pixel;
+        if (albedo) {
+            albedo[3 * p + 0] = alb.x / n;
+            albedo[3 * p + 1] = alb.y / n;
+            albedo[3 * p + 2] = alb.z / n;
+        }
+        if (normal) {
+            normal[3 * p + 0] = nrm.x / n;
+            normal[3 * p + 1] = nrm.y / n;
+            normal[3 * p + 2] = nrm.z / n;
+        }
+        if (depth) depth[p] = hits ? dsum / (float)hits : CUDART_INF_F;
+        if (coverage) coverage[p] = (float)hits / n;
+    }
+    unsigned long long w_rays = n_rays, w_nodes = tc.nodes, w_prims = tc.prims;
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        w_rays += __shfl_xor_sync(0xFFFFFFFFu, w_rays, off);
+        w_nodes += __shfl_xor_sync(0xFFFFFFFFu, w_nodes, off);
+        w_prims += __shfl_xor_sync(0xFFFFFFFFu, w_prims, off);
+    }
+    if (lane == 0 && w_rays) {
+        atomicAdd(&counters[3], w_nodes);
+        atomicAdd(&counters[4], w_prims);
+        atomicAdd(&counters[0], w_rays);
+    }
+}
+#endif
+
 // vk_eval_batch: the shading-side parity hook (include/vecchio_gpu.h).  One record per thread through the same
 // device functions the render kernels call.
 __global__ void __launch_bounds__(VK_BLOCK) k_eval(const DScene sc, vk_eval* __restrict__ recs, size_t n, uint32_t n_materials,
@@ -488,6 +588,20 @@ cudaError_t launch_intersect(const DScene& sc, const FlatProgram* flat, const vk
     else k_intersect<<<grid, VK_BLOCK, 0, st>>>(sc, rays, n, medium_xi, out);
     return cudaGetLastError();
 }
+#if !VK_LIGHT0
+// a.tiles_x / a.tiles_y: 8x4 tiles of one frame; one warp per tile and frame
+cudaError_t launch_aov(const DScene& sc, const FlatProgram& flat, bool use_flat, const DCamera* cams, uint32_t n_frames, const RenderArgs& a,
+                       uint32_t aov_spp, float* albedo, float* normal, float* depth, float* coverage, unsigned long long* counters,
+                       cudaStream_t st) {
+    const uint64_t threads = (uint64_t)a.tiles_x * a.tiles_y * n_frames * 32u;
+    const unsigned grid = (unsigned)((threads + VK_BLOCK - 1) / VK_BLOCK);
+#define VK_LA(F, M) k_aov<F, M><<<grid, VK_BLOCK, 0, st>>>(sc, flat, cams, n_frames, a, aov_spp, albedo, normal, depth, coverage, counters)
+    if (use_flat) { if (sc.has_media) VK_LA(true, true); else VK_LA(true, false); }
+    else { if (sc.has_media) VK_LA(false, true); else VK_LA(false, false); }
+#undef VK_LA
+    return cudaGetLastError();
+}
+#endif
 cudaError_t megakernel_occupancy(bool flat, bool media, bool legacy, int* blocks_per_sm, int* block_threads) {
     *block_threads = VK_BLOCK;
     cudaError_t e = cudaSuccess;

@@ -194,6 +194,35 @@ int vkh_write_ppm(const char* path, const uint8_t* rgb8, uint32_t width, uint32_
     return VK_OK;
 }
 
+int vkh_write_pfm(const char* path, const float* data, uint32_t width, uint32_t height, uint32_t channels) {
+    if (!path || !data || (channels != 1 && channels != 3)) {
+        g_err = "vkh_write_pfm: null argument or channels other than 1 and 3";
+        return VK_ERR_INVALID;
+    }
+    FILE* f = std::fopen(path, "wb");
+    if (!f) {
+        g_err = std::string("vkh_write_pfm: cannot create ") + path + ": " + std::strerror(errno);
+        return VK_ERR_INVALID;
+    }
+    bool ok = std::fprintf(f, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height) > 0;
+    // the floats as little-endian bytes whatever the host's byte order, one row at a time
+    std::vector<unsigned char> row((size_t)width * channels * 4);
+    for (uint32_t y = 0; ok && y < height; ++y) {
+        const float* src = data + (size_t)y * width * channels;
+        for (size_t i = 0; i < (size_t)width * channels; ++i) {
+            uint32_t b;
+            std::memcpy(&b, src + i, 4);
+            for (int k = 0; k < 4; ++k) row[4 * i + k] = (unsigned char)(b >> (8 * k));
+        }
+        ok = std::fwrite(row.data(), 1, row.size(), f) == row.size();
+    }
+    if (std::fclose(f) != 0 || !ok) {
+        g_err = std::string("vkh_write_pfm: write failed on ") + path;
+        return VK_ERR_INVALID;
+    }
+    return VK_OK;
+}
+
 int vkh_frame_filename(const char* dir, uint32_t file_idx, char* buf, size_t buf_len) {
     if (!buf) return -1;
     const bool has_dir = dir && dir[0];

@@ -43,6 +43,7 @@ struct Options {
     uint32_t batch = 1; // cameras per launch (vk_render_frames_rgb8); 1 = one vk_render_rgb8 per camera
     float adaptive = -1.0f; // >= 0: vk_render_adaptive_rgb8 with this max_error, --spp the cap
     uint32_t pass_spp = 0;  // its samples per pass (0 = not given: 64)
+    uint32_t aov = 0;       // > 0: feature planes of this many samples next to every frame (vk_render_aov)
     bool quiet = false;
 };
 
@@ -68,6 +69,10 @@ void usage(FILE* f) {
         "                     (the cap).  E = 0 writes the same files as without --adaptive.  The stopping rule\n"
         "                     makes the estimate slightly biased.  One device, --batch 1 (DESIGN.md section 7)\n"
         "  --pass-spp M       samples per adaptive pass (default 64)\n"
+        "  --aov N            also write albedo_NNNN.pfm, normal_NNNN.pfm (PF) and depth_NNNN.pfm (Pf) next to\n"
+        "                     output_NNNN.ppm: the first-hit albedo, normal and depth of the frame's camera rays\n"
+        "                     for samples 0..N-1 (vk_render_aov, same camera and seed; 1 <= N <= 65536).  Little-\n"
+        "                     endian, rows bottom-to-top; depth is +inf where no sample hit\n"
         "  --scene-seed S     host RNG seed for scene generation and BVH axis choices (default 1)\n"
         "  --gpus N           render each frame on devices 0..N-1 (spp split N ways)\n"
         "  --devices a,b,..   explicit device list\n"
@@ -140,6 +145,12 @@ int parse(int argc, char** argv, Options& o) {
         } else if (a == "--pass-spp") {
             if (!need(v) || !parse_u32(v, o.pass_spp) || o.pass_spp == 0) {
                 std::fprintf(stderr, "vecchio_gpu_render: --pass-spp needs an integer >= 1\n");
+                return 2;
+            }
+        } else if (a == "--aov") {
+            if (!need(v)) return 2;
+            if (!parse_u32(v, o.aov) || o.aov == 0 || o.aov > VK_AOV_MAX_SPP) {
+                std::fprintf(stderr, "vecchio_gpu_render: --aov needs a sample count 1 .. %u\n", VK_AOV_MAX_SPP);
                 return 2;
             }
         } else if (a == "--first-frame") {
@@ -227,6 +238,40 @@ void destroy_all(Gpus& g, vkh_scene* scene) {
     if (scene) vkh_scene_free(scene);
 }
 
+// --aov N: the feature planes of the n frames just rendered -- the same cameras, size, seed (frame f: P.seed + f) and flags --
+// written as albedo / normal / depth_NNNN.pfm next to their output_NNNN.ppm (file numbers first_idx + f).  Returns false
+// after printing the error.
+bool write_aov(const Options& opt, Gpus& gpus, const vk_camera* cams, uint32_t n, const vk_render_params& P, uint32_t first_idx) {
+    const size_t n_pix = (size_t)P.width * P.height;
+    std::vector<float> albedo(n_pix * 3 * n), normal(n_pix * 3 * n), depth(n_pix * n);
+    const int rc = gpus.many ? vk_multi_render_aov(gpus.many, cams, n, &P, opt.aov, albedo.data(), normal.data(), depth.data(), nullptr, nullptr)
+                             : vk_render_aov(gpus.one, cams, n, &P, opt.aov, albedo.data(), normal.data(), depth.data(), nullptr, nullptr);
+    if (rc != VK_OK) {
+        std::fprintf(stderr, "vecchio_gpu_render: %s\n", gpus.error());
+        return false;
+    }
+    const struct {
+        const char* kind;
+        const std::vector<float>& plane;
+        uint32_t channels;
+    } files[] = {{"albedo", albedo, 3}, {"normal", normal, 3}, {"depth", depth, 1}};
+    const bool has_dir = !opt.out_dir.empty(), slash = has_dir && opt.out_dir.back() == '/';
+    for (uint32_t f = 0; f < n; f++)
+        for (const auto& file : files) {
+            char name[4096]; // output_NNNN.ppm's directory and number (vkh_frame_filename)
+            const int len = std::snprintf(name, sizeof name, "%s%s%s_%04u.pfm", opt.out_dir.c_str(), has_dir && !slash ? "/" : "", file.kind, first_idx + f);
+            if (len < 0 || (size_t)len >= sizeof name) {
+                std::fprintf(stderr, "vecchio_gpu_render: output path too long\n");
+                return false;
+            }
+            if (vkh_write_pfm(name, file.plane.data() + f * n_pix * file.channels, P.width, P.height, file.channels) != VK_OK) {
+                std::fprintf(stderr, "vecchio_gpu_render: %s\n", vkh_last_error());
+                return false;
+            }
+        }
+    return true;
+}
+
 // --batch K > 1: the frame loop with up to K cameras of cam_iter per vk_render_frames_rgb8 (or
 // vk_multi_render_frames_rgb8) call.  Frame f of a batch is file number n0 + f with seed + n0 + f -- the numbers and seeds
 // of the one-camera loop, so the files are the same byte for byte whenever the batch runs the kernel a single frame runs:
@@ -298,6 +343,10 @@ int render_batched(const Options& opt, Gpus& gpus, vkh_scene* scene, uint32_t wi
         if ((world == 1 ? vk_render_frames_rgb8(gpus.one, cams.data(), n, &P, rgb8.data(), &stats)
                         : vk_multi_render_frames_rgb8(gpus.many, cams.data(), n, &P, rgb8.data(), &stats)) != VK_OK) {
             std::fprintf(stderr, "vecchio_gpu_render: %s\n", gpus.error());
+            finish_pending();
+            return 1;
+        }
+        if (opt.aov && !write_aov(opt, gpus, cams.data(), n, P, first_idx)) {
             finish_pending();
             return 1;
         }
@@ -431,6 +480,11 @@ int main(int argc, char** argv) {
             return 1;
         }
         const uint64_t rays = stats.rays;
+        if (opt.aov && !write_aov(opt, gpus, &cam, 1, P, file_idx)) {
+            finish_pending();
+            destroy_all(gpus, scene);
+            return 1;
+        }
 
         // Write output (main.rs:200-214), overlapped with the next frame's render.  At most one write is in
         // flight, so the other buffer is free by the time the next frame is converted into it.
